@@ -16,6 +16,13 @@ Chains are sharded over ranks (32 / N per GPU, strong scaling); the only exchang
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the UNMODIFIED reference (oracle/_ref, oracle/make_ref.py) on the host cores
+    python bench.py --gpus 1 --steps 20 --warmup 3 --dump-outputs DIR
+
+--dump-outputs DIR writes, after the run, what each timed leg computed in its last step as DIR/<name>.npy (float64):
+mh_* and e2e_* are the chain state a caller reads back after the last of the K steps (every chain's logLik, logPrior,
+logPost, temperature, acceptance_rate, n_accepted; the weights of the first DUMP_CHAINS chains), predict_mean /
+predict_votes the posterior summaries of DUMP_ROWS rows drawn once with default_rng(0).  Inputs, seeds and the step
+count depend only on the arguments, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -34,8 +41,8 @@ N_ROWS = 1_000_000
 N_CHAINS = 32
 SWAP_FREQUENCY = 100
 CPU_SAMPLE_ROWS = 100_000
-MIN_TIMED_S = 1.0            # the K-step block is repeated until this much device time has been measured
-MAX_BLOCKS = 64
+DUMP_CHAINS = 256            # --dump-outputs keeps the weights of at most this many chains (13 MB per leg) and the
+DUMP_ROWS = 65_536           # summaries of at most this many rows (10 MB), so that the dump stays under 64 MB
 PRED_SAMPLES = 1024          # posterior samples of the forward rows/s leg (c5 shape; S >= 1,000 so that the sample upload and the
                               # one all-reduce of the rows x samples grid are amortised as they are at the full 10k)
 
@@ -51,7 +58,14 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-mc3-leg", action="store_true", help="reference arm: skip the np_bnn.MC3.run_mcmc() swap period")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed legs computed in their last step to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm runs in a subprocess and returns only its rate)")
+    return args
 
 
 class ClockSampler:
@@ -169,6 +183,23 @@ def workload_config(args):
             "l2": "inputs larger than L2 (X = %.0f MB streamed once per step)" % (args.rows * 64 * 8 / 1e6)}
 
 
+def chain_outputs(prefix, st, first_chain):
+    """What bnn_chains_read hands back for the local chains first_chain, ... as float64 arrays '<prefix>_<field>';
+    weights only of the chains below DUMP_CHAINS."""
+    out = {k: getattr(st, k) for k in ("logLik", "logPrior", "logPost", "temperature", "acceptance_rate", "n_accepted")}
+    out["weights"] = st.w[:max(0, DUMP_CHAINS - first_chain)]
+    return {"%s_%s" % (prefix, k): np.asarray(v, dtype=np.float64) for k, v in out.items()}
+
+
+def write_outputs(path, parts):
+    """parts: every rank's dict of arrays, in rank order (chains and row blocks are contiguous in rank order)."""
+    arrays = {name: np.concatenate([p[name] for p in parts if name in p]) for name in parts[0]}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "--dump-outputs would exceed 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 _JSON_FD = None
 
 
@@ -236,6 +267,7 @@ def main():
     w0 = np.stack([flatten_weights(w) for w in wl.c4_init_weights(n_local, start)])
     net = NetShape(64, list(wl.C4_SHAPES), act="swish", lik=L.LIK_CATEGORICAL)
     K, W = args.steps, max(args.warmup, 3)
+    dump = {} if args.dump_outputs else None          # name -> this rank's share of the array (--dump-outputs)
 
     # ------------------------------------------------------------------ device-resident leg (value)
     eng = Engine(net, device=local_rank)
@@ -275,33 +307,27 @@ def main():
     clocks = ClockSampler(local_rank)
     clocks.start()
     time.sleep(0.25)
-    # The timed unit is a block of EXACTLY K steps (barrier + synchronize on both sides, CUDA events, max over ranks).
-    # The block is repeated until at least MIN_TIMED_S of device time has been measured (a K=20 block is 0.35 s at one
-    # GPU and 45 ms at eight: too short for the clock sampler and for a sustained-clock claim); the reported time is
-    # the MEDIAN block, every block time is listed in "blocks_ms".
-    blocks_ms, fwd_ms, fwd_n, launches = [], 0.0, 0, 0
-    t_wall0 = time.perf_counter()
+    # The timed region is EXACTLY K steps (barrier + synchronize on both sides, CUDA events, max over ranks), with at
+    # least one MC3 swap in it even when K < SWAP_FREQUENCY.
     swaps_before = n_swaps[0]
-    while True:
-        launches0 = eng.launch_count
-        ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        barrier()
-        ev0.record()
-        temps_all = run_steps(K, temps_all, force_swap=(len(blocks_ms) == 0))
-        ev1.record()
-        barrier()
-        blocks_ms.append(max_over_ranks(ev0.elapsed_time(ev1)))
-        if len(blocks_ms) == 1:
-            launches = eng.launch_count - launches0          # kernels launched inside one K-step block
-        if sum(blocks_ms) >= 1e3 * MIN_TIMED_S or len(blocks_ms) >= MAX_BLOCKS:
-            break
+    launches0 = eng.launch_count
+    ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    barrier()
+    t_wall0 = time.perf_counter()
+    ev0.record()
+    temps_all = run_steps(K, temps_all, force_swap=True)
+    ev1.record()
+    barrier()
     t_wall1 = time.perf_counter()
-    ms = float(np.median(blocks_ms))
+    ms = max_over_ranks(ev0.elapsed_time(ev1))
+    launches = eng.launch_count - launches0
     clk = clocks.stop(t_wall0, t_wall1)
     fwd_ms, fwd_n = eng.forward_time(reset=True)
     eng.set_option("time_forward", 0)
     value = args.chains * K / (ms * 1e-3)
-    st = eng.read_state(weights=False)
+    st = eng.read_state(weights=dump is not None)
+    if dump is not None:
+        dump.update(chain_outputs("mh", st, start))
     kernel_name = eng.last_kernel
 
     # roofline of the dominant kernel (forward + likelihood): algorithmic FLOPs per launch / its mean duration
@@ -320,7 +346,7 @@ def main():
                 "peak_source": "measured live on this GPU: back-to-back FP64 DMMA (bnn_measure_fp64_peak); "
                                "MEASURED_PEAKS.json has no FP64 entry",
                 "flop_per_launch": flop_per_launch, "launch_ms": fwd_avg_ms, "launches_timed": int(fwd_n),
-                "kernel_share_of_step": fwd_ms / float(sum(blocks_ms)) if fwd_n else None,
+                "kernel_share_of_step": fwd_ms / ms if fwd_n else None,
                 "traffic": ncu.get("dram_bytes_per_launch"),
                 "hbm": {"algorithmic_bytes_per_launch": args.rows * (64 * 8 + 4),
                         "achieved_gbs": args.rows * (64 * 8 + 4) / (fwd_avg_ms * 1e-3) / 1e9 if fwd_n else None}}
@@ -333,7 +359,7 @@ def main():
     from npbnn_b200 import predshard
     predict = None
     try:
-        rows_p, sets_p, grid_p, _, _ = predshard.partition(args.rows, PRED_SAMPLES, world, rank)
+        rows_p, sets_p, grid_p, _, sg_p = predshard.partition(args.rows, PRED_SAMPLES, world, rank)
         xd = x_pin[rows_p[0]:rows_p[1]].to(dev)
         rs_p = np.random.default_rng(5)
         w_all = w0[:1].repeat(PRED_SAMPLES, 0) + rs_p.normal(0, 0.05, (PRED_SAMPLES, w0.shape[1])) if n_local else None
@@ -364,6 +390,14 @@ def main():
                             "collective": "none" if grid_p[1] == 1 else "all-reduce of [rows, 10] partial sums within a row group"},
                    "includes": "upload (pinned host memory) + packing of the rank's posterior samples, the all-reduce of the grid, X row block resident",
                    "mean_prob_sum": float(out_p["mean"].sum().item()) / max(rows_p[1] - rows_p[0], 1)}
+        if dump is not None:
+            # the sampled rows of this rank's row block; the Q ranks of a row group hold the same summaries, the one of
+            # sample group 0 contributes them
+            idx = np.sort(np.random.default_rng(0).choice(args.rows, min(args.rows, DUMP_ROWS), replace=False))
+            idx = idx[(idx >= rows_p[0]) & (idx < rows_p[1])] - rows_p[0] if sg_p == 0 else idx[:0]
+            sel = torch.from_numpy(idx).to(dev)
+            dump["predict_mean"] = out_p["mean"][sel].cpu().numpy()
+            dump["predict_votes"] = out_p["votes"][sel].cpu().numpy()
         del xd, out_p
     except Exception as e:                                 # the headline must not depend on this leg
         predict = {"error": repr(e)}
@@ -434,21 +468,17 @@ def main():
             st2 = e2e_step()
         h2d = K * sum(a.nbytes for a in inj.values())
         d2h = K * (st2.f64.nbytes + st2.i32.nbytes)
-        # as for `value`: the timed unit is a block of EXACTLY K steps (barrier + synchronize on both sides, max over
-        # ranks), repeated until MIN_TIMED_S has been measured (a K=20 block is 45 ms at eight GPUs); median block
-        e2e_blocks = []
-        while True:
-            torch.cuda.synchronize(dev)
-            barrier()
-            t0 = time.perf_counter()
-            for s in range(K):
-                st2 = e2e_step()
-            torch.cuda.synchronize(dev)
-            barrier()
-            e2e_blocks.append(max_over_ranks(time.perf_counter() - t0))
-            if sum(e2e_blocks) >= MIN_TIMED_S or len(e2e_blocks) >= MAX_BLOCKS:
-                break
-        t_e2e = float(np.median(e2e_blocks))
+        # as for `value`: the timed region is EXACTLY K steps (barrier + synchronize on both sides, max over ranks)
+        torch.cuda.synchronize(dev)
+        barrier()
+        t0 = time.perf_counter()
+        for s in range(K):
+            st2 = e2e_step()
+        torch.cuda.synchronize(dev)
+        barrier()
+        t_e2e = max_over_ranks(time.perf_counter() - t0)
+        if dump is not None:
+            dump.update(chain_outputs("e2e", eng2.read_state(), start))
         e2e = {"value": args.chains * K / t_e2e, "unit": "chain-steps/s", "h2d_bytes_per_step": h2d / K,
                "d2h_bytes_per_step": d2h / K,
                "includes": "every step, per rank: proposals of all local chains drawn on the host (numpy; a host thread "
@@ -456,8 +486,7 @@ def main():
                            "bnn_mh_steps(1, inj), one MH iteration, chain state read back (bnn_chains_read, "
                            "synchronises); X is resident (staged once by bnn_set_data from pinned "
                            "host memory: setup_seconds, not timed)",
-               "seconds": t_e2e, "blocks": len(e2e_blocks), "blocks_s": [round(b, 5) for b in e2e_blocks],
-               "reported": "median block", "setup_seconds": t_setup, "setup_h2d_bytes": x_pin.numel() * 8 + y_pin.numel() * 4 + w0.nbytes,
+               "seconds": t_e2e, "setup_seconds": t_setup, "setup_h2d_bytes": x_pin.numel() * 8 + y_pin.numel() * 4 + w0.nbytes,
                "finite_logLik": bool(np.all(np.isfinite(st2.logLik)))}
         nxt[0].result()
         pool.shutdown()
@@ -474,14 +503,21 @@ def main():
             cpu = {"value": ref["value"], "unit": "chain-steps/s", "cores": ref["chains"], "kind": "reference",
                    "sample": ref["sample"], "wall_s": ref["chains_leg"]["wall_s"]}
 
+    if dump is not None:
+        parts = [dump]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, dump)
+        if rank == 0:
+            write_outputs(args.dump_outputs, parts)
+
     if rank == 0:
         line = {"metric": "MH iterations/sec (chains x steps / s)", "value": value, "unit": "chain-steps/s",
                 "n_gpus": world, "steps": K, "warmup": W, "ms_per_step": ms / K, "higher_is_better": True,
                 "scaling": "strong", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                 "config": workload_config(args), "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e,
                 "gpu_launches": int(launches), "clocks": clk,
-                "timing": {"blocks": len(blocks_ms), "steps_per_block": K, "blocks_ms": [round(b, 4) for b in blocks_ms],
-                           "reported": "median block", "timed_seconds": sum(blocks_ms) * 1e-3}, "predict": predict,
+                "timing": {"timed_steps": K, "timed_seconds": ms * 1e-3}, "predict": predict,
                 "swaps_in_timed_region": n_swaps[0] - swaps_before,
                 "check": {"logLik_finite": bool(np.all(np.isfinite(st.logLik))),
                           "mean_acceptance": float(np.mean(st.n_accepted / np.maximum(st.iteration, 1)))}}
