@@ -34,8 +34,17 @@ enum { BNN_ACT_RELU = 0, BNN_ACT_LEAKY = 1, BNN_ACT_SWISH = 2, BNN_ACT_TANH = 3 
 /* output transform + likelihood:
  *   CATEGORICAL   SoftMax (BNN_lib.py:166-168) + calc_likelihood (BNN_lib.py:100-121)
  *   GAUSSIAN      RegressTransform (BNN_lib.py:174) + calc_likelihood_regression (BNN_lib.py:123-131)
- *   GAUSSIAN_HEAD RegressTransformError (BNN_lib.py:177-182) + calc_likelihood_regression_error (:134-143) */
-enum { BNN_LIK_CATEGORICAL = 0, BNN_LIK_GAUSSIAN = 1, BNN_LIK_GAUSSIAN_HEAD = 2 };
+ *   GAUSSIAN_HEAD RegressTransformError (BNN_lib.py:177-182) + calc_likelihood_regression_error (:134-143)
+ * count data (estimation_mode="custom", RegressTransform outputs z, counts k; lik_temp is not applied, as there):
+ *   POISSON       poi_likelihood (BNN_lik.py:5-14): sum xlogy(k, exp(z0)) - gammaln(k+1) - exp(z0); K = 1 modelled
+ *                 column (output column 0), any output width
+ *   NEGBIN        negbin_likelihood / negbin_likelihood2d (BNN_lik.py:16-50): per modelled column j < K = O/2,
+ *                 nbinom.logpmf(k_j; n, p) with mean = exp(z_j), p = 1/(1+exp(-z_{K+j})), n = p mean/(1-p); even O
+ *   NEGBIN10      negbin_likelihood_base10 (BNN_lik.py:52-66): NEGBIN with 10** in place of exp
+ * For the count kinds the residual sums (sums_dev, BNN_F_SUM_R*) are of r = mean - k (mean = exp(z0), 10**z0):
+ * poi_acc / negbin_acc / negbin2d_acc / negbin_acc_base10 = sum r^2 / (N K). */
+enum { BNN_LIK_CATEGORICAL = 0, BNN_LIK_GAUSSIAN = 1, BNN_LIK_GAUSSIAN_HEAD = 2,
+       BNN_LIK_POISSON = 3, BNN_LIK_NEGBIN = 4, BNN_LIK_NEGBIN10 = 5 };
 /* npBNN prior_f, BNN_env.py:135-150 */
 enum { BNN_PRIOR_UNIFORM = 0, BNN_PRIOR_NORMAL = 1, BNN_PRIOR_CAUCHY = 2, BNN_PRIOR_LAPLACE = 3 };
 /* error parameter of the Gaussian likelihood: fixed sigma[O] per chain, or the population std of the
@@ -162,9 +171,10 @@ int64_t bnn_n_params(const bnn_ctx* ctx);
 
 /* Stage the data set once (npBNN._data/_labels/_test_data/_test_labels, BNN_env.py:35-49; the
  * reference re-copies X every step, BNN_env.py:388).  x_dev is [n_train + n_test, F] row-major,
- * training rows first.  labels_dev (int32 [n]) for CATEGORICAL, targets_dev (f64 [n, O]) for the
- * Gaussian likelihoods.  inst_w_dev [n_train] and class_w_dev [K] may be NULL
- * (calc_likelihood's instance_weight / class_weight, BNN_lib.py:100-121). */
+ * training rows first.  labels_dev (int32 [n]) for CATEGORICAL, targets_dev (f64 [n, K]) for the
+ * Gaussian and count likelihoods (K modelled columns: O, O/2 with the sigma head or NEGBIN*, 1 for POISSON).
+ * inst_w_dev [n_train] and class_w_dev [K] may be NULL (calc_likelihood's instance_weight / class_weight,
+ * BNN_lib.py:100-121); the count likelihoods refuse both (BNN_lik.py ignores them). */
 int bnn_set_data(bnn_ctx* ctx, const double* x_dev, int64_t n_train, int64_t n_test,
                  const int32_t* labels_dev, const double* targets_dev,
                  const double* inst_w_dev, const double* class_w_dev, void* stream);

@@ -14,6 +14,8 @@ MAX_OUT = 32
 
 ACT = {"ReLU": 0, "genReLU": 1, "swish": 2, "tanh": 3}
 LIK_CATEGORICAL, LIK_GAUSSIAN, LIK_GAUSSIAN_HEAD = 0, 1, 2
+LIK_POISSON, LIK_NEGBIN, LIK_NEGBIN10 = 3, 4, 5          # count likelihoods (estimation_mode="custom")
+LIK_COUNT = (LIK_POISSON, LIK_NEGBIN, LIK_NEGBIN10)
 PRIOR_UNIFORM, PRIOR_NORMAL, PRIOR_CAUCHY, PRIOR_LAPLACE = 0, 1, 2, 3
 SIGMA_FIXED, SIGMA_EMPIRICAL = 0, 1
 

@@ -7,6 +7,8 @@ CUDA library behind the C ABI (include/npbnn_b200.h).  There is no CPU fallback.
 What is on the device path            reference
   npBNN.calc_prior                    BNN_env.py:180-194
   MCMC.__init__ / MCMC.mh_step        BNN_env.py:274-532   (update_function = UpdateNormal)
+  count likelihoods (custom mode)     BNN_lik.py:5-66      (poi_likelihood, negbin_likelihood, negbin_likelihood2d,
+                                                          negbin_likelihood_base10 and their accuracy functions)
   run_mcmc                            BNN_mcmc.py:153-170
   MC3.run_mcmc                        BNN_mc3.py:87-126
   RunPredict / RunPredictInd / predict  BNN_lib.py:245-272, BNN_env.py:662-670
@@ -22,8 +24,13 @@ proposals on the device and never leaves it between logging points.
 
 Trainable activation parameters (ActFun(trainable=True)), init_additional_prob, mh_step(additional_prob=), weight
 indicators (freq_indicator > 0) and feature indicators (feature_indicators=True) run on the device from host-drawn
-numbers (rng="host"); hyper-prior scales (hyper_p) are drawn on the host and evaluated on the device.  Options of the reference that are not on the device path raise
-NotImplementedError: user-supplied likelihood / proposal / output functions, and the regression error-parameter proposal (estimate_error with empirical_error=False once the
+numbers (rng="host"); hyper-prior scales (hyper_p) are drawn on the host and evaluated on the device.
+
+estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
+MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
+companion MSE.  Options of the reference that are not on the device path raise
+NotImplementedError: other user-supplied likelihood / proposal / output functions (gamma_likelihood among them), count
+likelihoods under row sharding, and the regression error-parameter proposal (estimate_error with empirical_error=False once the
 iteration passes `_estimate_error` -- a branch on which the reference itself raises AttributeError as soon as one
 proposal has been accepted before that iteration, BNN_mcmc.py:105).
 """
@@ -46,7 +53,9 @@ small_number = 1e-10
 # callers around the path
 from .hostlib import (CalcAccuracy, CalcAccuracyRegression, CalcLabelAccuracy, CalcLabelAccuracyRegression,  # noqa: E402,F401
                       CalcLabelFreq, RegressTransform, RegressTransformError, SoftMax, UpdateNormal, calc_likelihood,
-                      calc_likelihood_regression, calc_likelihood_regression_error, load_obj, log_header)
+                      calc_likelihood_regression, calc_likelihood_regression_error, gamma_likelihood, load_obj, log_header,
+                      negbin2d_acc, negbin_acc, negbin_acc_base10, negbin_likelihood, negbin_likelihood2d,
+                      negbin_likelihood_base10, poi_acc, poi_likelihood)
 
 
 class ActFun:
@@ -117,11 +126,49 @@ def create_mask(w_layers, indx_input_list, nodes_per_feature_list):
     return masks
 
 
-_LIK = {"classification": L.LIK_CATEGORICAL, "regression": L.LIK_GAUSSIAN, "regression-error": L.LIK_GAUSSIAN_HEAD}
+# device likelihood of each estimation mode.  A custom model's own engine (prior, identity prediction) is the Gaussian
+# one; its sampler's kind is the count likelihood that MCMC(likelihood_f=) selects (_count_likelihood).
+_LIK = {"classification": L.LIK_CATEGORICAL, "regression": L.LIK_GAUSSIAN, "regression-error": L.LIK_GAUSSIAN_HEAD,
+        "custom": L.LIK_GAUSSIAN}
+
+# custom likelihoods on the device (BNN_lik.py), selected by function identity: likelihood_f -> (device kind, companion
+# accuracy_f)
+_COUNT_LIK = {poi_likelihood: (L.LIK_POISSON, poi_acc), negbin_likelihood: (L.LIK_NEGBIN, negbin_acc),
+              negbin_likelihood2d: (L.LIK_NEGBIN, negbin2d_acc),
+              negbin_likelihood_base10: (L.LIK_NEGBIN10, negbin_acc_base10)}
 
 
-def _net_of(weights, n_features, act_fun, estimation_mode):
-    return NetShape.from_weights(weights, n_features, act=act_fun._function, lik=_LIK[estimation_mode])
+def _count_likelihood(bnn, likelihood_f, accuracy_f, accuracy_lab_f, row_shard=False):
+    """The device likelihood kind and accuracy function of a sampler: None for a built-in estimation mode (which takes
+    no user functions), the count kind of likelihood_f for estimation_mode="custom"."""
+    if bnn._estimation_mode != "custom":
+        if likelihood_f is not None or accuracy_f is not None or accuracy_lab_f is not None:
+            raise NotImplementedError("user-supplied likelihood / accuracy functions are not on the device path")
+        return None, None
+    if likelihood_f is gamma_likelihood:
+        raise NotImplementedError("gamma_likelihood is not on the device path: it passes its second parameter as scipy's "
+                                  "location (BNN_lik.py:83) and broadcasts [N, 1] labels against [N] parameters into an "
+                                  "N x N table")
+    if likelihood_f not in _COUNT_LIK:
+        raise NotImplementedError("estimation_mode='custom' runs on the device with likelihood_f = poi_likelihood, "
+                                  "negbin_likelihood, negbin_likelihood2d or negbin_likelihood_base10")
+    kind, companion = _COUNT_LIK[likelihood_f]
+    if accuracy_f is not None and accuracy_f is not companion:
+        raise NotImplementedError("accuracy_f of %s must be %s (or None)" % (likelihood_f.__name__, companion.__name__))
+    if accuracy_lab_f is not None:
+        raise NotImplementedError("user-supplied accuracy_lab_f is not on the device path")
+    if row_shard:
+        raise NotImplementedError("row sharding of the count likelihoods is not implemented")
+    o, n_lab = bnn._size_output, bnn._labels.shape[1]
+    if likelihood_f is negbin_likelihood2d and o != 2 * n_lab:
+        raise ValueError("negbin_likelihood2d needs size_output = 2 x the label columns (%d), not %d" % (2 * n_lab, o))
+    if kind != L.LIK_POISSON and likelihood_f is not negbin_likelihood2d and o != 2:
+        raise NotImplementedError("%s on the device needs size_output=2 (mean, dispersion)" % likelihood_f.__name__)
+    return kind, companion
+
+
+def _net_of(weights, n_features, act_fun, estimation_mode, lik=None):
+    return NetShape.from_weights(weights, n_features, act=act_fun._function, lik=_LIK[estimation_mode] if lik is None else lik)
 
 
 class npBNN:
@@ -138,8 +185,14 @@ class npBNN:
         if estimation_mode not in _LIK:
             raise NotImplementedError("estimation_mode=%r (custom likelihoods) is not on the device path" % (estimation_mode,))
         if output_act_fun is not None and not (estimation_mode == "regression-error" and output_act_fun is RegressTransformError) \
-                and not (estimation_mode == "regression" and output_act_fun is RegressTransform):
+                and not (estimation_mode in ("regression", "custom") and output_act_fun is RegressTransform):
             raise NotImplementedError("user-supplied output_act_fun is not on the device path")
+        if estimation_mode == "custom":
+            # the count likelihoods read identity outputs; the reference crashes on None (RunPredict calls it)
+            if output_act_fun is not RegressTransform:
+                raise NotImplementedError("estimation_mode='custom' runs on the device with output_act_fun=RegressTransform")
+            if size_output is None:
+                raise ValueError("estimation_mode='custom' needs size_output")
         data, labels = dat["data"], dat["labels"]
         self._seed = seed
         self._data = np.ascontiguousarray(data, dtype=np.float64)
@@ -160,6 +213,10 @@ class npBNN:
             self._size_output = self._labels.shape[1]
             self._n_output_prm = self._labels.shape[1]
             self._error_prm = np.ones(self._size_output)
+        elif estimation_mode == "custom":
+            self._output_act_fun = RegressTransform
+            self._size_output = int(size_output)
+            self._n_output_prm = self._labels.shape[1]
         else:
             self._output_act_fun = RegressTransformError
             self._size_output = self._labels.shape[1] * 2
@@ -316,9 +373,9 @@ class _ChainGroup:
 
     def __init__(self, bnn, weights_per_chain, temperatures, update_f, update_ws, lik_temp, adapt_f, adapt_fM,
                  adapt_freq, adapt_stop, sample_from_prior, seed, device=0, init_additional_prob=0.0, row_shard=False,
-                 chain_offset=0):
+                 chain_offset=0, lik=None):
         self.bnn = bnn
-        net = _net_of(weights_per_chain[0], bnn._n_features, bnn._act_fun, bnn._estimation_mode)
+        net = _net_of(weights_per_chain[0], bnn._n_features, bnn._act_fun, bnn._estimation_mode, lik)
         self.net = net
         self.eng = Engine(net, device=device)
         cw = bnn._class_w if len(bnn._class_w) else None
@@ -456,8 +513,7 @@ class MCMC:
                  _group=None, _slot=0):
         if update_function is not UpdateNormal:
             raise NotImplementedError("only update_function=UpdateNormal runs on the device")
-        if likelihood_f is not None or accuracy_f is not None or accuracy_lab_f is not None:
-            raise NotImplementedError("user-supplied likelihood / accuracy functions are not on the device path")
+        count_kind, count_acc = _count_likelihood(bnn_obj, likelihood_f, accuracy_f, accuracy_lab_f, row_shard)
         if rng not in ("host", "philox"):
             raise ValueError("rng must be 'host' or 'philox'")
         if rng == "philox" and bnn_obj._freq_indicator and bnn_obj._n_layers < 4:
@@ -491,7 +547,7 @@ class MCMC:
             _group = _ChainGroup(bnn_obj, [bnn_obj._w_layers], [temperature], list(update_f)[:nl], list(update_ws)[:nl],
                                  likelihood_tempering, adapt_f, adapt_fM, adapt_freq, self._adapt_stop, sample_from_prior,
                                  seed=int(bnn_obj._seed) + 7919 * int(mcmc_id), device=device,
-                                 init_additional_prob=init_additional_prob, row_shard=row_shard)
+                                 init_additional_prob=init_additional_prob, row_shard=row_shard, lik=count_kind)
         elif bnn_obj._act_fun._trainable or init_additional_prob:
             raise NotImplementedError("trainable activation parameters / init_additional_prob inside an MC3 group")
         self._group, self._slot = _group, _slot
@@ -499,10 +555,13 @@ class MCMC:
         self._bnn_shapes = [w.shape for w in bnn_obj._w_layers]
         # the function attributes user scripts call on host tables (bnn_regress.py:55: mcmc._accuracy_lab_f(mcmc._y, ...))
         cls = bnn_obj._estimation_mode == "classification"
-        self._likelihood_f = {"classification": calc_likelihood, "regression": calc_likelihood_regression,
-                              "regression-error": calc_likelihood_regression_error}[bnn_obj._estimation_mode]
-        self._accuracy_f = CalcAccuracy if cls else CalcAccuracyRegression
-        self._accuracy_lab_f = CalcLabelAccuracy if cls else CalcLabelAccuracyRegression
+        if count_kind is not None:
+            self._likelihood_f, self._accuracy_f, self._accuracy_lab_f = likelihood_f, count_acc, None
+        else:
+            self._likelihood_f = {"classification": calc_likelihood, "regression": calc_likelihood_regression,
+                                  "regression-error": calc_likelihood_regression_error}[bnn_obj._estimation_mode]
+            self._accuracy_f = CalcAccuracy if cls else CalcAccuracyRegression
+            self._accuracy_lab_f = CalcLabelAccuracy if cls else CalcLabelAccuracyRegression
         self._bnn_view = bnn_obj
         self._sync(bnn_obj, self._group.eng.read_state())
 
@@ -529,6 +588,14 @@ class MCMC:
             self._label_acc = st.class_correct[c][present] / g.labels_count[present]
             self._label_freq = st.pred_hist[c] / n
             self._test_accuracy = st.n_correct_test[c] / nt if nt else 0
+        elif bnn_obj._estimation_mode == "custom":
+            # the companion MSE of the count likelihood (poi_acc, negbin_acc, ...): mean of (mean - k)^2 over the K
+            # modelled columns; no per-output accuracies
+            o = g.eng.K
+            self._accuracy = float(np.sum(st.sum_r2[c]) / (n * o))
+            self._label_acc = []
+            self._label_freq = None
+            self._test_accuracy = float(np.sum(st.sum_r2_test[c]) / (nt * o)) if nt else 0
         else:
             o = bnn_obj._n_output_prm
             self._accuracy = float(np.sum(st.sum_r2[c]) / (n * o))
@@ -809,8 +876,7 @@ class MC3:
     def __init__(self, data, logger, n_post_samples=100, sampling_f=100, n_chains=4, swap_frequency=100, verbose=1,
                  print_f=100, temperatures=None, min_temperature=0.8, likelihood_f=None, accuracy_f=None, adapt_freq=50,
                  adapt_f=0.1, adapt_fM=0.6, adapt_stop=1000, n_iteration=100000, rng="host", device=0, swap_seed=None):
-        if likelihood_f is not None or accuracy_f is not None:
-            raise NotImplementedError("user-supplied likelihood / accuracy functions are not on the device path")
+        count_kind, _ = _count_likelihood(data, likelihood_f, accuracy_f, None)
         import torch.distributed as dist
         self.n_chains = n_chains
         self.swap_frequency = swap_frequency
@@ -850,7 +916,7 @@ class MC3:
         self._group = _ChainGroup(data, [data._w_layers] * self.n_local,
                                   self.temperatures[self.start:self.start + self.n_local], [0.05] * nl, [0.075] * nl,
                                   1, adapt_f, adapt_fM, adapt_freq, adapt_stop, 0, seed=int(self.rseeds[0]), device=device,
-                                  chain_offset=self.start)
+                                  chain_offset=self.start, lik=count_kind)
         # per-chain views with the reference's attribute surface (singleChainArgs[i] = [bnn, mcmc])
         self.singleChainArgs = []
         for i in range(self.n_local):
@@ -859,7 +925,7 @@ class MC3:
             m = MCMC(b, temperature=self.temperatures[self.start + i], n_iteration=swap_frequency, sampling_f=sampling_f,
                      print_f=swap_frequency * 10, n_post_samples=n_post_samples, mcmc_id=self.start + i, randomize_seed=True,
                      adapt_freq=adapt_freq, adapt_f=adapt_f, adapt_fM=adapt_fM, adapt_stop=adapt_stop, rng=rng,
-                     _group=self._group, _slot=i)
+                     likelihood_f=likelihood_f, accuracy_f=accuracy_f, _group=self._group, _slot=i)
             self.singleChainArgs.append([b, m])
         self.current_temperatures = self.temperatures.copy()
 

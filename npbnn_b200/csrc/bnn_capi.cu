@@ -61,7 +61,7 @@ struct bnn_ctx {
   NetGeom g_base{};                 // minimal padding (bnn_set_net)
   NetGeom wp_geom{};                // layout the zero padding of wp_scratch was prepared for
   // staged data
-  DevBuf xs, labels, targets, inst_w, class_w;
+  DevBuf xs, labels, targets, lgk1, inst_w, class_w;     // lgk1: lgamma(k + 1) of the targets (count likelihoods)
   bool has_iw = false, has_cw = false;
   long long n_train = 0, n_test = 0, n_total = 0, n_pad = 0, n_tiles16 = 0;
   // workspaces
@@ -195,6 +195,7 @@ static FwdParams base_params(const bnn_ctx* c) {
   p.n_tiles16 = c->n_tiles16;
   p.labels = c->labels.as<int>();
   p.targets = c->targets.as<double>();
+  p.lgk1 = c->lgk1.as<double>();
   p.inst_w = c->has_iw ? c->inst_w.as<double>() : nullptr;
   p.class_w = c->has_cw ? c->class_w.as<double>() : nullptr;
   p.exp_tab = c->exp_tab.as<double>();
@@ -407,7 +408,7 @@ int bnn_set_net(bnn_ctx* c, const bnn_net_spec* s) {
   REQUIRE(s->n_layers >= 1 && s->n_layers <= BNN_MAX_LAYERS, "bnn_set_net: n_layers must be in [1, 8]");
   REQUIRE(s->n_features >= 1, "bnn_set_net: n_features must be positive");
   REQUIRE(s->act >= BNN_ACT_RELU && s->act <= BNN_ACT_TANH, "bnn_set_net: unknown activation");
-  REQUIRE(s->lik >= BNN_LIK_CATEGORICAL && s->lik <= BNN_LIK_GAUSSIAN_HEAD, "bnn_set_net: unknown likelihood");
+  REQUIRE(s->lik >= BNN_LIK_CATEGORICAL && s->lik <= BNN_LIK_NEGBIN10, "bnn_set_net: unknown likelihood");
   NetGeom g{};
   g.L = s->n_layers;
   g.F = s->n_features;
@@ -443,6 +444,11 @@ int bnn_set_net(bnn_ctx* c, const bnn_net_spec* s) {
   if (g.lik == BNN_LIK_GAUSSIAN_HEAD) {
     REQUIRE(g.O % 2 == 0, "bnn_set_net: the sigma-head likelihood needs an even output width");
     g.K = g.O / 2;
+  } else if (g.lik == BNN_LIK_POISSON) {
+    g.K = 1;                                     // poi_likelihood reads output column 0 only (BNN_lik.py:5-14)
+  } else if (g.lik == BNN_LIK_NEGBIN || g.lik == BNN_LIK_NEGBIN10) {
+    REQUIRE(g.O % 2 == 0, "bnn_set_net: the negative-binomial likelihood needs an even output width (mean | dispersion)");
+    g.K = g.O / 2;
   } else {
     g.K = g.O;
   }
@@ -471,6 +477,7 @@ int bnn_set_data(bnn_ctx* c, const double* x_dev, int64_t n_train, int64_t n_tes
   if (g.lik == BNN_LIK_CATEGORICAL) REQUIRE(labels_dev != nullptr, "bnn_set_data: labels_dev required for the categorical likelihood");
   else REQUIRE(targets_dev != nullptr, "bnn_set_data: targets_dev required for the Gaussian likelihoods");
   if (g.lik != BNN_LIK_CATEGORICAL) REQUIRE(inst_w_dev == nullptr, "instance_weight not implemented for regression (BNN_lib.py:129-130)");
+  if (bnn_lik_is_count(g.lik)) REQUIRE(class_w_dev == nullptr, "class_weight is not used by the count likelihoods (BNN_lik.py)");
   REQUIRE(!(inst_w_dev && class_w_dev), "class_weight together with instance_weight is an AxisError in the reference (BNN_lib.py:105)");
   CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
@@ -495,6 +502,11 @@ int bnn_set_data(bnn_ctx* c, const double* x_dev, int64_t n_train, int64_t n_tes
   } else {
     CUDA_TRY(c->targets.ensure(sizeof(double) * c->n_total * g.K, false, st));
     CUDA_TRY(cudaMemcpyAsync(c->targets.p, targets_dev, sizeof(double) * c->n_total * g.K, cudaMemcpyDeviceToDevice, st));
+    if (bnn_lik_is_count(g.lik)) {
+      CUDA_TRY(c->lgk1.ensure(sizeof(double) * c->n_total * g.K, false, st));
+      CUDA_TRY(bnn_launch_lgamma1(c->targets.as<double>(), c->lgk1.as<double>(), c->n_total * g.K, st));
+      c->launches++;
+    }
   }
   c->has_iw = inst_w_dev != nullptr;
   if (c->has_iw) {
@@ -1176,6 +1188,7 @@ int bnn_rowshard_config(bnn_ctx* c, int64_t n_train_global) {
   REQUIRE(c && c->have_data, "bnn_rowshard_config: call bnn_set_data (this rank's rows) first");
   invalidate_graphs(c);
   REQUIRE(n_train_global >= c->n_train, "bnn_rowshard_config: n_train_global is smaller than the local shard");
+  REQUIRE(!bnn_lik_is_count(c->g.lik), "bnn_rowshard_config: row sharding of the count likelihoods is not implemented");
   c->rowshard = true;
   c->n_train_global = n_train_global;
   c->have_chains = false;

@@ -921,6 +921,65 @@ __device__ __forceinline__ void quad_gauss_lik(const FwdParams& p, int c, long l
   if (lane == 0) p.part[((long long)c * p.NF) * nt + wt] = ll;
 }
 
+// Count likelihoods (BNN_LIK_POISSON / NEGBIN / NEGBIN10, BNN_lik.py:5-66) on the same fragment: per row and modelled
+// column j the log-pmf of bnn_count_loglik (the dispersion output K + j fetched from the lane that holds it, as the
+// sigma head does), summed over the training rows; sum r, sum r^2 (train) and sum r^2 (test) of r = mean - k for the
+// companion MSE.  Same xor trees and slots as quad_gauss_lik, so finalize_loglik and the accept step read them alike.
+template <int N3>
+__device__ __forceinline__ void quad_count_lik(const FwdParams& p, int c, long long wt, int lane,
+                                               const double (&acc)[N3 / 8][4]) {
+  static_assert(N3 == 8, "count outputs fit one 8-column tile");
+  const int K = p.g.K, lik = p.g.lik;
+  const int gq = lane >> 2, t = lane & 3;
+  const long long nt = p.n_tiles16;
+  double ll = 0.0, sr[2] = {0.0, 0.0}, sr2[2] = {0.0, 0.0}, st2[2] = {0.0, 0.0};
+#pragma unroll
+  for (int e = 0; e < 2; ++e) {
+    const int col = 2 * t + e;
+    const int dcol = (col + K) & 7;                                // column of this output's dispersion (NEGBIN*)
+    const int src = (gq << 2) | (dcol >> 1);
+    const double d00 = __shfl_sync(FULL_MASK, acc[0][0], src), d01 = __shfl_sync(FULL_MASK, acc[0][1], src);
+    const double d10 = __shfl_sync(FULL_MASK, acc[0][2], src), d11 = __shfl_sync(FULL_MASK, acc[0][3], src);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const long long row = wt * 16 + gq + 8 * h;
+      const bool active = row < p.n_total && col < K;
+      const bool train = active && row < p.n_train;
+      double r = 0.0;
+      if (active) {
+        const double zd = (dcol & 1) ? (h ? d11 : d01) : (h ? d10 : d00);
+        const double lr = bnn_count_loglik(lik, acc[0][2 * h + e], zd, p.targets[row * K + col], p.lgk1[row * K + col], &r);
+        if (train) ll += lr;
+      }
+      sr[e] += train ? r : 0.0;
+      sr2[e] += train ? r * r : 0.0;
+      st2[e] += (active && !train) ? r * r : 0.0;
+    }
+  }
+#pragma unroll
+  for (int o = 4; o <= 16; o <<= 1)                                 // rows: fixed xor tree over g => deterministic
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      sr[e] += __shfl_xor_sync(FULL_MASK, sr[e], o);
+      sr2[e] += __shfl_xor_sync(FULL_MASK, sr2[e], o);
+      st2[e] += __shfl_xor_sync(FULL_MASK, st2[e], o);
+    }
+#pragma unroll
+  for (int o = 1; o <= 16; o <<= 1) ll += __shfl_xor_sync(FULL_MASK, ll, o);
+  if (gq == 0) {
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const int col = 2 * t + e;
+      if (col < K) {
+        p.part[((long long)c * p.NF + 1 + col) * nt + wt] = sr[e];
+        p.part[((long long)c * p.NF + 1 + K + col) * nt + wt] = sr2[e];
+        p.part[((long long)c * p.NF + 1 + 2 * K + col) * nt + wt] = st2[e];
+      }
+    }
+  }
+  if (lane == 0) p.part[((long long)c * p.NF) * nt + wt] = ll;
+}
+
 // prediction mode: transformed outputs (identity, softplus on the sigma head) accumulated over the weight sets
 template <int N3>
 __device__ __forceinline__ void quad_gauss_pred(const FwdParams& p, int c, long long wt, int lane,
@@ -947,8 +1006,9 @@ __device__ __forceinline__ void quad_gauss_pred(const FwdParams& p, int c, long 
 
 // MODE: 0 likelihood, 1 likelihood with class / instance weights, 2 posterior prediction
 enum { FWD3_LIK = 0, FWD3_LIK_W = 1, FWD3_PRED = 2 };
-// LIKK: 0 categorical (softmax epilogue, software-pipelined into the next weight set), 1 Gaussian (plain or sigma head)
-enum { FWD3_CAT = 0, FWD3_GAUSS = 1 };
+// LIKK: 0 categorical (softmax epilogue, software-pipelined into the next weight set), 1 Gaussian (plain or sigma head),
+// 2 count likelihoods (likelihood modes only: their prediction is the Gaussian instantiation's identity output)
+enum { FWD3_CAT = 0, FWD3_GAUSS = 1, FWD3_COUNT = 2 };
 
 template <int ACT, int KP0, int N1, int N2, int N3, int NWARPS, int MODE, int LIKK = FWD3_CAT>
 __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__ FwdParams p) {
@@ -1326,6 +1386,9 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
         }
         if constexpr (CAT) {
           if (PREDICT) quad_epilogue_pred<N3>(p, c, wt, lane, acc3, tab, pacc, pvote);
+        } else if constexpr (LIKK == FWD3_COUNT) {
+          static_assert(!PREDICT, "count prediction runs the FWD3_GAUSS instantiation");
+          quad_count_lik<N3>(p, c, wt, lane, acc3);
         } else {
           if (PREDICT) quad_gauss_pred<N3>(p, c, wt, lane, acc3, pacc, tab);
           else quad_gauss_lik<N3>(p, c, wt, lane, acc3, tab);
@@ -2099,7 +2162,7 @@ static cudaError_t launch_fwd3(const FwdParams& p, int n_sms, cudaStream_t st) {
 }
 
 // k_fwd3 instantiations: two padded width families x four activations x {categorical (N3 = 16: likelihood, weighted
-// likelihood, prediction), Gaussian / sigma head (N3 = 8: likelihood, prediction)}
+// likelihood, prediction), Gaussian / sigma head (N3 = 8: likelihood, prediction), count (N3 = 8: likelihood)}
 //   family A   64 -> 64 -> 32 -> N3   12 warps per SM (BASELINE config 4 / 5 is its swish / categorical member)
 //   family B   32 -> 32 -> 16 -> N3   16 warps per SM
 template <int ACT, int KP0, int N1, int N2, int NWARPS>
@@ -2110,6 +2173,7 @@ static cudaError_t launch_fwd3_family(const FwdParams& p, bool predict, int n_sm
     return launch_fwd3<ACT, KP0, N1, N2, 16, NWARPS, FWD3_LIK, FWD3_CAT>(p, n_sms, st);
   }
   if (predict) return launch_fwd3<ACT, KP0, N1, N2, 8, NWARPS, FWD3_PRED, FWD3_GAUSS>(p, n_sms, st);
+  if (bnn_lik_is_count(p.g.lik)) return launch_fwd3<ACT, KP0, N1, N2, 8, NWARPS, FWD3_LIK, FWD3_COUNT>(p, n_sms, st);
   return launch_fwd3<ACT, KP0, N1, N2, 8, NWARPS, FWD3_LIK, FWD3_GAUSS>(p, n_sms, st);
 }
 

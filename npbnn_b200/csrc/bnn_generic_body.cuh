@@ -133,9 +133,10 @@ __device__ __forceinline__ void bnn_epilogue(const FwdParams& p, int c, long lon
     return;
   }
 
-  // Gaussian likelihoods: K modelled outputs, targets [n_total, K]
+  // Gaussian and count likelihoods: K modelled outputs, targets [n_total, K]
   const int K = g.K;
   const bool head = (g.lik == BNN_LIK_GAUSSIAN_HEAD);
+  const bool count = bnn_lik_is_count(g.lik);
   if (!PREDICT) {
     double ll = 0.0;
     for (int j = 0; j < K; ++j) {
@@ -143,7 +144,11 @@ __device__ __forceinline__ void bnn_epilogue(const FwdParams& p, int c, long lon
       if (active) {
         double t = tgt16 ? tgt16[rl * K + j] : p.targets[row * K + j];
         r = z[j] - t;
-        if (head && is_train) {
+        if (count) {
+          // (r is the residual of the count mean; test rows need it for the test MSE, the likelihood is train only)
+          const double lr = bnn_count_loglik(g.lik, z[j], z[K + j], t, p.lgk1[row * K + j], &r);
+          if (is_train) ll += lr;
+        } else if (head && is_train) {
           double s = softplus_ref(z[K + j]);
           double u = (t - z[j]) / s;
           ll += -0.5 * u * u - kLogSqrt2Pi - log(s);

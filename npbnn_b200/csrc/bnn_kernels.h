@@ -71,6 +71,8 @@ cudaError_t bnn_launch_pack_x(const double* x, double* xs, long long n, long lon
                               const int* ov_cols, const double* ov_vals, int n_ov, cudaStream_t st);
 // *flag |= 1 if a training label is outside [0, K) or a test label is negative (the reference raises IndexError there)
 cudaError_t bnn_launch_check_labels(const int* labels, long long n_train, long long n_total, int K, int* flag, cudaStream_t st);
+// out[i] = lgamma(k[i] + 1): the label-only term of the count likelihoods, once per data set
+cudaError_t bnn_launch_lgamma1(const double* k, double* out, long long n, cudaStream_t st);
 cudaError_t bnn_launch_pack_w(const NetGeom& g, const double* w, double* wp, int n_sets, cudaStream_t st);
 cudaError_t bnn_launch_finalize_lik(const NetGeom& g, const double* part, int NF, long long nt, long long n_train,
                                     double lik_temp, int sigma_mode, const double* sigma, double* loglik, double* sums,

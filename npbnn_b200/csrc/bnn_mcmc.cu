@@ -271,6 +271,20 @@ cudaError_t bnn_launch_check_labels(const int* labels, long long n_train, long l
   return cudaGetLastError();
 }
 
+// gammaln(k + 1) of the count likelihoods (BNN_lik.py:5-66) depends on the labels only
+__global__ void k_lgamma1(const double* __restrict__ k, double* __restrict__ out, long long n) {
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) out[i] = lgamma(k[i] + 1.0);
+}
+
+cudaError_t bnn_launch_lgamma1(const double* k, double* out, long long n, cudaStream_t st) {
+  long long blocks = (n + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  if (blocks < 1) blocks = 1;
+  k_lgamma1<<<(int)blocks, 256, 0, st>>>(k, out, n);
+  return cudaGetLastError();
+}
+
 cudaError_t bnn_measure_dmma_peak(int n_sms, double* tflops) {
   const int grid = n_sms * 2, threads = 256, iters = 2048;
   double* out = nullptr;

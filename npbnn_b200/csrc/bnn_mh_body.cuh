@@ -152,7 +152,8 @@ __device__ double finalize_loglik(const NetGeom& g, const double* part, int NF, 
     }
   }
   upd_sync<COH>();
-  return lik_temp * ll;
+  // the count likelihoods of BNN_lik.py take lik_temp and ignore it
+  return bnn_lik_is_count(g.lik) ? ll : lik_temp * ll;
 }
 
 #ifdef BNN_DBG_LOOPCLK       // tuning instrumentation: clocks per phase of the update body (thread 0 of chain 0)

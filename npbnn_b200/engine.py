@@ -129,7 +129,9 @@ class Engine:
         L.check(self.lib.bnn_set_net(h, C.byref(spec)))
         assert self.lib.bnn_n_params(h) == net.n_params
         out = net.shapes[-1][0]
-        self.K = out // 2 if net.lik == L.LIK_GAUSSIAN_HEAD else out
+        # modelled output columns: sigma head / negative binomial = (value | parameter) halves, Poisson = column 0
+        self.K = out // 2 if net.lik in (L.LIK_GAUSSIAN_HEAD, L.LIK_NEGBIN, L.LIK_NEGBIN10) else \
+            (1 if net.lik == L.LIK_POISSON else out)
         self.O = out
         self.n_train = self.n_test = 0
         self.n_chains = 0
@@ -171,7 +173,8 @@ class Engine:
 
     # ---------------------------------------------------------------- data
     def set_data(self, x, y, x_test=None, y_test=None, inst_w=None, class_w=None):
-        """Stage training (+ optional test) rows once (npBNN._data/_labels..., reference BNN_env.py:35-49)."""
+        """Stage training (+ optional test) rows once (npBNN._data/_labels..., reference BNN_env.py:35-49).  The count
+        likelihoods model the first K label columns (the ones BNN_lik.py reads)."""
         with torch.cuda.device(self.device):
             xs = [self._dev(x, torch.float64)]
             n_train, n_test = xs[0].shape[0], 0
@@ -187,6 +190,9 @@ class Engine:
             assert xd.shape[1] == self.net.n_features
             if not cat:
                 yd = yd.reshape(n_train + n_test, -1)
+                if self.net.lik in L.LIK_COUNT:
+                    assert yd.shape[1] >= self.K
+                    yd = yd[:, :self.K].contiguous()
                 assert yd.shape[1] == self.K
             iw, cw = self._dev(inst_w, torch.float64), self._dev(class_w, torch.float64)
             L.check(self.lib.bnn_set_data(self._h, _ptr(xd), n_train, n_test, _ptr(yd) if cat else None,

@@ -706,8 +706,9 @@ def GibbsSampleGammaRateExp(sd, a, alpha_0=1., beta_0=1.):
 
 
 # ------------------------------------------------------------------------------------------------------
-# count-data likelihoods of BNN_lik.py: host functions for estimation_mode="custom" users; custom likelihoods are not
-# on the device path (npBNN raises for them), the functions are exported so that post-processing code keeps working
+# count-data likelihoods of BNN_lik.py: host functions for estimation_mode="custom" users.  Inside MCMC / MC3
+# (likelihood_f=, accuracy_f=) the four count likelihoods and their accuracy functions are identity tokens that select
+# the device epilogue (BNN_LIK_POISSON / NEGBIN / NEGBIN10); gamma_likelihood is not on the device path
 # ------------------------------------------------------------------------------------------------------
 def _nbinom_logpmf(k, n, p):
     from scipy.special import gammaln, xlog1py, xlogy
