@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define BNN_ABI_VERSION 1
+#define BNN_ABI_VERSION 2
 #define BNN_MAX_LAYERS 8
 #define BNN_MAX_OUT 32          /* max width of the output layer (classes, or 2*O for the sigma head) */
 
@@ -313,13 +313,9 @@ int bnn_predict_sample_philox(bnn_ctx* ctx, const double* x_dev, int64_t n, cons
                               const double* alpha_dev, uint64_t seed, double* est_dev, int32_t* class_counts_dev,
                               double* post_pred_dev, void* stream);
 
-/* Debugging / tuning aids (no reference counterpart).
- * bnn_debug_read_part: per-warp-tile partial sums of the last forward pass, [sets in pass][slots][n_tiles16].
- * bnn_debug_counters : 48 clock counters of k_fwd3t, all zero unless the library was built with -DBNN_DBG_WAITCLK. */
+/* Debugging aid (no reference counterpart).
+ * bnn_debug_read_part: per-warp-tile partial sums of the last forward pass, [sets in pass][slots][n_tiles16]. */
 int bnn_debug_read_part(bnn_ctx* ctx, double* out_host, int64_t n_doubles);
-int bnn_debug_counters(bnn_ctx* ctx, unsigned long long* out48_host);
-/* bnn_debug_set_trace: device buffer [CTAs][uses][8 warps][2] for the checksums a -DBNN_DBG_CSUM build records. */
-int bnn_debug_set_trace(bnn_ctx* ctx, unsigned long long* trace_dev);
 /* Options: "force_generic" = 1 disables the shape-specialised forward kernels (cross-check in tests);
  * "time_forward" = 1 enables bnn_forward_time; "sparse" = 0 evaluates masked chains with the dense kernels;
  * "graphs" = 0 launches the free-running bnn_mh_steps loop eagerly instead of replaying a CUDA graph;
@@ -330,9 +326,7 @@ int bnn_debug_set_trace(bnn_ctx* ctx, unsigned long long* trace_dev);
  * "predict_tf32" = 1 (default 0) evaluates bnn_predict summaries (mean / votes) of the 64-64-32-16 categorical family on the
  * TF32 tensor cores in error-compensated 3xTF32 form with FP32 activations: class probabilities agree with the FP64 kernel
  * to ~1e-6 absolute (stated tolerance 5e-6); 2 = plain TF32 (one product, ~1e-4, stated 5e-3); bnn_mh_steps and the
- * likelihood calls never use reduced precision;
- * "tensor_l1" = 1 (layer 1 of the 64-64-32-10 swish network as exact int8 tensor-core products, k_fwd3t) exists only in
- * builds with -DBNN_EXPERIMENTAL_TENSOR_L1; the shipped library refuses it (DESIGN.md section 4). */
+ * likelihood calls never use reduced precision.  Any other name is refused. */
 int bnn_set_option(bnn_ctx* ctx, const char* name, int value);
 
 #ifdef __cplusplus

@@ -7,7 +7,8 @@ import ctypes as C
 import os
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("NPBNN_B200_LIB") or os.path.join(HERE, "libnpbnn_b200.so")   # override: tuning variants
+# NPBNN_B200_LIB loads another build of the library instead (e.g. to compare two builds on the same inputs)
+LIB_PATH = os.environ.get("NPBNN_B200_LIB") or os.path.join(HERE, "libnpbnn_b200.so")
 
 MAX_LAYERS = 8
 MAX_OUT = 32
@@ -103,8 +104,6 @@ _SIGNATURES = {
     "bnn_rowshard_commit": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_rowshard_update": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.POINTER(Injection), C.c_void_p]),
     "bnn_debug_read_part": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64]),
-    "bnn_debug_counters": (C.c_int, [C.c_void_p, C.c_void_p]),
-    "bnn_debug_set_trace": (C.c_int, [C.c_void_p, C.c_void_p]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_SIGNATURES))
@@ -125,7 +124,7 @@ def load(build_if_missing=True):
         fn = getattr(lib, name)       # AttributeError if the library does not export the symbol
         fn.restype = res
         fn.argtypes = args
-    if lib.bnn_abi_version() != 1:
+    if lib.bnn_abi_version() != 2:
         raise NpbnnError("libnpbnn_b200.so ABI version mismatch")
     _lib = lib
     return lib

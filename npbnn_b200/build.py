@@ -29,19 +29,6 @@ def _stale(target, deps):
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_variant(name, defines):
-    """Tuning helper: build csrc with extra -D defines into libnpbnn_b200_<name>.so (select with NPBNN_B200_LIB)."""
-    nvcc = _nvcc()
-    out = os.path.join(HERE, "libnpbnn_b200_%s.so" % name)
-    cmd = [nvcc] + [f for f in NVCC_FLAGS if f not in ("-Xptxas", "-v")] + ["-D%s" % d for d in defines] + \
-        ["-shared", "-o", out] + [os.path.join(CSRC, s) for s in SOURCES]
-    r = subprocess.run(cmd, capture_output=True, text=True)
-    if r.returncode:
-        sys.stderr.write(r.stdout + r.stderr)
-        raise RuntimeError("variant build failed")
-    return out
-
-
 def build(force=False, verbose=False):
     nvcc = _nvcc()
     hdrs = [os.path.join(CSRC, h) for h in HEADERS]

@@ -67,6 +67,7 @@ struct bnn_ctx {
   // workspaces
   DevBuf exp_tab, exp_tab_small, wp_scratch, part, counts_scratch, xs_pred, ov_cols, ov_vals;
   DevBuf h_w, h_alpha, h_sigma, h_loglik, h_sums, h_counts;    // device staging of the *_host entry points
+  DevBuf flag;                      // one int: bnn_set_data's label check
   // chains
   int C = 0;
   bnn_sampler_config cfg{};
@@ -90,11 +91,6 @@ struct bnn_ctx {
   cudaEvent_t inj_copied = nullptr;   // the last transfer out of inj_host
   const char* last_kernel = "";
   // block-masked networks: dataflow program of the chains' mask (k_fwd_sparse)
-  // tensor-core first layer (k_fwd3t): int8 slices of X (made once per data set) and of W1 (per scored batch)
-  DevBuf xsl, x_rowscale, wt, oz_flag;
-  long long n_tiles128 = 0;
-  bool tensor_ok = false;           // the staged data and the network shape qualify
-  int opt_tensor = 0;               // option "tensor_l1" (env NPBNN_TENSOR_L1): 1 = layer 1 on the int8 tensor cores (opt-in)
   DevBuf sp_items, sp_widx;
   int sp_prog_len = 0, sp_n_items = 0, sp_slots = 1, sp_wlen = 0;
   int sp_pair_nc1 = 0, sp_pair_nr1 = 0, sp_pair_nr2 = 0;   // uniform block pairs (k_fwd_sparse's fused path); nc1 == 0: none
@@ -136,30 +132,7 @@ static void invalidate_graphs(bnn_ctx* c) {
   c->mh_warm = false;
 }
 
-// network shapes with a k_fwd3t instantiation (BASELINE config 4 / 5: 64 -> 64 -> 32 -> 10 swish, categorical)
-static bool tensor_shape(const NetGeom& g) {
-#ifndef BNN_EXPERIMENTAL_TENSOR_L1
-  (void)g;
-  return false;                      // k_fwd3t is not part of the shipped library (bnn_forward.cu)
-#endif
-  return g.L == 3 && g.F_pad == 64 && g.l[0].out_pad == 64 && g.l[1].out_pad == 32 && g.l[2].out_pad == 16 &&
-         g.act == BNN_ACT_SWISH && g.lik == BNN_LIK_CATEGORICAL;
-}
-
-static cudaError_t timed_forward(bnn_ctx* c, const FwdParams& p_in, bool predict, cudaStream_t st) {
-  FwdParams p = p_in;
-  if (!predict && c->tensor_ok && c->opt_tensor && !c->force_generic && !p.sp_prog && p.x == c->xs.as<double>()) {
-    // slice W1 of every weight set of this pass for the integer tensor-core product
-    cudaError_t r = c->wt.ensure(bnn_slice_w1_bytes() * (size_t)p.C, false, st);
-    if (r != cudaSuccess) return r;
-    r = bnn_launch_slice_w1(p.wp, c->g.PB, c->wt.as<uint8_t>(), p.C, st);
-    if (r != cudaSuccess) return r;
-    c->launches++;
-    p.xsl = c->xsl.as<uint8_t>();
-    p.x_rowscale = c->x_rowscale.as<double>();
-    p.wt = c->wt.as<uint8_t>();
-    p.n_tiles128 = c->n_tiles128;
-  }
+static cudaError_t timed_forward(bnn_ctx* c, const FwdParams& p, bool predict, cudaStream_t st) {
   if (!c->time_forward) return bnn_launch_forward(p, predict, c->n_sms, c->force_generic, st, &c->last_kernel);
   if (c->ev_used + 2 > c->ev.size()) {
     for (int i = 0; i < 2; ++i) {
@@ -298,10 +271,6 @@ int bnn_ctx_create(bnn_ctx** out, int device) {
   c->force_generic = (fg && fg[0] == '1') ? 1 : 0;
   const char* pt = getenv("NPBNN_PREDICT_TF32");           // opt-in reduced-precision prediction summaries (bnn_pred_lp.cu)
   if (pt) c->opt_pred_tf32 = atoi(pt);
-#ifdef BNN_EXPERIMENTAL_TENSOR_L1
-  const char* tl = getenv("NPBNN_TENSOR_L1");
-  if (tl) c->opt_tensor = (tl[0] != '0');
-#endif
   std::vector<double> tab(BNN_EXP_TAB_SIZE);
   for (int j = 0; j < BNN_EXP_TAB_SIZE; ++j) tab[j] = exp2((double)j / BNN_EXP_TAB_SIZE);
   cudaError_t e = c->exp_tab.ensure(sizeof(double) * BNN_EXP_TAB_SIZE, false, 0);
@@ -321,12 +290,12 @@ int bnn_ctx_destroy(bnn_ctx* c) {
   if (!c) return 0;
   cudaSetDevice(c->device);
   cudaDeviceSynchronize();
-  DevBuf* bufs[] = {&c->xs, &c->labels, &c->targets, &c->inst_w, &c->class_w, &c->exp_tab, &c->exp_tab_small, &c->wp_scratch, &c->part,
-                    &c->counts_scratch, &c->xs_pred, &c->ov_cols, &c->ov_vals, &c->h_w, &c->h_alpha, &c->h_sigma,
-                    &c->h_loglik, &c->h_sums, &c->h_counts, &c->w_cur, &c->w_prop, &c->wp_prop, &c->mask, &c->owner,
-                    &c->sf, &c->si, &c->counts_prop, &c->alpha_chain, &c->inj_proposed, &c->inj_count, &c->inj_ix,
-                    &c->inj_iy, &c->inj_dz, &c->inj_logu, &c->inj_alpha_ix, &c->inj_alpha_dz, &c->inj_add_prob, &c->part_red, &c->part_sl, &c->sp_items, &c->sp_widx, &c->xsl, &c->x_rowscale, &c->wt,
-                    &c->oz_flag};
+  DevBuf* bufs[] = {&c->xs, &c->labels, &c->targets, &c->lgk1, &c->inst_w, &c->class_w, &c->exp_tab, &c->exp_tab_small,
+                    &c->wp_scratch, &c->part, &c->counts_scratch, &c->xs_pred, &c->ov_cols, &c->ov_vals, &c->h_w,
+                    &c->h_alpha, &c->h_sigma, &c->h_loglik, &c->h_sums, &c->h_counts, &c->w_cur, &c->w_prop,
+                    &c->wp_prop, &c->mask, &c->owner, &c->sf, &c->si, &c->counts_prop, &c->alpha_chain,
+                    &c->inj_proposed, &c->inj_count, &c->inj_ix, &c->inj_iy, &c->inj_dz, &c->inj_logu, &c->inj_alpha_ix,
+                    &c->inj_alpha_dz, &c->inj_add_prob, &c->part_red, &c->part_sl, &c->sp_items, &c->sp_widx, &c->flag};
   for (DevBuf* b : bufs) b->release();
   c->ps_entry.release(); c->pls_entry.release(); c->ps_tmp.release(); c->pls_tmp.release();
   for (DevBuf* b : {&c->ind_cur, &c->ind_prop, &c->fi_cur, &c->fi_prop, &c->feat_mean, &c->inj_ind_move, &c->inj_ind_flip,
@@ -354,14 +323,6 @@ int bnn_set_option(bnn_ctx* c, const char* name, int value) {
   if (strcmp(name, "force_generic") == 0) { c->force_generic = value; return 0; }
   if (strcmp(name, "time_forward") == 0) { c->time_forward = value; return 0; }
   if (strcmp(name, "sparse") == 0) { c->opt_sparse = value; return 0; }
-  if (strcmp(name, "tensor_l1") == 0) {
-#ifndef BNN_EXPERIMENTAL_TENSOR_L1
-    REQUIRE(value == 0, "tensor_l1: the experimental tensor-core first layer (k_fwd3t) is not compiled into this library "
-                        "(build with -DBNN_EXPERIMENTAL_TENSOR_L1)");
-#endif
-    c->opt_tensor = value;
-    return 0;
-  }
   if (strcmp(name, "graphs") == 0) { c->opt_graphs = value; return 0; }
   if (strcmp(name, "chain_loop") == 0) { c->opt_chain_loop = value; return 0; }
   if (strcmp(name, "predict_tf32") == 0) { c->opt_pred_tf32 = value; return 0; }
@@ -371,24 +332,6 @@ int bnn_set_option(bnn_ctx* c, const char* name, int value) {
     return 0;
   }
   return fail(std::string("bnn_set_option: unknown option ") + name);
-}
-
-// tuning instrumentation of k_fwd3t (all zeros unless the library was built with -DBNN_DBG_WAITCLK)
-int bnn_debug_counters(bnn_ctx* c, unsigned long long* out32_host) {
-  REQUIRE(c && out32_host, "bnn_debug_counters: null argument");
-  CUDA_TRY(cudaSetDevice(c->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(bnn_debug_counters_read(out32_host));
-  return 0;
-}
-
-// debugging aid: device buffer for the per-(CTA, use, warp) checksums of a -DBNN_DBG_CSUM build (NULL = off)
-int bnn_debug_set_trace(bnn_ctx* c, unsigned long long* dev_ptr) {
-  REQUIRE(c, "bnn_debug_set_trace: null context");
-  CUDA_TRY(cudaSetDevice(c->device));
-  CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(bnn_debug_set_trace_ptr(dev_ptr));
-  return 0;
 }
 
 // debugging aid: per-warp-tile partial sums of the last forward pass, [n_sets_in_pass][NF][n_tiles16]
@@ -490,12 +433,12 @@ int bnn_set_data(bnn_ctx* c, const double* x_dev, int64_t n_train, int64_t n_tes
   if (g.lik == BNN_LIK_CATEGORICAL) {
     CUDA_TRY(c->labels.ensure(sizeof(int) * c->n_total, false, st));
     CUDA_TRY(cudaMemcpyAsync(c->labels.p, labels_dev, sizeof(int) * c->n_total, cudaMemcpyDeviceToDevice, st));
-    CUDA_TRY(c->oz_flag.ensure(sizeof(int), false, st));
-    CUDA_TRY(cudaMemsetAsync(c->oz_flag.p, 0, sizeof(int), st));
-    CUDA_TRY(bnn_launch_check_labels(c->labels.as<int>(), n_train, c->n_total, g.K, c->oz_flag.as<int>(), st));
+    CUDA_TRY(c->flag.ensure(sizeof(int), false, st));
+    CUDA_TRY(cudaMemsetAsync(c->flag.p, 0, sizeof(int), st));
+    CUDA_TRY(bnn_launch_check_labels(c->labels.as<int>(), n_train, c->n_total, g.K, c->flag.as<int>(), st));
     c->launches++;
     int bad_label = 0;
-    CUDA_TRY(cudaMemcpyAsync(&bad_label, c->oz_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaMemcpyAsync(&bad_label, c->flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
     REQUIRE(bad_label == 0, "bnn_set_data: class labels must lie in [0, K) with K = the output width of the network "
                             "(the reference raises IndexError at BNN_lib.py:104)");
@@ -517,21 +460,6 @@ int bnn_set_data(bnn_ctx* c, const double* x_dev, int64_t n_train, int64_t n_tes
   if (c->has_cw) {
     CUDA_TRY(c->class_w.ensure(sizeof(double) * g.K, false, st));
     CUDA_TRY(cudaMemcpyAsync(c->class_w.p, class_w_dev, sizeof(double) * g.K, cudaMemcpyDeviceToDevice, st));
-  }
-  c->tensor_ok = false;
-  if (tensor_shape(g)) {
-    c->n_tiles128 = (c->n_pad + 127) / 128;
-    CUDA_TRY(c->xsl.ensure(bnn_slice_x_tile_bytes() * (size_t)c->n_tiles128, false, st));
-    CUDA_TRY(c->x_rowscale.ensure(sizeof(double) * (size_t)c->n_tiles128 * 128, false, st));
-    CUDA_TRY(c->oz_flag.ensure(sizeof(int), false, st));
-    CUDA_TRY(cudaMemsetAsync(c->oz_flag.p, 0, sizeof(int), st));
-    CUDA_TRY(bnn_launch_slice_x(c->xs.as<double>(), c->n_pad, c->xsl.as<uint8_t>(), c->x_rowscale.as<double>(),
-                                c->n_tiles128, c->oz_flag.as<int>(), st));
-    c->launches++;
-    int bad = 0;
-    CUDA_TRY(cudaMemcpyAsync(&bad, c->oz_flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(cudaStreamSynchronize(st));
-    c->tensor_ok = (bad == 0);      // non-finite features: integer slices cannot carry inf / NaN, stay on FP64
   }
   c->have_data = true;
   c->have_chains = false;
@@ -1115,7 +1043,7 @@ int bnn_mh_steps(bnn_ctx* c, int32_t n_steps, const bnn_injection* inj, void* st
   // Small data sets (a few thousand rows, <= 2048 weights, dense generic forward path): all n_steps iterations run
   // inside ONE persistent launch, a thread-block cluster per chain (bnn_chainloop.cu) -- injected or device-generated
   // proposals alike.  Same update / forward bodies and reduction order as the launch sequence below: identical chains.
-  if (c->opt_chain_loop && !c->time_forward && !c->opt_tensor && !(c->use_sparse && c->opt_sparse) &&
+  if (c->opt_chain_loop && !c->time_forward && !(c->use_sparse && c->opt_sparse) &&
       (c->force_generic || !bnn_fwd3_family(c->g)) && !bnn_part_slices(c->n_tiles16) &&
       bnn_chain_loop_fits(c->g, d.NF, d.n_tiles16, c->C, c->n_sms, c->opt_chain_cluster, c->opt_chain_loop)) {
     FwdParams p = base_params(c);
@@ -1139,8 +1067,7 @@ int bnn_mh_steps(bnn_ctx* c, int32_t n_steps, const bnn_injection* inj, void* st
   // it is captured once per n_steps into a CUDA graph and replayed -- at small N the loop is bound by launch latency,
   // not by the kernels.  The first call after any (re)configuration runs eagerly (function attributes, lazily
   // allocated workspaces); capture uses a private stream because the caller's may be the legacy default stream.
-  const bool graphable = !inj && c->opt_graphs && c->mh_warm && !c->time_forward && !c->opt_tensor &&
-                         n_steps >= 2 && n_steps <= 512;
+  const bool graphable = !inj && c->opt_graphs && c->mh_warm && !c->time_forward && n_steps >= 2 && n_steps <= 512;
   if (graphable) {
     cudaGraphExec_t exec = nullptr;
     long long per_launch = 0;

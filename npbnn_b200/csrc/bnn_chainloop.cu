@@ -13,7 +13,6 @@
 //     straight into the leader's shared memory (distributed shared memory stores / atomics);
 //   * barrier.cluster; next step.
 // Chains are independent, so the C clusters of a launch need not be co-resident.
-#include <cstdio>
 #include <cstdlib>
 #include <cooperative_groups.h>
 #include "bnn_mh_body.cuh"
@@ -143,12 +142,6 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
   ctx.didx_sm = didx_sm; ctx.ddz_sm = ddz_sm; ctx.pk_sm = pk_sm; ctx.pp_mode = pp_mode;
   const double2* wsrc = reinterpret_cast<const double2*>(d.wp_prop + (long long)c * g.PB);
 
-#ifdef BNN_DBG_LOOPCLK
-  long long lt[6] = {0, 0, 0, 0, 0, 0}, l0 = clock64(), dbg_epi = 0;
-#define LOOP_STAMP(i) do { const long long now_ = clock64(); lt[i] += now_ - l0; l0 = now_; } while (0)
-#else
-#define LOOP_STAMP(i) do { } while (0)
-#endif
   for (int s = 0; s <= n_steps; ++s) {
     // leader CTA, first UPD_TEAM_THREADS threads: accept step s-1, propose step s (the packed proposal lands in wsm)
     if (leader && tid < UPD_TEAM_THREADS) {
@@ -157,9 +150,7 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
       if (s < n_steps && tid < g.L) alpha_sm[tid] = d.alpha_fwd[(long long)c * g.L + tid];   // written by thread 0 before the team's last barrier
     }
     if (s == n_steps) break;
-    LOOP_STAMP(0);
     cluster.sync();                          // the proposal of step s (packed weights, slopes, zeroed counters) is visible
-    LOOP_STAMP(1);
     if (!leader) {
       // packed proposal from L2 (a pull from the leader's shared memory by 15 CTAs at once is bound by that SM's
       // shared-memory port: 5.7k clk measured against 2k through L2)
@@ -168,7 +159,6 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
     }
     for (int i = tid; i < NC; i += NTHR) cnt_local[i] = 0;
     __syncthreads();
-    LOOP_STAMP(2);
     for (int i = 0; i < n_slots; ++i) {
       const long long wt = tile_of(i);
       if (wt >= nt) break;
@@ -176,21 +166,12 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
       const double* xt = XRES ? slot : p.x + wt * 16 * (long long)g.F_pad;
       const double* xrow0 = xt + gq * g.F_pad;
       const double* xrow1 = xrow0 + 8 * g.F_pad;
-#ifdef BNN_DBG_LOOPCLK
-      const long long f0 = clock64();
-#endif
       fwd_generic_layers<ACT, !XRES, false>(g, xrow0, xrow1, wsm, (ACT == BNN_ACT_LEAKY) ? alpha_sm : nullptr, h0, h1, zs,
                                             ZS, tab, lane);
-#ifdef BNN_DBG_LOOPCLK
-      const long long f1 = clock64();
-#endif
       bnn_epilogue<false, false, GEN_TB>(p, 0, wt, lane, zs, ZS, tab, cnt_local, nullptr, nullptr,
                                          (XRES && cat) ? reinterpret_cast<const int*>(slot + 16 * g.F_pad) : nullptr,
                                          (XRES && !cat) ? slot + 16 * g.F_pad : nullptr);
       __syncwarp();
-#ifdef BNN_DBG_LOOPCLK
-      if (tid == 0) { lt[5] += f1 - f0; dbg_epi += clock64() - f1; }
-#endif
     }
     // the leader's team is done with its few tiles long before the workers: it pre-proposes iteration s + 1 (layer
     // choice, scalar draws, the proposal's draws) in the time it would otherwise wait at the barrier
@@ -199,25 +180,11 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
       mh_update_body<true>(d, c, 0, 3, s + 1, ctx);
     }
     __syncthreads();
-    LOOP_STAMP(3);
     if (cat)
       for (int i = tid; i < NC; i += NTHR)
         if (cnt_local[i]) atomicAdd(&cnt_dst[i], cnt_local[i]);
     cluster.sync();                          // partials and counters of step s are in the leader's shared memory
-    LOOP_STAMP(4);
   }
-#ifdef BNN_DBG_LOOPCLK
-  if (tid == 0 && c == 0 && (rank == 0 || rank == 1) && n_steps >= 50) {
-    printf("rank %d per step (clk): update %lld | barrier A %lld | weights %lld | forward %lld (warp 0: layers %lld, epilogue %lld) | flush + barrier B %lld\n", rank,
-           lt[0] / n_steps, lt[1] / n_steps, lt[2] / n_steps, lt[3] / n_steps, lt[5] / n_steps, dbg_epi / n_steps, lt[4] / n_steps);
-    if (rank == 0) {
-      printf("  update body: load %lld finalize %lld accept %lld thread0 %lld copy/ind %lld owner %lld reflect %lld sum %lld writeback %lld\n",
-             g_dbg_upd[0] / n_steps, g_dbg_upd[1] / n_steps, g_dbg_upd[2] / n_steps, g_dbg_upd[3] / n_steps, g_dbg_upd[4] / n_steps,
-             g_dbg_upd[5] / n_steps, g_dbg_upd[6] / n_steps, g_dbg_upd[7] / n_steps, g_dbg_upd[8] / n_steps);
-      for (int i = 0; i < 16; ++i) g_dbg_upd[i] = 0;
-    }
-  }
-#endif
   // no CTA may exit while others can still address its shared memory
   cluster.sync();
 }

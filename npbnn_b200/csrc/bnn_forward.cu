@@ -14,7 +14,6 @@
 //                 copies + mbarriers, hidden activations never leave registers.
 //   k_fwd_generic any depth/width: hidden activations staged in per-warp shared memory, weights read
 //                 through L1/L2.
-#include <cstdio>
 #include <type_traits>
 #include "bnn_common.cuh"
 #include "bnn_generic_body.cuh"
@@ -222,31 +221,10 @@ __device__ __forceinline__ void sparse_pair(const int* it, int nc1_rt, int O, co
 #pragma unroll
     for (int i = 0; i < NR1; ++i) care |= bnn_act_needs_care<ACT>(h1[q][i]);
   if (!__any_sync(FULL_MASK, care)) {
-#ifndef SPARSE_STAGED_ACT
 #pragma unroll
     for (int q = 0; q < NCH; ++q)
 #pragma unroll
       for (int i = 0; i < NR1; ++i) h1[q][i] = bnn_act_fast<ACT>(h1[q][i], alpha1[q], tab);
-#else
-    // all NCH * NR1 evaluations level by level (ActPipe): the program order ptxas gets is already interleaved
-    ActPipe<ACT, NCH * NR1> ap;
-#pragma unroll
-    for (int q = 0; q < NCH; ++q)
-#pragma unroll
-      for (int i = 0; i < NR1; ++i) ap.z[q * NR1 + i] = h1[q][i];
-    static_for<0, ActPipe<ACT, NCH * NR1>::STAGES>([&](auto st) {
-      if constexpr (ACT == BNN_ACT_LEAKY) {
-#pragma unroll
-        for (int q = 0; q < NCH; ++q) ap.template stage_range<decltype(st)::value>(q * NR1, (q + 1) * NR1, alpha1[q], tab);
-      } else {
-        ap.template stage<decltype(st)::value>(0.0, tab);
-      }
-    });
-#pragma unroll
-    for (int q = 0; q < NCH; ++q)
-#pragma unroll
-      for (int i = 0; i < NR1; ++i) h1[q][i] = ap.z[q * NR1 + i];
-#endif
   } else {
 #pragma unroll
     for (int q = 0; q < NCH; ++q)
@@ -277,30 +255,10 @@ __device__ __forceinline__ void sparse_pair(const int* it, int nc1_rt, int O, co
 #pragma unroll
     for (int j = 0; j < NR2; ++j) care |= bnn_act_needs_care<ACT>(h2[q][j]);
   if (!__any_sync(FULL_MASK, care)) {
-#ifndef SPARSE_STAGED_ACT
 #pragma unroll
     for (int q = 0; q < NCH; ++q)
 #pragma unroll
       for (int j = 0; j < NR2; ++j) h2[q][j] = bnn_act_fast<ACT>(h2[q][j], alpha2[q], tab);
-#else
-    ActPipe<ACT, NCH * NR2> ap;
-#pragma unroll
-    for (int q = 0; q < NCH; ++q)
-#pragma unroll
-      for (int j = 0; j < NR2; ++j) ap.z[q * NR2 + j] = h2[q][j];
-    static_for<0, ActPipe<ACT, NCH * NR2>::STAGES>([&](auto st) {
-      if constexpr (ACT == BNN_ACT_LEAKY) {
-#pragma unroll
-        for (int q = 0; q < NCH; ++q) ap.template stage_range<decltype(st)::value>(q * NR2, (q + 1) * NR2, alpha2[q], tab);
-      } else {
-        ap.template stage<decltype(st)::value>(0.0, tab);
-      }
-    });
-#pragma unroll
-    for (int q = 0; q < NCH; ++q)
-#pragma unroll
-      for (int j = 0; j < NR2; ++j) h2[q][j] = ap.z[q * NR2 + j];
-#endif
   } else {
 #pragma unroll
     for (int q = 0; q < NCH; ++q)
@@ -570,25 +528,8 @@ struct Fwd3Geom {
   static constexpr int PB = B3_OFF + N3;
 };
 
-#ifndef FWD3_WARPS
-#define FWD3_WARPS 12
-#endif
-#ifndef FWD3_ACT_MODE
-#define FWD3_ACT_MODE 0         // how layer-1 activations interleave with the layer-2 MMAs (tuning variants 1, 2)
-#endif
-
 template <int ACT, bool FAST = false, int TB = BNN_EXP_TAB_BITS>
 __device__ __forceinline__ void act_tile(double (&a)[4], double alpha, const double* tab) {
-#ifdef BNN_DBG_NOACT      // tuning experiment only: how fast is the kernel without activations?
-  return;
-#endif
-#ifdef BNN_DBG_ACTCHAIN   // tuning experiment only: N dependent register DFMAs per element instead of the activation
-#pragma unroll
-  for (int s = 0; s < BNN_DBG_ACTCHAIN; ++s)
-#pragma unroll
-    for (int e = 0; e < 4; ++e) a[e] = fma(a[e], 0.999, alpha);
-  return;
-#endif
 #pragma unroll
   for (int e = 0; e < 4; ++e) a[e] = FAST ? bnn_act_fast<ACT>(a[e], alpha, tab) : bnn_act<ACT, TB>(a[e], alpha, tab);
 }
@@ -1016,11 +957,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
   constexpr bool PREDICT = (MODE == FWD3_PRED);
   constexpr bool CAT = (LIKK == FWD3_CAT);
   constexpr bool DEFER = !PREDICT && CAT;        // categorical likelihood: epilogue pipelined into the next set's layer 1
-#ifdef BNN_DBG_NOEPI      // tuning experiment only: no likelihood epilogue at all (results are garbage)
-  constexpr bool EPI = false;
-#else
-  constexpr bool EPI = DEFER;
-#endif
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const NetGeom& g = p.g;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -1132,10 +1068,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
       }
     }
   };
-#ifdef BNN_DBG_RINGCLK
-  long long dbg_ring = 0;
-  const long long dbg_start = clock64();
-#endif
   long long q = 0;
   uint32_t x_uses = 0;               // X tiles this warp has loaded (parity of its mbarrier)
   bool x_prefetched = false;         // the X tile of this iteration was requested during the previous one
@@ -1193,13 +1125,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
     for (int c = c_lo; c < c_hi; ++c, ++q) {
       const int b = (int)(q & 1);
       __syncwarp();
-#ifdef BNN_DBG_RINGCLK      // tuning experiment only: clocks this warp spends waiting for the weight ring
-      const long long dbg_t0 = clock64();
-#endif
       mbar_wait(&full1[b], (uint32_t)((q >> 1) & 1));
-#ifdef BNN_DBG_RINGCLK
-      dbg_ring += clock64() - dbg_t0;
-#endif
       if (have_tile) {
         const double* W = w1buf + b * W1_D;                          // part 0; layers 2 / 3 index W23 with the same offsets
         const double* W23 = w23buf + b * W23_D - G3::W2_OFF;
@@ -1217,9 +1143,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
           const double* xr1 = xs + (gq + 8) * KP0;
           const double* wr = W + G3::W1_OFF + gq * KP0;
           const int sw = (gq & 1) * G3::SW0;
-          // Software pipeline over weight sets: the epilogue of the PREVIOUS set (softmax, log-likelihood,
-          // counters -- latency-bound FP64 chains and shuffles) sits in the same basic block as the first two
-          // k-groups of this set's layer 1, whose 64 DMMAs need no FP64 issue slots of their own.
           // Software pipeline over weight sets: the epilogue of the PREVIOUS set (softmax statistics, log-
           // likelihood: latency-bound FP64 chains and shuffles) is cut into four stages that are placed
           // between the MMA groups of the first two k-groups of this set's layer 1, whose DMMAs leave the
@@ -1232,7 +1155,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
             const int col = (8 * kg + 2 * t) ^ sw;
             const double2 alo = *reinterpret_cast<const double2*>(xr0 + col);
             const double2 ahi = *reinterpret_cast<const double2*>(xr1 + col);
-            if (EPI) {
+            if (DEFER) {
               if (kg == 0) qs_max<N3>(acc3, K, t, rs);
               else qs_exp<N3, 1, true>(acc3, K, t, ep_y, tab, rs);
             }
@@ -1241,7 +1164,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
               const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * KP0 + col);
               dmma16x8x8(acc1[j], alo.x, ahi.x, alo.y, ahi.y, bb.x, bb.y);
             }
-            if (EPI) {
+            if (DEFER) {
               if (kg == 0) qs_exp<N3, 0, true>(acc3, K, t, ep_y, tab, rs);
               else {
                 qs_reduce<N3, true>(rs);
@@ -1254,9 +1177,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
               dmma16x8x8(acc1[j], alo.x, ahi.x, alo.y, ahi.y, bb.x, bb.y);
             }
           }
-#ifndef BNN_DBG_NOCOMMIT      // tuning experiment only: counters / partial store of the previous set
-          if (EPI) quad_lik_commit<N3>(p, ep_c, ep_wt, lane, cnt, lr, prev_valid);
-#endif
+          if (DEFER) quad_lik_commit<N3>(p, ep_c, ep_wt, lane, cnt, lr, prev_valid);
 #pragma unroll 2
           for (int kg = 2; kg < KP0 / 8 - 2; ++kg) {
             const int col = (8 * kg + 2 * t) ^ sw;
@@ -1341,12 +1262,8 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
             }
           }
         };
-#ifdef FWD3_NO_FAST_ACT
-        layer2(std::false_type{});
-#else
         if (frag_needs_care<ACT, N1 / 8>(acc1)) layer2(std::false_type{});
         else layer2(std::true_type{});
-#endif
         // ---------------- layer 3: [16 x N2] x [N2 x N3]
 #pragma unroll
         for (int j = 0; j < N3 / 8; ++j) {
@@ -1369,12 +1286,8 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
             }
           }
         };
-#ifdef FWD3_NO_FAST_ACT
-        layer3(std::false_type{});
-#else
         if (frag_needs_care<ACT, N2 / 8>(acc2)) layer3(std::false_type{});
         else layer3(std::true_type{});
-#endif
         // weights of this use are no longer needed by this warp
         __syncwarp();
         release_part(1, q);
@@ -1419,11 +1332,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
       }
     }
   }
-#ifdef BNN_DBG_RINGCLK
-  if (lane == 0 && (blockIdx.x == 0 || blockIdx.x == 77) && p.C >= 32)
-    printf("cta %d warp %2d (smsp %d): ring wait %lld of %lld clk (%.1f%%)\n", blockIdx.x, warp, warp & 3, dbg_ring,
-           clock64() - dbg_start, 100.0 * dbg_ring / (double)(clock64() - dbg_start));
-#endif
   // drain the software pipeline: the epilogue of the last (tile, weight set) this warp ran
   if (DEFER && prev_valid) {
     RowStats<N3> rs;
@@ -1437,698 +1345,6 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
       if (cnt[i]) atomicAdd(&p.counts[i], cnt[i]);
   }
 }
-
-// The int8 tensor-core first layer (k_fwd3t, below) is EXPERIMENTAL and compiled only with -DBNN_EXPERIMENTAL_TENSOR_L1:
-// with its helper warps allowed to run two weight sets ahead an intermittent corruption was observed whose cause is not
-// understood (DESIGN.md section 4), so the shipped library does not contain the kernel and "tensor_l1" cannot be enabled.
-#ifndef BNN_EXPERIMENTAL_TENSOR_L1
-cudaError_t bnn_debug_set_trace_ptr(unsigned long long*) { return cudaErrorNotSupported; }
-cudaError_t bnn_debug_counters_read(unsigned long long* out48) {
-  for (int i = 0; i < 48; ++i) out48[i] = 0;
-  return cudaSuccess;
-}
-cudaError_t bnn_launch_slice_x(const double*, long long, uint8_t*, double*, long long, int*, cudaStream_t) {
-  return cudaErrorNotSupported;
-}
-cudaError_t bnn_launch_slice_w1(const double*, int, uint8_t*, int, cudaStream_t) { return cudaErrorNotSupported; }
-size_t bnn_slice_x_tile_bytes() { return 0; }
-size_t bnn_slice_w1_bytes() { return 0; }
-#else
-// =============================================================================================
-// k_fwd3t: the 3-layer kernel with layer 1 on the 5th-generation tensor cores (tcgen05 + TMEM)
-// =============================================================================================
-// tcgen05 has no FP64 kind, but the first-layer contraction X W1^T can be evaluated EXACTLY in integer
-// arithmetic (Ozaki splitting): every row of X and every row of W1 is scaled by a power of two and rounded to a
-// 47-bit signed integer, which is cut into 6 balanced base-256 digits (int8 "slices"):
-//     x_ik = 2^(e_i - 46) * sum_s a_s[i,k] 256^s          w_nk = 2^(f_n - 46) * sum_t b_t[n,k] 256^t
-//     sum_k x_ik w_nk = 2^(e_i + f_n - 92) * sum_T 256^T * ( sum_{s+t=T} sum_k a_s[i,k] b_t[n,k] )
-// The inner sums are int8 x int8 -> int32 tensor-core products (tcgen05.mma kind::i8, exact, no overflow:
-// 6 pairs * 64 * 128^2 < 2^31); the 6 most significant diagonals T = 10..5 (21 slice pairs) are kept, the
-// dropped ones are zero-mean and below 2^-41 of max|x_i| * max|w_n| (measured: log-likelihood within 1e-12
-// relative of the FP64 kernels).  X is sliced once at bnn_set_data (k_slice_x), W1 once per proposal
-// (k_slice_w1); both are stored in HBM in the tensor core's K-major core-matrix layout, so a plain bulk copy
-// brings them to shared memory.  Layers 2 and 3 stay on the FP64 DMMA path of k_fwd3 -- their A operand is a
-// per-chain activation, so the chains cannot share an MMA and a 32- or 16-column tcgen05.mma costs as much as
-// a 128-column one (70 clk floor, tools/umma_probe.cu).
-//
-// CTA = one 128-row tile at a time: 8 compute warps (16 rows each, the TMEM lane quarter of warp w is w & 3)
-// + 1 control warp whose elected lane streams the operands (bulk copies) and issues the MMAs.  Per chain:
-//   control : wait weights(q) and "TMEM drained(q-1)" -> 42 MMAs into 6 x 64 TMEM columns -> commit
-//   compute : wait commit(q) -> tcgen05.ld.16x256b (= the m16n8 accumulator fragment layout) -> recombine the
-//             6 diagonals to FP64 in registers (two int64 groups, 5 FP64 instructions per element) ->
-//             signal "drained" -> activation, layers 2/3, likelihood epilogue exactly as k_fwd3
-// so the integer MMAs of chain q+1 run under the FP64 work of chain q.
-constexpr int OZ_S = 6;                               // slices per operand
-constexpr int OZ_P = 46;                              // operands are rounded to |v| <= 2^46
-constexpr int OZ_XROW = OZ_S * 64;                    // bytes of one row of X slices
-constexpr int OZ_XTILE = 128 * OZ_XROW;
-constexpr int OZ_WPLANE = 64 * 64;
-constexpr int OZ_W1_BYTES = OZ_S * OZ_WPLANE + 64 * 8;   // 6 planes + colscale[64]
-constexpr int OZ_LBO = 128, OZ_SBO = 512;             // K-major, no swizzle: 8-row x 16-byte core matrices
-
-__host__ __device__ inline int oz_kmajor_offset(int r, int k) {
-  return (r >> 3) * OZ_SBO + (k >> 4) * OZ_LBO + (r & 7) * 16 + (k & 15);
-}
-
-// 47-bit integer image of v * 2^(46 - e) as 6 balanced base-256 digits
-__device__ __forceinline__ void oz_digits(double v, int e, int8_t (&d)[OZ_S]) {
-  long long q = __double2ll_rn(scalbn(v, OZ_P - e));
-#pragma unroll
-  for (int s = 0; s < OZ_S - 1; ++s) {
-    const int b = (int)((q + 128) & 255) - 128;
-    d[s] = (int8_t)b;
-    q = (q - b) >> 8;
-  }
-  d[OZ_S - 1] = (int8_t)q;
-}
-// exponent e with max < 2^e (0 for an all-zero row)
-__device__ __forceinline__ int oz_exponent(double mx) { return mx > 0.0 ? ilogb(mx) + 1 : 0; }
-
-// X (swizzled rows, F_pad = 64) -> slices [n_rows128][6][64 B] (a row's 6 x 64 bytes are contiguous: the helper
-// thread that owns the row copies them to TMEM, where they are the A operand) + rowscale[n_rows128] = 2^e_i.
-// One thread per row.  flag is set when a row holds a non-finite value (the tensor path is then not used).
-__global__ void k_slice_x(const double* __restrict__ x, long long n_pad16, uint8_t* __restrict__ xsl,
-                          double* __restrict__ rowscale, long long n_rows128, int* __restrict__ flag) {
-  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (r >= n_rows128) return;
-  const int sw = (int)(r & 1) * 8;
-  double mx = 0.0;
-  bool bad = false;
-  if (r < n_pad16)
-    for (int k = 0; k < 64; ++k) {
-      const double v = x[r * 64 + (k ^ sw)];
-      bad |= !isfinite(v);
-      mx = fmax(mx, fabs(v));
-    }
-  if (bad) { atomicExch(flag, 1); mx = 0.0; }
-  const int e = oz_exponent(mx);
-  rowscale[r] = scalbn(1.0, e);
-  uint32_t* out = reinterpret_cast<uint32_t*>(xsl + r * (long long)(OZ_S * 64));
-  for (int k4 = 0; k4 < 16; ++k4) {
-    uint32_t w[OZ_S] = {0, 0, 0, 0, 0, 0};
-    for (int kk = 0; kk < 4; ++kk) {
-      const int k = 4 * k4 + kk;
-      int8_t d[OZ_S];
-      const double v = (r < n_pad16 && !bad) ? x[r * 64 + (k ^ sw)] : 0.0;
-      oz_digits(v, e, d);
-#pragma unroll
-      for (int sl = 0; sl < OZ_S; ++sl) w[sl] |= (uint32_t)(uint8_t)d[sl] << (8 * kk);
-    }
-#pragma unroll
-    for (int sl = 0; sl < OZ_S; ++sl) out[sl * 16 + k4] = w[sl];
-  }
-}
-
-// packed weight sets (W1 = [64][64] swizzled rows at offset 0) -> per set: 6 slice planes + colscale[n] = 2^(f_n - 48)
-__global__ void k_slice_w1(const double* __restrict__ wp, int PB, uint8_t* __restrict__ wt) {
-  const int c = blockIdx.x, n = threadIdx.x;       // 64 threads: one per output unit
-  const double* w = wp + (long long)c * PB + n * 64;
-  const int sw = (n & 1) * 8;
-  double mx = 0.0;
-  for (int k = 0; k < 64; ++k) mx = fmax(mx, fabs(w[k ^ sw]));
-  const int f = oz_exponent(mx);
-  uint8_t* out = wt + (long long)c * OZ_W1_BYTES;
-  reinterpret_cast<double*>(out + OZ_S * OZ_WPLANE)[n] = scalbn(1.0, f - 48);   // 2^(f - 92) * 2^44: the helpers park the recombined sum scaled by 2^-44
-  for (int k = 0; k < 64; ++k) {
-    int8_t d[OZ_S];
-    oz_digits(w[k ^ sw], f, d);
-#pragma unroll
-    for (int s = 0; s < OZ_S; ++s) out[s * OZ_WPLANE + oz_kmajor_offset(n, k)] = (uint8_t)d[s];
-  }
-}
-
-__device__ __forceinline__ uint64_t oz_smem_desc(uint32_t saddr) {
-  // cute::UMMA::SmemDescriptor: start address [0,14), LBO [16,30), SBO [32,46) (all >> 4), version 1 at [46,48),
-  // layout type SWIZZLE_NONE (0) at [61,64)
-  return (uint64_t)((saddr >> 4) & 0x3fff) | ((uint64_t)(OZ_LBO >> 4) << 16) | ((uint64_t)(OZ_SBO >> 4) << 32) |
-         ((uint64_t)1 << 46);
-}
-__device__ __forceinline__ void oz_mma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, {%5, %5, %5, %5}, p;\n\t}\n" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc), "r"(0u)
-      : "memory");
-}
-__device__ __forceinline__ void oz_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
-               : "memory");
-}
-// 16 TMEM lanes x 16 columns in the m16n8 accumulator-fragment layout (verified by tools/umma_probe.cu):
-// v[4h + {0,1,2,3}] = (row g, col 8h+2t), (g, 8h+2t+1), (g+8, 8h+2t), (g+8, 8h+2t+1)
-__device__ __forceinline__ void oz_ld_frag(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr));
-}
-// (hi * 65536 + mid * 256 + lo) as a double: |value| < 2^51, so adding it to the integer image of 1.5 * 2^52 and
-// subtracting 1.5 * 2^52 converts exactly with ONE FP64 instruction (I2F.F64 runs at a fraction of the DFMA rate)
-__device__ __forceinline__ double oz_group(int hi, int mid, int lo) {
-  const long long v = (long long)hi * 65536 + (long long)mid * 256 + (long long)lo;
-  return __longlong_as_double(v + 0x4338000000000000LL) - 6755399441055744.0;
-}
-
-// 32 TMEM lanes (thread = lane = row) x 8 consecutive 32-bit columns
-__device__ __forceinline__ void oz_ld_row8(uint32_t taddr, uint32_t (&v)[8]) {
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
-               : "r"(taddr));
-}
-
-constexpr int FWD3T_COMPUTE_WARPS = 8;     // 16 rows each: layers 2 / 3 (DMMA) + likelihood epilogue
-constexpr int FWD3T_HELPER_WARPS = 4;      // one per TMEM lane quarter: drain, recombine, activate layer 1
-constexpr int FWD3T_CONTROL_WARP = 12;     // lane 0: weight streaming + MMA issue (warps 13-15 only donate registers)
-constexpr int FWD3T_THREADS = 16 * 32;
-// registers per thread after setmaxnreg (the kernel is launched with 512 x 128): 8 x 168 + 4 x 128 + 4 x 40 <= 2048
-constexpr int FWD3T_REGS_COMPUTE = 168, FWD3T_REGS_CONTROL = 40;
-
-// activated layer-1 outputs of the 128-row tile in shared memory: row r, 16-byte chunk c (columns 2c, 2c+1) at
-// r * 512 + ((c ^ s(r)) * 16), s(r) = ((r & 1) << 2) | ((r >> 1) & 3): conflict-free both for the helpers'
-// stores (lane = row, same chunk) and for the compute warps' A-fragment loads (rows g, chunks 4kg + t)
-__device__ __forceinline__ int a1_swz(int r) { return ((r & 1) << 2) | ((r >> 1) & 3); }
-
-__device__ __forceinline__ void oz_mma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], [%1], %2, %3, {%5, %5, %5, %5}, p;\n\t}\n" ::"r"(tmem_d),
-      "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc), "r"(0u)
-      : "memory");
-}
-__device__ __forceinline__ void oz_ld_row16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void oz_st_row16(uint32_t taddr, const uint4 (&w)[4]) {
-  asm volatile(
-      "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};" ::"r"(taddr),
-      "r"(w[0].x), "r"(w[0].y), "r"(w[0].z), "r"(w[0].w), "r"(w[1].x), "r"(w[1].y), "r"(w[1].z), "r"(w[1].w), "r"(w[2].x),
-      "r"(w[2].y), "r"(w[2].z), "r"(w[2].w), "r"(w[3].x), "r"(w[3].y), "r"(w[3].z), "r"(w[3].w)
-      : "memory");
-}
-
-// tuning instrumentation (build with -DBNN_DBG_WAITCLK): clocks spent per wait site / phase, summed over lane 0 of
-// every warp; slots 0-15 helper 0 (control), 16-31 helpers 1-3, 32-47 compute warps.  Read and reset with bnn_debug_counters().
-__device__ unsigned long long g_dbg_clk[48];
-__device__ unsigned long long* g_dbg_trace = nullptr;   // BNN_DBG_CSUM: [CTA][use][warp][2] checksums (a1 read, logits)
-cudaError_t bnn_debug_set_trace_ptr(unsigned long long* dev_ptr) { return cudaMemcpyToSymbol(g_dbg_trace, &dev_ptr, sizeof(dev_ptr)); }
-#ifdef BNN_DBG_WAITCLK
-#define DBG_T0() const long long dbg_t0 = clock64()
-#define DBG_ADD(slot) dbg[slot] += clock64() - dbg_t0
-#define DBG_WAIT(slot, bar, par) do { const long long t0__ = clock64(); mbar_wait_sleep(bar, par); dbg[slot] += clock64() - t0__; } while (0)
-#else
-#define DBG_T0()
-#define DBG_ADD(slot)
-#define DBG_WAIT(slot, bar, par) mbar_wait_sleep(bar, par)
-#endif
-cudaError_t bnn_debug_counters_read(unsigned long long* out48) {
-  cudaError_t e = cudaMemcpyFromSymbol(out48, g_dbg_clk, sizeof(unsigned long long) * 48);
-  if (e != cudaSuccess) return e;
-  unsigned long long z[48] = {0};
-  return cudaMemcpyToSymbol(g_dbg_clk, z, sizeof(z));
-}
-
-constexpr uint32_t OZ_TMEM_X = OZ_S * 64;     // TMEM columns [384, 480): X slices (A operand), 16 columns per slice
-
-template <int ACT, int MODE>
-__global__ void __launch_bounds__(FWD3T_THREADS, 1) k_fwd3t(const __grid_constant__ FwdParams p) {
-  constexpr int KP0 = 64, N1 = 64, N2 = 32, N3 = 16;
-  using G3 = Fwd3Geom<KP0, N1, N2, N3>;
-  constexpr bool PREDICT = (MODE == FWD3_PRED);
-  constexpr int TB = 8;                                            // 256-entry exp table (shared memory is short)
-  constexpr int REST = G3::PB - G3::W2_OFF;                       // FP64 part for the compute warps: W2, b2, W3, b3
-  constexpr uint32_t W1_BYTES = OZ_S * OZ_WPLANE;                  // slice planes of W1
-  constexpr uint32_t RSLOT_BYTES = REST * 8;
-  constexpr uint32_t HSLOT_BYTES = 2 * 64 * 8;                     // colscale[64] + b1[64] for the helpers
-  extern __shared__ __align__(128) unsigned char smem_raw[];
-  const NetGeom& g = p.g;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int gq = lane >> 2, t = lane & 3;
-  long long dbg[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
-  (void)dbg;
-
-  // ---- shared memory carve-up
-  uint8_t* w1ring = smem_raw;                                      // [2][W1_BYTES]
-  uint8_t* rring = w1ring + 2 * W1_BYTES;                          // [2][RSLOT_BYTES]
-  double* a1s = reinterpret_cast<double*>(rring + 2 * RSLOT_BYTES);  // [2][128][64] layer-1 outputs (double buffer)
-  double* tab = a1s + 2 * 128 * 64;
-  uint8_t* hring = reinterpret_cast<uint8_t*>(tab + (1 << TB));     // [4][HSLOT_BYTES]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(hring + 4 * HSLOT_BYTES);
-  uint64_t* w1full = bars;          // [2] W1 slices of a use have landed
-  uint64_t* rfull = bars + 2;       // [2] colscale + FP64 part of a use have landed
-  uint64_t* rempty = bars + 4;      // [2] all compute warps are done with the slot
-  uint64_t* tfull = bars + 6;       // layer-1 accumulators of a use are complete in TMEM
-  uint64_t* tfree = bars + 7;       // all helpers have drained the accumulators (and refreshed X at a tile change)
-  uint64_t* a1full = bars + 8;      // [4][2] activated layer-1 rows of a lane quarter are in a1s buffer b
-  uint64_t* a1free = bars + 16;     // [4][2] both compute warps of the quarter have consumed them
-  uint64_t* hfull = bars + 24;      // [4] colscale + b1 of a use have landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 28);
-  int* cnt = reinterpret_cast<int*>(bars + 30);
-  const int n_cnt = PREDICT ? 0 : p.C * (2 + 2 * g.K);
-#ifdef BNN_DBG_CSUM            // debugging aid: checksums of the activation hand-off
-  volatile unsigned long long* dbg_cs = reinterpret_cast<volatile unsigned long long*>(cnt + ((n_cnt + 3) & ~3));   // [2][8]
-#endif
-
-  for (int i = threadIdx.x; i < (1 << TB); i += blockDim.x) tab[i] = p.exp_tab_small[i];
-  for (int i = threadIdx.x; i < n_cnt; i += blockDim.x) cnt[i] = 0;
-  if (threadIdx.x == 0) {
-    rel[0] = rel[1] = 0;
-    for (int i = 0; i < 2; ++i) { mbar_init(&w1full[i], 1); mbar_init(&rfull[i], 1); mbar_init(&rempty[i], FWD3T_COMPUTE_WARPS); }
-    mbar_init(tfull, 1); mbar_init(tfree, FWD3T_HELPER_WARPS);
-    for (int i = 0; i < 8; ++i) { mbar_init(&a1full[i], 1); mbar_init(&a1free[i], 2); }
-    for (int i = 0; i < 4; ++i) mbar_init(&hfull[i], 1);
-    mbar_fence_init();
-  }
-  if (warp == FWD3T_COMPUTE_WARPS) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem = *tmem_slot;
-
-  const long long n_iter = (p.n_tiles128 + gridDim.x - 1) / gridDim.x;
-  const long long total_q = n_iter * p.C;            // weight-set uses, identical for every warp of the CTA
-
-  if (warp >= FWD3T_CONTROL_WARP) {
-    // ======================= control warp: lane 0 streams the weights and issues the MMAs; it owns no data, so
-    // none of its waits delays a warp that computes.  Its warpgroup gives its registers to the compute warps.
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(FWD3T_REGS_CONTROL));
-    if (warp == FWD3T_CONTROL_WARP && lane == 0) {
-      // instruction descriptor (cute::UMMA::InstrDescriptor): S32 accumulate, S8 x S8, K-major, N = 64, M = 128
-      const uint32_t idesc = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(64 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-      auto load_w1 = [&](long long use) {
-        const int b = (int)(use & 1), c = (int)(use % p.C);
-        mbar_arrive_expect_tx(&w1full[b], W1_BYTES);
-        bulk_g2s(w1ring + (size_t)b * W1_BYTES, p.wt + (size_t)c * OZ_W1_BYTES, W1_BYTES, &w1full[b]);
-      };
-      auto load_rest = [&](long long use) {
-        const int b = (int)(use & 1), c = (int)(use % p.C);
-        mbar_arrive_expect_tx(&rfull[b], RSLOT_BYTES);
-        bulk_g2s(rring + (size_t)b * RSLOT_BYTES, p.wp + (size_t)c * G3::PB + G3::W2_OFF, RSLOT_BYTES, &rfull[b]);
-      };
-      auto load_hslot = [&](long long use) {
-        const int b = (int)(use & 3), c = (int)(use % p.C);
-        uint8_t* slot = hring + (size_t)b * HSLOT_BYTES;
-        mbar_arrive_expect_tx(&hfull[b], HSLOT_BYTES);
-        bulk_g2s(slot, p.wt + (size_t)c * OZ_W1_BYTES + W1_BYTES, 64 * 8, &hfull[b]);
-        bulk_g2s(slot + 64 * 8, p.wp + (size_t)c * G3::PB + G3::B1_OFF, 64 * 8, &hfull[b]);
-      };
-      auto issue_mma = [&](long long use) {
-#ifdef BNN_DBG_NOMMA          // tuning experiment only
-        return;
-#endif
-        // all 21 slice pairs: A = X slices in TMEM, B = W1 slices of `use` in shared memory
-        const uint64_t wdesc = oz_smem_desc(smem_u32(w1ring + (size_t)(use & 1) * W1_BYTES));
-#pragma unroll 1
-        for (int d = 0; d < OZ_S; ++d) {               // diagonal T = 10 - d -> TMEM columns [64 d, 64 d + 64)
-          const int T = 2 * (OZ_S - 1) - d;
-          uint32_t acc = 0;
-          for (int sx = T - (OZ_S - 1); sx <= OZ_S - 1; ++sx) {
-            const int sw = T - sx;
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks) {
-              oz_mma_ts(tmem + 64 * d, tmem + OZ_TMEM_X + 16 * sx + 8 * ks,
-                        wdesc + (uint64_t)((sw * OZ_WPLANE + ks * 2 * OZ_LBO) >> 4), idesc, acc);
-              acc = 1;
-            }
-          }
-        }
-      };
-      for (long long u = 0; u < 2 && u < total_q; ++u) { load_w1(u); load_rest(u); load_hslot(u); }
-      // use 0: the helpers have staged the first tile's X slices (phase 0 of tfree)
-      mbar_wait_sleep(tfree, 0);
-      mbar_wait_sleep(&w1full[0], 0);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      if ((long long)blockIdx.x < p.n_tiles128) issue_mma(0);
-      oz_commit(tfull);
-      for (long long q = 0; q + 1 < total_q; ++q) {
-        const long long it = q / p.C;
-        const int c = (int)(q - it * p.C);
-        const long long tile = it * gridDim.x + blockIdx.x;
-        // the MMAs of use q are complete: their W1 slot takes the slices of use q + 2 (every helper has finished
-        // pass 1 of use q - 1, so the helper slot of use q - 2 is free as well)
-        DBG_WAIT(1, tfull, (uint32_t)(q & 1));
-        if (q + 2 < total_q) { load_w1(q + 2); load_hslot(q + 2); }
-        // the helpers have drained use q (and staged the next tile's X slices at a tile change)
-        DBG_WAIT(3, tfree, (uint32_t)((q + 1) & 1));
-        DBG_WAIT(4, &w1full[(q + 1) & 1], (uint32_t)(((q + 1) >> 1) & 1));
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const long long ntile = (c + 1 == p.C) ? tile + gridDim.x : tile;
-        {
-          DBG_T0();
-          if (ntile < p.n_tiles128) issue_mma(q + 1);
-          oz_commit(tfull);          // arrives when every MMA issued so far is complete (also with none issued)
-          DBG_ADD(8);
-        }
-        // FP64 part of use q + 1 goes into the slot of use q - 1 once the compute warps have released it
-        if (q >= 1) {
-          DBG_WAIT(5, &rempty[(q + 1) & 1], (uint32_t)(((q - 1) >> 1) & 1));
-          load_rest(q + 1);
-        }
-      }
-    }
-  } else if (warp >= FWD3T_COMPUTE_WARPS) {
-    // ======================= helper warps: X slices -> TMEM, accumulators -> activated layer-1 outputs in a1s
-    const int h = warp - FWD3T_COMPUTE_WARPS;                     // TMEM lane quarter (== warp & 3)
-    const int r = 32 * h + lane;                                   // row inside the 128-row tile
-    const uint32_t tlane = (uint32_t)(32 * h) << 16;
-    // this thread's row of X slices (6 x 64 bytes, contiguous) -> TMEM columns [384, 480) of its lane
-    auto stage_x = [&](long long tile) {
-      const uint4* src = reinterpret_cast<const uint4*>(p.xsl + ((size_t)tile * 128 + r) * OZ_XROW);
-#pragma unroll
-      for (int sl = 0; sl < OZ_S; ++sl) {
-        uint4 w[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) w[i] = __ldg(src + 4 * sl + i);
-        oz_st_row16(tmem + tlane + OZ_TMEM_X + 16 * sl, w);
-      }
-      asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-    };
-    if ((long long)blockIdx.x < p.n_tiles128) stage_x(blockIdx.x);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncwarp();
-    if (lane == 0) mbar_arrive(tfree);                       // phase 0 of tfree: the first tile's X is in TMEM
-    long long q = 0;
-    for (long long it = 0; it < n_iter; ++it) {
-      const long long tile = it * gridDim.x + blockIdx.x;
-      const bool tile_ok = tile < p.n_tiles128;
-      const double rsc = tile_ok ? p.x_rowscale[tile * 128 + r] : 0.0;
-      for (int c = 0; c < p.C; ++c, ++q) {
-        const int b = (int)(q & 1);
-        DBG_WAIT(0, &hfull[q & 3], (uint32_t)((q >> 2) & 1));
-        DBG_WAIT(1, tfull, (uint32_t)(q & 1));
-        if (q > 1) DBG_WAIT(2, &a1free[2 * h + b], (uint32_t)(((q >> 1) - 1) & 1));
-        // ... and stay at most ONE weight set ahead of this quarter's compute warps (wait until they have consumed
-        // use q - 1 from the other buffer).  Without this bound -- helpers two sets ahead at the moment the next
-        // tile's X slices are stored to TMEM -- a few rows of ONE weight set per launch came out wrong (always the
-        // third-from-last set of an early tile, rows of TMEM lane quarter 0; tools/race_probe.py).  In failing runs
-        // the compute warps read exactly the activations the helper wrote (-DBNN_DBG_CSUM), so the fault is not in
-        // this hand-off; any added delay (trace stores, weights read from global memory) hides it.  The cause is
-        // not understood; with the bound 64 launches over 8 chain counts were clean.  The kernel is opt-in.
-#ifndef BNN_DBG_NOLOCKSTEP
-        if (q > 0) mbar_wait_sleep(&a1free[2 * h + (b ^ 1)], (uint32_t)(((q - 1) >> 1) & 1));
-#endif
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        const uint8_t* slot = hring + (size_t)(q & 3) * HSLOT_BYTES;
-        const double* csc = reinterpret_cast<const double*>(slot);
-        const double* b1 = reinterpret_cast<const double*>(slot + 64 * 8);
-        const double al = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[c * 3 + 0] : 0.0;
-        double* arow = a1s + (size_t)b * 128 * 64 + r * 64;
-        const int sw = a1_swz(r);
-        const long long dbg_p1 = clock64(); (void)dbg_p1;
-        // ---- pass 1: drain the accumulators (the tensor core is idle until this is done).  Integer instructions
-        // only -- the FP64 pipe is busy with the compute warps' DMMAs, and every FP64 instruction here would
-        // queue behind them: the 6 diagonals are folded into one 64-bit integer per element,
-        // (a0 2^16 + a1 2^8 + a2) 2^20 + ((a3 2^16 + a4 2^8 + a5) >> 4)   (|.| < 2^60; the 4 dropped bits are
-        // 2^-64 of full scale), which is parked in a1s
-#ifdef BNN_DBG_NOHELPER       // tuning experiment only
-        if (false)
-#endif
-#pragma unroll 1
-        for (int cb = 0; cb < N1 / 16; ++cb) {
-          uint32_t v[OZ_S][16];
-#pragma unroll
-          for (int d = 0; d < OZ_S; ++d) oz_ld_row16(tmem + tlane + 64 * d + 16 * cb, v[d]);
-          asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            long long w[2];
-#pragma unroll
-            for (int e2 = 0; e2 < 2; ++e2) {
-              const int e = 2 * i + e2;
-              const long long hi = (long long)(int)v[0][e] * 65536 + (long long)(int)v[1][e] * 256 + (long long)(int)v[2][e];
-              const long long lo = (long long)(int)v[3][e] * 65536 + (long long)(int)v[4][e] * 256 + (long long)(int)v[5][e];
-              w[e2] = hi * 1048576 + (lo >> 4);
-            }
-            *reinterpret_cast<longlong2*>(arow + 2 * ((8 * cb + i) ^ sw)) = make_longlong2(w[0], w[1]);
-          }
-        }
-        dbg[6] += clock64() - dbg_p1;
-        // a new tile follows: its X slices replace the current ones (no MMA is in flight: tfull(q) was waited for)
-        if (c + 1 == p.C && tile + gridDim.x < p.n_tiles128) {
-          DBG_T0();
-          stage_x(tile + gridDim.x);
-          DBG_ADD(9);
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive(tfree);
-        const long long dbg_p2 = clock64(); (void)dbg_p2;
-        // ---- pass 2 (under the MMAs of the next weight set): integer -> FP64, scale, bias, activation, in place
-        // on this thread's own row.  v = vh 2^32 + vl with the two halves converted by the 2^52 trick.
-#ifdef BNN_DBG_NOHELPER
-        if (false)
-#endif
-#ifdef BNN_DBG_CSUM
-        unsigned long long csum = 0;
-#endif
-#pragma unroll 1
-        for (int cb = 0; cb < N1 / 8; ++cb) {
-          double z[8];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            const longlong2 ww = *reinterpret_cast<const longlong2*>(arow + 2 * ((4 * cb + i) ^ sw));
-            const long long w2[2] = {ww.x, ww.y};
-#pragma unroll
-            for (int e2 = 0; e2 < 2; ++e2) {
-              const int e = 2 * i + e2;
-              const int vh = (int)(w2[e2] >> 32);
-              const unsigned vl = (unsigned)w2[e2];
-              const double dh = __hiloint2double(0x43300000, vh ^ 0x80000000) - 4503601774854144.0;   // 2^52 + 2^31
-              const double dl = __hiloint2double(0x43300000, (int)vl) - 4503599627370496.0;           // 2^52
-              const double hsum = fma(dh, 4294967296.0, dl);
-              z[e] = fma(hsum * rsc, csc[8 * cb + e], b1[8 * cb + e]);
-            }
-          }
-#pragma unroll
-          for (int e = 0; e < 8; ++e) z[e] = bnn_act<ACT, TB>(z[e], al, tab);
-#ifdef BNN_DBG_CSUM
-#pragma unroll
-          for (int e = 0; e < 8; ++e) csum ^= (unsigned long long)__double_as_longlong(z[e]);
-#endif
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            *reinterpret_cast<double2*>(arow + 2 * ((4 * cb + i) ^ sw)) = make_double2(z[2 * i], z[2 * i + 1]);
-        }
-#ifdef BNN_DBG_CSUM
-        for (int o = 8; o > 0; o >>= 1) csum ^= __shfl_xor_sync(FULL_MASK, csum, o);
-        if ((lane & 15) == 0) dbg_cs[b * 8 + 2 * h + (lane >> 4)] = csum;
-#endif
-        __syncwarp();
-        dbg[7] += clock64() - dbg_p2;
-        if (lane == 0) mbar_arrive(&a1full[2 * h + b]);
-      }
-    }
-  } else {
-    // ======================= compute warps
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(FWD3T_REGS_COMPUTE));
-    const int h = warp & 3;
-    const int rbase = 32 * h + 16 * (warp >> 2);                // rows of this warp inside the 128-row tile
-    long long q = 0;
-    for (long long it = 0; it < n_iter; ++it) {
-      const long long tile = it * gridDim.x + blockIdx.x;
-      const long long wt = tile * 8 + (rbase >> 4);
-      const bool have_tile = tile < p.n_tiles128 && wt < p.n_tiles16;
-      int y[2] = {0, 0};
-      double wgt[2] = {1.0, 1.0};
-      double acc3[N3 / 8][4];
-      bool prev_valid = false;
-#pragma unroll
-      for (int j = 0; j < N3 / 8; ++j) acc3[j][0] = acc3[j][1] = acc3[j][2] = acc3[j][3] = 0.0;
-      if (have_tile) {
-#pragma unroll
-        for (int hh = 0; hh < 2; ++hh) {
-          const long long row = wt * 16 + gq + 8 * hh;
-          if (row < p.n_total) {
-            y[hh] = p.labels[row];
-            if (MODE == FWD3_LIK_W) {
-              if (p.class_w) wgt[hh] *= p.class_w[y[hh]];
-              if (p.inst_w && row < p.n_train) wgt[hh] *= p.inst_w[row];
-            }
-          }
-        }
-      }
-      for (int c = 0; c < p.C; ++c, ++q) {
-        const int b = (int)(q & 1);
-        DBG_WAIT(0, &rfull[b], (uint32_t)((q >> 1) & 1));
-        DBG_WAIT(1, &a1full[2 * h + b], (uint32_t)((q >> 1) & 1));
-        const long long dbg_c0 = clock64(); (void)dbg_c0;
-        const double* W = reinterpret_cast<const double*>(rring + (size_t)b * RSLOT_BYTES) - G3::W2_OFF;
-        const double a2 = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[c * 3 + 1] : 0.0;
-        // ---------------- layer 2: [16 x N1] x [N1 x N2], A operand = activated layer-1 rows from a1s.  The
-        // likelihood epilogue of the previous weight set (latency-bound FP64 chains and shuffles) is cut into
-        // stages between the MMA groups of the first k-groups.
-        double acc2[N2 / 8][4];
-#pragma unroll
-        for (int j = 0; j < N2 / 8; ++j) {
-          const double2 bb = *reinterpret_cast<const double2*>(W + G3::B2_OFF + 8 * j + 2 * t);
-          acc2[j][0] = bb.x; acc2[j][1] = bb.y; acc2[j][2] = bb.x; acc2[j][3] = bb.y;
-        }
-        RowStats<N3> rs;
-        LikRow lr;
-        const int K = g.K;
-#ifdef BNN_DBG_CSUM
-        unsigned long long ccs = 0;
-        const unsigned long long want_cs = dbg_cs[b * 8 + 2 * h + (warp >> 2)];
-#endif
-#ifdef BNN_DBG_NOCOMPUTE      // tuning experiment only
-        if (p.C < 0)
-#endif
-        {
-          const double* wr = W + G3::W2_OFF + gq * N1;
-          const int sw = (gq & 1) * G3::SW1;
-          const double* ar0 = a1s + (size_t)b * 128 * 64 + (rbase + gq) * 64;
-          const double* ar1 = ar0 + 8 * 64;
-          const int asw = a1_swz(gq);                            // rows g and g + 8 share the swizzle
-#pragma unroll
-          for (int kg = 0; kg < N1 / 8; ++kg) {
-            const double2 alo = *reinterpret_cast<const double2*>(ar0 + 2 * ((4 * kg + t) ^ asw));
-            const double2 ahi = *reinterpret_cast<const double2*>(ar1 + 2 * ((4 * kg + t) ^ asw));
-#ifdef BNN_DBG_CSUM
-            ccs ^= (unsigned long long)__double_as_longlong(alo.x) ^ (unsigned long long)__double_as_longlong(alo.y) ^
-                   (unsigned long long)__double_as_longlong(ahi.x) ^ (unsigned long long)__double_as_longlong(ahi.y);
-#endif
-            if (!PREDICT) {
-              if (kg == 0) qs_max<N3>(acc3, K, t, rs);
-              else if (kg == 1) qs_exp<N3, 0, true, TB>(acc3, K, t, y, tab, rs);
-              else if (kg == 2) qs_exp<N3, 1, true, TB>(acc3, K, t, y, tab, rs);
-              else if (kg == 3) {
-                qs_reduce<N3, true>(rs);
-                lr = quad_lik_finish<N3, MODE == FWD3_LIK_W>(p, wt, lane, rs, y, wgt, prev_valid && have_tile);
-              }
-            }
-            const int col = (8 * kg + 2 * t) ^ sw;
-#pragma unroll
-            for (int j = 0; j < N2 / 8; ++j) {
-              const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + col);
-              dmma16x8x8(acc2[j], alo.x, ahi.x, alo.y, ahi.y, bb.x, bb.y);
-            }
-          }
-        }
-#ifdef BNN_DBG_CSUM
-        for (int o = 16; o > 0; o >>= 1) ccs ^= __shfl_xor_sync(FULL_MASK, ccs, o);
-        if (lane == 0 && ccs != want_cs && have_tile) {
-          atomicAdd(&g_dbg_clk[40], 1ULL);
-          g_dbg_clk[41] = (unsigned long long)q; g_dbg_clk[42] = (unsigned long long)warp; g_dbg_clk[43] = (unsigned long long)it;
-        }
-#endif
-        // the activated layer-1 rows have been consumed: the helpers may overwrite this buffer (two weight sets on)
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&a1free[2 * h + b]);
-        dbg[2] += clock64() - dbg_c0;
-        if (!PREDICT) quad_lik_commit<N3>(p, c - 1, wt, lane, cnt, lr, prev_valid && have_tile);
-        // ---------------- layer 3: [16 x N2] x [N2 x N3]
-#pragma unroll
-        for (int j = 0; j < N3 / 8; ++j) {
-          const double2 bb = *reinterpret_cast<const double2*>(W + G3::B3_OFF + 8 * j + 2 * t);
-          acc3[j][0] = bb.x; acc3[j][1] = bb.y; acc3[j][2] = bb.x; acc3[j][3] = bb.y;
-        }
-#ifdef BNN_DBG_NOCOMPUTE
-        if (p.C < 0)
-#endif
-        {
-          const double* wr = W + G3::W3_OFF + gq * N2;
-          const int sw = (gq & 1) * G3::SW2;
-          act_tile<ACT, false, TB>(acc2[0], a2, tab);
-#pragma unroll
-          for (int kg = 0; kg < N2 / 8; ++kg) {
-            if (kg + 1 < N2 / 8) act_tile<ACT, false, TB>(acc2[kg + 1], a2, tab);
-            const int col = (8 * kg + 2 * t) ^ sw;
-#pragma unroll
-            for (int j = 0; j < N3 / 8; ++j) {
-              const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N2 + col);
-              dmma16x8x8(acc3[j], acc2[kg][0], acc2[kg][2], acc2[kg][1], acc2[kg][3], bb.x, bb.y);
-            }
-          }
-        }
-#ifdef BNN_DBG_CSUM
-        {
-          unsigned long long lcs = 0;
-#pragma unroll
-          for (int j = 0; j < N3 / 8; ++j)
-#pragma unroll
-            for (int e = 0; e < 4; ++e) lcs ^= (unsigned long long)__double_as_longlong(acc3[j][e]) * (unsigned long long)(2 * (4 * j + e) + 1);
-          for (int o = 16; o > 0; o >>= 1) lcs ^= __shfl_xor_sync(FULL_MASK, lcs, o);
-          if (lane == 0 && g_dbg_trace) {
-            unsigned long long* tr = g_dbg_trace + (((size_t)blockIdx.x * total_q + q) * 8 + warp) * 2;
-            tr[0] = ccs; tr[1] = lcs;
-          }
-        }
-#endif
-        // weights of this use are no longer needed by this warp
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&rempty[b]);
-        dbg[3] += clock64() - dbg_c0;
-        prev_valid = true;
-      }
-      if (have_tile && !PREDICT) {
-        // drain the software pipeline: epilogue of the last weight set of this tile
-        RowStats<N3> rs;
-        quad_softmax_stats<N3, true, TB>(acc3, g.K, t, y, tab, rs);
-        const LikRow lr = quad_lik_finish<N3, MODE == FWD3_LIK_W>(p, wt, lane, rs, y, wgt, true);
-        quad_lik_commit<N3>(p, p.C - 1, wt, lane, cnt, lr, true);
-      }
-    }
-  }
-#ifdef BNN_DBG_WAITCLK
-  if (lane == 0)
-    for (int i = 0; i < 12; ++i) atomicAdd(&g_dbg_clk[(warp >= FWD3T_CONTROL_WARP ? 0 : warp >= FWD3T_COMPUTE_WARPS ? 16 : 32) + i], (unsigned long long)dbg[i]);
-#endif
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-  __syncthreads();
-  if (warp == FWD3T_COMPUTE_WARPS)
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
-  if (n_cnt) {
-    for (int i = threadIdx.x; i < n_cnt; i += blockDim.x)
-      if (cnt[i]) atomicAdd(&p.counts[i], cnt[i]);
-  }
-}
-
-cudaError_t bnn_launch_slice_x(const double* x, long long n_pad16, uint8_t* xsl, double* rowscale, long long n_tiles128,
-                               int* flag, cudaStream_t st) {
-  const long long rows = n_tiles128 * 128;
-  k_slice_x<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(x, n_pad16, xsl, rowscale, rows, flag);
-  return cudaGetLastError();
-}
-cudaError_t bnn_launch_slice_w1(const double* wp, int PB, uint8_t* wt, int n_sets, cudaStream_t st) {
-  k_slice_w1<<<n_sets, 64, 0, st>>>(wp, PB, wt);
-  return cudaGetLastError();
-}
-size_t bnn_slice_x_tile_bytes() { return OZ_XTILE; }
-size_t bnn_slice_w1_bytes() { return OZ_W1_BYTES; }
-
-static size_t fwd3t_smem_bytes(int C, int K) {
-  using G3 = Fwd3Geom<64, 64, 32, 16>;
-  return 2 * (size_t)(OZ_S * OZ_WPLANE) + 2 * (size_t)(G3::PB - G3::W2_OFF) * 8 + 2 * 128 * 64 * sizeof(double) +
-         256 * sizeof(double) + 4 * 1024 + 30 * sizeof(uint64_t) + (size_t)C * (2 + 2 * K) * sizeof(int)
-#ifdef BNN_DBG_CSUM
-         + 256
-#endif
-      ;
-}
-
-template <int ACT, int MODE>
-static cudaError_t launch_fwd3t(const FwdParams& p, int n_sms, cudaStream_t st) {
-  auto kern = k_fwd3t<ACT, MODE>;
-  const size_t smem = fwd3t_smem_bytes(p.C, p.g.K);
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
-  if (smem > 232448) return cudaErrorInvalidConfiguration;
-  int grid = (int)(p.n_tiles128 < n_sms ? p.n_tiles128 : n_sms);
-  kern<<<grid, FWD3T_THREADS, smem, st>>>(p);
-  return cudaGetLastError();
-}
-
-#endif  // BNN_EXPERIMENTAL_TENSOR_L1
 
 // =============================================================================================
 // host-side launchers
@@ -2296,9 +1512,7 @@ static int sparse_pair_shape(const FwdParams& p) {
   const int pr = p.sp_pair_nc1 > 0 ? p.sp_pair_nr1 * 16 + p.sp_pair_nr2 : 0;
   return (pr == 3 * 16 + 2 || pr == 2 * 16 + 1 || pr == 2 * 16 + 2 || pr == 4 * 16 + 2) ? pr : 0;
 }
-#ifndef SPARSE_PAIR_NCH
-#define SPARSE_PAIR_NCH 2
-#endif
+constexpr int SPARSE_PAIR_NCH = 2;      // chains a thread of k_fwd_pairs evaluates together
 // shared-memory plan of k_fwd_pairs: resident chains, warps per group, warps
 static bool pairs_plan(const FwdParams& p, int nch, int* group, int* share, int* nwarps, size_t* bytes) {
   const size_t cap = 232448;
@@ -2407,7 +1621,7 @@ cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int 
     const int fam = bnn_fwd3_family(g);
     if (fam) {
       if (which) *which = names[fam - 1][g.act];
-      return fam == 1 ? launch_fwd3_act<64, 64, 32, FWD3_WARPS>(p, predict, n_sms, st)
+      return fam == 1 ? launch_fwd3_act<64, 64, 32, 12>(p, predict, n_sms, st)
                       : launch_fwd3_act<32, 32, 16, 16>(p, predict, n_sms, st);
     }
   }

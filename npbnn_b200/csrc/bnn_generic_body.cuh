@@ -2,7 +2,6 @@
 // activations staged in per-warp shared memory, and the likelihood / prediction epilogue on the staged outputs.
 // Shared by k_fwd_generic (bnn_forward.cu) and the persistent small-data chain loop (k_chain_loop, bnn_chainloop.cu).
 #pragma once
-#include <type_traits>
 #include "bnn_common.cuh"
 
 #define FULL_MASK 0xffffffffu
@@ -13,14 +12,6 @@
 constexpr int GEN_TB = 8;
 constexpr int GEN_TAB_SIZE = 1 << GEN_TB;
 
-// compile-time loop: f(std::integral_constant<int, I>{}) for I in [I0, N)
-template <int I0, int N, class F>
-__device__ __forceinline__ void static_for(F&& f) {
-  if constexpr (I0 < N) {
-    f(std::integral_constant<int, I0>{});
-    static_for<I0 + 1, N>(f);
-  }
-}
 #ifndef BNN_HAVE_LOGSQRT2PI
 #define BNN_HAVE_LOGSQRT2PI
 static constexpr double kLogSqrt2Pi = 0.91893853320467274178;

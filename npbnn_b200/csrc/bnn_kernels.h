@@ -59,14 +59,6 @@ bool bnn_pred_tf32_fits(const FwdParams& p);
 cudaError_t bnn_launch_pred_tf32(const FwdParams& p, int n_sms, int passes, cudaStream_t st, const char** which);
 // k_fwd3 width family the padded geometry matches exactly: 1 = 64->64->32, 2 = 32->32->16, 0 = none (generic kernel)
 int bnn_fwd3_family(const NetGeom& g);
-// tensor-core first layer (k_fwd3t): operand slicing
-cudaError_t bnn_launch_slice_x(const double* x, long long n_pad16, uint8_t* xsl, double* rowscale, long long n_tiles128,
-                               int* flag, cudaStream_t st);
-cudaError_t bnn_launch_slice_w1(const double* wp, int PB, uint8_t* wt, int n_sets, cudaStream_t st);
-size_t bnn_slice_x_tile_bytes();
-size_t bnn_slice_w1_bytes();
-cudaError_t bnn_debug_counters_read(unsigned long long* out32);
-cudaError_t bnn_debug_set_trace_ptr(unsigned long long* dev_ptr);
 cudaError_t bnn_launch_pack_x(const double* x, double* xs, long long n, long long n_pad, int F, int F_pad, int swz,
                               const int* ov_cols, const double* ov_vals, int n_ov, cudaStream_t st);
 // *flag |= 1 if a training label is outside [0, K) or a test label is negative (the reference raises IndexError there)

@@ -156,13 +156,6 @@ __device__ double finalize_loglik(const NetGeom& g, const double* part, int NF, 
   return bnn_lik_is_count(g.lik) ? ll : lik_temp * ll;
 }
 
-#ifdef BNN_DBG_LOOPCLK       // tuning instrumentation: clocks per phase of the update body (thread 0 of chain 0)
-__device__ long long g_dbg_upd[16];
-#define UPD_STAMP(i) do { if (threadIdx.x == 0 && c == 0) { const long long now_ = clock64(); g_dbg_upd[i] += now_ - dbg_t_; dbg_t_ = now_; } } while (0)
-#else
-#define UPD_STAMP(i) do { } while (0)
-#endif
-
 struct Draw { int ix, iy; double dz; };
 // k-th proposal of layer l of chain c at iteration it
 __device__ __forceinline__ Draw philox_draw(uint64_t seed, int c, int it, int l, int k, int rows, int cols, double ws) {
@@ -248,9 +241,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
   int* const gsi = d.si + (long long)c * BNN_I_STRIDE;
   const bool resident = COH && lp_ctx.w_sm != nullptr;            // persistent loop: state stays in shared memory
   const bool load_state = !resident || lp_ctx.first, store_state = !resident || lp_ctx.last;
-#ifdef BNN_DBG_LOOPCLK
-  long long dbg_t_ = clock64();
-#endif
   double* wc = d.w_cur + (long long)c * g.P;
   double* wn = d.w_prop + (long long)c * g.P;
   int* owner = d.owner + (long long)c * g.P;
@@ -275,7 +265,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
     upd_sync<COH>();
   }
   if (resident) { wc = lp_ctx.w_sm; wn = lp_ctx.w_sm + g.P; owner = lp_ctx.owner_sm; }
-  UPD_STAMP(0);
   double* sf = ssf;
   int* si = ssi;
   auto write_back = [&]() {
@@ -409,7 +398,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
     const double* sg_in = (g.lik == BNN_LIK_GAUSSIAN && smode == BNN_SIGMA_FIXED) ? sf + BNN_F_SIGMA : nullptr;
     const double* part_chain = lp_ctx.part_c ? lp_ctx.part_c : d.part + (long long)c * d.NF * d.n_tiles16;
     double ll = finalize_loglik<COH>(g, part_chain, d.NF, d.n_tiles16, d.n_train, d.cfg.lik_temp, smode, sg_in, red, sig);
-    UPD_STAMP(1);
     if (d.cfg.sample_from_prior) ll = 0.0;
     if (tid == 0) {
       double lp = sf[BNN_F_LOGPRIOR_PROP];
@@ -474,7 +462,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
       }
     }
     upd_sync<COH>();
-    UPD_STAMP(2);
   }
   if (!propose_mode) { write_back(); return; }
 
@@ -582,7 +569,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
       sf[BNN_F_ADD_PROB] = d.cfg.init_additional_prob;
     }
   }
-  UPD_STAMP(3);
   // zero the proposal's counters (the forward kernel accumulates into them)
   if (g.lik == BNN_LIK_CATEGORICAL)
 #pragma unroll 1
@@ -630,7 +616,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
     fi_p = dst;
   }
   if (d.ind_cur || d.fi_cur) upd_sync<COH>();
-  UPD_STAMP(4);
 
   // ------------------------------------------------------------------ UpdateNormal (BNN_mcmc.py:57-69)
   // z[Ix,Iy] = z[Ix,Iy] + N(0, d): fancy assignment => for duplicate (ix,iy) the LAST draw wins and
@@ -695,7 +680,6 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
     }
   }
 
-  UPD_STAMP(5);
   // ------------------------------------------------------------------ reflect, mask, prior, pack
   const double hi = d.cfg.w_bound, lo = -d.cfg.w_bound;
   double lp = 0.0;
@@ -735,9 +719,7 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
     wpk[pi] = z;
     if (lp_ctx.wpk_sm) lp_ctx.wpk_sm[pi] = z;
   }
-  UPD_STAMP(6);
   double s = block_sum_fixed<COH>(lp, sh);
-  UPD_STAMP(7);
   if (ind_p && d.cfg.use_indicators) {
     // + sum(ind) log(pi1) + (size - sum(ind)) log(1 - pi1)   (BNN_env.py:191-193)
     double n1 = 0.0;
@@ -768,5 +750,4 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
   }
   if (tid == 0) sf[BNN_F_LOGPRIOR_PROP] = s + sf[BNN_F_ADD_PROB];     // calc_prior(...) + additional_prob (BNN_env.py:481)
   write_back();
-  UPD_STAMP(8);
 }

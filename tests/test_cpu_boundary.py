@@ -16,7 +16,9 @@ def header_functions():
     return sorted(set(re.findall(r"\b(bnn_[a-z0-9_]+)\s*\(", src)))
 
 
-def test_library_builds_and_exports_header_symbols():
+def test_library_builds_and_exports_header_symbols_of_abi_2():
+    """ABI version 2: the header's entry points, and not the two debugging entry points of the removed tensor-core
+    first layer that version 1 exported."""
     import __graft_entry__ as ge
     ge.build()
     from npbnn_b200 import _lib
@@ -28,7 +30,9 @@ def test_library_builds_and_exports_header_symbols():
         assert hasattr(h, n), "library does not export %s" % n
     # the ctypes binding covers exactly the header
     assert set(_lib.EXPORTED_SYMBOLS) == set(names)
-    assert h.bnn_abi_version() == 1
+    assert h.bnn_abi_version() == 2
+    for n in ("bnn_debug_counters", "bnn_debug_set_trace"):
+        assert not hasattr(h, n), n
 
 
 def test_state_slot_constants_match_header():

@@ -523,53 +523,19 @@ def test_c5_full_size_prediction_properties():
     eng.close()
 
 
-@pytest.mark.parametrize("n", [16, 130, 1000, 4099, 50000])
-def test_c4_shape_tensor_core_first_layer(n):
-    """k_fwd3t: layer 1 as 21 exact int8 tensor-core products (Ozaki slices of X and W1, tcgen05 + TMEM) against
-    the oracle, the FP64 DMMA kernel (option tensor_l1=0) and with wide dynamic range in X and W1.
-    Tolerance: 1e-9 relative as for the FP64 kernels; the measured agreement is ~1e-13."""
-    from npbnn_b200.engine import Engine, NetShape
-    x, labels, sets = _c4_like(n, 5)
-    rng = np.random.default_rng(n)
-    x = x * np.exp(rng.normal(0, 2.0, (n, 1))) * np.where(rng.random((n, 64)) < 0.1, 1e-6, 1.0)   # ragged magnitudes
-    x[n // 2] = 0.0                                                                              # an all-zero row
-    sets[1][0][3] = 0.0                                                                          # an all-zero unit
-    sets[2][0] *= 1e-3
-    m = orc.Model(x=x, labels=labels, weights=sets[0], act="swish", mode="classification")
-    net = NetShape.from_weights(sets[0], 64, act="swish", lik=0)
-    eng = Engine(net)
-    eng.set_data(x[: n - n // 5], labels[: n - n // 5], x[n - n // 5:], labels[n - n // 5:])
-    m = orc.Model(x=x[: n - n // 5], labels=labels[: n - n // 5], weights=sets[0], act="swish", mode="classification",
-                  x_test=x[n - n // 5:], labels_test=labels[n - n // 5:])
+def test_unknown_options_are_refused():
+    """bnn_set_option refuses a name it does not know, including the removed tensor-core first layer ("tensor_l1"),
+    and leaves the context usable."""
     from npbnn_b200 import _lib as L
-    try:
-        eng.set_option("tensor_l1", 1)                   # experimental path, only in -DBNN_EXPERIMENTAL_TENSOR_L1 builds
-    except L.NpbnnError as e:
-        assert "not compiled" in str(e)
-        eng.close()
-        pytest.skip("k_fwd3t is not compiled into the shipped library")
-    res = eng.forward_lik(sets)
-    assert eng.last_kernel == "k_fwd3t<swish,64,64,32,16>", eng.last_kernel
-    eng.set_option("tensor_l1", 0)
-    f64 = eng.forward_lik(sets)
-    assert eng.last_kernel == "k_fwd3<swish,64,64,32,16>", eng.last_kernel
-    for i, w in enumerate(sets):
-        ref = oracle_score(m, w)
-        assert rel_close(res["loglik"][i], ref["loglik"]), (i, res["loglik"][i], ref["loglik"])
-        assert rel_close(res["loglik"][i], f64["loglik"][i], rtol=1e-11), (i, res["loglik"][i], f64["loglik"][i])
-        c = res["counts"][i]
-        assert c[0] == ref["n_correct"] and c[1] == ref["n_correct_test"]
-        assert np.array_equal(c[2:12], ref["class_correct"]) and np.array_equal(c[12:22], ref["pred_hist"])
-    # chains: same decisions and weights as the FP64 path
-    states = []
-    for tensor in (1, 0):
-        eng.set_option("tensor_l1", tensor)
-        eng.chains_init(sets, temperature=[1.0, 0.95, 0.9, 0.85, 0.8], seed=3)
-        eng.mh_steps(30)
-        states.append(eng.read_state())
-    a, b = states
-    assert np.array_equal(a.n_accepted, b.n_accepted) and np.array_equal(a.w, b.w)
-    assert rel_close(a.logLik, b.logLik, rtol=1e-11)
+    from npbnn_b200.engine import Engine, NetShape
+    x, labels, sets = _c4_like(16, 1)
+    eng = Engine(NetShape.from_weights(sets[0], 64, act="swish", lik=0))
+    eng.set_data(x, labels)
+    for name, value in (("tensor_l1", 1), ("tensor_l1", 0), ("no_such_option", 1)):
+        with pytest.raises(L.NpbnnError, match="unknown option " + name):
+            eng.set_option(name, value)
+    eng.set_option("force_generic", 0)
+    assert np.isfinite(eng.forward_lik(sets)["loglik"][0])
     eng.close()
 
 

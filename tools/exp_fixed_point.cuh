@@ -37,11 +37,7 @@ __device__ __forceinline__ void bnn_exp_split(double z, const double* __restrict
   static_assert(SCALE == -1 || SCALE == 1 || SCALE == 2, "exp(-z), exp(z) or exp(2z)");
   const double t = fma(z, (double)SCALE * 2954.639443740597, 393216.0);
   const unsigned hi = (unsigned)__double2hiint(t), F = (unsigned)__double2loint(t);
-#ifdef BNN_DBG_NOTAB          // tuning experiment only: what do the table lookups (random shared-memory reads) cost?
-  const double T = 1.0;
-#else
   const double T = *reinterpret_cast<const double*>(reinterpret_cast<const char*>(tab) + ((hi << 1) & 0x3FF8u));
-#endif
   Ts = __hiloint2double(__double2hiint(T) + (int)((hi & 0x000FE000u) << 7), __double2loint(T));
   // second-order terms in FP32: y = 1 + (23 leading bits of f); f re-centred on its truncation interval
   const float y = __uint_as_float((__funnelshift_r(F, hi, 11) & 0x007FFFFFu) | 0x3F800000u);

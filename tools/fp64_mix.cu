@@ -91,63 +91,6 @@ __global__ void __launch_bounds__(NW * 32, 1) k_mix(double* out, int iters, doub
   out[blockIdx.x * blockDim.x + threadIdx.x] = s;
 }
 
-// staged swish (ActPipe): 8 elements, one dependency level after each MMA
-template <int NW, int NA>
-__global__ void __launch_bounds__(NW * 32, 1) k_staged(double* out, int iters, double x, double y, const double* gtab) {
-  __shared__ double tab[BNN_EXP_TAB_SIZE];
-  for (int i = threadIdx.x; i < BNN_EXP_TAB_SIZE; i += blockDim.x) tab[i] = gtab[i];
-  __syncthreads();
-  double c[NA][4];
-#pragma unroll
-  for (int i = 0; i < NA; ++i) c[i][0] = c[i][1] = c[i][2] = c[i][3] = 0.0;
-  double a[4], b[2];
-#pragma unroll
-  for (int i = 0; i < 4; ++i) a[i] = x + threadIdx.x * 1e-6 + i * 1e-3;
-  b[0] = y + threadIdx.x * 1e-6; b[1] = y * 0.5;
-  ActPipe<BNN_ACT_SWISH, 8> ap;
-#pragma unroll
-  for (int i = 0; i < 8; ++i) ap.z[i] = 0.3 * i + threadIdx.x * 1e-3;
-  const double off = 0.25 + (threadIdx.x & 31) * 0.37;
-  for (int it = 0; it < iters; ++it) {
-    static_assert(NA >= 6, "");
-    dmma16x8x8(c[0], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<0>(0.0, tab); ap.template stage<1>(0.0, tab);
-    dmma16x8x8(c[1], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<2>(0.0, tab); ap.template stage<3>(0.0, tab);
-    dmma16x8x8(c[2], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<4>(0.0, tab); ap.template stage<5>(0.0, tab);
-    dmma16x8x8(c[3], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<6>(0.0, tab); ap.template stage<7>(0.0, tab);
-    dmma16x8x8(c[4], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<8>(0.0, tab); ap.template stage<9>(0.0, tab);
-    dmma16x8x8(c[5], a[0], a[1], a[2], a[3], b[0], b[1]); ap.template stage<10>(0.0, tab);
-#pragma unroll
-    for (int i = 6; i < NA; ++i) dmma16x8x8(c[i], a[0], a[1], a[2], a[3], b[0], b[1]);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) ap.z[i] += off;
-  }
-  double s = 0;
-#pragma unroll
-  for (int i = 0; i < NA; ++i) s += c[i][0] + c[i][1] + c[i][2] + c[i][3];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) s += ap.z[i];
-  out[blockIdx.x * blockDim.x + threadIdx.x] = s;
-}
-template <int NW, int NA>
-void run_staged(int sms, double* out, const double* tab) {
-  const int iters = 4096 / NA;
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
-  k_staged<NW, NA><<<sms, NW * 32>>>(out, iters, 1.0000001, 1e-9, tab);
-  cudaEventRecord(e0);
-  for (int r = 0; r < 5; ++r) k_staged<NW, NA><<<sms, NW * 32>>>(out, iters, 1.0000001, 1e-9, tab);
-  cudaEventRecord(e1);
-  cudaEventSynchronize(e1);
-  float ms;
-  cudaEventElapsedTime(&ms, e0, e1);
-  ms /= 5;
-  const double clk = ms * 1e-3 * 1.965e9, wps = NW / 4.0;
-  const double per_smsp_mma = (double)iters * NA * wps, per_smsp_fp = (double)iters * 8 * 13 * wps;
-  printf("%-34s warps=%2d mma/it=%d act/it= 8  %.3f ms  clk/mma(all-in) %.1f  clk per FP64 instr beyond 64.4/mma: %.2f  err=%s\n",
-         "staged fast swish (ActPipe)", NW, NA, ms, clk / per_smsp_mma, (clk - 64.4 * per_smsp_mma) / per_smsp_fp,
-         cudaGetErrorString(cudaGetLastError()));
-}
-
 template <int NW, int NA, int NCH, int MODE, int NI>
 void run(int sms, double* out, const double* tab, const char* what) {
   const int iters = 4096 / (NA > 0 ? NA : 4);
@@ -171,7 +114,7 @@ void run(int sms, double* out, const double* tab, const char* what) {
          cudaGetErrorString(cudaGetLastError()));
 }
 
-int main(int argc, char**) {
+int main() {
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, 0);
   const int sms = prop.multiProcessorCount;
@@ -182,14 +125,6 @@ int main(int argc, char**) {
   for (int i = 0; i < BNN_EXP_TAB_SIZE; ++i) h[i] = exp2((double)i / BNN_EXP_TAB_SIZE);
   cudaMemcpy(tab, h, sizeof(h), cudaMemcpyHostToDevice);
   printf("%s, %d SMs\n", prop.name, sms);
-  if (argc > 1) {
-    run_staged<12, 8>(sms, out, tab); run_staged<12, 16>(sms, out, tab); run_staged<12, 24>(sms, out, tab);
-    run<12, 8, 8, 5, 0>(sms, out, tab, "fast swish x8 unstaged, 8 mma");
-    run<12, 16, 8, 5, 0>(sms, out, tab, "fast swish x8 unstaged, 16 mma");
-    run<12, 24, 8, 5, 0>(sms, out, tab, "fast swish x8 unstaged, 24 mma");
-    run<12, 8, 8, 0, 0>(sms, out, tab, "12 dfma chain x8, 8 mma");
-    return 0;
-  }
   run<12, 8, 0, 0, 0>(sms, out, tab, "mma only");
   run<12, 4, 4, 0, 0>(sms, out, tab, "12 dfma chain");
   run<12, 4, 4, 1, 0>(sms, out, tab, "dfma/dadd/dmul + immediates");
