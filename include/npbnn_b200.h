@@ -287,7 +287,10 @@ const char* bnn_last_kernel(const bnn_ctx* ctx);
  *     bnn_rowshard_commit(red)                                 the accept step will see the global sums
  *     bnn_rowshard_update(accept_mode = 1, propose = 0, NULL)  accept / reject: identical on every rank
  * After bnn_chains_init the same local / all-reduce / commit sequence is followed by accept_mode = 2 (initial state).
- * The reductions are fixed-order, so every rank holds bit-identical chain states. */
+ * The reductions are fixed-order, so every rank holds bit-identical chain states.  Every likelihood kind is served.
+ * The count kinds exchange the same 1 + 3K slots as the Gaussian one (log-likelihood, then sum r, sum r^2 and the
+ * test sum r^2 per modelled column); lgamma(k + 1) is staged by bnn_set_data from the rank's own targets, and the
+ * companion MSE is the exchanged sum over the global row count, which the caller divides by. */
 int bnn_rowshard_config(bnn_ctx* ctx, int64_t n_train_global);
 int bnn_rowshard_n_values(const bnn_ctx* ctx);                 /* doubles per chain in the exchanged vector */
 int bnn_rowshard_local(bnn_ctx* ctx, double* red_dev, void* stream);

@@ -29,10 +29,12 @@ numbers (rng="host"); hyper-prior scales (hyper_p) are drawn on the host and eva
 estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
 MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
 companion MSE.  Options of the reference that are not on the device path raise
-NotImplementedError: other user-supplied likelihood / proposal / output functions (gamma_likelihood among them), count
-likelihoods under row sharding, and the regression error-parameter proposal (estimate_error with empirical_error=False once the
-iteration passes `_estimate_error` -- a branch on which the reference itself raises AttributeError as soon as one
-proposal has been accepted before that iteration, BNN_mcmc.py:105).
+NotImplementedError: other user-supplied likelihood / proposal / output functions (gamma_likelihood among them),
+MCMC(row_shard=True) with a count likelihood outside an initialised torch.distributed process group, MC3 with
+more ranks than chains (row-sharded chain blocks) together with host-drawn weight or feature indicators (rng="host" and
+freq_indicator > 0 or feature_indicators=True), and the regression error-parameter proposal (estimate_error with
+empirical_error=False once the iteration passes `_estimate_error` -- a branch on which the reference itself raises
+AttributeError as soon as one proposal has been accepted before that iteration, BNN_mcmc.py:105).
 """
 import csv
 import os
@@ -138,7 +140,7 @@ _COUNT_LIK = {poi_likelihood: (L.LIK_POISSON, poi_acc), negbin_likelihood: (L.LI
               negbin_likelihood_base10: (L.LIK_NEGBIN10, negbin_acc_base10)}
 
 
-def _count_likelihood(bnn, likelihood_f, accuracy_f, accuracy_lab_f, row_shard=False):
+def _count_likelihood(bnn, likelihood_f, accuracy_f, accuracy_lab_f):
     """The device likelihood kind and accuracy function of a sampler: None for a built-in estimation mode (which takes
     no user functions), the count kind of likelihood_f for estimation_mode="custom"."""
     if bnn._estimation_mode != "custom":
@@ -157,8 +159,6 @@ def _count_likelihood(bnn, likelihood_f, accuracy_f, accuracy_lab_f, row_shard=F
         raise NotImplementedError("accuracy_f of %s must be %s (or None)" % (likelihood_f.__name__, companion.__name__))
     if accuracy_lab_f is not None:
         raise NotImplementedError("user-supplied accuracy_lab_f is not on the device path")
-    if row_shard:
-        raise NotImplementedError("row sharding of the count likelihoods is not implemented")
     o, n_lab = bnn._size_output, bnn._labels.shape[1]
     if likelihood_f is negbin_likelihood2d and o != 2 * n_lab:
         raise ValueError("negbin_likelihood2d needs size_output = 2 x the label columns (%d), not %d" % (2 * n_lab, o))
@@ -369,31 +369,30 @@ def _has_test(bnn):
 
 class _ChainGroup:
     """C chains of one model on one GPU: engine + the host bookkeeping that turns numpy draws into the
-    injection arrays of bnn_mh_steps."""
+    injection arrays of bnn_mh_steps.  row_shard = (R, r): this GPU holds row shard r of R of the training and test rows,
+    and the R ranks of process group `row_group` (None: the default group) run the same chains (rowshard.py)."""
 
     def __init__(self, bnn, weights_per_chain, temperatures, update_f, update_ws, lik_temp, adapt_f, adapt_fM,
-                 adapt_freq, adapt_stop, sample_from_prior, seed, device=0, init_additional_prob=0.0, row_shard=False,
-                 chain_offset=0, lik=None):
+                 adapt_freq, adapt_stop, sample_from_prior, seed, device=0, init_additional_prob=0.0, row_shard=(1, 0),
+                 row_group=None, chain_offset=0, lik=None):
         self.bnn = bnn
         net = _net_of(weights_per_chain[0], bnn._n_features, bnn._act_fun, bnn._estimation_mode, lik)
         self.net = net
         self.eng = Engine(net, device=device)
         cw = bnn._class_w if len(bnn._class_w) else None
-        import torch.distributed as dist
-        world = dist.get_world_size() if (row_shard and dist.is_available() and dist.is_initialized()) else 1
-        if world > 1:
-            # rows split over the ranks, same chains everywhere, one all-reduce per MH iteration (rowshard.py)
+        R, r = row_shard
+        if R > 1:
+            # rows split over the R ranks of the group, same chains on each, one all-reduce per MH iteration (rowshard.py)
             from . import rowshard
-            rank = dist.get_rank()
-            a, b = rowshard.row_partition(len(bnn._data), world, rank)
+            a, b = rowshard.row_partition(len(bnn._data), R, r)
             iw = None if bnn._instance_weights is None else bnn._instance_weights[a:b]
             if _has_test(bnn):
-                ta, tb = rowshard.row_partition(len(bnn._test_data), world, rank)
+                ta, tb = rowshard.row_partition(len(bnn._test_data), R, r)
                 self.eng.set_data(bnn._data[a:b], bnn._labels[a:b], bnn._test_data[ta:tb], bnn._test_labels[ta:tb],
                                   inst_w=iw, class_w=cw)
             else:
                 self.eng.set_data(bnn._data[a:b], bnn._labels[a:b], inst_w=iw, class_w=cw)
-            self.eng.enable_rowshard(len(bnn._data), rowshard.dist_all_reduce_sum)
+            self.eng.enable_rowshard(len(bnn._data), lambda t: rowshard.dist_all_reduce_sum(t, row_group))
         else:
             self.eng.set_data(bnn._data, bnn._labels, bnn._test_data if _has_test(bnn) else None,
                               bnn._test_labels if _has_test(bnn) else None, inst_w=bnn._instance_weights, class_w=cw)
@@ -513,7 +512,13 @@ class MCMC:
                  _group=None, _slot=0):
         if update_function is not UpdateNormal:
             raise NotImplementedError("only update_function=UpdateNormal runs on the device")
-        count_kind, count_acc = _count_likelihood(bnn_obj, likelihood_f, accuracy_f, accuracy_lab_f, row_shard)
+        count_kind, count_acc = _count_likelihood(bnn_obj, likelihood_f, accuracy_f, accuracy_lab_f)
+        import torch.distributed as dist
+        if count_kind is not None and row_shard and not (dist.is_available() and dist.is_initialized()):
+            # a count model is row-sharded over the ranks of a process group; without one there are no ranks to shard
+            # over, and the request stays refused rather than silently running unsharded
+            raise NotImplementedError("row_shard=True with a count likelihood shards the rows over the ranks of "
+                                      "torch.distributed: initialise the process group first")
         if rng not in ("host", "philox"):
             raise ValueError("rng must be 'host' or 'philox'")
         if rng == "philox" and bnn_obj._freq_indicator and bnn_obj._n_layers < 4:
@@ -544,10 +549,13 @@ class MCMC:
         self.update_function = update_function
         self._own_group = _group is None
         if _group is None:
+            shard = (1, 0)
+            if row_shard and dist.is_available() and dist.is_initialized():
+                shard = (dist.get_world_size(), dist.get_rank())
             _group = _ChainGroup(bnn_obj, [bnn_obj._w_layers], [temperature], list(update_f)[:nl], list(update_ws)[:nl],
                                  likelihood_tempering, adapt_f, adapt_fM, adapt_freq, self._adapt_stop, sample_from_prior,
                                  seed=int(bnn_obj._seed) + 7919 * int(mcmc_id), device=device,
-                                 init_additional_prob=init_additional_prob, row_shard=row_shard, lik=count_kind)
+                                 init_additional_prob=init_additional_prob, row_shard=shard, lik=count_kind)
         elif bnn_obj._act_fun._trainable or init_additional_prob:
             raise NotImplementedError("trainable activation parameters / init_additional_prob inside an MC3 group")
         self._group, self._slot = _group, _slot
@@ -870,8 +878,11 @@ def _chain_view(bnn):
 
 class MC3:
     """Metropolis-coupled chains (BNN_mc3.py:8-126).  All chains live on the GPU(s); there is no fork pool
-    and nothing is pickled between swap periods.  With torch.distributed initialised the chains are
-    sharded over the ranks and the swap step all-gathers the log-posteriors (npbnn_b200/mc3.py)."""
+    and nothing is pickled between swap periods.  With torch.distributed initialised the ranks form Q chain blocks x
+    R row shards (mc3.chain_grid): the chains are sharded over the blocks, the R ranks of a block split its rows
+    (rowshard.py), and the swap step all-gathers the log-posteriors (npbnn_b200/mc3.py)."""
+
+    R = 1          # row shards per chain block
 
     def __init__(self, data, logger, n_post_samples=100, sampling_f=100, n_chains=4, swap_frequency=100, verbose=1,
                  print_f=100, temperatures=None, min_temperature=0.8, likelihood_f=None, accuracy_f=None, adapt_freq=50,
@@ -899,13 +910,21 @@ class MC3:
         self.logger = logger
         self.world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
         self.rank = dist.get_rank() if self.world > 1 else 0
-        if n_chains < self.world:
-            raise ValueError("MC3: n_chains=%d is smaller than the number of ranks (%d); every rank needs a chain"
-                             % (n_chains, self.world))
+        self.Q, self.R = _mc3.chain_grid(n_chains, self.world)
+        q, r = divmod(self.rank, self.R)
+        if self.R > 1 and rng == "host" and (data._freq_indicator or data._feature_indicators is not None):
+            # the indicator flips come from numpy's global generator (_ChainGroup.draw_steps), whose state differs
+            # between the ranks of a block
+            raise NotImplementedError("MC3 with more ranks (%d) than chains (%d) and rng='host' does not run weight or "
+                                      "feature indicators; use rng='philox'" % (self.world, n_chains))
         if self.world > 1:
             # every rank must hold the same chain seeds and swap generator whatever its own numpy state is
             self.rseeds = np.asarray(_mc3.broadcast_from_rank0(self.rseeds))
-        self.start, self.n_local = _mc3.chain_partition(n_chains, self.world, self.rank)
+        self.start, self.n_local = _mc3.chain_partition(n_chains, self.Q, q)
+        row_group = None
+        if 1 < self.R < self.world:
+            from .predshard import block_group
+            row_group = block_group(self.world, self.R, q)
         self._rng_mode = rng
         if swap_seed is None and self.world == 1:
             self._swap_rng = _mc3.GlobalSwapRNG()      # the reference's own stream (np.random, BNN_mc3.py:99,109)
@@ -916,7 +935,7 @@ class MC3:
         self._group = _ChainGroup(data, [data._w_layers] * self.n_local,
                                   self.temperatures[self.start:self.start + self.n_local], [0.05] * nl, [0.075] * nl,
                                   1, adapt_f, adapt_fM, adapt_freq, adapt_stop, 0, seed=int(self.rseeds[0]), device=device,
-                                  chain_offset=self.start, lik=count_kind)
+                                  row_shard=(self.R, r), row_group=row_group, chain_offset=self.start, lik=count_kind)
         # per-chain views with the reference's attribute surface (singleChainArgs[i] = [bnn, mcmc])
         self.singleChainArgs = []
         for i in range(self.n_local):
@@ -993,7 +1012,7 @@ class MC3:
             self._run_period()
             if self.n_chains > 1:
                 temps, swapped, (j, k), lp = _mc3.exchange(g.eng.gather(L.F_LOGPOST), self.current_temperatures,
-                                                           self._swap_rng, None, self.world)
+                                                           self._swap_rng, None, self.world, self.R)
                 if swapped:
                     if self.verbose > 0 and self.rank == 0:
                         print(mc3_it, "SWAPPED", lp[j], lp[k], self.current_temperatures[j], self.current_temperatures[k])
@@ -1018,13 +1037,13 @@ class MC3:
 
     def _log_on_rank0(self, cold):
         """Chains sharded over ranks: the cold temperature migrates between ranks with the swaps, the files belong to
-        rank 0.  The rank holding the cold chain sends its exported state (statistics + weights, a few kB) to rank 0,
-        which is the only rank that writes the .log / .pkl and keeps the posterior sample list."""
+        rank 0.  The r = 0 rank of the block holding the cold chain sends its exported state (statistics + weights, a
+        few kB) to rank 0, which is the only rank that writes the .log / .pkl and keeps the posterior sample list."""
         import torch.distributed as dist
         cold_chain = int(np.flatnonzero(self.current_temperatures == 1)[0]) if np.any(self.current_temperatures == 1) else -1
         if cold_chain < 0:
             return
-        owner = _mc3.owner_of(cold_chain, self.n_chains, self.world)
+        owner = _mc3.owner_of(cold_chain, self.n_chains, self.world, self.R)
         box = [None]
         if self.rank == owner:
             b, m = cold

@@ -1115,7 +1115,6 @@ int bnn_rowshard_config(bnn_ctx* c, int64_t n_train_global) {
   REQUIRE(c && c->have_data, "bnn_rowshard_config: call bnn_set_data (this rank's rows) first");
   invalidate_graphs(c);
   REQUIRE(n_train_global >= c->n_train, "bnn_rowshard_config: n_train_global is smaller than the local shard");
-  REQUIRE(!bnn_lik_is_count(c->g.lik), "bnn_rowshard_config: row sharding of the count likelihoods is not implemented");
   c->rowshard = true;
   c->n_train_global = n_train_global;
   c->have_chains = false;

@@ -12,6 +12,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
+from . import rowshard
 
 
 @dataclass
@@ -306,8 +307,7 @@ class Engine:
                                          _np_ptr(uws), _np_ptr(al), _np_ptr(sg), self._stream()))
         self.n_chains = n
         if callable(self._rowshard):
-            self._rowshard_exchange()
-            self.rowshard_update(2, False)
+            rowshard.exchange([self], self._all_reduce_own, 2)
 
     def _pack_injection(self, injection, n_steps):
         arrs = {k: np.ascontiguousarray(injection[k], dtype=(np.float64 if k in ("dz", "log_u") else np.int32))
@@ -364,19 +364,13 @@ class Engine:
         L.check(self.lib.bnn_rowshard_commit(self._h, _ptr(red), self._stream()))
         torch.cuda.current_stream(self.device).synchronize()      # red may be released by the caller
 
-    def _rowshard_exchange(self):
-        red = self.rowshard_local()
-        self._rowshard(red)                       # the exchange step: C * n_values doubles
-        self.rowshard_commit(red)
+    def _all_reduce_own(self, reds):
+        self._rowshard(reds[0])                   # the exchange step: C * n_values doubles
 
     def _mh_steps_rowshard(self, n_steps, injection):
         if not callable(self._rowshard):
             raise L.NpbnnError("manual row sharding: drive rowshard_update / rowshard_local / rowshard_commit yourself")
-        for s in range(n_steps):
-            one = None if injection is None else {k: v[s:s + 1] for k, v in injection.items() if v is not None}
-            self.rowshard_update(0, True, one)
-            self._rowshard_exchange()
-            self.rowshard_update(1, False)
+        rowshard.mh_steps([self], n_steps, injection, self._all_reduce_own)
 
     def read_state(self, weights=True) -> ChainState:
         n = self.n_chains

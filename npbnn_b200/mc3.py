@@ -4,7 +4,8 @@ Replaces the fork pool of the reference (BNN_mc3.py:87-126), which pickles every
 of the data) to a worker and back each swap period.  Here the chains never leave their GPU; the only
 exchange is an all-gather of the per-chain log-posteriors (8 bytes per chain) over NCCL/NVLink, after
 which every rank evaluates the same swap with the same seeded generator and updates the temperatures
-of its own chains.  No tensor of the data path is communicated.
+of its own chains.  No tensor of the data path is communicated.  With more ranks than chains the ranks form a grid of
+chain blocks x row shards (chain_grid): the ranks of a block run the same chains on their own rows (rowshard.py).
 """
 from typing import Optional, Tuple
 
@@ -25,6 +26,20 @@ def chain_partition(n_chains: int, world_size: int, rank: int) -> Tuple[int, int
     base, rem = divmod(n_chains, world_size)
     start = rank * base + min(rank, rem)
     return start, base + (1 if rank < rem else 0)
+
+
+def chain_grid(n_chains: int, world_size: int) -> Tuple[int, int]:
+    """(Q, R): Q chain blocks x R row shards with Q * R == world_size.  Up to one rank per chain the ranks hold whole
+    chains (R = 1, the partition of chain_partition over all ranks).  With more ranks than chains, Q is the largest
+    divisor of world_size that does not exceed n_chains, and the R ranks of a block split its rows (rowshard.py), so
+    every GPU has work: 4 chains on 8 GPUs run as 4 x 2, one chain on 8 GPUs as 1 x 8.  Rank = q * R + r: the R ranks
+    of a block, which all-reduce every MH iteration, are neighbours."""
+    if n_chains < 1 or world_size < 1:
+        raise ValueError("chain_grid: %d chains on %d ranks" % (n_chains, world_size))
+    if world_size <= n_chains:
+        return world_size, 1
+    q = max(d for d in range(1, n_chains + 1) if world_size % d == 0)
+    return q, world_size // q
 
 
 class SwapRNG:
@@ -65,12 +80,14 @@ def broadcast_from_rank0(obj, group: Optional[dist.ProcessGroup] = None):
     return box[0]
 
 
-def owner_of(chain: int, n_chains: int, world_size: int) -> int:
-    """Rank that holds global chain index `chain` under chain_partition."""
-    for r in range(world_size):
-        start, n = chain_partition(n_chains, world_size, r)
+def owner_of(chain: int, n_chains: int, world_size: int, R: int = 1) -> int:
+    """Rank that holds global chain index `chain` under chain_partition over the world_size / R chain blocks: the r = 0
+    rank of its block."""
+    Q = world_size // R
+    for q in range(Q):
+        start, n = chain_partition(n_chains, Q, q)
         if start <= chain < start + n:
-            return r
+            return q * R
     raise ValueError("chain %d of %d" % (chain, n_chains))
 
 
@@ -87,7 +104,7 @@ def swap_temperatures(log_post: np.ndarray, temps: np.ndarray, j: int, k: int, l
 
 def gather_log_post(local: torch.Tensor, counts, group: Optional[dist.ProcessGroup] = None) -> np.ndarray:
     """All-gather of the local chains' log-posteriors -> host vector over all chains (rank order).
-    `counts[r]` = chains owned by rank r.  Uses the process group's backend (NCCL on GPUs, gloo in tests)."""
+    `counts[r]` = chains rank r contributes.  Uses the process group's backend (NCCL on GPUs, gloo in tests)."""
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
         return local.detach().cpu().numpy().astype(np.float64)
     world = dist.get_world_size(group)
@@ -101,11 +118,15 @@ def gather_log_post(local: torch.Tensor, counts, group: Optional[dist.ProcessGro
 
 
 def exchange(local_log_post: torch.Tensor, temps_all: np.ndarray, rng: SwapRNG,
-             group: Optional[dist.ProcessGroup] = None, world_size: int = 1):
-    """One swap step.  Returns (new temperatures of ALL chains, swapped?, (j, k), gathered log-posteriors)."""
+             group: Optional[dist.ProcessGroup] = None, world_size: int = 1, R: int = 1, gather=gather_log_post):
+    """One swap step on a grid of world_size / R chain blocks x R row shards (chain_grid).  Returns (new temperatures of
+    ALL chains, swapped?, (j, k), gathered log-posteriors).  The R ranks of a block hold bit-identical copies of its
+    log-posteriors; only the r = 0 copy enters the swap (the others count zero chains in the gather).
+    gather(local, counts, group): the all-gather (a test substitutes an in-process one)."""
     n = len(temps_all)
-    counts = [chain_partition(n, world_size, r)[1] for r in range(world_size)]
-    lp = gather_log_post(local_log_post, counts, group)
+    Q = world_size // R
+    counts = [chain_partition(n, Q, p // R)[1] if p % R == 0 else 0 for p in range(world_size)]
+    lp = gather(local_log_post, counts, group)
     if n < 2:
         return np.array(temps_all, dtype=np.float64), False, (0, 0), lp
     j, k = rng.pair(n)

@@ -52,12 +52,14 @@ def partition(n_rows: int, n_sets: int, world: int, rank: int, grid: Optional[Tu
 _GROUPS = {}
 
 
-def _row_group(world: int, q: int, rg: int):
-    """Process group of the Q ranks that share row group rg (every rank must create all groups, in the same order)."""
-    key = (world, q)
+def block_group(world: int, size: int, index: int):
+    """Process group of the `size` consecutive ranks of block `index` (ranks index * size ... + size - 1): the Q ranks
+    that share a row group here, the R row shards of a chain block in MC3 (mc3.chain_grid).  Every rank creates all
+    blocks' groups at its first call, in the same order, as torch.distributed requires."""
+    key = (world, size)
     if key not in _GROUPS:
-        _GROUPS[key] = [dist.new_group(list(range(g * q, (g + 1) * q))) for g in range(world // q)]
-    return _GROUPS[key][rg]
+        _GROUPS[key] = [dist.new_group(list(range(g * size, (g + 1) * size))) for g in range(world // size)]
+    return _GROUPS[key][index]
 
 
 def combine(local_sum: torch.Tensor, n_sets_total: int, world: int, rank: int, grid: Tuple[int, int]) -> torch.Tensor:
@@ -65,7 +67,7 @@ def combine(local_sum: torch.Tensor, n_sets_total: int, world: int, rank: int, g
     mean over all n_sets_total samples of the row block, identical on the Q ranks of the row group."""
     r, q = grid
     if q > 1:
-        dist.all_reduce(local_sum, op=dist.ReduceOp.SUM, group=_row_group(world, q, rank // q))
+        dist.all_reduce(local_sum, op=dist.ReduceOp.SUM, group=block_group(world, q, rank // q))
     return local_sum / float(n_sets_total)
 
 
