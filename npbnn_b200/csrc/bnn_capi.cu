@@ -26,9 +26,14 @@ static int fail(const std::string& msg) {
     if (!(cond)) return fail(msg); \
   } while (0)
 
+// device buffer that frees itself; one owner, so not copyable
 struct DevBuf {
   void* p = nullptr;
   size_t bytes = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { release(); }
   // grow-only; newly allocated memory is zero-filled when `zero`
   cudaError_t ensure(size_t n, bool zero, cudaStream_t st, bool* grew = nullptr) {
     if (grew) *grew = false;
@@ -82,7 +87,7 @@ struct bnn_ctx {
   long long n_train_global = 0;
   DevBuf part_red;
   DevBuf part_sl;                   // [C, NF, n_slices]: slice sums of the tile partials (k_reduce_part), read by k_mh_update
-  DevBuf inj_proposed, inj_count, inj_ix, inj_iy, inj_dz, inj_logu, inj_alpha_ix, inj_alpha_dz, inj_add_prob;
+  DevBuf inj_alpha_ix, inj_alpha_dz, inj_add_prob;
   // the six arrays every injection carries travel in ONE host-to-device transfer: packed into a pinned staging buffer
   // (so the caller's arrays are free on return whatever memory they live in), copied into one device arena
   DevBuf inj_arena;
@@ -96,7 +101,6 @@ struct bnn_ctx {
   int sp_pair_nc1 = 0, sp_pair_nr1 = 0, sp_pair_nr2 = 0;   // uniform block pairs (k_fwd_sparse's fused path); nc1 == 0: none
   bool use_sparse = false;
   int opt_sparse = 1;               // option "sparse": 0 forces the dense kernels for masked chains
-  long long sp_fma = 0, dense_fma = 0;
   // optional per-launch timing of the forward kernel (bench.py roofline): event pairs on the launch stream
   int time_forward = 0;
   std::vector<cudaEvent_t> ev;      // start/stop pairs, recorded but not yet read
@@ -110,8 +114,14 @@ struct bnn_ctx {
     size_t bytes = 0;
     cudaEvent_t staged = nullptr, done = nullptr;
     bool pending = false;
+    ~Snap() {
+      if (host) cudaFreeHost(host);
+      if (staged) cudaEventDestroy(staged);
+      if (done) cudaEventDestroy(done);
+    }
   };
-  std::vector<Snap> snaps;
+  static constexpr int kSnapSlots = 64;
+  Snap snaps[kSnapSlots];
   cudaStream_t copy_stream = nullptr;
   // CUDA graphs of the free-running MH loop (bnn_mh_steps without injection): launch-bound at small N
   struct StepGraph { int n_steps; cudaGraphExec_t exec; long long launches; };
@@ -123,6 +133,17 @@ struct bnn_ctx {
   int opt_chain_cluster = 16;       // option "chain_loop_cluster": largest thread-block cluster per chain
   int opt_pred_tf32 = 0;            // option "predict_tf32": opt-in 3xTF32 prediction summaries (bnn_pred_lp.cu), never the MH path
   bool mh_warm = false;             // one eager bnn_mh_steps has run since the last (re)configuration
+
+  // the owner of the device resources above (the DevBufs and Snaps free themselves); the caller has made this context's
+  // device current and synchronised it
+  ~bnn_ctx() {
+    for (auto& gph : graphs) cudaGraphExecDestroy(gph.exec);
+    if (capture_stream) cudaStreamDestroy(capture_stream);
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+    if (inj_host) cudaFreeHost(inj_host);
+    if (inj_copied) cudaEventDestroy(inj_copied);
+    for (cudaEvent_t e : ev) cudaEventDestroy(e);
+  }
 };
 
 // every call that changes what a captured launch sequence would contain (pointers, kernel choice, chain count)
@@ -152,29 +173,34 @@ static cudaError_t timed_forward(bnn_ctx* c, const FwdParams& p, bool predict, c
 }
 
 static int sets_per_pass(const NetGeom& g) {
-  int nc = 2 + 2 * g.K;
+  int nc = bnn_n_counts(g.K);
   int byc = 16384 / (nc * 4);
   int v = byc < BNN_MAX_SETS_PER_PASS ? byc : BNN_MAX_SETS_PER_PASS;
   return v < 1 ? 1 : v;
 }
-static int n_slots(const NetGeom& g) { return g.lik == BNN_LIK_CATEGORICAL ? 1 : 1 + 3 * g.K; }
-
-static FwdParams base_params(const bnn_ctx* c) {
+// the forward parameters every launch over the packed rows x (n_total rows, the first n_train of them training rows) shares
+static FwdParams fwd_params(const bnn_ctx* c, const NetGeom& g, const double* x, long long n_train, long long n_total) {
   FwdParams p{};
-  p.g = c->g;
-  p.x = c->xs.as<double>();
-  p.n_train = c->n_train;
-  p.n_total = c->n_total;
-  p.n_tiles16 = c->n_tiles16;
+  p.g = g;
+  p.x = x;
+  p.n_train = n_train;
+  p.n_total = n_total;
+  p.n_tiles16 = (n_total + 15) / 16;
+  p.exp_tab = c->exp_tab.as<double>();
+  p.exp_tab_small = c->exp_tab_small.as<double>();
+  p.NF = bnn_n_slots(g);
+  p.inv_sets = 1.0;
+  return p;
+}
+
+// ... over the staged data set
+static FwdParams base_params(const bnn_ctx* c) {
+  FwdParams p = fwd_params(c, c->g, c->xs.as<double>(), c->n_train, c->n_total);
   p.labels = c->labels.as<int>();
   p.targets = c->targets.as<double>();
   p.lgk1 = c->lgk1.as<double>();
   p.inst_w = c->has_iw ? c->inst_w.as<double>() : nullptr;
   p.class_w = c->has_cw ? c->class_w.as<double>() : nullptr;
-  p.exp_tab = c->exp_tab.as<double>();
-  p.exp_tab_small = c->exp_tab_small.as<double>();
-  p.NF = n_slots(c->g);
-  p.inv_sets = 1.0;
   return p;
 }
 
@@ -267,8 +293,6 @@ int bnn_ctx_create(bnn_ctx** out, int device) {
   bnn_ctx* c = new bnn_ctx();
   c->device = device;
   c->n_sms = prop.multiProcessorCount;
-  const char* fg = getenv("NPBNN_FORCE_GENERIC");
-  c->force_generic = (fg && fg[0] == '1') ? 1 : 0;
   const char* pt = getenv("NPBNN_PREDICT_TF32");           // opt-in reduced-precision prediction summaries (bnn_pred_lp.cu)
   if (pt) c->opt_pred_tf32 = atoi(pt);
   std::vector<double> tab(BNN_EXP_TAB_SIZE);
@@ -290,29 +314,6 @@ int bnn_ctx_destroy(bnn_ctx* c) {
   if (!c) return 0;
   cudaSetDevice(c->device);
   cudaDeviceSynchronize();
-  DevBuf* bufs[] = {&c->xs, &c->labels, &c->targets, &c->lgk1, &c->inst_w, &c->class_w, &c->exp_tab, &c->exp_tab_small,
-                    &c->wp_scratch, &c->part, &c->counts_scratch, &c->xs_pred, &c->ov_cols, &c->ov_vals, &c->h_w,
-                    &c->h_alpha, &c->h_sigma, &c->h_loglik, &c->h_sums, &c->h_counts, &c->w_cur, &c->w_prop,
-                    &c->wp_prop, &c->mask, &c->owner, &c->sf, &c->si, &c->counts_prop, &c->alpha_chain,
-                    &c->inj_proposed, &c->inj_count, &c->inj_ix, &c->inj_iy, &c->inj_dz, &c->inj_logu, &c->inj_alpha_ix,
-                    &c->inj_alpha_dz, &c->inj_add_prob, &c->part_red, &c->part_sl, &c->sp_items, &c->sp_widx, &c->flag};
-  for (DevBuf* b : bufs) b->release();
-  c->ps_entry.release(); c->pls_entry.release(); c->ps_tmp.release(); c->pls_tmp.release();
-  for (DevBuf* b : {&c->ind_cur, &c->ind_prop, &c->fi_cur, &c->fi_prop, &c->feat_mean, &c->inj_ind_move, &c->inj_ind_flip,
-                    &c->inj_fi_move, &c->inj_fi_flip}) b->release();
-  for (auto& sn : c->snaps) {
-    sn.dev.release();
-    if (sn.host) cudaFreeHost(sn.host);
-    if (sn.staged) cudaEventDestroy(sn.staged);
-    if (sn.done) cudaEventDestroy(sn.done);
-  }
-  c->inj_arena.release();
-  if (c->inj_host) cudaFreeHost(c->inj_host);
-  if (c->inj_copied) cudaEventDestroy(c->inj_copied);
-  if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-  invalidate_graphs(c);
-  if (c->capture_stream) cudaStreamDestroy(c->capture_stream);
-  for (cudaEvent_t e : c->ev) cudaEventDestroy(e);
   delete c;
   return 0;
 }
@@ -357,31 +358,21 @@ int bnn_set_net(bnn_ctx* c, const bnn_net_spec* s) {
   g.F = s->n_features;
   g.act = s->act;
   g.lik = s->lik;
-  int in = s->n_features, off = 0, coff = 0;
-  g.max_w = 8;
+  int in = s->n_features, coff = 0;
+  int out_pad[BNN_MAX_LAYERS];
   for (int l = 0; l < g.L; ++l) {
     LayerGeom& lg = g.l[l];
     REQUIRE(s->out_dim[l] >= 1, "bnn_set_net: layer width must be positive");
     lg.in = in;
     lg.out = s->out_dim[l];
     lg.bias = s->has_bias[l] ? 1 : 0;
-    lg.in_pad = bnn_round_up(in, 8);
-    lg.out_pad = bnn_round_up(lg.out, 8);
-    lg.stride = lg.in_pad;
-    lg.swz = bnn_swz_for(lg.stride);
-    lg.w_off = off;
-    off += lg.out_pad * lg.stride;
-    lg.b_off = off;
-    off += lg.out_pad;
     lg.c_off = coff;
     coff += lg.out * (lg.in + lg.bias);
-    if (l >= 1 && lg.in_pad > g.max_w) g.max_w = lg.in_pad;
+    out_pad[l] = bnn_round_up(lg.out, 8);
     in = lg.out;
   }
-  g.F_pad = g.l[0].in_pad;
-  g.x_swz = g.l[0].swz;
+  geom_layout(g, bnn_round_up(g.F, 8), out_pad);
   g.P = coff;
-  g.PB = off;
   g.O = g.l[g.L - 1].out;
   REQUIRE(g.O <= BNN_MAX_OUT, "bnn_set_net: output layer wider than BNN_MAX_OUT (32)");
   if (g.lik == BNN_LIK_GAUSSIAN_HEAD) {
@@ -474,7 +465,7 @@ int bnn_forward_lik(bnn_ctx* c, const double* w_dev, int32_t n_sets, const doubl
   CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
   const NetGeom& g = c->g;
-  const int NC = 2 + 2 * g.K;
+  const int NC = bnn_n_counts(g.K);
   if (int rc = ensure_wp_scratch(c, g, (size_t)n_sets, st)) return rc;
   CUDA_TRY(bnn_launch_pack_w(g, w_dev, c->wp_scratch.as<double>(), n_sets, st));
   c->launches++;
@@ -512,7 +503,7 @@ int bnn_forward_lik_host(bnn_ctx* c, const double* w_host, int32_t n_sets, const
   CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
   const NetGeom& g = c->g;
-  const int NC = 2 + 2 * g.K;
+  const int NC = bnn_n_counts(g.K);
   CUDA_TRY(c->h_w.ensure(sizeof(double) * (size_t)n_sets * g.P, false, st));
   CUDA_TRY(cudaMemcpyAsync(c->h_w.p, w_host, sizeof(double) * (size_t)n_sets * g.P, cudaMemcpyHostToDevice, st));
   if (alpha_host) {
@@ -649,8 +640,6 @@ static bool build_sparse_program(bnn_ctx* c, const double* mask_host, std::vecto
         for (int k = 0; k < it.nc; ++k) readers[l - 1][it.c0 + k]++;
   }
   sp += (long long)lo.out * lo.in;
-  c->sp_fma = sp;
-  c->dense_fma = dense;
   if (sp * 4 > dense) return false;
 
   // weight stream starts with the output-layer bias (8 entries)
@@ -772,7 +761,7 @@ static ChainDev chain_dev(bnn_ctx* c) {
   d.sf = c->sf.as<double>();
   d.si = c->si.as<int>();
   d.part = c->part.as<double>();
-  d.NF = n_slots(c->g);
+  d.NF = bnn_n_slots(c->g);
   d.counts_prop = c->counts_prop.as<int>();
   d.alpha_fwd = c->alpha_chain.as<double>();
   if (const int ns = bnn_part_slices(c->n_tiles16)) {     // chains_forward folds the tile partials into ns slices per chain
@@ -790,7 +779,7 @@ static ChainDev chain_dev(bnn_ctx* c) {
 // forward pass of every chain's packed proposal -> partials + proposal counters
 static int chains_forward(bnn_ctx* c, cudaStream_t st) {
   const NetGeom& g = c->g;
-  const int NC = 2 + 2 * g.K;
+  const int NC = bnn_n_counts(g.K);
   const int per = sets_per_pass(g);
   FwdParams p = base_params(c);
   if (c->use_sparse && c->opt_sparse) {
@@ -833,7 +822,7 @@ int bnn_chains_init(bnn_ctx* c, int32_t n_chains, const bnn_sampler_config* cfg,
   CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
   const NetGeom& g = c->g;
-  const int C = n_chains, NC = 2 + 2 * g.K;
+  const int C = n_chains, NC = bnn_n_counts(g.K);
   c->C = C;
   c->have_ps_entry = false;          // per-entry prior scales belong to the previous set of chains
   for (auto& sn : c->snaps) sn.pending = false;
@@ -849,9 +838,9 @@ int bnn_chains_init(bnn_ctx* c, int32_t n_chains, const bnn_sampler_config* cfg,
   CUDA_TRY(c->si.ensure(sizeof(int) * (size_t)C * BNN_I_STRIDE, false, st));
   CUDA_TRY(c->counts_prop.ensure(sizeof(int) * (size_t)C * NC, false, st));
   CUDA_TRY(c->alpha_chain.ensure(sizeof(double) * (size_t)C * g.L, false, st));
-  CUDA_TRY(c->part.ensure(sizeof(double) * (size_t)n_slots(g) * C * c->n_tiles16, false, st));
-  if (c->rowshard) CUDA_TRY(c->part_red.ensure(sizeof(double) * (size_t)C * n_slots(g), true, st));
-  CUDA_TRY(c->part_sl.ensure(sizeof(double) * (size_t)C * n_slots(g) * 64, false, st));
+  CUDA_TRY(c->part.ensure(sizeof(double) * (size_t)bnn_n_slots(g) * C * c->n_tiles16, false, st));
+  if (c->rowshard) CUDA_TRY(c->part_red.ensure(sizeof(double) * (size_t)C * bnn_n_slots(g), true, st));
+  CUDA_TRY(c->part_sl.ensure(sizeof(double) * (size_t)C * bnn_n_slots(g) * 64, false, st));
   c->use_sparse = false;
   if (cfg->use_mask) {
     CUDA_TRY(c->mask.ensure(sizeof(double) * g.P, false, st));
@@ -1121,14 +1110,14 @@ int bnn_rowshard_config(bnn_ctx* c, int64_t n_train_global) {
   return 0;
 }
 
-int bnn_rowshard_n_values(const bnn_ctx* c) { return c ? n_slots(c->g) + 2 + 2 * c->g.K : 0; }
+int bnn_rowshard_n_values(const bnn_ctx* c) { return c ? bnn_n_slots(c->g) + bnn_n_counts(c->g.K) : 0; }
 
 int bnn_rowshard_local(bnn_ctx* c, double* red_dev, void* stream) {
   REQUIRE(c && c->have_chains && c->rowshard && red_dev, "bnn_rowshard_local: bad arguments");
   CUDA_TRY(cudaSetDevice(c->device));
   const NetGeom& g = c->g;
   const int* counts = (g.lik == BNN_LIK_CATEGORICAL) ? c->counts_prop.as<int>() : nullptr;
-  CUDA_TRY(bnn_launch_rowshard_local(g, c->part.as<double>(), n_slots(g), c->n_tiles16, counts, 2 + 2 * g.K, red_dev, c->C,
+  CUDA_TRY(bnn_launch_rowshard_local(g, c->part.as<double>(), bnn_n_slots(g), c->n_tiles16, counts, bnn_n_counts(g.K), red_dev, c->C,
                                      (cudaStream_t)stream));
   c->launches++;
   return 0;
@@ -1139,7 +1128,7 @@ int bnn_rowshard_commit(bnn_ctx* c, const double* red_global_dev, void* stream) 
   CUDA_TRY(cudaSetDevice(c->device));
   const NetGeom& g = c->g;
   int* counts = (g.lik == BNN_LIK_CATEGORICAL) ? c->counts_prop.as<int>() : nullptr;
-  CUDA_TRY(bnn_launch_rowshard_commit(red_global_dev, n_slots(g), 2 + 2 * g.K, c->part_red.as<double>(), counts, c->C,
+  CUDA_TRY(bnn_launch_rowshard_commit(red_global_dev, bnn_n_slots(g), bnn_n_counts(g.K), c->part_red.as<double>(), counts, c->C,
                                       (cudaStream_t)stream));
   c->launches++;
   return 0;
@@ -1180,10 +1169,9 @@ static size_t snap_bytes(const bnn_ctx* c) {
 
 int bnn_chains_snapshot(bnn_ctx* c, int32_t slot, void* stream) {
   REQUIRE(c && c->have_chains, "bnn_chains_snapshot: call bnn_chains_init first");
-  REQUIRE(slot >= 0 && slot < 64, "bnn_chains_snapshot: slot must be in [0, 64)");
+  REQUIRE(slot >= 0 && slot < bnn_ctx::kSnapSlots, "bnn_chains_snapshot: slot must be in [0, 64)");
   CUDA_TRY(cudaSetDevice(c->device));
   cudaStream_t st = (cudaStream_t)stream;
-  if ((size_t)slot >= c->snaps.size()) c->snaps.resize(slot + 1);
   bnn_ctx::Snap& sn = c->snaps[slot];
   REQUIRE(!sn.pending, "bnn_chains_snapshot: slot still holds an unread snapshot");
   const size_t nb = snap_bytes(c);
@@ -1216,7 +1204,7 @@ int bnn_chains_snapshot(bnn_ctx* c, int32_t slot, void* stream) {
 }
 
 int bnn_snapshot_ready(bnn_ctx* c, int32_t slot) {
-  if (!c || slot < 0 || (size_t)slot >= c->snaps.size() || !c->snaps[slot].pending) return -1;
+  if (!c || slot < 0 || slot >= bnn_ctx::kSnapSlots || !c->snaps[slot].pending) return -1;
   cudaError_t e = cudaEventQuery(c->snaps[slot].done);
   if (e == cudaSuccess) return 1;
   if (e == cudaErrorNotReady) return 0;
@@ -1225,7 +1213,7 @@ int bnn_snapshot_ready(bnn_ctx* c, int32_t slot) {
 }
 
 int bnn_snapshot_read(bnn_ctx* c, int32_t slot, double* f64_host, int32_t* i32_host, double* w_host) {
-  REQUIRE(c && slot >= 0 && (size_t)slot < c->snaps.size() && c->snaps[slot].pending,
+  REQUIRE(c && slot >= 0 && slot < bnn_ctx::kSnapSlots && c->snaps[slot].pending,
           "bnn_snapshot_read: no snapshot pending in this slot");
   CUDA_TRY(cudaSetDevice(c->device));
   bnn_ctx::Snap& sn = c->snaps[slot];
@@ -1375,18 +1363,12 @@ static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double
   CUDA_TRY(bnn_launch_pack_x(x_dev, c->xs_pred.as<double>(), n, n_pad, g.F, g.F_pad, g.x_swz, ovc, ovv, n_override, st));
   if (int rc = ensure_wp_scratch(c, g, (size_t)n_sets, st)) return rc;
   CUDA_TRY(bnn_launch_pack_w(g, w_dev, c->wp_scratch.as<double>(), n_sets, st));
-  FwdParams p{};
-  p.g = g;
-  p.x = c->xs_pred.as<double>();
-  p.n_train = n; p.n_total = n; p.n_tiles16 = n_pad / 16;
+  FwdParams p = fwd_params(c, g, c->xs_pred.as<double>(), n, n);
   p.wp = c->wp_scratch.as<double>();
   p.alpha = alpha_dev;
   p.C = n_sets;
-  p.NF = n_slots(g);
   p.mean_out = mean_dev; p.votes_out = votes_dev; p.dense_out = dense_dev;
   p.inv_sets = (double)n_sets;   // divisor (np.mean and the vote share divide, BNN_lib.py:390-392)
-  p.exp_tab = c->exp_tab.as<double>();
-  p.exp_tab_small = c->exp_tab_small.as<double>();
   p.samp_u = u_dev; p.samp_counts = class_counts_dev; p.samp_dense = post_pred_dev;
   p.samp_philox = samp_philox ? 1 : 0; p.samp_seed = samp_seed;
   if (class_counts_dev) CUDA_TRY(cudaMemsetAsync(class_counts_dev, 0, sizeof(int32_t) * (size_t)n_sets * g.K, st));

@@ -13,7 +13,6 @@
 //     straight into the leader's shared memory (distributed shared memory stores / atomics);
 //   * barrier.cluster; next step.
 // Chains are independent, so the C clusters of a launch need not be co-resident.
-#include <cstdlib>
 #include <cooperative_groups.h>
 #include "bnn_mh_body.cuh"
 #include "bnn_generic_body.cuh"
@@ -45,7 +44,7 @@ __host__ __device__ inline size_t chain_loop_per_warp(const NetGeom& g) {
   return 2 * 16 * (size_t)g.max_w + 16 * (size_t)ZS;
 }
 __host__ __device__ inline size_t chain_loop_common_doubles(const NetGeom& g, int NF, long long nt, int warps) {
-  const int NC = 2 + 2 * g.K;
+  const int NC = bnn_n_counts(g.K);
   return GEN_TAB_SIZE + (((size_t)NF * nt + 1) & ~(size_t)1) + (size_t)g.PB + ((BNN_MAX_LAYERS + 1) & ~1) +
          (size_t)warps * chain_loop_per_warp(g) + (size_t)((NC + 3) & ~3);      // (2 * NC4 ints = NC4 doubles)
 }
@@ -59,7 +58,7 @@ __host__ __device__ inline size_t chain_loop_tile_doubles(const NetGeom& g) {
 template <int ACT, bool XRES>
 __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __grid_constant__ ChainDev d,
                                                                       const __grid_constant__ FwdParams p0, int n_steps,
-                                                                      int tw, int tl, int n_worker_tiles, int pp_mode) {
+                                                                      int tw, int tl, int n_worker_tiles) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ FwdParams sp;                  // this chain's forward parameters (partials -> the leader's shared memory)
   cg::cluster_group cluster = cg::this_cluster();
@@ -70,7 +69,7 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int NTHR = (int)blockDim.x, NW = NTHR >> 5;
   const int gq = lane >> 2;
-  const int NC = 2 + 2 * g.K, NC4 = (NC + 3) & ~3;
+  const int NC = bnn_n_counts(g.K), NC4 = (NC + 3) & ~3;
   const int ZS = g.l[g.L - 1].out_pad + 1;
   const long long nt = d.n_tiles16;
   const bool leader = (rank == 0);
@@ -139,7 +138,7 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
   const FwdParams& p = sp;
   UpdLoop ctx;
   ctx.part_c = part_sm; ctx.counts_c = cnt_leader; ctx.w_sm = wstate; ctx.owner_sm = owner_sm; ctx.wpk_sm = wsm;
-  ctx.didx_sm = didx_sm; ctx.ddz_sm = ddz_sm; ctx.pk_sm = pk_sm; ctx.pp_mode = pp_mode;
+  ctx.didx_sm = didx_sm; ctx.ddz_sm = ddz_sm; ctx.pk_sm = pk_sm;
   const double2* wsrc = reinterpret_cast<const double2*>(d.wp_prop + (long long)c * g.PB);
 
   for (int s = 0; s <= n_steps; ++s) {
@@ -175,7 +174,7 @@ __global__ void __launch_bounds__(CL_MAX_WARPS * 32, 1) k_chain_loop(const __gri
     }
     // the leader's team is done with its few tiles long before the workers: it pre-proposes iteration s + 1 (layer
     // choice, scalar draws, the proposal's draws) in the time it would otherwise wait at the barrier
-    if (pp_mode && leader && tid < UPD_TEAM_THREADS && s + 1 < n_steps) {
+    if (leader && tid < UPD_TEAM_THREADS && s + 1 < n_steps) {
       ctx.first = false; ctx.last = false;
       mh_update_body<true>(d, c, 0, 3, s + 1, ctx);
     }
@@ -200,6 +199,13 @@ static size_t chain_loop_static_smem() {
   return v;
 }
 
+// dynamic shared memory a CTA of the kernel may use: what the static part leaves of BNN_MAX_DYN_SMEM
+static size_t chain_loop_max_dyn_smem() { return BNN_MAX_DYN_SMEM - chain_loop_static_smem(); }
+template <typename Kern>
+static cudaError_t prepare_chain_loop(Kern kern) {
+  return bnn_prepare_kernel((const void*)kern, (int)chain_loop_max_dyn_smem(), true);
+}
+
 // clusters of `cl` CTAs (warps * 32 threads, smem bytes each) the GPU can hold at the same time; cached per shape
 static int chain_loop_max_clusters(int cl, int warps, size_t smem) {
   struct Key { int cl, warps; size_t smem; int n; };
@@ -208,8 +214,7 @@ static int chain_loop_max_clusters(int cl, int warps, size_t smem) {
   for (int i = 0; i < n_cache; ++i)
     if (cache[i].cl == cl && cache[i].warps == warps && cache[i].smem == smem) return cache[i].n;
   auto kern = k_chain_loop<BNN_ACT_TANH, true>;          // (every instantiation has the same footprint up to a few registers)
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(232448 - chain_loop_static_smem()));
-  cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+  if (prepare_chain_loop(kern) != cudaSuccess) { cudaGetLastError(); return 0; }
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)cl);
   cfg.blockDim = dim3((unsigned)warps * 32);
@@ -226,7 +231,7 @@ static int chain_loop_max_clusters(int cl, int warps, size_t smem) {
 
 // The tile assignment of one cluster size: warps per CTA, tile slots, residency.
 static bool chain_loop_plan_for(const NetGeom& g, int NF, long long nt, int cl, ChainLoopPlan* plan) {
-  const size_t cap = (232448 - chain_loop_static_smem()) / sizeof(double);
+  const size_t cap = chain_loop_max_dyn_smem() / sizeof(double);
   const size_t tile_d = chain_loop_tile_doubles(g), lead_d = chain_loop_leader_doubles(g);
   const int workers = cl - 1;
   ChainLoopPlan best{};
@@ -297,14 +302,7 @@ template <int ACT, bool XRES>
 static cudaError_t launch_chain_loop_t(const ChainDev& d, const FwdParams& p, int n_steps, const ChainLoopPlan& plan,
                                        cudaStream_t st) {
   auto kern = k_chain_loop<ACT, XRES>;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)(232448 - chain_loop_static_smem()));
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
+  if (cudaError_t e = prepare_chain_loop(kern)) return e;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)(d.C * plan.cluster));
   cfg.blockDim = dim3((unsigned)plan.warps * 32);
@@ -318,10 +316,7 @@ static cudaError_t launch_chain_loop_t(const ChainDev& d, const FwdParams& p, in
   cfg.attrs = at;
   cfg.numAttrs = 1;
   int tw = plan.tw, tl = plan.tl, nwt = plan.n_worker_tiles;
-  // NPBNN_CHAIN_PP (debugging aid): 0 = no pre-proposal, 1 = scalar draws only, 2 (default) = scalar draws + proposal draws
-  static int pp_mode = -1;
-  if (pp_mode < 0) { const char* e = getenv("NPBNN_CHAIN_PP"); pp_mode = e ? atoi(e) : 2; }
-  return cudaLaunchKernelEx(&cfg, kern, d, p, n_steps, tw, tl, nwt, pp_mode);
+  return cudaLaunchKernelEx(&cfg, kern, d, p, n_steps, tw, tl, nwt);
 }
 
 template <int ACT>
@@ -338,10 +333,5 @@ cudaError_t bnn_launch_chain_loop(const ChainDev& d, const FwdParams& p, int n_s
   ChainLoopPlan plan;
   if (!chain_loop_plan(d.g, d.NF, d.n_tiles16, d.C, n_sms, max_cluster, mode, &plan)) return cudaErrorNotSupported;
   if (cluster_out) *cluster_out = plan.cluster;
-  switch (d.g.act) {
-    case BNN_ACT_RELU: return launch_chain_loop_a<BNN_ACT_RELU>(d, p, n_steps, plan, st);
-    case BNN_ACT_LEAKY: return launch_chain_loop_a<BNN_ACT_LEAKY>(d, p, n_steps, plan, st);
-    case BNN_ACT_SWISH: return launch_chain_loop_a<BNN_ACT_SWISH>(d, p, n_steps, plan, st);
-    default: return launch_chain_loop_a<BNN_ACT_TANH>(d, p, n_steps, plan, st);
-  }
+  return bnn_with_act(d.g.act, [&](auto a) { return launch_chain_loop_a<decltype(a)::value>(d, p, n_steps, plan, st); });
 }

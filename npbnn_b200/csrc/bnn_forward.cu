@@ -14,8 +14,10 @@
 //                 copies + mbarriers, hidden activations never leave registers.
 //   k_fwd_generic any depth/width: hidden activations staged in per-warp shared memory, weights read
 //                 through L1/L2.
-#include <type_traits>
-#include "bnn_common.cuh"
+#include <mutex>
+#include <set>
+#include <utility>
+#include "bnn_kernels.h"
 #include "bnn_generic_body.cuh"
 
 // =============================================================================================
@@ -42,7 +44,7 @@ __global__ void __launch_bounds__(GEN_WARPS * 32) k_fwd_generic(const __grid_con
   int* ibase = reinterpret_cast<int*>(hbase + GEN_WARPS * per_warp);
   int* pvote = ibase + warp * (PREDICT ? 16 * PW : 0);
   int* cnt = ibase;   // likelihood mode: [C][2+2K]
-  const int n_cnt = (!PREDICT && g.lik == BNN_LIK_CATEGORICAL) ? p.C * (2 + 2 * g.K) : 0;
+  const int n_cnt = PREDICT ? 0 : bnn_smem_counts(g, p.C);
 
   for (int i = threadIdx.x; i < GEN_TAB_SIZE; i += blockDim.x) tab[i] = p.exp_tab_small[i];
   for (int i = threadIdx.x; i < n_cnt; i += blockDim.x) cnt[i] = 0;
@@ -300,7 +302,7 @@ __global__ void __launch_bounds__(NCH == 4 ? 320 : 512, 1) k_fwd_sparse(const __
   double* buf = wsm + (size_t)G * p.sp_wlen + warp * per_warp;
   double* zs = buf + (g.F + NCH * p.sp_slots) * SP_US;
   int* cnt = reinterpret_cast<int*>(wsm + (size_t)G * p.sp_wlen + nwarps * per_warp);
-  const int n_cnt = (g.lik == BNN_LIK_CATEGORICAL) ? p.C * (2 + 2 * g.K) : 0;
+  const int n_cnt = bnn_smem_counts(g, p.C);
   int* next_unit = cnt + n_cnt;
   int* prog = reinterpret_cast<int*>((reinterpret_cast<uintptr_t>(next_unit + 1) + 15) & ~(uintptr_t)15);
 
@@ -429,7 +431,7 @@ __global__ void __launch_bounds__(NCH == 1 ? 768 : 512, 1) k_fwd_pairs(const __g
   double* tile = wsm + (size_t)G * p.sp_wlen + (size_t)grp * g.F * SP_US;       // [n_groups][F][33]
   double* zs = wsm + (size_t)G * p.sp_wlen + (size_t)n_groups * g.F * SP_US + (size_t)warp * 32 * ZS;
   int* cnt = reinterpret_cast<int*>(wsm + (size_t)G * p.sp_wlen + (size_t)n_groups * g.F * SP_US + (size_t)nwarps * 32 * ZS);
-  const int n_cnt = (g.lik == BNN_LIK_CATEGORICAL) ? p.C * (2 + 2 * g.K) : 0;
+  const int n_cnt = bnn_smem_counts(g, p.C);
   int* prog = cnt + ((n_cnt + 3) & ~3);                        // 16-byte aligned: the areas before it are
 
   for (int i = threadIdx.x; i < BNN_EXP_TAB_SIZE; i += blockDim.x) tab[i] = p.exp_tab[i];
@@ -689,7 +691,7 @@ __device__ __forceinline__ void quad_lik_commit(const FwdParams& p, int c, long 
                                                 const LikRow& o, bool valid) {
   static_assert(N3 < 32, "one lane per class plus one for the totals");
   const int K = p.g.K;
-  int* cc = cnt + c * (2 + 2 * K);
+  int* cc = cnt + c * bnn_n_counts(K);
   // Counters without data-dependent control flow: one ballot per class and table (independent VOTEs that pipeline),
   // lane k keeps the count of class k, then ONE predicated shared-memory atomic per table with distinct addresses per
   // lane.  (Measured: the counters cost nothing -- a build without them runs in the same 17.3 ms.)
@@ -977,7 +979,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
   uint64_t* xbar = bars + 4 + warp; // [NWARPS]
   int* rel = reinterpret_cast<int*>(bars + 4 + NWARPS);   // [4] warps that released slot b of part 0 / part 1
   int* cnt = reinterpret_cast<int*>(bars + 6 + NWARPS);
-  const int n_cnt = DEFER ? p.C * (2 + 2 * g.K) : 0;
+  const int n_cnt = DEFER ? p.C * bnn_n_counts(g.K) : 0;
   const int PW = CAT ? g.K : g.O;                 // columns of a prediction row
 
   for (int i = threadIdx.x; i < BNN_EXP_TAB_SIZE; i += blockDim.x) tab[i] = p.exp_tab[i];
@@ -1349,27 +1351,35 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
 // =============================================================================================
 // host-side launchers
 // =============================================================================================
+cudaError_t bnn_prepare_kernel(const void* fn, int max_dyn_smem, bool nonportable_cluster) {
+  static std::mutex mu;
+  static std::set<std::pair<const void*, int>> done;      // (kernel, device) pairs already prepared
+  int dev = 0;
+  cudaError_t e = cudaGetDevice(&dev);
+  if (e != cudaSuccess) return e;
+  std::lock_guard<std::mutex> lock(mu);
+  if (done.count({fn, dev})) return cudaSuccess;
+  e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, max_dyn_smem);
+  if (e == cudaSuccess && nonportable_cluster) e = cudaFuncSetAttribute(fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+  if (e == cudaSuccess) done.insert({fn, dev});
+  return e;
+}
+
 template <int KP0, int N1, int N2, int N3, int NWARPS, int MODE, int LIKK>
 static size_t fwd3_smem_bytes(const FwdParams& p) {
   constexpr bool DEFER = (MODE != FWD3_PRED) && (LIKK == FWD3_CAT);
   using G3 = Fwd3Geom<KP0, N1, N2, N3>;
   size_t d = 2 * (size_t)G3::PB + (size_t)NWARPS * 16 * KP0 + BNN_EXP_TAB_SIZE;
   size_t bytes = d * sizeof(double) + (6 + NWARPS) * sizeof(uint64_t);     // barriers + the ring's release counters
-  size_t ints = DEFER ? (size_t)p.C * (2 + 2 * p.g.K) : 0;
-  return bytes + ints * sizeof(int);
+  return bytes + (DEFER ? bnn_smem_counts(p.g, p.C) : 0) * sizeof(int);
 }
 
 template <int ACT, int KP0, int N1, int N2, int N3, int NWARPS, int MODE, int LIKK>
 static cudaError_t launch_fwd3(const FwdParams& p, int n_sms, cudaStream_t st) {
   auto kern = k_fwd3<ACT, KP0, N1, N2, N3, NWARPS, MODE, LIKK>;
   size_t smem = fwd3_smem_bytes<KP0, N1, N2, N3, NWARPS, MODE, LIKK>(p);
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
-  if (smem > 232448) return cudaErrorInvalidConfiguration;
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
+  if (smem > BNN_MAX_DYN_SMEM) return cudaErrorInvalidConfiguration;
   long long ctas = (p.n_tiles16 + NWARPS - 1) / NWARPS;
   if (MODE != FWD3_PRED) ctas *= p.C;          // likelihood modes deal (tile group, weight set) pairs out over the CTAs
   int grid = (int)(ctas < n_sms ? ctas : n_sms);
@@ -1395,12 +1405,9 @@ static cudaError_t launch_fwd3_family(const FwdParams& p, bool predict, int n_sm
 
 template <int KP0, int N1, int N2, int NWARPS>
 static cudaError_t launch_fwd3_act(const FwdParams& p, bool predict, int n_sms, cudaStream_t st) {
-  switch (p.g.act) {
-    case BNN_ACT_RELU: return launch_fwd3_family<BNN_ACT_RELU, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
-    case BNN_ACT_LEAKY: return launch_fwd3_family<BNN_ACT_LEAKY, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
-    case BNN_ACT_SWISH: return launch_fwd3_family<BNN_ACT_SWISH, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
-    default: return launch_fwd3_family<BNN_ACT_TANH, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
-  }
+  return bnn_with_act(p.g.act, [&](auto a) {
+    return launch_fwd3_family<decltype(a)::value, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
+  });
 }
 
 // which k_fwd3 family the padded geometry matches exactly: 1 = A, 2 = B, 0 = none
@@ -1420,16 +1427,11 @@ static cudaError_t launch_generic_t(const FwdParams& p, int n_sms, cudaStream_t 
   const int PW = (p.g.lik == BNN_LIK_CATEGORICAL) ? p.g.K : p.g.O;
   size_t per_warp = 2 * 16 * (size_t)p.g.max_w + 16 * ZS + (PREDICT ? 16 * PW : 0);
   size_t bytes = (GEN_TAB_SIZE + GEN_WARPS * per_warp) * sizeof(double);
-  size_t ints = PREDICT ? (size_t)GEN_WARPS * 16 * PW
-                        : (p.g.lik == BNN_LIK_CATEGORICAL ? (size_t)p.C * (2 + 2 * p.g.K) : 0);
+  size_t ints = PREDICT ? (size_t)GEN_WARPS * 16 * PW : bnn_smem_counts(p.g, p.C);
   bytes += ints * sizeof(int);
-  if (bytes > 232448) return cudaErrorInvalidConfiguration;
-  static size_t attr_bytes = 0;
-  if (bytes > 48 * 1024 && bytes > attr_bytes) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess) return e;
-    attr_bytes = 232448;
-  }
+  if (bytes > BNN_MAX_DYN_SMEM) return cudaErrorInvalidConfiguration;
+  if (bytes > 48 * 1024)
+    if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
   long long ctas = (p.n_tiles16 + GEN_WARPS - 1) / GEN_WARPS;
   // resident CTAs per SM limited by shared memory; cap the grid at a few waves of resident CTAs
   long long max_grid = (long long)n_sms * 8;
@@ -1445,25 +1447,19 @@ static cudaError_t launch_generic_t(const FwdParams& p, int n_sms, cudaStream_t 
 
 template <bool PREDICT>
 static cudaError_t launch_generic(const FwdParams& p, int n_sms, cudaStream_t st) {
-  switch (p.g.act) {
-    case BNN_ACT_RELU: return launch_generic_t<BNN_ACT_RELU, PREDICT>(p, n_sms, st);
-    case BNN_ACT_LEAKY: return launch_generic_t<BNN_ACT_LEAKY, PREDICT>(p, n_sms, st);
-    case BNN_ACT_SWISH: return launch_generic_t<BNN_ACT_SWISH, PREDICT>(p, n_sms, st);
-    default: return launch_generic_t<BNN_ACT_TANH, PREDICT>(p, n_sms, st);
-  }
+  return bnn_with_act(p.g.act, [&](auto a) { return launch_generic_t<decltype(a)::value, PREDICT>(p, n_sms, st); });
 }
 
 // shared-memory plan of k_fwd_sparse: chains per unit, chains per resident weight group and warps per CTA
 static size_t sparse_fixed_bytes(const FwdParams& p, int C) {
-  return BNN_EXP_TAB_SIZE * sizeof(double) +
-         (p.g.lik == BNN_LIK_CATEGORICAL ? (size_t)C * (2 + 2 * p.g.K) * sizeof(int) : 0) +
+  return BNN_EXP_TAB_SIZE * sizeof(double) + (size_t)bnn_smem_counts(p.g, C) * sizeof(int) +
          (size_t)(p.sp_prog_len + 8) * sizeof(int) + 16;
 }
 static size_t sparse_warp_bytes(const FwdParams& p, int nch) {
   return ((size_t)(p.g.F + nch * p.sp_slots) * SP_US + 32 * (SP_MAX_O + 1)) * sizeof(double);
 }
 static bool sparse_plan(const FwdParams& p, int C, int nch, int* group, int* nwarps) {
-  const size_t cap = 232448;
+  const size_t cap = BNN_MAX_DYN_SMEM;
   const size_t fixed = sparse_fixed_bytes(p, C), per_warp = sparse_warp_bytes(p, nch);
   const size_t per_chain = (size_t)p.sp_wlen * sizeof(double);
   const int c_up = (C + nch - 1) / nch * nch;
@@ -1497,12 +1493,7 @@ static cudaError_t launch_sparse_n(const FwdParams& p0, int n_sms, cudaStream_t 
   if (units < nwarps) nwarps = (int)units;
   const size_t bytes = sparse_fixed_bytes(p, p.C) + (size_t)group * p.sp_wlen * sizeof(double) +
                        (size_t)nwarps * sparse_warp_bytes(p, NCH);
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
   kern<<<grid, nwarps * 32, bytes, st>>>(p);
   return cudaGetLastError();
 }
@@ -1513,13 +1504,15 @@ static int sparse_pair_shape(const FwdParams& p) {
   return (pr == 3 * 16 + 2 || pr == 2 * 16 + 1 || pr == 2 * 16 + 2 || pr == 4 * 16 + 2) ? pr : 0;
 }
 constexpr int SPARSE_PAIR_NCH = 2;      // chains a thread of k_fwd_pairs evaluates together
+// dynamic shared memory of k_fwd_pairs: `group` resident chains, `nwarps` warps that share one X tile per `share`
+static size_t pairs_bytes(const FwdParams& p, int group, int share, int nwarps) {
+  const size_t n_cnt = bnn_smem_counts(p.g, p.C);
+  return BNN_EXP_TAB_SIZE * sizeof(double) + (((n_cnt + 3) & ~(size_t)3) + p.sp_prog_len + 4) * sizeof(int) +
+         (size_t)group * p.sp_wlen * sizeof(double) + (size_t)(nwarps / share) * p.g.F * SP_US * sizeof(double) +
+         (size_t)nwarps * 32 * (SP_MAX_O + 1) * sizeof(double);
+}
 // shared-memory plan of k_fwd_pairs: resident chains, warps per group, warps
 static bool pairs_plan(const FwdParams& p, int nch, int* group, int* share, int* nwarps, size_t* bytes) {
-  const size_t cap = 232448;
-  const size_t n_cnt = (p.g.lik == BNN_LIK_CATEGORICAL) ? (size_t)p.C * (2 + 2 * p.g.K) : 0;
-  const size_t fixed = BNN_EXP_TAB_SIZE * sizeof(double) + (((n_cnt + 3) & ~(size_t)3) + p.sp_prog_len + 4) * sizeof(int);
-  const size_t per_chain = (size_t)p.sp_wlen * sizeof(double), tile_b = (size_t)p.g.F * SP_US * sizeof(double);
-  const size_t zs_b = 32 * (SP_MAX_O + 1) * sizeof(double);
   const int max_warps = (nch == 1) ? 24 : 16;
   const int c_up = (p.C + nch - 1) / nch * nch;
   // all chains resident if they fit next to a useful number of warps, else as many as fit with the full set of warps
@@ -1528,8 +1521,8 @@ static bool pairs_plan(const FwdParams& p, int nch, int* group, int* share, int*
     int gw = n_sub < 8 ? n_sub : 8;
     while (max_warps % gw) --gw;                       // groups tile the CTA exactly
     for (int w = max_warps; w >= gw; w -= gw) {
-      const size_t need = fixed + (size_t)gch * per_chain + (size_t)(w / gw) * tile_b + (size_t)w * zs_b;
-      if (need <= cap && (w >= max_warps / 2 || gch == nch)) {
+      const size_t need = pairs_bytes(p, gch, gw, w);
+      if (need <= BNN_MAX_DYN_SMEM && (w >= max_warps / 2 || gch == nch)) {
         *group = gch; *share = gw; *nwarps = w; *bytes = need;
         return true;
       }
@@ -1558,17 +1551,9 @@ static cudaError_t launch_pairs(const FwdParams& p0, int n_sms, cudaStream_t st)
   const long long tiles_per_cta = (n_tiles32 + grid - 1) / grid;
   if (tiles_per_cta * share < nwarps) {
     nwarps = (int)tiles_per_cta * share;
-    const size_t n_cnt = (p.g.lik == BNN_LIK_CATEGORICAL) ? (size_t)p.C * (2 + 2 * p.g.K) : 0;
-    bytes = BNN_EXP_TAB_SIZE * sizeof(double) + (((n_cnt + 3) & ~(size_t)3) + p.sp_prog_len + 4) * sizeof(int) +
-            (size_t)group * p.sp_wlen * sizeof(double) + (size_t)(nwarps / share) * p.g.F * SP_US * sizeof(double) +
-            (size_t)nwarps * 32 * (SP_MAX_O + 1) * sizeof(double);
+    bytes = pairs_bytes(p, group, share, nwarps);
   }
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
   kern<<<grid, nwarps * 32, bytes, st>>>(p);
   return cudaGetLastError();
 }
@@ -1597,12 +1582,7 @@ bool bnn_sparse_fits(const FwdParams& p) {
 }
 
 static cudaError_t launch_sparse(const FwdParams& p, int n_sms, cudaStream_t st) {
-  switch (p.g.act) {
-    case BNN_ACT_RELU: return launch_sparse_t<BNN_ACT_RELU>(p, n_sms, st);
-    case BNN_ACT_LEAKY: return launch_sparse_t<BNN_ACT_LEAKY>(p, n_sms, st);
-    case BNN_ACT_SWISH: return launch_sparse_t<BNN_ACT_SWISH>(p, n_sms, st);
-    default: return launch_sparse_t<BNN_ACT_TANH>(p, n_sms, st);
-  }
+  return bnn_with_act(p.g.act, [&](auto a) { return launch_sparse_t<decltype(a)::value>(p, n_sms, st); });
 }
 
 // Dispatch: specialised kernel when the padded shape is one of the compiled instantiations.

@@ -81,12 +81,12 @@ __device__ __forceinline__ void bnn_epilogue(const FwdParams& p, int c, long lon
           ll = (d < -745.1332191019412) ? -INFINITY : d - log(S);
           if (p.class_w) ll *= p.class_w[y];
           if (p.inst_w) ll *= p.inst_w[row];
-          int* cc = cnt_smem + c * (2 + 2 * K);
+          int* cc = cnt_smem + c * bnn_n_counts(K);
           if (ok) atomicAdd(&cc[2 + y], 1);
           atomicAdd(&cc[2 + K + arg], 1);
           if (ok) atomicAdd(&cc[0], 1);
         } else if (ok) {
-          atomicAdd(&cnt_smem[c * (2 + 2 * K) + 1], 1);
+          atomicAdd(&cnt_smem[c * bnn_n_counts(K) + 1], 1);
         }
       }
       double s = warp16_sum(is_train ? ll : 0.0);

@@ -1,6 +1,26 @@
 // Internal interface between the kernel translation units and the C-ABI layer (bnn_capi.cu).
 #pragma once
+#include <type_traits>
 #include "bnn_common.cuh"
+
+// Most dynamic shared memory a block of sm_100 may opt in to (227 KB).
+constexpr int BNN_MAX_DYN_SMEM = 232448;
+
+// Lets kernel `fn` use up to max_dyn_smem bytes of dynamic shared memory (and non-portable cluster sizes, if asked) on
+// the current device.  Function attributes belong to a device's context, so they are set once per (kernel, device);
+// safe when several host threads launch at once.
+cudaError_t bnn_prepare_kernel(const void* fn, int max_dyn_smem, bool nonportable_cluster = false);
+
+// f(std::integral_constant<int, ACT>{}) for the run-time activation `act`: where launchers pick a kernel's ACT.
+template <typename F>
+inline auto bnn_with_act(int act, F&& f) {
+  switch (act) {
+    case BNN_ACT_RELU: return f(std::integral_constant<int, BNN_ACT_RELU>{});
+    case BNN_ACT_LEAKY: return f(std::integral_constant<int, BNN_ACT_LEAKY>{});
+    case BNN_ACT_SWISH: return f(std::integral_constant<int, BNN_ACT_SWISH>{});
+    default: return f(std::integral_constant<int, BNN_ACT_TANH>{});
+  }
+}
 
 struct PriorScales {
   double s[BNN_MAX_LAYERS];    // npBNN._prior_scale
@@ -25,7 +45,7 @@ struct ChainDev {
   int* si;              // [C, BNN_I_STRIDE]
   const double* part;   // forward partials [C, NF, n_tiles16]
   int NF;
-  int* counts_prop;     // [C, 2 + 2K]
+  int* counts_prop;     // [C, bnn_n_counts(K)]
   // injected draws of the current bnn_mh_steps call (device copies) or null
   const int* inj_proposed;
   const int* inj_count;

@@ -190,7 +190,6 @@ struct UpdLoop {
   int* didx_sm;               // [2][UPD_DRAW_CAP] draw cache (entry index), one buffer per iteration parity -- k_mh_update
   double* ddz_sm;             // [2][UPD_DRAW_CAP] draw cache (increment)      keeps a single one in static shared memory
   int* pk_sm;                 // [P] per canonical entry: layer << 24 | offset in the packed set (filled when `first`)
-  int pp_mode;                // pre-proposal: 0 off, 1 scalar draws, 2 scalar draws + the proposal's draws
   bool first, last;
 };
 
@@ -281,7 +280,7 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
       for (int i = tid; i < g.P; i += NT) { gwc[i] = wc[i]; gwn[i] = wn[i]; }
     }
   };
-  const int NC = 2 + 2 * g.K;
+  const int NC = bnn_n_counts(g.K);
   const int P0 = g.l[0].out * (g.l[0].in + g.l[0].bias);      // size of the first weight matrix (indicator shape)
   // The free-running generator's scalar draws of iteration it_x (layer choice, accept uniform, indicator / slope
   // moves) are independent Philox blocks: the lanes of warp 0 evaluate them side by side, thread 0 consumes them.
@@ -373,7 +372,7 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
       upd_sync<COH>();
       if (can) {
         const int nd = s_off_n[g.L - 1] + s_cnt_n[g.L - 1];
-        if (nd <= UPD_DRAW_CAP && lp_ctx.pp_mode >= 2) {
+        if (nd <= UPD_DRAW_CAP) {
           int* di = didx_base + (itn & 1) * UPD_DRAW_CAP;
           double* dd = ddz_base + (itn & 1) * UPD_DRAW_CAP;
 #pragma unroll 1

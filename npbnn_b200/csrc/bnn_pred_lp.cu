@@ -275,12 +275,7 @@ template <int ACT, int PASSES>
 cudaError_t launch_lp(const FwdParams& p, int n_sms, cudaStream_t st) {
   auto kern = k_pred_tf32x3<ACT, PASSES>;
   const size_t bytes = 2 * (size_t)PBF * sizeof(double);
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) return e;
-    attr_done = true;
-  }
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, (int)bytes)) return e;
   {
     const long long n_pairs = (long long)p.C * PBF / 2;
     k_split_w_tf32<<<(unsigned)((n_pairs + 255) / 256), 256, 0, st>>>(const_cast<double*>(p.wp), n_pairs);
@@ -304,18 +299,8 @@ cudaError_t bnn_launch_pred_tf32(const FwdParams& p, int n_sms, int passes, cuda
   static const char* const names[2][4] = {{"k_pred_tf32x3<relu>", "k_pred_tf32x3<leaky>", "k_pred_tf32x3<swish>", "k_pred_tf32x3<tanh>"},
                                           {"k_pred_tf32x1<relu>", "k_pred_tf32x1<leaky>", "k_pred_tf32x1<swish>", "k_pred_tf32x1<tanh>"}};
   if (which) *which = names[passes == 1][p.g.act];
-  if (passes == 1) {
-    switch (p.g.act) {
-      case BNN_ACT_RELU: return launch_lp<BNN_ACT_RELU, 1>(p, n_sms, st);
-      case BNN_ACT_LEAKY: return launch_lp<BNN_ACT_LEAKY, 1>(p, n_sms, st);
-      case BNN_ACT_SWISH: return launch_lp<BNN_ACT_SWISH, 1>(p, n_sms, st);
-      default: return launch_lp<BNN_ACT_TANH, 1>(p, n_sms, st);
-    }
-  }
-  switch (p.g.act) {
-    case BNN_ACT_RELU: return launch_lp<BNN_ACT_RELU, 3>(p, n_sms, st);
-    case BNN_ACT_LEAKY: return launch_lp<BNN_ACT_LEAKY, 3>(p, n_sms, st);
-    case BNN_ACT_SWISH: return launch_lp<BNN_ACT_SWISH, 3>(p, n_sms, st);
-    default: return launch_lp<BNN_ACT_TANH, 3>(p, n_sms, st);
-  }
+  return bnn_with_act(p.g.act, [&](auto a) {
+    constexpr int ACT = decltype(a)::value;
+    return passes == 1 ? launch_lp<ACT, 1>(p, n_sms, st) : launch_lp<ACT, 3>(p, n_sms, st);
+  });
 }
