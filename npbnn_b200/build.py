@@ -9,7 +9,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnpbnn_b200.so")
-SOURCES = ["bnn_forward.cu", "bnn_mcmc.cu", "bnn_chainloop.cu", "bnn_pred_lp.cu", "bnn_capi.cu"]
+SOURCES = ["bnn_forward.cu", "bnn_sparse.cu", "bnn_mcmc.cu", "bnn_chainloop.cu", "bnn_pred_lp.cu", "bnn_capi.cu"]
 HEADERS = ["bnn_common.cuh", "bnn_kernels.h", "bnn_mh_body.cuh", "bnn_generic_body.cuh", os.path.join("..", "..", "include", "npbnn_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

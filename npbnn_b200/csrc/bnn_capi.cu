@@ -95,11 +95,8 @@ struct bnn_ctx {
   size_t inj_host_bytes = 0;
   cudaEvent_t inj_copied = nullptr;   // the last transfer out of inj_host
   const char* last_kernel = "";
-  // block-masked networks: dataflow program of the chains' mask (k_fwd_sparse)
-  DevBuf sp_items, sp_widx;
-  int sp_prog_len = 0, sp_n_items = 0, sp_slots = 1, sp_wlen = 0;
-  int sp_pair_nc1 = 0, sp_pair_nr1 = 0, sp_pair_nr2 = 0;   // uniform block pairs (k_fwd_sparse's fused path); nc1 == 0: none
-  bool use_sparse = false;
+  // block-masked networks: dataflow program of the chains' mask (bnn_sparse.cu); sp.prog null: the dense kernels run
+  struct { DevBuf prog, widx; SparseParams sp{}; } sparse;
   int opt_sparse = 1;               // option "sparse": 0 forces the dense kernels for masked chains
   // optional per-launch timing of the forward kernel (bench.py roofline): event pairs on the launch stream
   int time_forward = 0;
@@ -578,167 +575,6 @@ int bnn_log_prior_entries(bnn_ctx* c, const double* w_dev, int32_t n_sets, int32
   return 0;
 }
 
-// Dataflow program of a block-masked network for k_fwd_sparse (format: bnn_forward.cu).
-// Per hidden layer, consecutive rows whose kept columns span the same range [c0, c0+nc) form a block
-// (create_mask, BNN_lib.py:16-47 produces exactly such blocks); blocks are cut into items of at most 4 rows.
-// Columns inside the range that the mask drops are harmless (their weights are exactly zero).  Items are
-// emitted in dependency order starting from the last hidden layer, each unit of an earlier layer gets a
-// scratch slot that is released after its last reader.  The output layer is evaluated densely.
-// Returns false when the cover is not worth it (more than a quarter of the dense work).
-namespace {
-struct SpItem { int r0, nr, c0, nc; };
-}
-static bool build_sparse_program(bnn_ctx* c, const double* mask_host, std::vector<int>& prog, std::vector<int>& widx) {
-  const NetGeom& g = c->g;
-  const int US = 33;                            // SP_US of bnn_forward.cu
-  prog.clear();
-  widx.clear();
-  c->sp_n_items = 0;
-  c->sp_slots = 1;
-  if (g.L < 2 || g.O > 8) return false;
-  const int H = g.L - 1;                        // hidden layers
-  const LayerGeom& lo = g.l[H];
-  const int op = (lo.out + 1) & ~1;
-  std::vector<std::vector<SpItem>> items(H);
-  std::vector<std::vector<int>> unit_item(H), readers(H), slot(H);
-  long long sp = 0, dense = 0;
-  for (int l = 0; l < g.L; ++l) dense += (long long)g.l[l].out * g.l[l].in;
-  for (int l = 0; l < H; ++l) {
-    const LayerGeom& lg = g.l[l];
-    const int cols = lg.in + lg.bias;
-    auto range_of = [&](int row, int& c0, int& nc) {
-      int lo_ = -1, hi = -1;
-      for (int k = 0; k < lg.in; ++k)
-        if (mask_host[lg.c_off + row * cols + lg.bias + k] != 0.0) { if (lo_ < 0) lo_ = k; hi = k; }
-      c0 = lo_ < 0 ? 0 : lo_;
-      nc = lo_ < 0 ? 0 : hi - lo_ + 1;
-    };
-    unit_item[l].assign(lg.out, -1);
-    readers[l].assign(lg.out, 0);
-    slot[l].assign(lg.out, -1);
-    int r = 0;
-    while (r < lg.out) {
-      int c0, nc;
-      range_of(r, c0, nc);
-      int r1 = r + 1;
-      while (r1 < lg.out) {
-        int d0, dn;
-        range_of(r1, d0, dn);
-        if (d0 != c0 || dn != nc) break;
-        ++r1;
-      }
-      for (int q = r; q < r1; q += 4) {
-        const int nr = (r1 - q < 4) ? r1 - q : 4;
-        for (int i = 0; i < nr; ++i) unit_item[l][q + i] = (int)items[l].size();
-        items[l].push_back({q, nr, c0, nc});
-        sp += (long long)nr * nc;
-      }
-      r = r1;
-    }
-    if (l > 0)
-      for (const SpItem& it : items[l])
-        for (int k = 0; k < it.nc; ++k) readers[l - 1][it.c0 + k]++;
-  }
-  sp += (long long)lo.out * lo.in;
-  if (sp * 4 > dense) return false;
-
-  // weight stream starts with the output-layer bias (8 entries)
-  for (int o = 0; o < 8; ++o) widx.push_back(o < lo.out ? lo.b_off + o : -1);
-
-  std::vector<std::vector<char>> done(H);
-  for (int l = 0; l < H; ++l) done[l].assign(items[l].size(), 0);
-  std::vector<int> free_slots;                  // released slots, reused lowest first
-  int n_slots = 0;
-  auto take_slot = [&]() {
-    if (free_slots.empty()) return n_slots++;
-    size_t best = 0;
-    for (size_t i = 1; i < free_slots.size(); ++i) if (free_slots[i] < free_slots[best]) best = i;
-    int v = free_slots[best];
-    free_slots.erase(free_slots.begin() + best);
-    return v;
-  };
-  // explicit stack instead of recursion: (layer, item, next column to check)
-  struct Frame { int l, idx, k; };
-  for (size_t top = 0; top < items[H - 1].size(); ++top) {
-    std::vector<Frame> st{{H - 1, (int)top, 0}};
-    while (!st.empty()) {
-      Frame& f = st.back();
-      const SpItem it = items[f.l][f.idx];
-      if (done[f.l][f.idx]) { st.pop_back(); continue; }
-      bool pushed = false;
-      if (f.l > 0) {
-        for (; f.k < it.nc; ++f.k) {
-          const int prod = unit_item[f.l - 1][it.c0 + f.k];
-          if (!done[f.l - 1][prod]) { st.push_back({f.l - 1, prod, 0}); pushed = true; break; }
-        }
-      }
-      if (pushed) continue;
-      // emit the item: program entry ...
-      const int l = f.l, idx = f.idx;
-      const LayerGeom& lg = g.l[l];
-      const bool to_out = (l == H - 1);
-      prog.push_back(l | (it.nr << 8) | (to_out ? (1 << 16) : 0));
-      prog.push_back(it.nc);
-      prog.push_back(l > 0 ? 1 : 0);
-      prog.push_back(0);
-      for (int i = 0; i < 4; ++i) {
-        int off = 0;
-        if (!to_out && i < it.nr) {
-          const int s = take_slot();
-          slot[l][it.r0 + i] = s;
-          off = (g.F + s) * US;
-        }
-        prog.push_back(off);
-      }
-      for (int k = 0; k < it.nc; ++k)
-        prog.push_back(l == 0 ? (it.c0 + k) * US : (g.F + slot[l - 1][it.c0 + k]) * US);
-      while (prog.size() % 4) prog.push_back(0);
-      // ... and its weights in consumption order
-      const int nrp = (it.nr + 1) & ~1;
-      for (int i = 0; i < nrp; ++i) widx.push_back(i < it.nr ? lg.b_off + it.r0 + i : -1);
-      for (int k = 0; k < it.nc; ++k)
-        for (int i = 0; i < nrp; ++i) {
-          const int r = it.r0 + i, cc = it.c0 + k;
-          widx.push_back(i < it.nr ? lg.w_off + r * lg.stride + (cc ^ ((r & 1) * lg.swz)) : -1);
-        }
-      if (to_out)
-        for (int i = 0; i < it.nr; ++i)
-          for (int o = 0; o < op; ++o) {
-            const int u = it.r0 + i;
-            widx.push_back(o < lo.out ? lo.w_off + o * lo.stride + (u ^ ((o & 1) * lo.swz)) : -1);
-          }
-      if (l > 0)
-        for (int k = 0; k < it.nc; ++k)
-          if (--readers[l - 1][it.c0 + k] == 0) free_slots.push_back(slot[l - 1][it.c0 + k]);
-      done[l][idx] = 1;
-      c->sp_n_items++;
-      st.pop_back();
-    }
-  }
-  c->sp_slots = n_slots < 1 ? 1 : n_slots;
-  // Uniform block pairs: two hidden layers, and the program is (first-layer item, the second-layer item that reads
-  // exactly its units) repeated with the same shape -- then k_fwd_sparse keeps the hidden units in registers.
-  c->sp_pair_nc1 = c->sp_pair_nr1 = c->sp_pair_nr2 = 0;
-  if (H == 2 && c->sp_n_items >= 2 && c->sp_n_items % 2 == 0) {
-    bool uniform = true;
-    int nc1 = 0, nr1 = 0, nr2 = 0;
-    size_t pos = 0;
-    for (int n = 0; n < c->sp_n_items && uniform; n += 2) {
-      const int* a = prog.data() + pos;
-      const int a_nr = (a[0] >> 8) & 0xff, a_nc = a[1];
-      const int* b = a + 8 + ((a_nc + 3) & ~3);
-      const int b_nr = (b[0] >> 8) & 0xff, b_nc = b[1];
-      uniform = (a[0] & 0xff) == 0 && !((a[0] >> 16) & 1) && (b[0] & 0xff) == 1 && ((b[0] >> 16) & 1) && b_nc == a_nr;
-      for (int i = 0; i < a_nr && uniform; ++i) uniform = (b[8 + i] == a[4 + i]);     // reads the slots the first item wrote, in order
-      if (n == 0) { nc1 = a_nc; nr1 = a_nr; nr2 = b_nr; }
-      uniform = uniform && a_nc == nc1 && a_nr == nr1 && b_nr == nr2;
-      pos += 16 + ((a_nc + 3) & ~3) + ((b_nc + 3) & ~3);
-    }
-    if (uniform && nc1 > 0) { c->sp_pair_nc1 = nc1; c->sp_pair_nr1 = nr1; c->sp_pair_nr2 = nr2; }
-  }
-  return true;
-}
-
 static ChainDev chain_dev(bnn_ctx* c) {
   ChainDev d{};
   d.g = c->g;
@@ -782,15 +618,7 @@ static int chains_forward(bnn_ctx* c, cudaStream_t st) {
   const int NC = bnn_n_counts(g.K);
   const int per = sets_per_pass(g);
   FwdParams p = base_params(c);
-  if (c->use_sparse && c->opt_sparse) {
-    p.sp_prog = c->sp_items.as<int>();
-    p.sp_widx = c->sp_widx.as<int>();
-    p.sp_wlen = c->sp_wlen;
-    p.sp_prog_len = c->sp_prog_len;
-    p.sp_n_items = c->sp_n_items;
-    p.sp_slots = c->sp_slots;
-    p.sp_pair_nc1 = c->sp_pair_nc1; p.sp_pair_nr1 = c->sp_pair_nr1; p.sp_pair_nr2 = c->sp_pair_nr2;
-  }
+  if (c->opt_sparse) p.sp = c->sparse.sp;
   for (int s0 = 0; s0 < c->C; s0 += per) {
     const int n = (c->C - s0 < per) ? c->C - s0 : per;
     p.wp = c->wp_prop.as<double>() + (size_t)s0 * g.PB;
@@ -841,27 +669,22 @@ int bnn_chains_init(bnn_ctx* c, int32_t n_chains, const bnn_sampler_config* cfg,
   CUDA_TRY(c->part.ensure(sizeof(double) * (size_t)bnn_n_slots(g) * C * c->n_tiles16, false, st));
   if (c->rowshard) CUDA_TRY(c->part_red.ensure(sizeof(double) * (size_t)C * bnn_n_slots(g), true, st));
   CUDA_TRY(c->part_sl.ensure(sizeof(double) * (size_t)C * bnn_n_slots(g) * 64, false, st));
-  c->use_sparse = false;
+  c->sparse.sp = SparseParams{};
   if (cfg->use_mask) {
     CUDA_TRY(c->mask.ensure(sizeof(double) * g.P, false, st));
     CUDA_TRY(cudaMemcpyAsync(c->mask.p, mask_host, sizeof(double) * g.P, cudaMemcpyHostToDevice, st));
     // block-sparse forward: only when the cover is thin and the initial weights respect the mask (the
     // reference applies the mask at construction, BNN_env.py:259-267; proposals are masked in k_mh_update)
-    std::vector<int> items, widx;
-    bool ok = build_sparse_program(c, mask_host, items, widx);
+    SparseProgram sp;
+    bool ok = bnn_sparse_build(g, mask_host, &sp);
     for (size_t i = 0; ok && i < (size_t)C * g.P; ++i)
       if (mask_host[i % g.P] == 0.0 && w0_host[i] != 0.0) ok = false;
     if (ok) {
-      FwdParams probe{};
-      probe.g = g; probe.sp_slots = c->sp_slots; probe.sp_prog_len = (int)items.size(); probe.sp_wlen = (int)widx.size();
-      ok = bnn_sparse_fits(probe);
-    }
-    if (ok) {
-      if (upload(c->sp_items, items.data(), items.size(), st)) return 1;
-      if (upload(c->sp_widx, widx.data(), widx.size(), st)) return 1;
-      c->sp_prog_len = (int)items.size();
-      c->sp_wlen = (int)widx.size();
-      c->use_sparse = true;
+      if (upload(c->sparse.prog, sp.prog.data(), sp.prog.size(), st)) return 1;
+      if (upload(c->sparse.widx, sp.widx.data(), sp.widx.size(), st)) return 1;
+      c->sparse.sp = sp.sp;
+      c->sparse.sp.prog = c->sparse.prog.as<int>();
+      c->sparse.sp.widx = c->sparse.widx.as<int>();
     }
   }
   CUDA_TRY(cudaMemcpyAsync(c->w_cur.p, w0_host, sizeof(double) * (size_t)C * g.P, cudaMemcpyHostToDevice, st));
@@ -1032,7 +855,7 @@ int bnn_mh_steps(bnn_ctx* c, int32_t n_steps, const bnn_injection* inj, void* st
   // Small data sets (a few thousand rows, <= 2048 weights, dense generic forward path): all n_steps iterations run
   // inside ONE persistent launch, a thread-block cluster per chain (bnn_chainloop.cu) -- injected or device-generated
   // proposals alike.  Same update / forward bodies and reduction order as the launch sequence below: identical chains.
-  if (c->opt_chain_loop && !c->time_forward && !(c->use_sparse && c->opt_sparse) &&
+  if (c->opt_chain_loop && !c->time_forward && !(c->sparse.sp.prog && c->opt_sparse) &&
       (c->force_generic || !bnn_fwd3_family(c->g)) && !bnn_part_slices(c->n_tiles16) &&
       bnn_chain_loop_fits(c->g, d.NF, d.n_tiles16, c->C, c->n_sms, c->opt_chain_cluster, c->opt_chain_loop)) {
     FwdParams p = base_params(c);

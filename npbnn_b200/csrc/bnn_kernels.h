@@ -1,6 +1,7 @@
 // Internal interface between the kernel translation units and the C-ABI layer (bnn_capi.cu).
 #pragma once
 #include <type_traits>
+#include <vector>
 #include "bnn_common.cuh"
 
 // Most dynamic shared memory a block of sm_100 may opt in to (227 KB).
@@ -72,7 +73,15 @@ struct ChainDev {
 
 cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int force_generic, cudaStream_t st,
                                const char** which);
-bool bnn_sparse_fits(const FwdParams& p);
+// Block-masked networks (bnn_sparse.cu).  bnn_sparse_build writes the dataflow program of `mask` and its FwdParams::sp
+// (device pointers null) to *out; false: the dense kernels run instead (the block cover is not thin enough, or the
+// program does not fit the kernels' shared memory).  bnn_launch_sparse runs the program in p.sp; *which = its kernel.
+struct SparseProgram {
+  std::vector<int> prog, widx;    // program ints, weight-index stream
+  SparseParams sp;
+};
+bool bnn_sparse_build(const NetGeom& g, const double* mask, SparseProgram* out);
+cudaError_t bnn_launch_sparse(const FwdParams& p, int n_sms, cudaStream_t st, const char** which);
 // opt-in reduced-precision posterior prediction (bnn_pred_lp.cu): 3xTF32 tensor-core contractions, FP32 activations /
 // softmax, FP64 accumulation over the samples; summaries of the 64-64-32-16 categorical family only
 bool bnn_pred_tf32_fits(const FwdParams& p);
