@@ -249,6 +249,15 @@ int bnn_chains_write(bnn_ctx* ctx, const double* f64_host, const int32_t* i32_ho
  * (npBNN.sample_prior_scale, BNN_env.py:196-219; GibbsSampleNormStdGamma*, BNN_mcmc.py:124-141).  The proposals of
  * the following bnn_mh_steps are scored with these scales. */
 int bnn_chains_set_prior_scales(bnn_ctx* ctx, const double* entry_scale_host, void* stream);
+/* The additional_prob argument of mh_step (BNN_env.py:381,481) for chains whose proposals are drawn on the device
+ * (host [C], finite; synchronises the stream).  Every following proposal of chain c adds per_chain_host[c] to its
+ * log-prior, with the Exp(10) term of trainable activation parameters on top, until the next call.  Injected steps read
+ * it too: a bnn_injection that carries add_prob takes precedence for its steps, one without add_prob (NULL) uses this
+ * value, as free-running steps do.  The value lives in a buffer of the context whose address is
+ * fixed from the first call after bnn_chains_init on, so a change reaches the captured graphs of bnn_mh_steps (the
+ * copy runs in stream order before their next replay).  NULL, and never calling this, mean 0 for every chain.
+ * bnn_chains_init clears it. */
+int bnn_chains_set_additional_prob(bnn_ctx* ctx, const double* per_chain_host, void* stream);
 /* Device pointers to the live chain state (same layout as bnn_chains_read; e.g. the log-posteriors for
  * the MC3 all-gather are f64_dev[c * BNN_F_STRIDE + BNN_F_LOGPOST]).  Any pointer may be NULL. */
 int bnn_chains_state_dev(bnn_ctx* ctx, double** f64_dev, int32_t** i32_dev, double** w_dev);

@@ -80,6 +80,7 @@ _SIGNATURES = {
     "bnn_chains_read_indicators": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_write": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_set_prior_scales": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bnn_chains_set_additional_prob": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_init": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(SamplerConfig), C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_mh_steps": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(Injection), C.c_void_p]),

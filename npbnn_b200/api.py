@@ -23,8 +23,10 @@ log-likelihood differs in the last bits because of the summation order).  `rng="
 proposals on the device and never leaves it between logging points.
 
 Trainable activation parameters (ActFun(trainable=True)), init_additional_prob, mh_step(additional_prob=), weight
-indicators (freq_indicator > 0) and feature indicators (feature_indicators=True) run on the device from host-drawn
-numbers (rng="host"); hyper-prior scales (hyper_p) are drawn on the host and evaluated on the device.
+indicators (freq_indicator > 0) and feature indicators (feature_indicators=True) run on the device with either source of
+random numbers; hyper-prior scales (hyper_p) are drawn on the host and evaluated on the device.  With rng="philox",
+mh_step(additional_prob=a) copies a into the chain's device value when it changes (bnn_chains_set_additional_prob).
+MC3 runs trainable activation parameters in every chain, on every rank layout.
 
 estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
 MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
@@ -32,7 +34,8 @@ companion MSE.  Options of the reference that are not on the device path raise
 NotImplementedError: other user-supplied likelihood / proposal / output functions (gamma_likelihood among them),
 MCMC(row_shard=True) with a count likelihood outside an initialised torch.distributed process group, MC3 with
 more ranks than chains (row-sharded chain blocks) together with host-drawn weight or feature indicators (rng="host" and
-freq_indicator > 0 or feature_indicators=True), and the regression error-parameter proposal (estimate_error with
+freq_indicator > 0 or feature_indicators=True), init_additional_prob inside an MC3 group (the reference's MC3 never
+passes it, BNN_mc3.py:61-75), and the regression error-parameter proposal (estimate_error with
 empirical_error=False once the iteration passes `_estimate_error` -- a branch on which the reference itself raises
 AttributeError as soon as one proposal has been accepted before that iteration, BNN_mcmc.py:105).
 """
@@ -556,9 +559,11 @@ class MCMC:
                                  likelihood_tempering, adapt_f, adapt_fM, adapt_freq, self._adapt_stop, sample_from_prior,
                                  seed=int(bnn_obj._seed) + 7919 * int(mcmc_id), device=device,
                                  init_additional_prob=init_additional_prob, row_shard=shard, lik=count_kind)
-        elif bnn_obj._act_fun._trainable or init_additional_prob:
-            raise NotImplementedError("trainable activation parameters / init_additional_prob inside an MC3 group")
+        elif init_additional_prob:
+            # the reference's MC3 builds its chains without it (BNN_mc3.py:61-75)
+            raise NotImplementedError("init_additional_prob inside an MC3 group")
         self._group, self._slot = _group, _slot
+        self._dev_add_prob = 0.0          # additional_prob the device holds for rng="philox" (set_additional_prob)
         self._seen_version = bnn_obj.__dict__.get("_data_version", 0)
         self._bnn_shapes = [w.shape for w in bnn_obj._w_layers]
         # the function attributes user scripts call on host tables (bnn_regress.py:55: mcmc._accuracy_lab_f(mcmc._y, ...))
@@ -677,11 +682,11 @@ class MCMC:
         if bnn_obj.__dict__.get("_data_version", 0) != self._seen_version:
             raise RuntimeError("npBNN.update_data / reset_weights was called after this MCMC staged the model on the device; "
                                "construct a new MCMC (the device state would silently ignore the change)")
-        if additional_prob and self._rng_mode == "philox":
-            raise NotImplementedError("additional_prob is injected with the host-drawn numbers (rng='host')")
         g = self._group
         if not self._own_group:
             raise RuntimeError("this MCMC belongs to an MC3 group; step the group instead")
+        if self._rng_mode == "philox":
+            self._set_device_additional_prob(additional_prob)
         done = 0
         while done < n_steps:
             if self._rng_mode == "philox":
@@ -700,6 +705,13 @@ class MCMC:
                 g.eng.mh_steps(k, inj)
                 done += k
         self._sync(bnn_obj, g.eng.read_state())
+
+    def _set_device_additional_prob(self, a):
+        """Device-drawn proposals read additional_prob from the chain's device value: copy it there when it changes."""
+        a = float(a)
+        if a != self._dev_add_prob:
+            self._group.eng.set_additional_prob([a])
+            self._dev_add_prob = a
 
     def mh_step(self, bnn_obj, additional_prob=0, return_bnn=False):
         self.run(bnn_obj, 1, additional_prob)
@@ -812,6 +824,7 @@ def _run_mcmc_pipelined(bnn, mcmc, logger, depth):
     the same files as the synchronous loop."""
     from collections import deque
     eng = mcmc._group.eng
+    mcmc._set_device_additional_prob(0)      # the loop's mh_step passes none (BNN_mcmc.py:153-170)
     it = mcmc._current_iteration
     pending, free = deque(), list(range(depth))
     if hasattr(logger, "begin_async"):

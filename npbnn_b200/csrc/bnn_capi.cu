@@ -82,6 +82,11 @@ struct bnn_ctx {
   DevBuf ind_cur, ind_prop, fi_cur, fi_prop, feat_mean, inj_ind_move, inj_ind_flip, inj_fi_move, inj_fi_flip;   // indicators
   bool have_feat_mean = false;
   bool have_ps_entry = false;
+  // additional_prob of free-running chains (bnn_chains_set_additional_prob): [C], read by the proposal step when no
+  // injection carries one.  Allocated by the first set after bnn_chains_init and kept at that address, so that captured
+  // graphs see a new value through the copy into it.
+  DevBuf add_prob;
+  bool have_add_prob = false;
   // row sharding: the chains' accept step reads the all-reduced sums from part_red (one pseudo tile)
   bool rowshard = false;
   long long n_train_global = 0;
@@ -600,6 +605,7 @@ static ChainDev chain_dev(bnn_ctx* c) {
   d.NF = bnn_n_slots(c->g);
   d.counts_prop = c->counts_prop.as<int>();
   d.alpha_fwd = c->alpha_chain.as<double>();
+  d.add_prob = c->have_add_prob ? c->add_prob.as<double>() : nullptr;
   if (const int ns = bnn_part_slices(c->n_tiles16)) {     // chains_forward folds the tile partials into ns slices per chain
     d.part = c->part_sl.as<double>();
     d.n_tiles16 = ns;
@@ -653,6 +659,7 @@ int bnn_chains_init(bnn_ctx* c, int32_t n_chains, const bnn_sampler_config* cfg,
   const int C = n_chains, NC = bnn_n_counts(g.K);
   c->C = C;
   c->have_ps_entry = false;          // per-entry prior scales belong to the previous set of chains
+  c->have_add_prob = false;          // and so does their additional_prob
   for (auto& sn : c->snaps) sn.pending = false;
   c->cfg = *cfg;
   fill_prior_scales(c->ps, cfg->prior_scale, g.L);
@@ -1104,6 +1111,29 @@ int bnn_chains_set_prior_scales(bnn_ctx* c, const double* entry_scale_host, void
   ChainDev d = chain_dev(c);
   CUDA_TRY(bnn_launch_prior_refresh(d, st));
   c->launches++;
+  return 0;
+}
+
+int bnn_chains_set_additional_prob(bnn_ctx* c, const double* per_chain_host, void* stream) {
+  REQUIRE(c && c->have_chains, "bnn_chains_set_additional_prob: call bnn_chains_init first");
+  CUDA_TRY(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (!per_chain_host) {
+    if (c->have_add_prob) invalidate_graphs(c);      // the captured sequences read the buffer
+    c->have_add_prob = false;
+    return 0;
+  }
+  for (int ch = 0; ch < c->C; ++ch)
+    REQUIRE(std::isfinite(per_chain_host[ch]), "bnn_chains_set_additional_prob: values must be finite");
+  if (!c->have_add_prob) {
+    // the first value after bnn_chains_init: the proposal step starts reading the buffer, the captured sequences did not
+    invalidate_graphs(c);
+    CUDA_TRY(c->add_prob.ensure(sizeof(double) * (size_t)c->C, false, st));
+  }
+  // in stream order: the steps queued before this call use the old value, the ones after it (a graph replay too) the new
+  CUDA_TRY(cudaMemcpyAsync(c->add_prob.p, per_chain_host, sizeof(double) * (size_t)c->C, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaStreamSynchronize(st));   // the caller's array is free on return
+  c->have_add_prob = true;
   return 0;
 }
 

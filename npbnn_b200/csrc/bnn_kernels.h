@@ -69,6 +69,9 @@ struct ChainDev {
   const uint8_t* inj_ind_flip;
   const int* inj_fi_move;
   const uint8_t* inj_fi_flip;
+  // additional_prob of every chain when no injection carries one ([C], bnn_chains_set_additional_prob) or null (0).
+  // Appended, so that the offsets of the fields above stay those of the kernels that do not read it.
+  const double* add_prob;
 };
 
 cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int force_generic, cudaStream_t st,

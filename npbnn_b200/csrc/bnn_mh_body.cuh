@@ -527,8 +527,9 @@ __device__ void mh_update_body(const ChainDev& d, const int c, int accept_mode, 
 #pragma unroll 1
       for (int l = 0; l < g.L; ++l) si[BNN_I_PROPOSED + l] = s_prop[l];
       // trainable activation parameters (BNN_env.py:416-421): UpdateNormal1D(_acc_prm, d=0.05, n=1, Mb=1, mb=0) with
-      // the injected draw, both reflections over every entry (BNN_mcmc.py:46-56), Exp(10) term into additional_prob
-      double addp = d.inj_add_prob ? d.inj_add_prob[(long long)step * d.C + c] : 0.0;
+      // the injected draw, both reflections over every entry (BNN_mcmc.py:46-56), Exp(10) term into additional_prob.
+      // additional_prob itself: the injected value of this step, else the chain's device value, else 0
+      double addp = d.inj_add_prob ? d.inj_add_prob[(long long)step * d.C + c] : (d.add_prob ? d.add_prob[c] : 0.0);
 #pragma unroll 1
       for (int l = 0; l < g.L; ++l) sf[BNN_F_ALPHA_PROP + l] = sf[BNN_F_ALPHA + l];
       if (d.cfg.n_act_prm > 0 && (d.inj_alpha_ix || !d.inj_proposed)) {

@@ -421,6 +421,13 @@ class Engine:
             assert e.shape == (self.n_chains, self.net.n_params), e.shape
         L.check(self.lib.bnn_chains_set_prior_scales(self._h, _np_ptr(e), self._stream()))
 
+    def set_additional_prob(self, values):
+        """additional_prob [C] of the chains' device-drawn proposals (bnn_chains_set_additional_prob); None: 0."""
+        a = None
+        if values is not None:
+            a = np.ascontiguousarray(np.broadcast_to(np.asarray(values, dtype=np.float64), (self.n_chains,)))
+        L.check(self.lib.bnn_chains_set_additional_prob(self._h, _np_ptr(a), self._stream()))
+
     def set_temperature(self, temps):
         t = np.ascontiguousarray(temps, dtype=np.float64)
         assert t.shape == (self.n_chains,)
