@@ -233,12 +233,23 @@ int bnn_chains_read(bnn_ctx* ctx, double* f64_host, int32_t* i32_host, double* w
 int bnn_chains_snapshot(bnn_ctx* ctx, int32_t slot, void* stream);
 int bnn_snapshot_ready(bnn_ctx* ctx, int32_t slot);
 int bnn_snapshot_read(bnn_ctx* ctx, int32_t slot, double* f64_host, int32_t* i32_host, double* w_host);
+/* The indicators the same snapshot holds for chains that carry them (layouts of bnn_chains_read_indicators; either may
+ * be NULL): waits for the slot and copies them out without freeing it, so call it before bnn_snapshot_read.  A snapshot
+ * is one iteration's state, indicators included, however many steps were queued behind it. */
+int bnn_snapshot_read_indicators(bnn_ctx* ctx, int32_t slot, double* ind_host, double* fi_host);
 /* Training means of the features (host [n_features]) for the feature-indicator transform; call before
  * bnn_chains_init with cfg.use_feature_indicators. */
 int bnn_set_feature_means(bnn_ctx* ctx, const double* mean_host, void* stream);
 /* Current indicators of every chain: ind_host [C, size of the first weight matrix], fi_host [C, n_features]
  * (doubles 0/1; either may be NULL; synchronises). */
 int bnn_chains_read_indicators(bnn_ctx* ctx, double* ind_host, double* fi_host, void* stream);
+/* The counterpart: set the current indicators of every chain (same layouts, values 0 or 1; either may be NULL;
+ * synchronises) and score the chains' current weights under them as bnn_chains_init scores w0 -- logLik, logPrior with
+ * the indicator term, logPost and the accuracy counters of the initial state.  So it starts chains from indicators that
+ * are not all ones (npBNN._indicators / _feature_indicators set before MCMC.__init__), and it is the indicator step of
+ * restoring a saved chain, which ends with bnn_chains_write of the saved state.  Drops the captured graphs of
+ * bnn_mh_steps.  Row-sharded chains stop before the accept step, as bnn_chains_init does. */
+int bnn_chains_write_indicators(bnn_ctx* ctx, const double* ind_host, const double* fi_host, void* stream);
 /* Write the state arrays back (same layout as bnn_chains_read; synchronises the stream): the host edits what it
  * read -- MCMC.reset_update_n / reset_update_f / reset_update_ws (BNN_env.py:540-547), the iteration count after
  * a Gibbs step.  Any pointer may be NULL. */

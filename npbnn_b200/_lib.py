@@ -76,8 +76,10 @@ _SIGNATURES = {
     "bnn_chains_snapshot": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "bnn_snapshot_ready": (C.c_int, [C.c_void_p, C.c_int32]),
     "bnn_snapshot_read": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bnn_snapshot_read_indicators": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
     "bnn_set_feature_means": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_read_indicators": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bnn_chains_write_indicators": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_write": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_set_prior_scales": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_chains_set_additional_prob": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -26,7 +26,16 @@ Trainable activation parameters (ActFun(trainable=True)), init_additional_prob, 
 indicators (freq_indicator > 0) and feature indicators (feature_indicators=True) run on the device with either source of
 random numbers; hyper-prior scales (hyper_p) are drawn on the host and evaluated on the device.  With rng="philox",
 mh_step(additional_prob=a) copies a into the chain's device value when it changes (bnn_chains_set_additional_prob).
-MC3 runs trainable activation parameters in every chain, on every rank layout.
+MC3 runs trainable activation parameters in every chain, on every rank layout.  Chains start from the model's
+indicators, all ones or not.
+
+Resuming.  The [bnn, mcmc, logger] pickle that postLogger.log_weights writes carries the chain's device state as of
+the logging point (state rows, indicators, additional_prob, the host generator _rs); load_obj it, raise
+mcmc._n_iterations and run_mcmc(bnn, mcmc, logger) continues the chain bit for bit.  A pickled MC3 continues all its
+chains on the next run_mcmc; the caller restores np.random's state where the run draws from it (swaps of a single-process
+MC3, host-drawn indicator flips).  Not resumable: pickles written before samplers carried their state (RuntimeError: use
+npBNN(pickle_file=)), the cold-chain mcmc that MC3's logger pickles (RuntimeError: resume the MC3 object), and samplers
+run over torch.distributed ranks -- MCMC(row_shard=True) and MC3 with world > 1 (NotImplementedError).
 
 estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
 MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
@@ -43,12 +52,13 @@ import csv
 import os
 import pickle
 from copy import deepcopy
+from types import SimpleNamespace
 
 import numpy as np
 
 from . import _lib as L
 from . import mc3 as _mc3
-from .engine import Engine, NetShape, flatten_weights, unflatten_weights
+from .engine import ChainState, Engine, NetShape, flatten_weights, unflatten_weights
 
 small_number = 1e-10
 
@@ -377,7 +387,9 @@ class _ChainGroup:
 
     def __init__(self, bnn, weights_per_chain, temperatures, update_f, update_ws, lik_temp, adapt_f, adapt_fM,
                  adapt_freq, adapt_stop, sample_from_prior, seed, device=0, init_additional_prob=0.0, row_shard=(1, 0),
-                 row_group=None, chain_offset=0, lik=None):
+                 row_group=None, chain_offset=0, lik=None, saved=None):
+        """saved: one MCMC._chain_state per chain (an unpickled sampler): the chains continue from it instead of
+        starting from the weights as MCMC.__init__ does."""
         self.bnn = bnn
         net = _net_of(weights_per_chain[0], bnn._n_features, bnn._act_fun, bnn._estimation_mode, lik)
         self.net = net
@@ -419,11 +431,29 @@ class _ChainGroup:
                              chain_offset=chain_offset, freq_indicator=float(bnn._freq_indicator))
         self.freq_indicator = float(bnn._freq_indicator)
         self.use_fi = bnn._feature_indicators is not None
-        if (self.freq_indicator or self.use_fi) and (np.any(np.asarray(bnn._indicators) != 1) or
-                                                     (self.use_fi and np.any(np.asarray(bnn._feature_indicators) != 1))):
-            raise NotImplementedError("chains start from all-one indicators (as npBNN.__init__ leaves them)")
         if not per_layer:        # a model that already carries sampled hyper-prior scales
             self.eng.set_prior_scales(np.tile(bnn._entry_scales(), (self.n, 1)))
+        # bnn_chains_init starts every chain from all-one indicators (as npBNN.__init__ leaves them); other values are
+        # written and the weights scored again under them
+        ind = fi = None
+        if saved is not None:
+            ind = np.stack([s["ind"] for s in saved]) if self.freq_indicator else None
+            fi = np.stack([s["fi"] for s in saved]) if self.use_fi else None
+        else:
+            if self.freq_indicator and np.any(np.asarray(bnn._indicators) != 1):
+                ind = np.broadcast_to(np.asarray(bnn._indicators, dtype=np.float64), (self.n,) + tuple(net.shapes[0]))
+            if self.use_fi and np.any(np.asarray(bnn._feature_indicators) != 1):
+                fi = np.broadcast_to(np.asarray(bnn._feature_indicators, dtype=np.float64), (self.n, net.n_features))
+        if ind is not None or fi is not None:
+            self.eng.write_indicators(ind, fi)
+        if saved is not None:
+            add_prob = [s["add_prob"] for s in saved]
+            if any(add_prob):
+                self.eng.set_additional_prob(add_prob)
+            # last: set_prior_scales and write_indicators recompute logPrior without the additional_prob / Exp(10) term
+            # of the last proposal, and the saved values must win
+            self.eng.write_state(ChainState(np.stack([s["f64"] for s in saved]), np.stack([s["i32"] for s in saved]),
+                                            None, net, self.eng.K))
         self.n_act_prm = bnn._act_fun.n_trainable()
         if self.n_act_prm > net.n_layers:
             raise ValueError("more trainable activation parameters than layers")
@@ -550,11 +580,15 @@ class MCMC:
         self._rng_mode = rng
         self._regression_error_proposal = (bnn_obj._estimation_mode == "regression" and not bnn_obj._empirical_error)
         self.update_function = update_function
+        self._dev_add_prob = 0.0          # additional_prob the device holds for rng="philox" (set_additional_prob)
         self._own_group = _group is None
+        self._device = device
+        self._row_sharded = False
         if _group is None:
             shard = (1, 0)
             if row_shard and dist.is_available() and dist.is_initialized():
                 shard = (dist.get_world_size(), dist.get_rank())
+            self._row_sharded = shard[0] > 1
             _group = _ChainGroup(bnn_obj, [bnn_obj._w_layers], [temperature], list(update_f)[:nl], list(update_ws)[:nl],
                                  likelihood_tempering, adapt_f, adapt_fM, adapt_freq, self._adapt_stop, sample_from_prior,
                                  seed=int(bnn_obj._seed) + 7919 * int(mcmc_id), device=device,
@@ -563,7 +597,6 @@ class MCMC:
             # the reference's MC3 builds its chains without it (BNN_mc3.py:61-75)
             raise NotImplementedError("init_additional_prob inside an MC3 group")
         self._group, self._slot = _group, _slot
-        self._dev_add_prob = 0.0          # additional_prob the device holds for rng="philox" (set_additional_prob)
         self._seen_version = bnn_obj.__dict__.get("_data_version", 0)
         self._bnn_shapes = [w.shape for w in bnn_obj._w_layers]
         # the function attributes user scripts call on host tables (bnn_regress.py:55: mcmc._accuracy_lab_f(mcmc._y, ...))
@@ -579,7 +612,8 @@ class MCMC:
         self._sync(bnn_obj, self._group.eng.read_state())
 
     # ---------------------------------------------------------------- state export
-    def _sync(self, bnn_obj, st):
+    def _sync(self, bnn_obj, st, indicators=None):
+        """indicators: (weight, feature) indicators of the same export as st (a snapshot); None reads the live ones."""
         c = self._slot
         g = self._group
         self._logLik = float(st.logLik[c])
@@ -623,12 +657,22 @@ class MCMC:
             bnn_obj._act_fun._prm = np.array(st.alpha_prop[c][:na])         # the last proposal (BNN_env.py:421)
         if st.w is not None:
             bnn_obj._w_layers = st.weights(c)        # fresh arrays: logged samples keep their own copies
+        ind = fi = None
         if g.freq_indicator or g.use_fi:
-            ind, fi = g.eng.read_indicators(weight=bool(g.freq_indicator), feature=g.use_fi)
+            ind, fi = indicators if indicators is not None else \
+                g.eng.read_indicators(weight=bool(g.freq_indicator), feature=g.use_fi)
             if ind is not None:
                 bnn_obj._indicators = ind[c]
             if fi is not None:
                 bnn_obj._feature_indicators = fi[c].astype(int)
+        # what a pickle of this sampler needs to continue the chain (_restage): the raw state rows (accept ring,
+        # counters, update sizes, temperature, slopes, sigma, iteration), the indicators and the device additional_prob.
+        # Fresh arrays and a fresh dict at every sync: the background pickle writer holds shallow copies of earlier ones.
+        self._chain_state = {"f64": np.array(st.f64[c]), "i32": np.array(st.i32[c]),
+                             "ind": None if ind is None else ind[c], "fi": None if fi is None else fi[c],
+                             "add_prob": self._dev_add_prob}
+        # the host generator as of this point: the next slice's draws advance _rs in place before the writer pickles
+        self._rs_state = self._rs.bit_generator.state
         self._bnn_view = bnn_obj
         self._y_cache = {}
 
@@ -678,6 +722,8 @@ class MCMC:
     # ---------------------------------------------------------------- stepping
     def run(self, bnn_obj, n_steps, additional_prob=0):
         """n_steps MH iterations (BNN_env.py:381-532 each) with as few host round trips as the rng mode allows."""
+        if self._group is None:
+            self._restage(bnn_obj)
         self._check_supported(n_steps)
         if bnn_obj.__dict__.get("_data_version", 0) != self._seen_version:
             raise RuntimeError("npBNN.update_data / reset_weights was called after this MCMC staged the model on the device; "
@@ -723,6 +769,8 @@ class MCMC:
         logPrior / logPost of the current weights under them (device) and one iteration counted."""
         if not self._own_group:
             raise RuntimeError("this MCMC belongs to an MC3 group")
+        if self._group is None:
+            self._restage(bnn_obj)
         bnn_obj.sample_prior_scale()
         eng = self._group.eng
         eng.set_prior_scales(bnn_obj._entry_scales()[None, :])
@@ -734,6 +782,14 @@ class MCMC:
     def _edit_state(self, edit):
         if not self._own_group:
             raise RuntimeError("this MCMC belongs to an MC3 group")
+        if self._group is None and "_chain_state" in self.__dict__:
+            # unpickled and not restaged yet: edit the saved rows, which the restaging writes to the device
+            cs = dict(self._chain_state)
+            st = SimpleNamespace(f64=cs["f64"][None].copy(), i32=cs["i32"][None].copy())
+            edit(st)
+            cs["f64"], cs["i32"] = st.f64[0], st.i32[0]
+            self._chain_state = cs
+            return
         eng = self._group.eng
         st = eng.read_state(weights=False)
         edit(st)
@@ -763,17 +819,63 @@ class MCMC:
 
     def reset_temperature(self, temp):
         self._temperature = temp
-        if self._own_group:
+        if self._own_group and self._group is None:
+            self._edit_state(lambda st: st.f64.__setitem__((slice(None), L.F_TEMPERATURE), temp))
+        elif self._own_group:
             self._group.eng.set_temperature([temp])
 
+    # ---------------------------------------------------------------- pickling and resuming
+    # postLogger pickles the live [bnn, mcmc, logger] at every sample (BNN_env.py:658); as in the reference,
+    # load_obj(pkl) -> raise mcmc._n_iterations -> run_mcmc(bnn, mcmc, logger) continues the chain.  The pickle holds no
+    # device handle: the first step of an unpickled sampler stages the model again (_restage) and writes the state saved
+    # at the last sync, so the chain continues bit for bit (device generators are keyed on seed, chain and iteration).
     def __getstate__(self):
         d = dict(self.__dict__)
         d["_group"] = None
-        d["_rs"] = None
         d["update_function"] = None
         d["_bnn_view"] = None
         d["_y_cache"] = {}
+        if "_rs_state" in d:
+            # the host generator travels as its state as of the last sync (the live one may have advanced since) and is
+            # rebuilt on first use (__getattr__): a logging point's shallow copy builds no generator
+            d.pop("_rs", None)
         return d
+
+    def __setstate__(self, d):
+        self.__dict__.update(d)
+        self.update_function = UpdateNormal
+
+    def __getattr__(self, name):
+        # only reached for attributes the instance lacks: _rs of an unpickled sampler
+        if name == "_rs" and "_rs_state" in self.__dict__:
+            rs = np.random.default_rng(0)
+            rs.bit_generator.state = self.__dict__["_rs_state"]
+            self.__dict__["_rs"] = rs
+            return rs
+        raise AttributeError(name)
+
+    def _restage(self, bnn_obj):
+        """Rebuild the device chain of an unpickled sampler from the pickled model (data, weights, mask, prior scales,
+        feature means) and this sampler's settings, then write its saved state (_ChainGroup(saved=))."""
+        if "_chain_state" not in self.__dict__:
+            raise RuntimeError("this MCMC was pickled without its chain state (by a version that could not resume "
+                               "samplers): rebuild it from npBNN(pickle_file=...), which restores the last weights")
+        if not self._own_group:
+            raise RuntimeError("this MCMC is a chain of an MC3 group (the cold chain its logger pickles): unpickle and "
+                               "run the MC3 object to resume the chains")
+        if self._row_sharded:
+            raise NotImplementedError("resuming a row-sharded MCMC is not built: only rank 0 writes the pickle, and it "
+                                      "holds rank 0's own chains alone")
+        cs = self._chain_state
+        nl = bnn_obj._n_layers
+        count_kind = _COUNT_LIK[self._likelihood_f][0] if self._likelihood_f in _COUNT_LIK else None
+        self._group = _ChainGroup(bnn_obj, [bnn_obj._w_layers], [float(cs["f64"][L.F_TEMPERATURE])],
+                                  list(cs["f64"][L.F_UPDATE_F:L.F_UPDATE_F + nl]),
+                                  list(cs["f64"][L.F_UPDATE_WS:L.F_UPDATE_WS + nl]), self._lik_temp, self._adapt_f,
+                                  self._adapt_fM, self._adapt_freq, self._adapt_stop, self._sample_from_prior,
+                                  seed=int(bnn_obj._seed) + 7919 * int(self._mcmc_id), device=self._device,
+                                  lik=count_kind, saved=[cs])
+        self._bnn_view = bnn_obj
 
 
 def _mirror_adaptation(st, c, it, adapt_freq, adapt_stop, adapt_f, adapt_fM, max_n, n_params):
@@ -830,9 +932,14 @@ def _run_mcmc_pipelined(bnn, mcmc, logger, depth):
     if hasattr(logger, "begin_async"):
         logger.begin_async()
 
+    g = mcmc._group
+
     def retire():
         slot = pending.popleft()
-        mcmc._sync(bnn, eng.snapshot_read(slot))
+        # the indicators of the snapshot's iteration: the live ones already belong to the steps queued behind it
+        ind = eng.snapshot_read_indicators(slot, weight=bool(g.freq_indicator), feature=g.use_fi) \
+            if g.freq_indicator or g.use_fi else None
+        mcmc._sync(bnn, eng.snapshot_read(slot), ind)
         free.append(slot)
         _report(bnn, mcmc, logger)
 
@@ -857,7 +964,10 @@ def _run_mcmc_pipelined(bnn, mcmc, logger, depth):
 def run_mcmc(bnn, mcmc, logger, pipeline_depth=4):
     """The driver loop of BNN_mcmc.py:153-170, batched: the device runs up to the next print / sampling /
     final iteration without returning to the host; with device-generated proposals (rng="philox") the logging
-    points are exported asynchronously and the loop never waits for the device (pipeline_depth=0: synchronous)."""
+    points are exported asynchronously and the loop never waits for the device (pipeline_depth=0: synchronous).
+    An unpickled mcmc continues its chain (MCMC._restage)."""
+    if mcmc._group is None:
+        mcmc._restage(bnn)
     if mcmc._rng_mode == "philox" and mcmc._own_group and pipeline_depth > 0 and mcmc._current_iteration < mcmc._n_iterations:
         return _run_mcmc_pipelined(bnn, mcmc, logger, int(pipeline_depth))
     # host-drawn proposals: the loop returns to the host at every logging point anyway, but the pickle of
@@ -945,6 +1055,7 @@ class MC3:
             self._swap_rng = _mc3.SwapRNG(int(self.rseeds[0]) if swap_seed is None else int(swap_seed))
         nl = data._n_layers
         self._bnn = data
+        self._device = device
         self._group = _ChainGroup(data, [data._w_layers] * self.n_local,
                                   self.temperatures[self.start:self.start + self.n_local], [0.05] * nl, [0.075] * nl,
                                   1, adapt_f, adapt_fM, adapt_freq, adapt_stop, 0, seed=int(self.rseeds[0]), device=device,
@@ -1010,6 +1121,8 @@ class MC3:
         # -- after every swap period (BNN_mc3.py:118-122 -> BNN_env.py:658).  As in run_mcmc above the writes go to the
         # logger's background writer (newest snapshot wins, the last one is on disk when this returns) so that the
         # device does not idle while the host pickles: tools/mc3_api_c4.py.
+        if self._group is None:
+            self._restage()
         lg = self.logger if hasattr(self.logger, "begin_async") and self.__dict__.get("async_pickle", True) else None
         if lg is not None:
             lg.begin_async()
@@ -1047,6 +1160,34 @@ class MC3:
                 b0, m0 = self.singleChainArgs[0]
                 print(mc3_it, m0._logPost, b0._w_layers[0][0][0:5])
 
+
+    # A pickled MC3 holds its chain views (each [bnn, mcmc] with its saved state, MCMC._chain_state), the temperatures,
+    # the logger and the swap generator (a seeded SwapRNG pickles its state); the next run_mcmc continues every chain.
+    # A single-process MC3 without swap_seed draws its swaps from numpy's global generator, as the reference does
+    # (GlobalSwapRNG), and so do host-drawn indicator flips: to continue those streams the caller restores np.random's
+    # state (np.random.set_state) before run_mcmc; unpickling neither saves nor touches it.
+    def __getstate__(self):
+        d = dict(self.__dict__)
+        d["_group"] = None
+        d.pop("_cold_view", None)
+        return d
+
+    def _restage(self):
+        """One chain group from the chain views of an unpickled MC3: each view's weights and saved state."""
+        import torch.distributed as dist
+        if self.world > 1 or (dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1):
+            raise NotImplementedError("resuming MC3 over torch.distributed ranks is not built: only rank 0 writes the "
+                                      "pickle, and it holds rank 0's own chains alone")
+        views = self.singleChainArgs
+        m0 = views[0][1]
+        count_kind = _COUNT_LIK[m0._likelihood_f][0] if m0._likelihood_f in _COUNT_LIK else None
+        nl = self._bnn._n_layers
+        self._group = _ChainGroup(self._bnn, [b._w_layers for b, _ in views], [m._temperature for _, m in views],
+                                  [0.05] * nl, [0.075] * nl, 1, self.adapt_f, self.adapt_fM, self.adapt_freq,
+                                  self.adapt_stop, 0, seed=int(self.rseeds[0]), device=self._device,
+                                  chain_offset=self.start, lik=count_kind, saved=[m._chain_state for _, m in views])
+        for b, m in views:
+            m._group, m._bnn_view = self._group, b
 
     def _log_on_rank0(self, cold):
         """Chains sharded over ranks: the cold temperature migrates between ranks with the swaps, the files belong to

@@ -993,8 +993,15 @@ int bnn_chains_read(bnn_ctx* c, double* f64_host, int32_t* i32_host, double* w_h
 }
 
 // ---- asynchronous snapshots (include/npbnn_b200.h) ----------------------------------------------------------
-static size_t snap_bytes(const bnn_ctx* c) {
-  return (size_t)c->C * (sizeof(double) * BNN_F_STRIDE + sizeof(int) * BNN_I_STRIDE + sizeof(double) * c->g.P);
+// a slot holds the f64 rows, the i32 rows, the weights, then the current weight / feature indicators of chains that
+// carry them (doubles; counts returned in n_ind, n_fi)
+static size_t snap_bytes(const bnn_ctx* c, size_t* n_ind = nullptr, size_t* n_fi = nullptr) {
+  const size_t ni = c->cfg.use_indicators ? (size_t)c->C * c->g.l[0].out * (c->g.l[0].in + c->g.l[0].bias) : 0;
+  const size_t nf = c->cfg.use_feature_indicators ? (size_t)c->C * c->g.F : 0;
+  if (n_ind) *n_ind = ni;
+  if (n_fi) *n_fi = nf;
+  return (size_t)c->C * (sizeof(double) * BNN_F_STRIDE + sizeof(int) * BNN_I_STRIDE + sizeof(double) * c->g.P) +
+         sizeof(double) * (ni + nf);
 }
 
 int bnn_chains_snapshot(bnn_ctx* c, int32_t slot, void* stream) {
@@ -1024,6 +1031,12 @@ int bnn_chains_snapshot(bnn_ctx* c, int32_t slot, void* stream) {
   CUDA_TRY(cudaMemcpyAsync(d, c->sf.p, nf, cudaMemcpyDeviceToDevice, st));
   CUDA_TRY(cudaMemcpyAsync(d + nf, c->si.p, ni, cudaMemcpyDeviceToDevice, st));
   CUDA_TRY(cudaMemcpyAsync(d + nf + ni, c->w_cur.p, nw, cudaMemcpyDeviceToDevice, st));
+  size_t n_ind, n_fi;
+  snap_bytes(c, &n_ind, &n_fi);
+  if (n_ind) CUDA_TRY(cudaMemcpyAsync(d + nf + ni + nw, c->ind_cur.p, sizeof(double) * n_ind, cudaMemcpyDeviceToDevice, st));
+  if (n_fi)
+    CUDA_TRY(cudaMemcpyAsync(d + nf + ni + nw + sizeof(double) * n_ind, c->fi_cur.p, sizeof(double) * n_fi,
+                             cudaMemcpyDeviceToDevice, st));
   CUDA_TRY(cudaEventRecord(sn.staged, st));
   // ... device-to-host on the copy stream, off the chains' critical path
   CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, sn.staged, 0));
@@ -1058,6 +1071,22 @@ int bnn_snapshot_read(bnn_ctx* c, int32_t slot, double* f64_host, int32_t* i32_h
   return 0;
 }
 
+int bnn_snapshot_read_indicators(bnn_ctx* c, int32_t slot, double* ind_host, double* fi_host) {
+  REQUIRE(c && slot >= 0 && slot < bnn_ctx::kSnapSlots && c->snaps[slot].pending,
+          "bnn_snapshot_read_indicators: no snapshot pending in this slot");
+  REQUIRE(!ind_host || c->cfg.use_indicators, "bnn_snapshot_read_indicators: the chains have no weight indicators");
+  REQUIRE(!fi_host || c->cfg.use_feature_indicators, "bnn_snapshot_read_indicators: the chains have no feature indicators");
+  CUDA_TRY(cudaSetDevice(c->device));
+  bnn_ctx::Snap& sn = c->snaps[slot];
+  CUDA_TRY(cudaEventSynchronize(sn.done));
+  size_t n_ind, n_fi;
+  const size_t nb = snap_bytes(c, &n_ind, &n_fi);
+  const char* h = static_cast<const char*>(sn.host) + nb - sizeof(double) * (n_ind + n_fi);
+  if (ind_host) memcpy(ind_host, h, sizeof(double) * n_ind);
+  if (fi_host) memcpy(fi_host, h + sizeof(double) * n_ind, sizeof(double) * n_fi);
+  return 0;
+}
+
 int bnn_set_feature_means(bnn_ctx* c, const double* mean_host, void* stream) {
   REQUIRE(c && c->have_net && mean_host, "bnn_set_feature_means: call bnn_set_net first");
   invalidate_graphs(c);
@@ -1083,6 +1112,35 @@ int bnn_chains_read_indicators(bnn_ctx* c, double* ind_host, double* fi_host, vo
     CUDA_TRY(cudaMemcpyAsync(fi_host, c->fi_cur.p, sizeof(double) * (size_t)c->C * c->g.F, cudaMemcpyDeviceToHost, st));
   }
   CUDA_TRY(cudaStreamSynchronize(st));
+  return 0;
+}
+
+int bnn_chains_write_indicators(bnn_ctx* c, const double* ind_host, const double* fi_host, void* stream) {
+  REQUIRE(c && c->have_chains, "bnn_chains_write_indicators: call bnn_chains_init first");
+  REQUIRE(!ind_host || c->cfg.use_indicators, "bnn_chains_write_indicators: the chains have no weight indicators");
+  REQUIRE(!fi_host || c->cfg.use_feature_indicators, "bnn_chains_write_indicators: the chains have no feature indicators");
+  const NetGeom& g = c->g;
+  const size_t P0 = (size_t)g.l[0].out * (g.l[0].in + g.l[0].bias);
+  for (size_t i = 0; ind_host && i < (size_t)c->C * P0; ++i)
+    REQUIRE(ind_host[i] == 0.0 || ind_host[i] == 1.0, "bnn_chains_write_indicators: weight indicators must be 0 or 1");
+  for (size_t i = 0; fi_host && i < (size_t)c->C * g.F; ++i)
+    REQUIRE(fi_host[i] == 0.0 || fi_host[i] == 1.0, "bnn_chains_write_indicators: feature indicators must be 0 or 1");
+  if (!ind_host && !fi_host) return 0;
+  invalidate_graphs(c);              // the captured sequences read the indicators
+  CUDA_TRY(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (ind_host) CUDA_TRY(cudaMemcpyAsync(c->ind_cur.p, ind_host, sizeof(double) * (size_t)c->C * P0, cudaMemcpyHostToDevice, st));
+  if (fi_host) CUDA_TRY(cudaMemcpyAsync(c->fi_cur.p, fi_host, sizeof(double) * (size_t)c->C * g.F, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(cudaStreamSynchronize(st));   // the caller's arrays are free on return
+  // the current weights are scored again under the new indicators, as bnn_chains_init scores w0 (the proposal step
+  // copies ind_cur / fi_cur into the proposal buffers)
+  ChainDev d = chain_dev(c);
+  CUDA_TRY(bnn_launch_mh_update(d, 0, 2, 0, st));
+  c->launches++;
+  if (int rc = chains_forward(c, st)) return rc;
+  if (c->rowshard) return 0;          // the caller reduces over the ranks first, then bnn_rowshard_update(accept = 2)
+  CUDA_TRY(bnn_launch_mh_update(d, 2, 0, 0, st));
+  c->launches++;
   return 0;
 }
 

@@ -396,6 +396,15 @@ class Engine:
         L.check(self.lib.bnn_snapshot_read(self._h, int(slot), _np_ptr(f64), _np_ptr(i32), _np_ptr(w)))
         return ChainState(f64, i32, w, self.net, self.K)
 
+    def snapshot_read_indicators(self, slot: int, weight=True, feature=True):
+        """The indicators ring slot `slot` holds (read_indicators' layouts); call before snapshot_read frees the slot."""
+        ind = np.empty((self.n_chains, self._p0)) if weight else None
+        fi = np.empty((self.n_chains, self.net.n_features)) if feature else None
+        L.check(self.lib.bnn_snapshot_read_indicators(self._h, int(slot), _np_ptr(ind), _np_ptr(fi)))
+        if ind is not None:
+            ind = ind.reshape((self.n_chains,) + tuple(self.net.shapes[0]))
+        return ind, fi
+
     def read_indicators(self, weight=True, feature=True):
         """(weight indicators [C, out0, in0+b0] or None, feature indicators [C, F] or None) of the chains' current state."""
         ind = np.empty((self.n_chains, self._p0)) if weight else None
@@ -404,6 +413,15 @@ class Engine:
         if ind is not None:
             ind = ind.reshape((self.n_chains,) + tuple(self.net.shapes[0]))
         return ind, fi
+
+    def write_indicators(self, ind=None, fi=None):
+        """Set the chains' current indicators (weight [C, out0, in0+b0], feature [C, F], 0/1; None: unchanged) and score
+        their current weights under them as chains_init scores w0 (bnn_chains_write_indicators)."""
+        ind = None if ind is None else np.ascontiguousarray(np.reshape(ind, (self.n_chains, self._p0)), dtype=np.float64)
+        fi = None if fi is None else np.ascontiguousarray(np.reshape(fi, (self.n_chains, self.net.n_features)), dtype=np.float64)
+        L.check(self.lib.bnn_chains_write_indicators(self._h, _np_ptr(ind), _np_ptr(fi), self._stream()))
+        if callable(self._rowshard) and (ind is not None or fi is not None):
+            rowshard.exchange([self], self._all_reduce_own, 2)
 
     def write_state(self, st: ChainState):
         """Write an edited host copy of the state arrays back (bnn_chains_write)."""
