@@ -336,6 +336,15 @@ int bnn_predict_sample_philox(bnn_ctx* ctx, const double* x_dev, int64_t n, cons
                               const double* alpha_dev, uint64_t seed, double* est_dev, int32_t* class_counts_dev,
                               double* post_pred_dev, void* stream);
 
+/* bnn_predict_sample_philox over a block of a larger prediction: x_dev holds rows row0 ... row0 + n - 1 and w_dev the
+ * weight sets set0 ... set0 + n_sets - 1 of it, and the uniforms are keyed on the global (row0 + row, set0 + set).  The
+ * block's outputs are then that block of the larger call's: post_pred_dev bit for bit where both run the same kernel,
+ * est_dev and class_counts_dev as the block's share and counts.  Ranks that split a prediction into row x sample blocks
+ * draw the single-process run's uniforms.  bnn_predict_sample_philox is this call with row0 = set0 = 0. */
+int bnn_predict_sample_philox_at(bnn_ctx* ctx, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,
+                                 const double* alpha_dev, uint64_t seed, int64_t row0, int32_t set0, double* est_dev,
+                                 int32_t* class_counts_dev, double* post_pred_dev, void* stream);
+
 /* Debugging aid (no reference counterpart).
  * bnn_debug_read_part: per-warp-tile partial sums of the last forward pass, [sets in pass][slots][n_tiles16]. */
 int bnn_debug_read_part(bnn_ctx* ctx, double* out_host, int64_t n_doubles);

@@ -96,6 +96,9 @@ _SIGNATURES = {
                               C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_predict_sample_philox": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_uint64,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bnn_predict_sample_philox_at": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p,
+                                               C.c_uint64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                               C.c_void_p]),
     "bnn_predict_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "bnn_launch_count": (C.c_int64, [C.c_void_p]),

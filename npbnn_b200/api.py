@@ -37,6 +37,13 @@ MC3, host-drawn indicator flips).  Not resumable: pickles written before sampler
 npBNN(pickle_file=)), the cold-chain mcmc that MC3's logger pickles (RuntimeError: resume the MC3 object), and samplers
 run over torch.distributed ranks -- MCMC(row_shard=True) and MC3 with world > 1 (NotImplementedError).
 
+Several GPUs.  Under an initialised torch.distributed process group of more than one rank, MC3 shards its chains
+(mc3.chain_grid), MCMC(row_shard=True) one chain's rows, and the posterior-prediction callers (get_posterior_cat_prob,
+sample_from_categorical, get_posterior_est, get_pdp / pdp, feature_importance, hostlib's predictBNN and
+get_posterior_threshold) are collective: every rank calls them with the same arguments (ValueError on every rank
+otherwise), scores its rows x samples block on its current device (predshard.predict_ranks) and returns the
+single-process result.  Rank 0 alone draws from numpy's global stream and writes files.
+
 estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
 MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
 companion MSE.  Options of the reference that are not on the device path raise
@@ -1242,11 +1249,22 @@ def _lik_of_output(output_act_fun):
 _ENGINE_CACHE = {}
 
 
+def _ranks():
+    """Ranks of the initialised torch.distributed process group (1 without one): the prediction callers below are
+    collective over them when there is more than one."""
+    from . import predshard
+    return predshard.ranks()[0]
+
+
 def _predict_engine(weights, n_features, actFun, output_act_fun):
-    key = (tuple(tuple(w.shape) for w in weights), n_features, actFun._function, _lik_of_output(output_act_fun))
+    """The cached prediction engine of a network shape: on GPU 0 in a single process, on the rank's current device
+    (torch.cuda.set_device of a torchrun script) under a process group of several ranks."""
+    import torch
+    device = torch.cuda.current_device() if _ranks() > 1 else 0
+    key = (tuple(tuple(w.shape) for w in weights), n_features, actFun._function, _lik_of_output(output_act_fun), device)
     if key not in _ENGINE_CACHE:
         _ENGINE_CACHE[key] = Engine(NetShape.from_weights(weights, n_features, act=actFun._function,
-                                                          lik=_lik_of_output(output_act_fun)))
+                                                          lik=_lik_of_output(output_act_fun)), device=device)
     return _ENGINE_CACHE[key]
 
 
@@ -1308,18 +1326,57 @@ def predict(bnn_obj, data):
 _HOST_UNIFORM_LIMIT = 1 << 26       # n x S above which mode 2 draws its uniforms inside the kernel (512 MB of float64)
 
 
+def _sampling_kind(n, s, rng):
+    """rng=None picks "host" while the (N, S) array of uniforms stays below 512 MB and "philox" beyond (BASELINE config
+    5: 80 GB)."""
+    if rng is None:
+        return "host" if n * s <= _HOST_UNIFORM_LIMIT else "philox"
+    if rng not in ("host", "philox"):
+        raise ValueError("rng must be None, 'host' or 'philox'")
+    return rng
+
+
 def _sampling_uniforms(n, s, rng):
     """(u, seed) of the posterior-predictive resampling.  rng="host": the reference's draw -- np.random.random(S) per
     instance in instance order = one (N, S) draw from the global stream (reproduces the reference for a seeded run).
-    rng="philox": uniforms generated inside the kernel, seeded from the global stream, O(1) extra memory.  rng=None
-    picks "host" while the (N, S) array stays below 512 MB and "philox" beyond (BASELINE config 5: 80 GB)."""
-    if rng is None:
-        rng = "host" if n * s <= _HOST_UNIFORM_LIMIT else "philox"
-    if rng == "host":
+    rng="philox": uniforms generated inside the kernel, seeded from the global stream, O(1) extra memory.  rng=None:
+    _sampling_kind."""
+    if _sampling_kind(n, s, rng) == "host":
         return np.random.random((n, s)), None
-    if rng != "philox":
-        raise ValueError("rng must be None, 'host' or 'philox'")
     return None, int(np.random.randint(0, 2 ** 31 - 1)) * 2654435761 + 1
+
+
+def _cat_prob_ranks(x, post_samples, feature_index_to_shuffle, post_summary_mode, unlink_features_within_block, actFun,
+                    output_act_fun, return_dense, rng):
+    """get_posterior_cat_prob under a process group of several ranks (module header, "Several GPUs"): the shuffled
+    feature blocks are permuted by rank 0's draws, and every rank builds its own rows of the permuted features."""
+    from . import predshard
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    if post_summary_mode not in (0, 1, 2):
+        raise ValueError("post_summary_mode must be 0 (argmax votes), 1 (mean softmax) or 2 (categorical resampling)")
+    weights = [s["weights"] for s in post_samples]
+    eng = _predict_engine(weights[0], x.shape[1], actFun, output_act_fun)
+    al = _alpha_rows([s["alphas"] for s in post_samples], actFun, len(weights[0]))
+    n, S = x.shape[0], len(weights)
+    shuffle = []
+    if feature_index_to_shuffle:
+        if unlink_features_within_block and type(feature_index_to_shuffle) == list:
+            shuffle = list(feature_index_to_shuffle)
+        else:
+            shuffle = [feature_index_to_shuffle]
+    sample = _sampling_kind(n, S, rng) if post_summary_mode == 2 else None
+
+    def draw():
+        # the single-process order: the permutations of the shuffled blocks, then the uniforms (np.random.permutation(N)
+        # makes the draws np.random.permutation(x[:, fi]) makes)
+        perms = [np.random.permutation(n) for _ in shuffle]
+        u, seed = _sampling_uniforms(n, S, sample) if sample else (None, None)
+        return perms, u, seed
+
+    out = predshard.predict_ranks(eng, x, weights, al, mean=post_summary_mode == 1, votes=post_summary_mode == 0,
+                                  dense=return_dense, sample=sample, shuffle=shuffle, draw=draw)
+    summary = {0: "votes", 1: "mean", 2: "predictions"}[post_summary_mode]
+    return out.get("dense"), out[summary]
 
 
 def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_shuffle=None, post_summary_mode=0,
@@ -1330,6 +1387,9 @@ def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_sh
     if len(pred_features) == 0:
         print("Data not found.")
         return 0
+    if _ranks() > 1:
+        return _cat_prob_ranks(pred_features, post_samples, feature_index_to_shuffle, post_summary_mode,
+                               unlink_features_within_block, actFun, output_act_fun, return_dense, rng)
     # a private copy only when columns are permuted below (512 MB and 0.2 s at BASELINE config 5 otherwise)
     x = np.array(pred_features, dtype=np.float64, copy=True) if feature_index_to_shuffle else \
         np.ascontiguousarray(pred_features, dtype=np.float64)
@@ -1365,6 +1425,13 @@ def sample_from_categorical(pred_features, post_samples, actFun=None, output_act
     weights = [s["weights"] for s in post_samples]
     eng = _predict_engine(weights[0], x.shape[1], actFun, output_act_fun)
     al = _alpha_rows([s["alphas"] for s in post_samples], actFun, len(weights[0]))
+    if _ranks() > 1:
+        from . import predshard
+        n, S = x.shape[0], len(weights)
+        sample = _sampling_kind(n, S, rng)
+        out = predshard.predict_ranks(eng, x, weights, al, sample=sample, post_predictions=post_predictions,
+                                      draw=lambda: ([],) + _sampling_uniforms(n, S, sample))
+        return {k: out[k] for k in ("predictions", "class_counts", "post_predictions")}
     u, seed = _sampling_uniforms(x.shape[0], len(weights), rng)
     return eng.predict_sample(x, weights, u, alphas=al, post_predictions=post_predictions, seed=seed)
 
@@ -1416,7 +1483,7 @@ def feature_importance(input_features, weights_pkl=None, weights_posterior=None,
                        "acc_with_feature_randomized_mean": np.mean(accuracies_wo_feature, axis=1),
                        "acc_with_feature_randomized_std": np.std(accuracies_wo_feature, axis=1)})
     df = df.sort_values("delta_acc_mean", ascending=False)
-    if write_to_file:
+    if write_to_file and _is_rank0():
         if predictions_outdir == "":
             predictions_outdir = os.path.dirname(weights_pkl) if weights_pkl else "."
         if not os.path.exists(predictions_outdir) and predictions_outdir != "":
@@ -1441,7 +1508,11 @@ def get_posterior_est(pkl_file):
         x = np.ascontiguousarray(x, dtype=np.float64)
         eng = _predict_engine(weights[0], x.shape[1], bnn_obj._act_fun, bnn_obj._output_act_fun)
         al = _alpha_rows([s["alphas"] for s in ps], bnn_obj._act_fun, len(weights[0]))
-        out = eng.predict(x, weights, alphas=al, mean=True, dense=True)
+        if _ranks() > 1:
+            from . import predshard
+            out = predshard.predict_ranks(eng, x, weights, al, mean=True, dense=True)
+        else:
+            out = eng.predict(x, weights, alphas=al, mean=True, dense=True)
         res["post_est" + key], res["prm_mean" + key] = out["dense"], out["mean"]
     return res
 
@@ -1471,12 +1542,18 @@ def get_pdp(data, focal_features, estimation_mode, size_output, actFun, output_a
     out = np.zeros((grid.shape[0], size_output, 3))
     eng = _predict_engine(weights[0], data.shape[1], actFun, output_act_fun)
     al = _alpha_rows(alphas, actFun, len(weights[0]))
+    if _ranks() > 1:
+        from . import predshard
+        # every rank scores its block and gets the full [N, K] mean: the row quantiles below need all rows
+        predict = lambda ov: predshard.predict_ranks(eng, data, weights, al, override=ov, mean=True)["mean"]  # noqa: E731
+    else:
+        predict = lambda ov: eng.predict(data, weights, alphas=al, override=ov, mean=True)["mean"]  # noqa: E731
     for n in range(grid.shape[0]):
         # the grid value is written first, the feature-indicator transform inside RunPredict then replaces masked
         # features by their mean (BNN_pdp.py:65-73, BNN_lib.py:248-249): the transform wins on a shared column
         ov = dict(zip([int(f) for f in focal_features], [float(v) for v in grid[n, :]]))
         ov.update(zip([int(cc) for cc in dt_cols], [float(v) for v in dt_vals]))
-        smean = eng.predict(data, weights, alphas=al, override=(list(ov.keys()), list(ov.values())), mean=True)["mean"]
+        smean = predict((list(ov.keys()), list(ov.values())))
         if estimation_mode == "classification":
             smean = np.cumsum(smean, axis=1)
         out[n, :, 0] = np.mean(smean, axis=0)

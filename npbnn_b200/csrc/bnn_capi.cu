@@ -1250,7 +1250,7 @@ static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double
                         const double* alpha_dev, const int32_t* override_cols, const double* override_vals,
                         int32_t n_override, double* mean_dev, double* votes_dev, double* dense_dev, const double* u_dev,
                         int32_t* class_counts_dev, double* post_pred_dev, void* stream, bool samp_philox = false,
-                        uint64_t samp_seed = 0) {
+                        uint64_t samp_seed = 0, int64_t samp_row0 = 0, int32_t samp_set0 = 0) {
   REQUIRE(c && c->have_net, "bnn_predict: call bnn_set_net first");
   REQUIRE(x_dev && w_dev && n >= 1 && n_sets >= 1, "bnn_predict: bad arguments");
   REQUIRE(mean_dev || votes_dev || dense_dev, "bnn_predict: no output requested");
@@ -1282,6 +1282,7 @@ static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double
   p.inv_sets = (double)n_sets;   // divisor (np.mean and the vote share divide, BNN_lib.py:390-392)
   p.samp_u = u_dev; p.samp_counts = class_counts_dev; p.samp_dense = post_pred_dev;
   p.samp_philox = samp_philox ? 1 : 0; p.samp_seed = samp_seed;
+  p.samp_row0 = samp_row0; p.samp_set0 = samp_set0;
   if (class_counts_dev) CUDA_TRY(cudaMemsetAsync(class_counts_dev, 0, sizeof(int32_t) * (size_t)n_sets * g.K, st));
   if (c->opt_pred_tf32 && !c->force_generic && bnn_pred_tf32_fits(p)) {
     // opt-in reduced precision (stated tolerance: class probabilities to ~1e-6 absolute); summaries only
@@ -1301,13 +1302,21 @@ int bnn_predict(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev,
                       votes_dev, dense_dev, nullptr, nullptr, nullptr, stream);
 }
 
+int bnn_predict_sample_philox_at(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,
+                                 const double* alpha_dev, uint64_t seed, int64_t row0, int32_t set0, double* est_dev,
+                                 int32_t* class_counts_dev, double* post_pred_dev, void* stream) {
+  REQUIRE(c && c->have_net && c->g.lik == BNN_LIK_CATEGORICAL, "bnn_predict_sample_philox: needs the categorical likelihood");
+  REQUIRE(est_dev, "bnn_predict_sample_philox: est_dev is required");
+  REQUIRE(row0 >= 0 && set0 >= 0, "bnn_predict_sample_philox_at: negative offset");
+  return predict_impl(c, x_dev, n, w_dev, n_sets, alpha_dev, nullptr, nullptr, 0, nullptr, est_dev, nullptr, nullptr,
+                      class_counts_dev, post_pred_dev, stream, true, seed, row0, set0);
+}
+
 int bnn_predict_sample_philox(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,
                               const double* alpha_dev, uint64_t seed, double* est_dev, int32_t* class_counts_dev,
                               double* post_pred_dev, void* stream) {
-  REQUIRE(c && c->have_net && c->g.lik == BNN_LIK_CATEGORICAL, "bnn_predict_sample_philox: needs the categorical likelihood");
-  REQUIRE(est_dev, "bnn_predict_sample_philox: est_dev is required");
-  return predict_impl(c, x_dev, n, w_dev, n_sets, alpha_dev, nullptr, nullptr, 0, nullptr, est_dev, nullptr, nullptr,
-                      class_counts_dev, post_pred_dev, stream, true, seed);
+  return bnn_predict_sample_philox_at(c, x_dev, n, w_dev, n_sets, alpha_dev, seed, 0, 0, est_dev, class_counts_dev,
+                                      post_pred_dev, stream);
 }
 
 int bnn_predict_sample(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,

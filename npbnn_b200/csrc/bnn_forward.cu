@@ -295,7 +295,7 @@ __device__ __forceinline__ void quad_epilogue_pred(const FwdParams& p, int c, lo
       const long long row = wt * 16 + gq + 8 * h;
       const bool live = row < p.n_total;
       const double inv = 1.0 / r.S[h];
-      const double u = live ? bnn_samp_uniform(p.samp_seed, row, c) : 2.0;
+      const double u = live ? bnn_samp_uniform(p.samp_seed, p.samp_row0 + row, p.samp_set0 + c) : 2.0;
       double base = 0.0;
       int drawn = 0x7fffffff;
 #pragma unroll

@@ -99,7 +99,7 @@ __device__ __forceinline__ void bnn_epilogue(const FwdParams& p, int c, long lon
         double* pa = pacc + (lane & 15) * K;
         // sample_from_categorical: first class whose running sum (np.cumsum order) reaches u; none => class 0
         const bool sampling = p.samp_u || p.samp_philox;
-        const double u = p.samp_u ? p.samp_u[row * p.C + c] : (p.samp_philox ? bnn_samp_uniform(p.samp_seed, row, c) : 0.0);
+        const double u = p.samp_u ? p.samp_u[row * p.C + c] : (p.samp_philox ? bnn_samp_uniform(p.samp_seed, p.samp_row0 + row, p.samp_set0 + c) : 0.0);
         double cum = 0.0;
         int drawn = -1;
         for (int k = 0; k < K; ++k) {

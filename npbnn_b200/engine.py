@@ -472,9 +472,10 @@ class Engine:
         torch.cuda.current_stream(self.device).synchronize()
 
     # ---------------------------------------------------------------- prediction
-    def predict(self, x, weight_sets, alphas=None, override=None, mean=True, votes=False, dense=False):
+    def predict(self, x, weight_sets, alphas=None, override=None, mean=True, votes=False, dense=False, device_out=False):
         """Posterior prediction over rows of x for every weight set (reference BNN_lib.py:376-392).
-        override: (cols, vals) PDP column overwrite (BNN_pdp.py:65).  Returns dict of numpy arrays."""
+        override: (cols, vals) PDP column overwrite (BNN_pdp.py:65).  Returns dict of numpy arrays (device_out: of
+        tensors on this engine's device)."""
         w = self._as_sets(weight_sets)
         with torch.cuda.device(self.device):
             xd = self._dev(x, torch.float64)
@@ -496,18 +497,20 @@ class Engine:
             torch.cuda.current_stream(self.device).synchronize()
             out = {}
             if mean:
-                out["mean"] = md.cpu().numpy()
+                out["mean"] = md
             if votes:
-                out["votes"] = vd.cpu().numpy()
+                out["votes"] = vd
             if dense:
-                out["dense"] = dd.cpu().numpy()
-            return out
+                out["dense"] = dd
+            return out if device_out else {k: v.cpu().numpy() for k, v in out.items()}
 
-    def predict_sample(self, x, weight_sets, u=None, alphas=None, post_predictions=True, seed=None):
+    def predict_sample(self, x, weight_sets, u=None, alphas=None, post_predictions=True, seed=None, row0=0, set0=0,
+                       device_out=False):
         """sample_from_categorical (BNN_lib.py:682-713) fused into the prediction pass.  u [n, S]: the reference's
         uniforms (np.random.random(S) per instance); u=None: uniforms generated in the kernel from `seed` (Philox,
-        nothing of size n x S is stored).  Returns dict(predictions [n,K], class_counts [S,K], post_predictions [n,S]
-        or None)."""
+        nothing of size n x S is stored), keyed on (row0 + row, set0 + set): rows row0... and sets set0... of a larger
+        call draw that call's uniforms.  Returns dict(predictions [n,K], class_counts [S,K], post_predictions [n,S]
+        or None) of numpy arrays (device_out: of float64 tensors on this engine's device)."""
         w = self._as_sets(weight_sets)
         with torch.cuda.device(self.device):
             xd, wd, ad = self._dev(x, torch.float64), self._dev(w, torch.float64), self._dev(alphas, torch.float64)
@@ -516,14 +519,16 @@ class Engine:
             cc = torch.empty((S, self.K), dtype=torch.int32, device=self.device)
             pp = torch.empty((n, S), dtype=torch.float64, device=self.device) if post_predictions else None
             if u is None:
-                L.check(self.lib.bnn_predict_sample_philox(self._h, _ptr(xd), n, _ptr(wd), S, _ptr(ad),
-                                                           int(0 if seed is None else seed) & (2 ** 64 - 1), _ptr(est), _ptr(cc),
-                                                           _ptr(pp), self._stream()))
+                L.check(self.lib.bnn_predict_sample_philox_at(self._h, _ptr(xd), n, _ptr(wd), S, _ptr(ad),
+                                                              int(0 if seed is None else seed) & (2 ** 64 - 1), int(row0),
+                                                              int(set0), _ptr(est), _ptr(cc), _ptr(pp), self._stream()))
             else:
                 ud = self._dev(u, torch.float64)
                 assert tuple(ud.shape) == (n, S)
                 L.check(self.lib.bnn_predict_sample(self._h, _ptr(xd), n, _ptr(wd), S, _ptr(ad), _ptr(ud), _ptr(est), _ptr(cc),
                                                     _ptr(pp), self._stream()))
             torch.cuda.current_stream(self.device).synchronize()
+            if device_out:
+                return {"predictions": est, "class_counts": cc.to(torch.float64), "post_predictions": pp}
             return {"predictions": est.cpu().numpy(), "class_counts": cc.cpu().numpy().astype(np.float64),
                     "post_predictions": None if pp is None else pp.cpu().numpy()}

@@ -269,7 +269,9 @@ def get_accuracy_threshold(probs, labels, threshold=0.75):
 
 
 def get_posterior_threshold(pkl_file, target_acc=0.9, post_summary_mode=1, output_file=None):
-    """Smallest posterior-probability cut-off (0.01 ... 0.99) at which the test accuracy reaches target_acc."""
+    """Smallest posterior-probability cut-off (0.01 ... 0.99) at which the test accuracy reaches target_acc.  Collective
+    under a process group of several ranks (predictBNN); only rank 0 writes output_file."""
+    from . import api
     bnn_obj, mcmc_obj, logger_obj = load_obj(pkl_file)
     res = predictBNN(bnn_obj._test_data, pickle_file=pkl_file, test_labels=bnn_obj._test_labels,
                      post_summary_mode=post_summary_mode, verbose=0)["post_prob_predictions"]
@@ -281,7 +283,7 @@ def get_posterior_threshold(pkl_file, target_acc=0.9, post_summary_mode=1, outpu
         except Exception:           # no instance above the cut-off
             pass
     tbl = np.array(rows)
-    if output_file is not None:
+    if output_file is not None and api._is_rank0():
         import pandas as pd
         np.round(pd.DataFrame(tbl, columns=["Threshold", "Accuracy", "Retained_data"]), 3).to_csv(
             path_or_buf=output_file, sep="\t", index=False, header=True)
@@ -308,7 +310,8 @@ def predictBNN(predict_features, pickle_file, test_labels=[], instance_id=[], pi
                post_cutoff=None, threshold=0.95, bf=150, post_summary_mode=0, fname="", wd="", verbose=1):
     """Posterior prediction for `predict_features` from the samples stored in `pickle_file`; all posterior samples are
     scored in one device pass (api.get_posterior_cat_prob).  Writes <fname_><pkl>_pred_pr.npy, _pred_mean_pr.txt and
-    (with labels) _accuracy.txt next to the pickle (or into `wd`)."""
+    (with labels) _accuracy.txt next to the pickle (or into `wd`).  Under a process group of several ranks the call is
+    collective (every rank passes the same arguments and gets the same result) and only rank 0 writes the files."""
     from . import api
     bnn_obj, mcmc_obj, logger_obj = load_obj(pickle_file)
     post_samples = logger_obj._post_weight_samples
@@ -321,6 +324,7 @@ def predictBNN(predict_features, pickle_file, test_labels=[], instance_id=[], pi
         fname = fname + "_"
     f_dense = os.path.join(outdir, fname + out_name + "_pred_pr.npy")
     f_mean = os.path.join(outdir, fname + out_name + "_pred_mean_pr.txt")
+    writer = api._is_rank0()
     if len(test_labels) > 0:
         accuracy = CalcAccuracy(post_prob, test_labels)
         tp = CalcTP(post_prob, test_labels, threshold=threshold)
@@ -333,8 +337,9 @@ def predictBNN(predict_features, pickle_file, test_labels=[], instance_id=[], pi
             print("True positive rate:", np.mean(tp))
             print("False positive rate:", np.mean(fp))
             print("Confusion matrix:\n", cm)
-        with open(os.path.join(outdir, fname + out_name + "_accuracy.txt"), "w") as outf:
-            outf.writelines("Mean accuracy: %s (TP: %s; FP: %s)" % (mean_accuracy, tp, fp))
+        if writer:
+            with open(os.path.join(outdir, fname + out_name + "_accuracy.txt"), "w") as outf:
+                outf.writelines("Mean accuracy: %s (TP: %s; FP: %s)" % (mean_accuracy, tp, fp))
     else:
         mean_accuracy, cm_out = np.nan, np.nan
     if pickle_file_prior:
@@ -351,6 +356,8 @@ def predictBNN(predict_features, pickle_file, test_labels=[], instance_id=[], pi
         keep = np.where(np.max(post_prob, axis=1) > cut)[0]
         post_prob = turn_low_pp_instances_to_nan(post_prob, keep)
         dense = np.array([turn_low_pp_instances_to_nan(i, keep) for i in dense])
+    if not writer:
+        return {"post_prob_predictions": post_prob, "mean_accuracy": mean_accuracy, "confusion_matrix": cm_out}
     if len(instance_id):
         instance_id = np.asarray(instance_id)
         tbl = np.hstack((instance_id.reshape(len(instance_id), 1), np.round(post_prob, 4).astype(str)))

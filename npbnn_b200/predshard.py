@@ -8,6 +8,10 @@ form R row groups x Q sample groups (R Q = world); a rank predicts its row block
 the Q partial sums of a row block ([rows, K] doubles, 20 MB at 250k rows) are added with ONE all-reduce over NCCL.
 `grid_for` picks the (R, Q) with the fewest rounds per GPU; Q = 1 (rows only, no collective) wins whenever the row
 split is already balanced.
+
+`predict_ranks` is the same grid behind the reference's prediction callers (api.get_posterior_cat_prob and everything
+built on it): every rank passes the caller's full arguments, scores its block and gets back the full arrays the
+single-process call returns.  It is collective: every rank of the process group calls it with the same arguments.
 """
 import math
 from typing import Optional, Tuple
@@ -131,3 +135,199 @@ def predict_sharded(engine, x_rows, weight_sets, n_rows_total: int, rank: int, w
         if votes:
             out["votes"] = combine(vsum, S, world, rank, grid)
     return out
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# collective prediction behind the reference's prediction callers
+# ---------------------------------------------------------------------------------------------------------------------
+def ranks() -> Tuple[int, int]:
+    """(world, rank) of the initialised default process group; (1, 0) without one."""
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_world_size(), dist.get_rank()
+    return 1, 0
+
+
+def comm_device() -> torch.device:
+    """Where the tensors of the collectives live: the current GPU under NCCL (one GPU per rank), host memory under
+    gloo (ranks that share GPUs)."""
+    if dist.get_backend() == "nccl":
+        return torch.device("cuda", torch.cuda.current_device())
+    return torch.device("cpu")
+
+
+def agree(call) -> None:
+    """Collective check that every rank passed the same arguments `call` (a small tuple of plain values).  Runs before
+    any other collective of the call: ranks that disagree on a shape would otherwise hang in a later collective or
+    exchange blocks of different problems.  A mismatch raises ValueError on every rank."""
+    calls = [None] * dist.get_world_size()
+    dist.all_gather_object(calls, call)
+    bad = [r for r, c in enumerate(calls) if c != calls[0]]
+    if bad:
+        raise ValueError("collective prediction called with different arguments: rank 0 passed %r, rank %d passed %r"
+                         % (calls[0], bad[0], calls[bad[0]]))
+
+
+def from_rank0(value, shape, dtype: torch.dtype) -> torch.Tensor:
+    """Rank 0's array `value` (ignored on the other ranks) on every rank, as a tensor of `shape` on comm_device()."""
+    dev = comm_device()
+    if dist.get_rank() == 0:
+        t = torch.as_tensor(np.ascontiguousarray(value)).to(device=dev, dtype=dtype).reshape(shape).contiguous()
+    else:
+        t = torch.empty(shape, dtype=dtype, device=dev)
+    dist.broadcast(t, src=0)
+    return t
+
+
+def _columns(selector, n_features: int):
+    """Distinct column indices of a feature selector x[:, selector] (an index or a list of indices)."""
+    return list(dict.fromkeys(int(c) % n_features for c in np.atleast_1d(np.asarray(selector)).ravel()))
+
+
+def permuted_rows(x: np.ndarray, lo: int, hi: int, shuffle, perms) -> np.ndarray:
+    """Rows lo..hi of x after `x[:, cols] = x[perm][:, cols]` for each (cols, perm) of zip(shuffle, perms), in order:
+    the rows of the reference's `x[:, fi] = np.random.permutation(x[:, fi])` (np.random.permutation(N) draws the
+    permutation np.random.permutation(x[:, fi]) applies), built from the full host copy without permuting it."""
+    rows = np.array(x[lo:hi], copy=True)
+    src = {}                      # column -> source row of each row after the permutations so far
+    for cols, perm in zip(shuffle, perms):
+        for col in _columns(cols, x.shape[1]):
+            src[col] = perm if col not in src else src[col][perm]
+    for col, s in src.items():
+        rows[:, col] = x[s[lo:hi], col]
+    return rows
+
+
+# the outputs in the order a rank packs its blocks for the all-gather
+_OUTPUTS = ("mean", "votes", "predictions", "class_counts", "post_predictions", "dense")
+
+
+def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False, votes=False, dense=False,
+                  sample=None, post_predictions=False, shuffle=(), draw=None, grid: Optional[Tuple[int, int]] = None):
+    """Posterior prediction of all N rows of x over all S posterior samples, split over the ranks of the default process
+    group.  Collective: every rank passes the same arguments (checked first, ValueError on every rank otherwise) and
+    returns the same dict of host arrays as the single-process engine calls:
+      mean [N, W], votes [N, W], dense [S, N, W]                     (Engine.predict; W = K, or the outputs)
+      predictions [N, K], class_counts [S, K], post_predictions [N, S] (Engine.predict_sample, with sample set)
+    x: the caller's full host features [N, F]; weight_sets: all S posterior samples; alphas: [S, L] or None; override:
+    (cols, vals) column overwrite.  sample: None, "host" (reference uniforms) or "philox" (in-kernel uniforms, keyed on
+    the global (row, sample) so the split does not change them).  shuffle: feature selectors whose rows are permuted.
+    draw(): run on rank 0 only, returns (permutations of range(N), one per shuffle entry; uniforms [N, S] or None; seed
+    or None) drawn from rank 0's numpy stream, which every rank then receives.
+
+    The rank scores rows x samples block `partition(N, S, world, rank, grid)`; a rank with an empty block makes no kernel
+    call but joins every collective.  Combination (one all-gather of every rank's block): means are sums over each sample
+    group, added in sample-group order and divided by S once (with one sample group: the block's own mean); votes and
+    resampled shares are integer counts, added and divided by S once; class_counts are added over the row groups."""
+    from . import _lib as L
+    world, rank = ranks()
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    n, f = x.shape
+    S = len(weight_sets)
+    W = engine.K if engine.net.lik == L.LIK_CATEGORICAL else engine.O
+    K = engine.K
+    ov = None if override is None else (tuple(int(c) for c in override[0]), tuple(float(v) for v in override[1]))
+    shuffle = list(shuffle)
+    agree((n, f, S, W, engine.net.n_params, engine.net.act, engine.net.lik, bool(mean), bool(votes), bool(dense), sample,
+           bool(post_predictions), [tuple(_columns(s, f)) for s in shuffle], ov, grid))
+    if sample not in (None, "host", "philox"):
+        raise ValueError("sample must be None, 'host' or 'philox'")
+    rows, sets, grid, _, _ = partition(n, S, world, rank, grid)
+    R, Q = grid
+    (a, b), (c, d) = rows, sets
+    n_loc, s_loc = b - a, d - c
+    dev = comm_device()
+
+    # draws from numpy's global stream: rank 0's, the ones a single-process run makes
+    drawn = draw() if rank == 0 and draw is not None else ([None] * len(shuffle), None, None)
+    perms = []
+    if shuffle:
+        pm = from_rank0(np.stack(drawn[0]) if rank == 0 else None, (len(shuffle), n), torch.int64)
+        perms = list(pm.cpu().numpy())
+    u = seed = None
+    if sample == "host":
+        u = from_rank0(drawn[1] if rank == 0 else None, (n, S), torch.float64)
+    elif sample == "philox":
+        seed = int(from_rank0(np.array([drawn[2] if rank == 0 else 0], dtype=np.int64), (1,), torch.int64).item())
+
+    names = [k for k, on in zip(_OUTPUTS, (mean, votes, sample, sample, sample and post_predictions, dense)) if on]
+
+    def sizes(nl, sl):
+        return {"mean": (nl, W), "votes": (nl, W), "predictions": (nl, K), "class_counts": (sl, K),
+                "post_predictions": (nl, sl), "dense": (sl, nl, W)}
+
+    parts = {}
+    if n_loc and s_loc:
+        xb = permuted_rows(x, a, b, shuffle, perms) if shuffle else x[a:b]
+        w = weight_sets[c:d]
+        al = None if alphas is None else np.asarray(alphas)[c:d]
+        if mean or votes or dense:
+            o = engine.predict(xb, w, alphas=al, override=override, mean=mean, votes=votes, dense=dense, device_out=True)
+            if mean:
+                parts["mean"] = o["mean"] if Q == 1 else o["mean"] * float(s_loc)
+            if votes:
+                parts["votes"] = torch.round(o["votes"] * float(s_loc))
+            if dense:
+                parts["dense"] = o["dense"]
+        if sample:
+            r = engine.predict_sample(xb, w, None if u is None else u[a:b, c:d], alphas=al,
+                                      post_predictions=post_predictions, seed=seed, row0=a, set0=c, device_out=True)
+            parts["predictions"] = torch.round(r["predictions"] * float(s_loc))
+            parts["class_counts"] = r["class_counts"]
+            if post_predictions:
+                parts["post_predictions"] = r["post_predictions"]
+
+    # one all-gather of every rank's blocks, packed into one vector padded to the longest
+    blocks = [partition(n, S, world, q, grid)[:2] for q in range(world)]
+    lens = [sum(int(np.prod(sizes(rb - ra, sb - sa)[k])) for k in names) for (ra, rb), (sa, sb) in blocks]
+    send = torch.zeros(max(lens), dtype=torch.float64, device=dev)
+    if parts:
+        send[:lens[rank]] = torch.cat([parts[k].to(device=dev, dtype=torch.float64).reshape(-1) for k in names])
+    recv = [torch.empty_like(send) for _ in range(world)]
+    dist.all_gather(recv, send)
+
+    def view(q):
+        (ra, rb), (sa, sb) = blocks[q]
+        out, o = {}, 0
+        for k in names:
+            shp = sizes(rb - ra, sb - sa)[k]
+            m = int(np.prod(shp))
+            out[k] = recv[q][o:o + m].reshape(shp)
+            o += m
+        return out
+
+    views = [view(q) for q in range(world)]
+    res = {}
+    for k in names:
+        if k in ("mean", "votes", "predictions"):
+            full = torch.empty((n, W if k != "predictions" else K), dtype=torch.float64, device=dev)
+            for g in range(R):
+                (ra, rb), _ = blocks[g * Q]
+                if rb == ra:
+                    continue
+                if k == "mean" and Q == 1:
+                    full[ra:rb] = views[g][k]
+                    continue
+                acc = views[g * Q][k].clone()
+                for q in range(1, Q):
+                    acc += views[g * Q + q][k]
+                full[ra:rb] = acc / float(S)
+        elif k == "class_counts":
+            full = torch.zeros((S, K), dtype=torch.float64, device=dev)
+            for q in range(world):
+                (ra, rb), (sa, sb) = blocks[q]
+                if rb > ra:
+                    full[sa:sb] += views[q][k]
+        elif k == "post_predictions":
+            full = torch.empty((n, S), dtype=torch.float64, device=dev)
+            for q in range(world):
+                (ra, rb), (sa, sb) = blocks[q]
+                full[ra:rb, sa:sb] = views[q][k]
+        else:
+            full = torch.empty((S, n, W), dtype=torch.float64, device=dev)
+            for q in range(world):
+                (ra, rb), (sa, sb) = blocks[q]
+                full[sa:sb, ra:rb] = views[q][k]
+        res[k] = full.cpu().numpy()
+    if sample and not post_predictions:
+        res["post_predictions"] = None
+    return res
