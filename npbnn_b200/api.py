@@ -38,11 +38,13 @@ npBNN(pickle_file=)), the cold-chain mcmc that MC3's logger pickles (RuntimeErro
 run over torch.distributed ranks -- MCMC(row_shard=True) and MC3 with world > 1 (NotImplementedError).
 
 Several GPUs.  Under an initialised torch.distributed process group of more than one rank, MC3 shards its chains
-(mc3.chain_grid), MCMC(row_shard=True) one chain's rows, and the posterior-prediction callers (get_posterior_cat_prob,
+(mc3.chain_grid) and MCMC(row_shard=True) one chain's rows.  The posterior-prediction callers (get_posterior_cat_prob,
 sample_from_categorical, get_posterior_est, get_pdp / pdp, feature_importance, hostlib's predictBNN and
-get_posterior_threshold) are collective: every rank calls them with the same arguments (ValueError on every rank
-otherwise), scores its rows x samples block on its current device (predshard.predict_ranks) and returns the
-single-process result.  Rank 0 alone draws from numpy's global stream and writes files.
+get_posterior_threshold) all go through one routine, predshard.predict_ranks, in one process and on many ranks alike.
+They are collective: every rank calls them with the same arguments (ValueError on every rank otherwise), scores its
+rows x samples block on its current device and returns the result of one process.  Rank 0 alone draws from numpy's
+global stream and writes files.  A single process is a group of one rank: it scores the whole problem on GPU 0 and
+makes no torch.distributed call.
 
 estimation_mode="custom" runs with output_act_fun=RegressTransform and one of the count likelihoods of BNN_lik.py as
 MCMC / MC3(likelihood_f=), recognised by identity (SURVEY.md, item 9 on pluggable callables); accuracy_f=None means the likelihood's
@@ -65,6 +67,7 @@ import numpy as np
 
 from . import _lib as L
 from . import mc3 as _mc3
+from . import predshard
 from .engine import ChainState, Engine, NetShape, flatten_weights, unflatten_weights
 
 small_number = 1e-10
@@ -1157,12 +1160,7 @@ class MC3:
                 m._sync(b, st)
                 if m._temperature == 1:                     # the logger follows the cold chain (BNN_mc3.py:118-122)
                     cold = (b, m)
-            if self.world == 1:
-                if cold is not None:
-                    self.logger.log_sample(*cold)
-                    self.logger.log_weights(*cold)
-            else:
-                self._log_on_rank0(cold)
+            self._log_on_rank0(cold)
             if mc3_it % self.print_f == 0 and self.rank == 0 and self.n_local:
                 b0, m0 = self.singleChainArgs[0]
                 print(mc3_it, m0._logPost, b0._w_layers[0][0][0:5])
@@ -1197,16 +1195,18 @@ class MC3:
             m._group, m._bnn_view = self._group, b
 
     def _log_on_rank0(self, cold):
-        """Chains sharded over ranks: the cold temperature migrates between ranks with the swaps, the files belong to
-        rank 0.  The r = 0 rank of the block holding the cold chain sends its exported state (statistics + weights, a
-        few kB) to rank 0, which is the only rank that writes the .log / .pkl and keeps the posterior sample list."""
+        """The logger follows the cold chain (`cold`: this rank's (bnn, mcmc) at temperature 1, or None), and the files
+        belong to rank 0.  In a single process, and whenever rank 0 holds the cold chain, rank 0 logs its own chain.
+        Chains sharded over ranks: the cold temperature migrates between ranks with the swaps, and the r = 0 rank of the
+        block holding the cold chain sends its exported state (statistics + weights, a few kB) to rank 0, which is the
+        only rank that writes the .log / .pkl and keeps the posterior sample list."""
         import torch.distributed as dist
         cold_chain = int(np.flatnonzero(self.current_temperatures == 1)[0]) if np.any(self.current_temperatures == 1) else -1
         if cold_chain < 0:
             return
         owner = _mc3.owner_of(cold_chain, self.n_chains, self.world, self.R)
         box = [None]
-        if self.rank == owner:
+        if owner != 0 and self.rank == owner:          # only a state that travels is exported
             b, m = cold
             box[0] = {"bnn": {k: getattr(b, k) for k in ("_w_layers", "_indicators", "_error_prm", "_feature_indicators",
                                                           "_prior_scale", "_seed")},
@@ -1249,18 +1249,11 @@ def _lik_of_output(output_act_fun):
 _ENGINE_CACHE = {}
 
 
-def _ranks():
-    """Ranks of the initialised torch.distributed process group (1 without one): the prediction callers below are
-    collective over them when there is more than one."""
-    from . import predshard
-    return predshard.ranks()[0]
-
-
 def _predict_engine(weights, n_features, actFun, output_act_fun):
     """The cached prediction engine of a network shape: on GPU 0 in a single process, on the rank's current device
     (torch.cuda.set_device of a torchrun script) under a process group of several ranks."""
     import torch
-    device = torch.cuda.current_device() if _ranks() > 1 else 0
+    device = torch.cuda.current_device() if predshard.ranks()[0] > 1 else 0
     key = (tuple(tuple(w.shape) for w in weights), n_features, actFun._function, _lik_of_output(output_act_fun), device)
     if key not in _ENGINE_CACHE:
         _ENGINE_CACHE[key] = Engine(NetShape.from_weights(weights, n_features, act=actFun._function,
@@ -1346,14 +1339,18 @@ def _sampling_uniforms(n, s, rng):
     return None, int(np.random.randint(0, 2 ** 31 - 1)) * 2654435761 + 1
 
 
-def _cat_prob_ranks(x, post_samples, feature_index_to_shuffle, post_summary_mode, unlink_features_within_block, actFun,
-                    output_act_fun, return_dense, rng):
-    """get_posterior_cat_prob under a process group of several ranks (module header, "Several GPUs"): the shuffled
-    feature blocks are permuted by rank 0's draws, and every rank builds its own rows of the permuted features."""
-    from . import predshard
-    x = np.ascontiguousarray(x, dtype=np.float64)
+def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_shuffle=None, post_summary_mode=0,
+                           unlink_features_within_block=False, actFun=None, output_act_fun=None, return_dense=True,
+                           rng=None):
+    """BNN_lib.py:352-397 with all posterior samples scored in ONE pass over the features.
+    return_dense=False skips the [S, N, K] tensor (it is 800 GB at BASELINE config 5) and returns None for it.  Mode 2
+    resamples as sample_from_categorical (BNN_lib.py:682-713), inside the prediction kernel."""
+    if len(pred_features) == 0:
+        print("Data not found.")
+        return 0
     if post_summary_mode not in (0, 1, 2):
         raise ValueError("post_summary_mode must be 0 (argmax votes), 1 (mean softmax) or 2 (categorical resampling)")
+    x = np.ascontiguousarray(pred_features, dtype=np.float64)
     weights = [s["weights"] for s in post_samples]
     eng = _predict_engine(weights[0], x.shape[1], actFun, output_act_fun)
     al = _alpha_rows([s["alphas"] for s in post_samples], actFun, len(weights[0]))
@@ -1367,7 +1364,7 @@ def _cat_prob_ranks(x, post_samples, feature_index_to_shuffle, post_summary_mode
     sample = _sampling_kind(n, S, rng) if post_summary_mode == 2 else None
 
     def draw():
-        # the single-process order: the permutations of the shuffled blocks, then the uniforms (np.random.permutation(N)
+        # the reference's order: the permutations of the shuffled blocks, then the uniforms (np.random.permutation(N)
         # makes the draws np.random.permutation(x[:, fi]) makes)
         perms = [np.random.permutation(n) for _ in shuffle]
         u, seed = _sampling_uniforms(n, S, sample) if sample else (None, None)
@@ -1379,43 +1376,6 @@ def _cat_prob_ranks(x, post_samples, feature_index_to_shuffle, post_summary_mode
     return out.get("dense"), out[summary]
 
 
-def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_shuffle=None, post_summary_mode=0,
-                           unlink_features_within_block=False, actFun=None, output_act_fun=None, return_dense=True,
-                           rng=None):
-    """BNN_lib.py:352-397 with all posterior samples scored in ONE pass over the features.
-    return_dense=False skips the [S, N, K] tensor (it is 800 GB at BASELINE config 5) and returns None for it."""
-    if len(pred_features) == 0:
-        print("Data not found.")
-        return 0
-    if _ranks() > 1:
-        return _cat_prob_ranks(pred_features, post_samples, feature_index_to_shuffle, post_summary_mode,
-                               unlink_features_within_block, actFun, output_act_fun, return_dense, rng)
-    # a private copy only when columns are permuted below (512 MB and 0.2 s at BASELINE config 5 otherwise)
-    x = np.array(pred_features, dtype=np.float64, copy=True) if feature_index_to_shuffle else \
-        np.ascontiguousarray(pred_features, dtype=np.float64)
-    if feature_index_to_shuffle:
-        if unlink_features_within_block and type(feature_index_to_shuffle) == list:
-            for fi in feature_index_to_shuffle:
-                x[:, fi] = np.random.permutation(x[:, fi])
-        else:
-            x[:, feature_index_to_shuffle] = np.random.permutation(x[:, feature_index_to_shuffle])
-    weights = [s["weights"] for s in post_samples]
-    if post_summary_mode not in (0, 1, 2):
-        raise ValueError("post_summary_mode must be 0 (argmax votes), 1 (mean softmax) or 2 (categorical resampling)")
-    eng = _predict_engine(weights[0], x.shape[1], actFun, output_act_fun)
-    al = _alpha_rows([s["alphas"] for s in post_samples], actFun, len(weights[0]))
-    if post_summary_mode == 2:
-        # sample_from_categorical (BNN_lib.py:682-713): the reference draws np.random.random(S) per instance in
-        # instance order; one (N, S) draw consumes the global stream identically.  The draw itself is fused into the
-        # prediction kernel, the [S, N, K] tensor is only produced when the caller wants it back.
-        dense = eng.predict(x, weights, alphas=al, mean=False, dense=True)["dense"] if return_dense else None
-        u, seed = _sampling_uniforms(x.shape[0], len(weights), rng)
-        res = eng.predict_sample(x, weights, u, alphas=al, post_predictions=False, seed=seed)
-        return dense, res["predictions"]
-    out = eng.predict(x, weights, alphas=al, mean=(post_summary_mode == 1), votes=(post_summary_mode == 0), dense=return_dense)
-    return out.get("dense"), out["votes" if post_summary_mode == 0 else "mean"]
-
-
 def sample_from_categorical(pred_features, post_samples, actFun=None, output_act_fun=None, rng=None,
                             post_predictions=True):
     """Posterior-predictive resampling with the outputs of the reference's sample_from_categorical
@@ -1425,15 +1385,10 @@ def sample_from_categorical(pred_features, post_samples, actFun=None, output_act
     weights = [s["weights"] for s in post_samples]
     eng = _predict_engine(weights[0], x.shape[1], actFun, output_act_fun)
     al = _alpha_rows([s["alphas"] for s in post_samples], actFun, len(weights[0]))
-    if _ranks() > 1:
-        from . import predshard
-        n, S = x.shape[0], len(weights)
-        sample = _sampling_kind(n, S, rng)
-        out = predshard.predict_ranks(eng, x, weights, al, sample=sample, post_predictions=post_predictions,
-                                      draw=lambda: ([],) + _sampling_uniforms(n, S, sample))
-        return {k: out[k] for k in ("predictions", "class_counts", "post_predictions")}
-    u, seed = _sampling_uniforms(x.shape[0], len(weights), rng)
-    return eng.predict_sample(x, weights, u, alphas=al, post_predictions=post_predictions, seed=seed)
+    n, S = x.shape[0], len(weights)
+    sample = _sampling_kind(n, S, rng)
+    return predshard.predict_ranks(eng, x, weights, al, sample=sample, post_predictions=post_predictions,
+                                   draw=lambda: ([],) + _sampling_uniforms(n, S, sample))
 
 
 def feature_importance(input_features, weights_pkl=None, weights_posterior=None, true_labels=[], fname_stem="",
@@ -1508,11 +1463,7 @@ def get_posterior_est(pkl_file):
         x = np.ascontiguousarray(x, dtype=np.float64)
         eng = _predict_engine(weights[0], x.shape[1], bnn_obj._act_fun, bnn_obj._output_act_fun)
         al = _alpha_rows([s["alphas"] for s in ps], bnn_obj._act_fun, len(weights[0]))
-        if _ranks() > 1:
-            from . import predshard
-            out = predshard.predict_ranks(eng, x, weights, al, mean=True, dense=True)
-        else:
-            out = eng.predict(x, weights, alphas=al, mean=True, dense=True)
+        out = predshard.predict_ranks(eng, x, weights, al, mean=True, dense=True)
         res["post_est" + key], res["prm_mean" + key] = out["dense"], out["mean"]
     return res
 
@@ -1542,18 +1493,14 @@ def get_pdp(data, focal_features, estimation_mode, size_output, actFun, output_a
     out = np.zeros((grid.shape[0], size_output, 3))
     eng = _predict_engine(weights[0], data.shape[1], actFun, output_act_fun)
     al = _alpha_rows(alphas, actFun, len(weights[0]))
-    if _ranks() > 1:
-        from . import predshard
-        # every rank scores its block and gets the full [N, K] mean: the row quantiles below need all rows
-        predict = lambda ov: predshard.predict_ranks(eng, data, weights, al, override=ov, mean=True)["mean"]  # noqa: E731
-    else:
-        predict = lambda ov: eng.predict(data, weights, alphas=al, override=ov, mean=True)["mean"]  # noqa: E731
     for n in range(grid.shape[0]):
         # the grid value is written first, the feature-indicator transform inside RunPredict then replaces masked
         # features by their mean (BNN_pdp.py:65-73, BNN_lib.py:248-249): the transform wins on a shared column
         ov = dict(zip([int(f) for f in focal_features], [float(v) for v in grid[n, :]]))
         ov.update(zip([int(cc) for cc in dt_cols], [float(v) for v in dt_vals]))
-        smean = predict((list(ov.keys()), list(ov.values())))
+        # every rank gets the full [N, K] mean: the row quantiles below need all rows
+        smean = predshard.predict_ranks(eng, data, weights, al, override=(list(ov.keys()), list(ov.values())),
+                                        mean=True)["mean"]
         if estimation_mode == "classification":
             smean = np.cumsum(smean, axis=1)
         out[n, :, 0] = np.mean(smean, axis=0)

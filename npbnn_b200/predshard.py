@@ -10,8 +10,10 @@ the Q partial sums of a row block ([rows, K] doubles, 20 MB at 250k rows) are ad
 split is already balanced.
 
 `predict_ranks` is the same grid behind the reference's prediction callers (api.get_posterior_cat_prob and everything
-built on it): every rank passes the caller's full arguments, scores its block and gets back the full arrays the
-single-process call returns.  It is collective: every rank of the process group calls it with the same arguments.
+built on it), in one process and on many ranks alike: every rank passes the caller's full arguments, scores its block
+and gets back the full arrays one process computes.  It is collective: every rank of the process group calls it with
+the same arguments.  One rank (no process group, or a group of one) scores the whole problem and makes no collective
+call.
 """
 import math
 from typing import Optional, Tuple
@@ -205,9 +207,10 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
                   sample=None, post_predictions=False, shuffle=(), draw=None, grid: Optional[Tuple[int, int]] = None):
     """Posterior prediction of all N rows of x over all S posterior samples, split over the ranks of the default process
     group.  Collective: every rank passes the same arguments (checked first, ValueError on every rank otherwise) and
-    returns the same dict of host arrays as the single-process engine calls:
+    returns the same dict of host arrays as the engine calls over the whole problem:
       mean [N, W], votes [N, W], dense [S, N, W]                     (Engine.predict; W = K, or the outputs)
-      predictions [N, K], class_counts [S, K], post_predictions [N, S] (Engine.predict_sample, with sample set)
+      predictions [N, K], class_counts [S, K], post_predictions [N, S] (Engine.predict_sample, with sample set;
+                                                                       post_predictions None unless asked for)
     x: the caller's full host features [N, F]; weight_sets: all S posterior samples; alphas: [S, L] or None; override:
     (cols, vals) column overwrite.  sample: None, "host" (reference uniforms) or "philox" (in-kernel uniforms, keyed on
     the global (row, sample) so the split does not change them).  shuffle: feature selectors whose rows are permuted.
@@ -217,7 +220,9 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
     The rank scores rows x samples block `partition(N, S, world, rank, grid)`; a rank with an empty block makes no kernel
     call but joins every collective.  Combination (one all-gather of every rank's block): means are sums over each sample
     group, added in sample-group order and divided by S once (with one sample group: the block's own mean); votes and
-    resampled shares are integer counts, added and divided by S once; class_counts are added over the row groups."""
+    resampled shares are integer counts, added and divided by S once; class_counts are added over the row groups.
+    With one rank the block is the whole problem and the engine's host outputs are returned as they are: no
+    torch.distributed call, no rescaling."""
     from . import _lib as L
     world, rank = ranks()
     x = np.ascontiguousarray(x, dtype=np.float64)
@@ -225,29 +230,51 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
     S = len(weight_sets)
     W = engine.K if engine.net.lik == L.LIK_CATEGORICAL else engine.O
     K = engine.K
-    ov = None if override is None else (tuple(int(c) for c in override[0]), tuple(float(v) for v in override[1]))
     shuffle = list(shuffle)
-    agree((n, f, S, W, engine.net.n_params, engine.net.act, engine.net.lik, bool(mean), bool(votes), bool(dense), sample,
-           bool(post_predictions), [tuple(_columns(s, f)) for s in shuffle], ov, grid))
+    if world > 1:
+        ov = None if override is None else (tuple(int(c) for c in override[0]), tuple(float(v) for v in override[1]))
+        agree((n, f, S, W, engine.net.n_params, engine.net.act, engine.net.lik, bool(mean), bool(votes), bool(dense),
+               sample, bool(post_predictions), [tuple(_columns(s, f)) for s in shuffle], ov, grid))
     if sample not in (None, "host", "philox"):
         raise ValueError("sample must be None, 'host' or 'philox'")
     rows, sets, grid, _, _ = partition(n, S, world, rank, grid)
     R, Q = grid
     (a, b), (c, d) = rows, sets
     n_loc, s_loc = b - a, d - c
-    dev = comm_device()
 
-    # draws from numpy's global stream: rank 0's, the ones a single-process run makes
-    drawn = draw() if rank == 0 and draw is not None else ([None] * len(shuffle), None, None)
-    perms = []
-    if shuffle:
-        pm = from_rank0(np.stack(drawn[0]) if rank == 0 else None, (len(shuffle), n), torch.int64)
-        perms = list(pm.cpu().numpy())
-    u = seed = None
-    if sample == "host":
-        u = from_rank0(drawn[1] if rank == 0 else None, (n, S), torch.float64)
-    elif sample == "philox":
-        seed = int(from_rank0(np.array([drawn[2] if rank == 0 else 0], dtype=np.int64), (1,), torch.int64).item())
+    # draws from numpy's global stream: rank 0's, the ones one process makes
+    perms, u, seed = draw() if rank == 0 and draw is not None else ([None] * len(shuffle), None, None)
+    if world > 1:
+        if shuffle:
+            perms = list(from_rank0(np.stack(perms) if rank == 0 else None, (len(shuffle), n), torch.int64).cpu().numpy())
+        if sample == "host":
+            u = from_rank0(u, (n, S), torch.float64)
+        elif sample == "philox":
+            seed = int(from_rank0(np.array([seed if rank == 0 else 0], dtype=np.int64), (1,), torch.int64).item())
+
+    out = {}
+    if (n_loc and s_loc) or world == 1:       # one rank calls the engine even on an empty problem, which it refuses
+        xb = permuted_rows(x, a, b, shuffle, perms) if shuffle else x[a:b]
+        w = weight_sets[c:d]
+        al = None if alphas is None else np.asarray(alphas)[c:d]
+        if mean or votes or dense:
+            out.update(engine.predict(xb, w, alphas=al, override=override, mean=mean, votes=votes, dense=dense,
+                                      device_out=world > 1))
+        if sample:
+            out.update(engine.predict_sample(xb, w, None if u is None else u[a:b, c:d], alphas=al,
+                                             post_predictions=post_predictions, seed=seed, row0=a, set0=c,
+                                             device_out=world > 1))
+    if world == 1:
+        return out
+
+    # the block as the combination adds it: sums over the rank's samples, integer counts
+    if out:
+        if mean and Q > 1:
+            out["mean"] = out["mean"] * float(s_loc)
+        if votes:
+            out["votes"] = torch.round(out["votes"] * float(s_loc))
+        if sample:
+            out["predictions"] = torch.round(out["predictions"] * float(s_loc))
 
     names = [k for k, on in zip(_OUTPUTS, (mean, votes, sample, sample, sample and post_predictions, dense)) if on]
 
@@ -255,33 +282,13 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
         return {"mean": (nl, W), "votes": (nl, W), "predictions": (nl, K), "class_counts": (sl, K),
                 "post_predictions": (nl, sl), "dense": (sl, nl, W)}
 
-    parts = {}
-    if n_loc and s_loc:
-        xb = permuted_rows(x, a, b, shuffle, perms) if shuffle else x[a:b]
-        w = weight_sets[c:d]
-        al = None if alphas is None else np.asarray(alphas)[c:d]
-        if mean or votes or dense:
-            o = engine.predict(xb, w, alphas=al, override=override, mean=mean, votes=votes, dense=dense, device_out=True)
-            if mean:
-                parts["mean"] = o["mean"] if Q == 1 else o["mean"] * float(s_loc)
-            if votes:
-                parts["votes"] = torch.round(o["votes"] * float(s_loc))
-            if dense:
-                parts["dense"] = o["dense"]
-        if sample:
-            r = engine.predict_sample(xb, w, None if u is None else u[a:b, c:d], alphas=al,
-                                      post_predictions=post_predictions, seed=seed, row0=a, set0=c, device_out=True)
-            parts["predictions"] = torch.round(r["predictions"] * float(s_loc))
-            parts["class_counts"] = r["class_counts"]
-            if post_predictions:
-                parts["post_predictions"] = r["post_predictions"]
-
     # one all-gather of every rank's blocks, packed into one vector padded to the longest
+    dev = comm_device()
     blocks = [partition(n, S, world, q, grid)[:2] for q in range(world)]
     lens = [sum(int(np.prod(sizes(rb - ra, sb - sa)[k])) for k in names) for (ra, rb), (sa, sb) in blocks]
     send = torch.zeros(max(lens), dtype=torch.float64, device=dev)
-    if parts:
-        send[:lens[rank]] = torch.cat([parts[k].to(device=dev, dtype=torch.float64).reshape(-1) for k in names])
+    if out:
+        send[:lens[rank]] = torch.cat([out[k].to(device=dev, dtype=torch.float64).reshape(-1) for k in names])
     recv = [torch.empty_like(send) for _ in range(world)]
     dist.all_gather(recv, send)
 

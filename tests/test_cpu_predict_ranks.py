@@ -4,7 +4,9 @@ output conventions, so that every rank layout can be compared with the single-pr
   * the combine and gather of row x sample blocks, empty row blocks (N < world) and empty sample blocks (S < Q) included;
   * the draws of rank 0 (permutations of shuffled feature blocks, host uniforms, Philox seeds) reach every rank, are the
     draws the single-process call makes, and leave the other ranks' np.random state as it was;
-  * ranks called with different arguments all raise ValueError."""
+  * ranks called with different arguments all raise ValueError;
+  * one rank, with no process group or in a group of one, returns the engine's own results for the whole problem, makes
+    the reference's draws and no collective call."""
 import json
 import os
 import subprocess
@@ -216,3 +218,107 @@ def test_rank_layouts_return_the_single_process_results(world, tmp_path):
             kept = [k for k in info if k.endswith("_kept")]
             assert len(kept) == 5 * 6 and all(info[k] for k in kept), (r, info)
         assert info["mismatch_raised"], (r, info)
+
+
+def _forbidden(name):
+    def call(*a, **k):
+        raise AssertionError("one rank made a collective call: torch.distributed.%s" % name)
+    return call
+
+
+def _one_rank_is_the_engine(eng):
+    """The callers on one rank against the engine calls on a copy of x permuted in place by
+    x[:, fi] = np.random.permutation(x[:, fi]): the same bits, and the same np.random state afterwards."""
+    import npbnn_b200 as bn
+    n, S = 37, 5
+    x = np.random.default_rng(2).standard_normal((n, 6))
+    rs = np.random.default_rng(3)
+    ps = [{"weights": [rs.normal(0, 1.0, (6, 4))], "alphas": [0.0]} for _ in range(S)]
+    w = [p["weights"] for p in ps]
+    af = bn.ActFun(fun="swish")
+    kw = dict(actFun=af, output_act_fun=bn.SoftMax)
+
+    def same(call, ref, seed):
+        np.random.seed(seed)
+        want = ref()
+        state = np.random.get_state()
+        np.random.seed(seed)
+        got = call()
+        assert np.array_equal(np.random.get_state()[1], state[1]) and np.random.get_state()[2] == state[2]
+        return got, want
+
+    for fis, unlink in ((None, False), ([0, 3], True), ([1, 2, 4], False), ([5, 5], True), (2, False)):
+        def ref_cat_prob(mode):
+            xr = x.copy()
+            if fis:
+                for fi in (fis if unlink and type(fis) == list else [fis]):
+                    xr[:, fi] = np.random.permutation(xr[:, fi])
+            if mode == 2:
+                dense = eng.predict(xr, w, mean=False, dense=True)["dense"]
+                return dense, eng.predict_sample(xr, w, np.random.random((n, S)), post_predictions=False)["predictions"]
+            o = eng.predict(xr, w, mean=mode == 1, votes=mode == 0, dense=True)
+            return o["dense"], o["votes" if mode == 0 else "mean"]
+
+        for mode in (0, 1, 2):
+            got, want = same(lambda: bn.get_posterior_cat_prob(x, ps, feature_index_to_shuffle=fis,
+                                                                unlink_features_within_block=unlink,
+                                                                post_summary_mode=mode, rng="host", **kw),
+                             lambda: ref_cat_prob(mode), 5)
+            assert all(np.array_equal(g, r) for g, r in zip(got, want)), (fis, mode)
+    # an invalid mode raises before any draw
+    np.random.seed(5)
+    state = np.random.get_state()[1].copy()
+    with pytest.raises(ValueError):
+        bn.get_posterior_cat_prob(x, ps, feature_index_to_shuffle=[0, 3], post_summary_mode=3, **kw)
+    assert np.array_equal(np.random.get_state()[1], state)
+
+    def ref_sample(rng):
+        if rng == "host":
+            return eng.predict_sample(x, w, np.random.random((n, S)))
+        return eng.predict_sample(x, w, seed=int(np.random.randint(0, 2 ** 31 - 1)) * 2654435761 + 1)
+
+    for rng in ("host", "philox"):
+        got, want = same(lambda: bn.sample_from_categorical(x, ps, rng=rng, **kw), lambda: ref_sample(rng), 11)
+        assert set(got) == set(want) and all(np.array_equal(got[k], want[k]) for k in want), rng
+
+    def ref_pdp():
+        grid = bn.make_pdp_features(x, [1])
+        out = np.zeros((len(grid), 4, 3))
+        for i, v in enumerate(grid[:, 0]):
+            m = np.cumsum(eng.predict(x, w, override=([1], [float(v)]), mean=True)["mean"], axis=1)
+            out[i, :, 0] = np.mean(m, axis=0)
+            out[i, :, 1], out[i, :, 2] = np.quantile(m, q=(0.025, 0.975), axis=0)
+        return out
+
+    got, want = same(lambda: bn.get_pdp(x, [1], "classification", 4, af, bn.SoftMax, w, [p["alphas"] for p in ps],
+                                        None)["pdp"], ref_pdp, 13)
+    assert np.array_equal(got, want)
+
+
+@pytest.fixture
+def fake_engine(monkeypatch):
+    from npbnn_b200 import api
+    ns = {}
+    exec(FAKE_ENGINE, ns)
+    eng = ns["FakeEngine"](6, 4)
+    monkeypatch.setattr(api, "_predict_engine", lambda *a, **k: eng)
+    return eng
+
+
+def test_one_process_returns_the_engine_results(fake_engine):
+    import torch.distributed as dist
+    assert not dist.is_initialized()
+    _one_rank_is_the_engine(fake_engine)
+
+
+def test_group_of_one_rank_makes_no_collective_call(fake_engine, monkeypatch, tmp_path):
+    import torch.distributed as dist
+    from npbnn_b200 import predshard
+    dist.init_process_group("gloo", init_method="file://%s" % (tmp_path / "store"), rank=0, world_size=1)
+    try:
+        assert predshard.ranks() == (1, 0)
+        for name in ("all_gather", "all_gather_object", "broadcast", "broadcast_object_list", "all_reduce"):
+            monkeypatch.setattr(dist, name, _forbidden(name))
+        _one_rank_is_the_engine(fake_engine)
+    finally:
+        dist.destroy_process_group()
