@@ -288,6 +288,20 @@ int bnn_predict(bnn_ctx* ctx, const double* x_dev, int64_t n, const double* w_de
                 const double* alpha_dev, const int32_t* override_cols, const double* override_vals,
                 int32_t n_override, double* mean_dev, double* votes_dev, double* dense_dev, void* stream);
 
+/* Zero pattern of the weight sets the prediction calls below will score: mask_host [n_params] in the canonical layout,
+ * 0 where every weight set is exactly zero (e.g. the union over the posterior samples of w != 0 of a block-masked
+ * network, create_mask / apply_mask), NULL clears it.  While a pattern is set and option "sparse" is 1, bnn_predict,
+ * bnn_predict_sample and bnn_predict_sample_philox(_at) run the block-sparse kernels on the program of the pattern
+ * (bnn_last_kernel: "k_fwd_sparse<pairs,predict>" or "k_fwd_sparse<predict>"): same outputs as the dense kernels up to
+ * the order of the sums, each row's sums over the sets in set order.  Each call first checks on the device that every
+ * weight set is zero outside the pattern and runs the dense kernels when one is not; that check reads one flag back, so
+ * with a pattern set these calls wait on the host for the stream's work up to the check (without one they stay
+ * asynchronous).  The program is built per pattern and padded layout and kept while the pattern does not change;
+ * bnn_set_net clears the pattern.  When the pattern's block cover is not thin enough (or
+ * the network has no hidden layer, more than 8 outputs, or a program too large for shared memory) the call succeeds and
+ * prediction stays dense.  Option "predict_tf32" does not apply to the block-sparse kernels. */
+int bnn_set_predict_mask(bnn_ctx* ctx, const double* mask_host);
+
 /* Number of kernel launches issued by this context so far (bench.py's gpu_launches). */
 int64_t bnn_launch_count(const bnn_ctx* ctx);
 /* With option "time_forward" = 1 every forward launch is bracketed by CUDA events on its stream; this

@@ -101,6 +101,7 @@ _SIGNATURES = {
                                                C.c_void_p]),
     "bnn_predict_sample": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "bnn_set_predict_mask": (C.c_int, [C.c_void_p, C.c_void_p]),
     "bnn_launch_count": (C.c_int64, [C.c_void_p]),
     "bnn_last_kernel": (C.c_char_p, [C.c_void_p]),
     "bnn_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int]),

@@ -1302,7 +1302,8 @@ def RunPredict(data, weights, actFun, output_act_fun, data_transform=None):
     if data_transform is not None:
         cols, vals = data_transform.override()
         ov = (cols, vals) if len(cols) else None
-    return eng.predict(data, [weights], alphas=al, override=ov, mean=False, dense=True)["dense"][0]
+    return eng.predict(data, [weights], alphas=al, override=ov, mean=False, dense=True,
+                       pattern=predshard.zero_pattern([weights], eng.net))["dense"][0]
 
 
 def RunPredictInd(data, weights, ind, actFun, output_act_fun, data_transform=None):
@@ -1345,6 +1346,19 @@ def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_sh
     """BNN_lib.py:352-397 with all posterior samples scored in ONE pass over the features.
     return_dense=False skips the [S, N, K] tensor (it is 800 GB at BASELINE config 5) and returns None for it.  Mode 2
     resamples as sample_from_categorical (BNN_lib.py:682-713), inside the prediction kernel."""
+    return _posterior_cat_prob(pred_features, post_samples, feature_index_to_shuffle, post_summary_mode,
+                               unlink_features_within_block, actFun, output_act_fun, return_dense, rng)
+
+
+def _samples_pattern(post_samples, n_features, actFun, output_act_fun):
+    """predshard.zero_pattern of the posterior samples (list of dicts), for callers that score them many times."""
+    weights = [s["weights"] for s in post_samples]
+    return predshard.engine_pattern(_predict_engine(weights[0], n_features, actFun, output_act_fun), weights)
+
+
+def _posterior_cat_prob(pred_features, post_samples, feature_index_to_shuffle, post_summary_mode,
+                        unlink_features_within_block, actFun, output_act_fun, return_dense, rng, pattern="auto"):
+    """get_posterior_cat_prob with the samples' zero pattern given (pattern="auto": computed here)."""
     if len(pred_features) == 0:
         print("Data not found.")
         return 0
@@ -1371,7 +1385,7 @@ def get_posterior_cat_prob(pred_features, post_samples=None, feature_index_to_sh
         return perms, u, seed
 
     out = predshard.predict_ranks(eng, x, weights, al, mean=post_summary_mode == 1, votes=post_summary_mode == 0,
-                                  dense=return_dense, sample=sample, shuffle=shuffle, draw=draw)
+                                  dense=return_dense, sample=sample, shuffle=shuffle, draw=draw, pattern=pattern)
     summary = {0: "votes", 1: "mean", 2: "predictions"}[post_summary_mode]
     return out.get("dense"), out[summary]
 
@@ -1416,8 +1430,11 @@ def feature_importance(input_features, weights_pkl=None, weights_posterior=None,
         bnn_obj, mcmc_obj, logger_obj = load_obj(weights_pkl)
         weights_posterior = logger_obj._post_weight_samples
         actFun, output_act_fun = bnn_obj._act_fun, bnn_obj._output_act_fun
-    kw = dict(post_summary_mode=post_summary_mode, actFun=actFun, output_act_fun=output_act_fun, return_dense=False)
-    _, pred = get_posterior_cat_prob(input_features, weights_posterior, **kw)
+    # the samples' zero pattern once for the 1 + blocks x n_permutations passes over the same samples
+    pattern = _samples_pattern(weights_posterior, np.asarray(input_features).shape[1], actFun, output_act_fun)
+    kw = dict(post_summary_mode=post_summary_mode, actFun=actFun, output_act_fun=output_act_fun, return_dense=False,
+              rng=None, pattern=pattern)
+    _, pred = _posterior_cat_prob(input_features, weights_posterior, None, unlink_features_within_block=False, **kw)
     ref_accuracy = CalcAccuracy(pred, true_labels)
     if verbose:
         print("Reference accuracy (mean):", np.mean(ref_accuracy))
@@ -1427,8 +1444,8 @@ def feature_importance(input_features, weights_pkl=None, weights_posterior=None,
             print("Processing feature block %i", block_id + 1)
         accs = []
         for _ in np.arange(n_permutations):
-            _, pred = get_posterior_cat_prob(input_features, weights_posterior, feature_index_to_shuffle=feature_block,
-                                             unlink_features_within_block=unlink_features_within_block, **kw)
+            _, pred = _posterior_cat_prob(input_features, weights_posterior, feature_block,
+                                          unlink_features_within_block=unlink_features_within_block, **kw)
             accs.append(CalcAccuracy(pred, true_labels))
         accuracies_wo_feature.append(accs)
     accuracies_wo_feature = np.array(accuracies_wo_feature)
@@ -1493,6 +1510,7 @@ def get_pdp(data, focal_features, estimation_mode, size_output, actFun, output_a
     out = np.zeros((grid.shape[0], size_output, 3))
     eng = _predict_engine(weights[0], data.shape[1], actFun, output_act_fun)
     al = _alpha_rows(alphas, actFun, len(weights[0]))
+    pattern = predshard.engine_pattern(eng, weights)        # once for all grid steps
     for n in range(grid.shape[0]):
         # the grid value is written first, the feature-indicator transform inside RunPredict then replaces masked
         # features by their mean (BNN_pdp.py:65-73, BNN_lib.py:248-249): the transform wins on a shared column
@@ -1500,7 +1518,7 @@ def get_pdp(data, focal_features, estimation_mode, size_output, actFun, output_a
         ov.update(zip([int(cc) for cc in dt_cols], [float(v) for v in dt_vals]))
         # every rank gets the full [N, K] mean: the row quantiles below need all rows
         smean = predshard.predict_ranks(eng, data, weights, al, override=(list(ov.keys()), list(ov.values())),
-                                        mean=True)["mean"]
+                                        mean=True, pattern=pattern)["mean"]
         if estimation_mode == "classification":
             smean = np.cumsum(smean, axis=1)
         out[n, :, 0] = np.mean(smean, axis=0)

@@ -102,7 +102,18 @@ struct bnn_ctx {
   const char* last_kernel = "";
   // block-masked networks: dataflow program of the chains' mask (bnn_sparse.cu); sp.prog null: the dense kernels run
   struct { DevBuf prog, widx; SparseParams sp{}; } sparse;
-  int opt_sparse = 1;               // option "sparse": 0 forces the dense kernels for masked chains
+  int opt_sparse = 1;               // option "sparse": 0 forces the dense kernels for masked chains and for prediction
+  // posterior prediction of block-masked networks (bnn_set_predict_mask): the zero pattern [P] (0/1) and its device copy,
+  // and the program built from it for the padded layout `geom` (sp.prog null: the builder declined, the dense kernels
+  // run).  Separate from the chains' program: prediction picks its padding from its own row count.
+  struct {
+    std::vector<double> mask;
+    bool active = false;            // a pattern is set (NULL clears it; the program is kept for the next same pattern)
+    bool built = false;
+    NetGeom geom{};
+    DevBuf mask_dev, prog, widx, flag;
+    SparseParams sp{};
+  } pred_sparse;
   // optional per-launch timing of the forward kernel (bench.py roofline): event pairs on the launch stream
   int time_forward = 0;
   std::vector<cudaEvent_t> ev;      // start/stop pairs, recorded but not yet read
@@ -395,6 +406,11 @@ int bnn_set_net(bnn_ctx* c, const bnn_net_spec* s) {
   c->have_net = true;
   c->have_data = false;
   c->have_chains = false;
+  // a prediction pattern belongs to the previous network (its length and layout): gone with it
+  c->pred_sparse.active = false;
+  c->pred_sparse.built = false;
+  c->pred_sparse.mask.clear();
+  c->pred_sparse.sp = SparseParams{};
   return 0;
 }
 
@@ -1246,6 +1262,30 @@ int bnn_chains_set_temperature(bnn_ctx* c, const double* temperature_host, void*
   return 0;
 }
 
+// the prediction program of the pattern set by bnn_set_predict_mask for the padded layout g (built once per pattern and
+// layout); c->pred_sparse.sp.prog stays null when the builder declines or the program does not fit the prediction kernel
+static int pred_program(bnn_ctx* c, const NetGeom& g, cudaStream_t st) {
+  auto& ps = c->pred_sparse;
+  if (ps.built && same_layout(ps.geom, g)) return 0;
+  ps.sp = SparseParams{};
+  SparseProgram sp;
+  if (bnn_sparse_build(g, ps.mask.data(), &sp)) {
+    FwdParams probe{};
+    probe.g = g;
+    probe.sp = sp.sp;
+    if (bnn_sparse_predict_fits(probe)) {
+      if (upload(ps.prog, sp.prog.data(), sp.prog.size(), st)) return 1;
+      if (upload(ps.widx, sp.widx.data(), sp.widx.size(), st)) return 1;
+      ps.sp = sp.sp;
+      ps.sp.prog = ps.prog.as<int>();
+      ps.sp.widx = ps.widx.as<int>();
+    }
+  }
+  ps.geom = g;
+  ps.built = true;
+  return 0;
+}
+
 static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,
                         const double* alpha_dev, const int32_t* override_cols, const double* override_vals,
                         int32_t n_override, double* mean_dev, double* votes_dev, double* dense_dev, const double* u_dev,
@@ -1283,8 +1323,22 @@ static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double
   p.samp_u = u_dev; p.samp_counts = class_counts_dev; p.samp_dense = post_pred_dev;
   p.samp_philox = samp_philox ? 1 : 0; p.samp_seed = samp_seed;
   p.samp_row0 = samp_row0; p.samp_set0 = samp_set0;
+  if (c->opt_sparse && c->pred_sparse.active && c->pred_sparse.mask.size() == (size_t)g.P) {
+    // block-masked network: its program, if every weight set is zero outside the pattern (else the dense kernels)
+    auto& ps = c->pred_sparse;
+    if (int rc = pred_program(c, g, st)) return rc;
+    if (ps.sp.prog) {
+      CUDA_TRY(ps.flag.ensure(sizeof(int), false, st));
+      CUDA_TRY(bnn_launch_mask_violations(w_dev, n_sets, g.P, ps.mask_dev.as<double>(), ps.flag.as<int>(), c->n_sms, st));
+      c->launches++;
+      int bad = 1;
+      CUDA_TRY(cudaMemcpyAsync(&bad, ps.flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+      CUDA_TRY(cudaStreamSynchronize(st));
+      if (!bad) p.sp = ps.sp;
+    }
+  }
   if (class_counts_dev) CUDA_TRY(cudaMemsetAsync(class_counts_dev, 0, sizeof(int32_t) * (size_t)n_sets * g.K, st));
-  if (c->opt_pred_tf32 && !c->force_generic && bnn_pred_tf32_fits(p)) {
+  if (c->opt_pred_tf32 && !c->force_generic && !p.sp.prog && bnn_pred_tf32_fits(p)) {
     // opt-in reduced precision (stated tolerance: class probabilities to ~1e-6 absolute); summaries only
     CUDA_TRY(bnn_launch_pred_tf32(p, c->n_sms, c->opt_pred_tf32 >= 2 ? 1 : 3, st, &c->last_kernel));
     c->launches += 3;
@@ -1300,6 +1354,25 @@ int bnn_predict(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev,
                 int32_t n_override, double* mean_dev, double* votes_dev, double* dense_dev, void* stream) {
   return predict_impl(c, x_dev, n, w_dev, n_sets, alpha_dev, override_cols, override_vals, n_override, mean_dev,
                       votes_dev, dense_dev, nullptr, nullptr, nullptr, stream);
+}
+
+int bnn_set_predict_mask(bnn_ctx* c, const double* mask_host) {
+  REQUIRE(c && c->have_net, "bnn_set_predict_mask: call bnn_set_net first");
+  auto& ps = c->pred_sparse;
+  if (!mask_host) {
+    ps.active = false;
+    return 0;
+  }
+  std::vector<double> m((size_t)c->g.P);
+  for (size_t i = 0; i < m.size(); ++i) m[i] = mask_host[i] != 0.0 ? 1.0 : 0.0;
+  ps.active = true;
+  if (m == ps.mask) return 0;                          // same pattern: the programs built for it stay
+  CUDA_TRY(cudaSetDevice(c->device));
+  ps.mask.swap(m);
+  ps.built = false;
+  CUDA_TRY(ps.mask_dev.ensure(sizeof(double) * ps.mask.size(), false, 0));
+  CUDA_TRY(cudaMemcpy(ps.mask_dev.p, ps.mask.data(), sizeof(double) * ps.mask.size(), cudaMemcpyHostToDevice));
+  return 0;
 }
 
 int bnn_predict_sample_philox_at(bnn_ctx* c, const double* x_dev, int64_t n, const double* w_dev, int32_t n_sets,

@@ -1017,7 +1017,7 @@ static cudaError_t launch_generic(const FwdParams& p, int n_sms, cudaStream_t st
 cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int force_generic, cudaStream_t st,
                                const char** which) {
   const NetGeom& g = p.g;
-  if (p.sp.prog && !predict) return bnn_launch_sparse(p, n_sms, st, which);
+  if (p.sp.prog) return predict ? bnn_launch_sparse_predict(p, n_sms, st, which) : bnn_launch_sparse(p, n_sms, st, which);
   if (!force_generic && !p.samp_u) {
     static const char* const names[2][4] = {
         {"k_fwd3<relu,64,64,32>", "k_fwd3<leaky,64,64,32>", "k_fwd3<swish,64,64,32,16>", "k_fwd3<tanh,64,64,32>"},

@@ -85,6 +85,13 @@ struct SparseProgram {
 };
 bool bnn_sparse_build(const NetGeom& g, const double* mask, SparseProgram* out);
 cudaError_t bnn_launch_sparse(const FwdParams& p, int n_sms, cudaStream_t st, const char** which);
+// Prediction mode of the same program (mean / votes / dense / resampling outputs of FwdParams): thread = row, the sets
+// of the launch summed in order 0 ... C-1.  bnn_sparse_predict_fits: the program fits the prediction kernel's shared
+// memory.  bnn_launch_mask_violations: *flag = 1 if an entry that `mask` [P] drops is nonzero in a canonical set of w.
+bool bnn_sparse_predict_fits(const FwdParams& p);
+cudaError_t bnn_launch_sparse_predict(const FwdParams& p, int n_sms, cudaStream_t st, const char** which);
+cudaError_t bnn_launch_mask_violations(const double* w, int n_sets, int P, const double* mask, int* flag, int n_sms,
+                                       cudaStream_t st);
 // opt-in reduced-precision posterior prediction (bnn_pred_lp.cu): 3xTF32 tensor-core contractions, FP32 activations /
 // softmax, FP64 accumulation over the samples; summaries of the 64-64-32-16 categorical family only
 bool bnn_pred_tf32_fits(const FwdParams& p);

@@ -731,3 +731,310 @@ static cudaError_t launch_sparse_t(const FwdParams& p, int n_sms, cudaStream_t s
 cudaError_t bnn_launch_sparse(const FwdParams& p, int n_sms, cudaStream_t st, const char** which) {
   return bnn_with_act(p.g.act, [&](auto a) { return launch_sparse_t<decltype(a)::value>(p, n_sms, st, which); });
 }
+
+// =============================================================================================
+// prediction mode: posterior summaries over S weight sets (bnn_predict / bnn_predict_sample*)
+// =============================================================================================
+// Same program, same weight stream, same item functions as the likelihood kernels above, but the loops are turned
+// around: a warp keeps ONE 32-row tile (thread = row) and walks every weight set in order 0, 1, ..., S-1, so each row's
+// sums over the sets run in that fixed order whatever n, the tile, the launch geometry or the GPU.  S can be 10,000:
+// the sets are streamed through shared memory in groups of sp.group, double-buffered (cp.async gathers group i + 1 from
+// the packed sets while group i is evaluated); the X tile and the per-row accumulators (mean [K_out], votes [K_out])
+// stay in the warp's shared memory for the whole walk.  A CTA owns a contiguous range of tiles and runs it in rounds
+// of one tile per warp.  The epilogue is the generic kernel's prediction epilogue (bnn_epilogue<true>) per thread.
+constexpr int SPP_NCH = 2;               // weight sets a thread evaluates together
+constexpr int SPP_MAX_WARPS = 16;        // <= 128 registers
+constexpr int SPP_ZS = SP_MAX_O + 1;     // per-row stride of the accumulators
+
+__device__ __forceinline__ void cp_async8(double* dst, const double* src) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(dst)), "l"(src) : "memory");
+}
+
+// transformed outputs of one (row, set) into the row's accumulators; sampling / dense outputs as the dense kernels.
+// This is the prediction branch of bnn_epilogue<true> (bnn_generic_body.cuh) for one thread's row with the outputs in
+// registers, in the same operation order; the two must change together.
+__device__ __forceinline__ void sparse_pred_epilogue(const FwdParams& p, int c, long long row, bool active,
+                                                     const double (&z)[SP_MAX_O], const double* tab, double* pa, int* pv) {
+  const NetGeom& g = p.g;
+  if (g.lik == BNN_LIK_CATEGORICAL) {
+    const int K = g.K;
+    double m = z[0];
+    int arg = 0;
+#pragma unroll
+    for (int k = 1; k < SP_MAX_O; ++k)
+      if (k < K && z[k] > m) { m = z[k]; arg = k; }    // first maximum wins, as np.argmax
+    double e[SP_MAX_O], S = 0.0;
+#pragma unroll
+    for (int k = 0; k < SP_MAX_O; ++k)
+      if (k < K) { e[k] = bnn_exp_neg<BNN_EXP_TAB_BITS>(z[k] - m, tab); S += e[k]; }
+    const double inv = 1.0 / S;
+    const bool sampling = p.samp_u || p.samp_philox;
+    double u = 0.0;
+    if (active && sampling)
+      u = p.samp_u ? p.samp_u[row * p.C + c] : bnn_samp_uniform(p.samp_seed, p.samp_row0 + row, p.samp_set0 + c);
+    double cum = 0.0;
+    int drawn = -1;
+#pragma unroll
+    for (int k = 0; k < SP_MAX_O; ++k) {
+      if (k < K) {
+        const double pk = e[k] * inv;
+        cum += pk;
+        if (drawn < 0 && cum - u >= 0.0) drawn = k;
+        if (active) {
+          pa[k] += pk;
+          if (p.dense_out) p.dense_out[((long long)c * p.n_total + row) * K + k] = pk;
+        }
+      }
+    }
+    if (sampling) {
+      arg = drawn < 0 ? 0 : drawn;
+      if (active && p.samp_dense) p.samp_dense[row * p.C + c] = (double)arg;
+    }
+    if (active) pv[arg] += 1;
+    if (sampling && p.samp_counts) {
+      // one atomic per distinct class among the rows of the tile
+      const unsigned grp = __match_any_sync(FULL_MASK, active ? arg : 64 + (int)(threadIdx.x & 31));
+      if (active && (int)(threadIdx.x & 31) == __ffs(grp) - 1) atomicAdd(&p.samp_counts[c * K + arg], __popc(grp));
+    }
+    return;
+  }
+  if (!active) return;
+  const int O = g.O, K = g.K;
+  const bool head = (g.lik == BNN_LIK_GAUSSIAN_HEAD);
+#pragma unroll
+  for (int j = 0; j < SP_MAX_O; ++j) {
+    if (j < O) {
+      double v = z[j];
+      if (head && j >= K) v = softplus_ref(v);
+      pa[j] += v;
+      if (p.dense_out) p.dense_out[((long long)c * p.n_total + row) * O + j] = v;
+    }
+  }
+}
+
+// NR1 == 0: the program interpreter (sparse_item); otherwise uniform block pairs (sparse_pair) of that shape
+template <int ACT, int NR1, int NR2, int NC1>
+__global__ void __launch_bounds__(SPP_MAX_WARPS * 32, 1) k_pred_sparse(const __grid_constant__ FwdParams p) {
+  constexpr int NCH = SPP_NCH;
+  constexpr bool PAIRS = NR1 > 0;
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  const NetGeom& g = p.g;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  const int O = g.O;
+  const int G = p.sp.group;                                   // weight sets per shared-memory buffer
+  const int wlen = p.sp.wlen;
+  const int sq = p.sp.slots * SP_US;
+  const int per_warp = (g.F + (PAIRS ? 0 : NCH * p.sp.slots)) * SP_US + 32 * SPP_ZS;
+
+  double* tab = reinterpret_cast<double*>(smem_raw);
+  double* wsm = tab + BNN_EXP_TAB_SIZE;                       // [2][G][wlen]
+  double* buf = wsm + 2 * (size_t)G * wlen + (size_t)warp * per_warp;           // X tile (+ scratch slots)
+  double* pacc = buf + (per_warp - 32 * SPP_ZS);              // [32][SPP_ZS]
+  const size_t n_dbl = (BNN_EXP_TAB_SIZE + 2 * (size_t)G * wlen + (size_t)nwarps * per_warp + 1) & ~(size_t)1;
+  int* prog = reinterpret_cast<int*>(reinterpret_cast<double*>(smem_raw) + n_dbl);
+  int* pvote = prog + ((p.sp.prog_len + 3) & ~3) + warp * 32 * SPP_ZS;
+
+  for (int i = threadIdx.x; i < BNN_EXP_TAB_SIZE; i += blockDim.x) tab[i] = p.exp_tab[i];
+  for (int i = threadIdx.x; i < p.sp.prog_len; i += blockDim.x) prog[i] = p.sp.prog[i];
+
+  const long long n_tiles32 = (p.n_tiles16 + 1) >> 1;
+  const long long n_pad = p.n_tiles16 * 16;
+  const long long t0 = n_tiles32 * blockIdx.x / gridDim.x, t1 = n_tiles32 * (blockIdx.x + 1) / gridDim.x;
+  const int n_grp = (p.C + G - 1) / G;
+  const double* bufl = buf + lane;
+  double* pa = pacc + lane * SPP_ZS;
+  int* pv = pvote + lane * SPP_ZS;
+
+  // group gi of the weight sets -> buffer b, gathered in program order (sp.widx)
+  auto load_group = [&](int gi, int b) {
+    const int s0 = gi * G, gc = min(G, p.C - s0);
+    double* dst = wsm + (size_t)b * G * wlen;
+    for (int i = threadIdx.x; i < gc * wlen; i += blockDim.x) {
+      const int c = i / wlen, j = i - c * wlen;
+      const int idx = __ldg(p.sp.widx + j);
+      if (idx < 0) dst[i] = 0.0;
+      else cp_async8(dst + i, p.wp + (long long)(s0 + c) * g.PB + idx);
+    }
+    asm volatile("cp.async.commit_group;" ::: "memory");
+  };
+
+  for (long long base = t0; base < t1; base += nwarps) {
+    const long long w32 = base + warp;
+    const bool have = w32 < t1;                                // (warps without a tile still join the barriers)
+    const long long row = w32 * 32 + lane;
+    const bool active = have && row < p.n_total;
+    if (have) {
+      // X tile -> [feature][row]; global reads are contiguous (32 * F_pad consecutive doubles).  The same staging as
+      // k_fwd_sparse's, kept as a copy so that the likelihood kernel's code and schedule stay as they are.
+      const double* xt = p.x + w32 * 32 * (long long)g.F_pad;
+      for (int j0 = 0; j0 < g.F_pad; j0 += 8) {
+        double v[8];
+#pragma unroll
+        for (int uu = 0; uu < 8; ++uu) {
+          const int idx = (j0 + uu) * 32 + lane;
+          v[uu] = (w32 * 32 + idx / g.F_pad < n_pad) ? __ldg(xt + idx) : 0.0;
+        }
+#pragma unroll
+        for (int uu = 0; uu < 8; ++uu) {
+          const int idx = (j0 + uu) * 32 + lane;
+          const int r = idx / g.F_pad, cp = idx - r * g.F_pad;
+          const int cidx = cp ^ ((r & 1) * g.x_swz);
+          if (cidx < g.F) buf[cidx * SP_US + r] = v[uu];
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < SPP_ZS; ++k) { pa[k] = 0.0; pv[k] = 0; }
+      __syncwarp();
+    }
+    load_group(0, 0);
+    for (int gi = 0; gi < n_grp; ++gi) {
+      asm volatile("cp.async.wait_all;" ::: "memory");
+      __syncthreads();                                         // group gi is resident, group gi - 1's readers are done
+      if (gi + 1 < n_grp) load_group(gi + 1, (gi + 1) & 1);
+      if (!have) continue;
+      const int s0 = gi * G, gc = min(G, p.C - s0);
+      const double* wg = wsm + (size_t)(gi & 1) * G * wlen;
+      for (int sub = 0; sub < gc; sub += NCH) {
+        // sets of this step (a short last step repeats its last set; the copy is not scored)
+        int ch[NCH];
+        const double* w[NCH];
+        double out[NCH][SP_MAX_O];
+#pragma unroll
+        for (int q = 0; q < NCH; ++q) {
+          ch[q] = min(sub + q, gc - 1);
+          w[q] = wg + (size_t)ch[q] * wlen;
+#pragma unroll
+          for (int o = 0; o < SP_MAX_O; ++o) out[q][o] = w[q][o];
+          w[q] += SP_MAX_O;
+        }
+        const int* it = prog;
+        if constexpr (PAIRS) {
+          double alpha1[NCH], alpha2[NCH];
+#pragma unroll
+          for (int q = 0; q < NCH; ++q) {
+            alpha1[q] = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[(long long)(s0 + ch[q]) * g.L + 0] : 0.0;
+            alpha2[q] = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[(long long)(s0 + ch[q]) * g.L + 1] : 0.0;
+          }
+          const int nc1 = p.sp.pair_nc1;
+          const int stride = 2 * SP_HDR + ((nc1 + 3) & ~3) + ((NR1 + 3) & ~3);
+          for (int n = 0; n < p.sp.n_items; n += 2, it += stride)
+            sparse_pair<ACT, NCH, NR1, NR2, NC1>(it, nc1, O, w, bufl, alpha1, alpha2, tab, out);
+        } else {
+          double* bufw = buf + lane;
+          for (int n = 0; n < p.sp.n_items; ++n) {
+            const int4 h = *reinterpret_cast<const int4*>(it);
+            const int layer = h.x & 0xff, nr = (h.x >> 8) & 0xff, nc = h.y;
+            const bool to_out = (h.x >> 16) & 1;
+            const int qs = h.z ? sq : 0;
+            double alpha[NCH];
+#pragma unroll
+            for (int q = 0; q < NCH; ++q)
+              alpha[q] = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[(long long)(s0 + ch[q]) * g.L + layer] : 0.0;
+            switch (nr) {
+              case 1: sparse_item<ACT, NCH, 1>(it, nc, qs, sq, to_out, O, w, bufw, alpha, tab, out); break;
+              case 2: sparse_item<ACT, NCH, 2>(it, nc, qs, sq, to_out, O, w, bufw, alpha, tab, out); break;
+              case 3: sparse_item<ACT, NCH, 3>(it, nc, qs, sq, to_out, O, w, bufw, alpha, tab, out); break;
+              default: sparse_item<ACT, NCH, 4>(it, nc, qs, sq, to_out, O, w, bufw, alpha, tab, out); break;
+            }
+            it += SP_HDR + ((nc + 3) & ~3);
+          }
+        }
+        // sets in order: this step's first set, then its second
+#pragma unroll
+        for (int q = 0; q < NCH; ++q)
+          if (sub + q < gc) sparse_pred_epilogue(p, s0 + sub + q, row, active, out[q], tab, pa, pv);
+      }
+    }
+    __syncthreads();                                           // the last group's readers are done with the buffers
+    if (active) {
+      const int W = bnn_pred_width(g);
+      for (int k = 0; k < W; ++k) {
+        if (p.mean_out) p.mean_out[row * W + k] = pa[k] / p.inv_sets;
+        if (p.votes_out) p.votes_out[row * W + k] = (double)pv[k] / p.inv_sets;
+      }
+    }
+  }
+}
+
+// dynamic shared memory of k_pred_sparse
+static size_t spred_bytes(const FwdParams& p, bool pairs, int group, int nwarps) {
+  const size_t per_warp = (size_t)(p.g.F + (pairs ? 0 : SPP_NCH * p.sp.slots)) * SP_US + 32 * SPP_ZS;
+  const size_t n_dbl = (BNN_EXP_TAB_SIZE + 2 * (size_t)group * p.sp.wlen + (size_t)nwarps * per_warp + 1) & ~(size_t)1;
+  const size_t n_int = ((p.sp.prog_len + 3) & ~3) + (size_t)nwarps * 32 * SPP_ZS;
+  return n_dbl * sizeof(double) + n_int * sizeof(int);
+}
+
+// launch plan of k_pred_sparse: CTAs, warps (tiles per round), sets per buffer.  Rounds first: the most warps that fit
+// next to a double-buffered group of SPP_NCH sets set the number of rounds over the CTA's tiles, the tiles are then
+// spread evenly over that many rounds, and what shared memory is left takes as many sets per group as fit.
+static bool spred_plan(const FwdParams& p, bool pairs, int n_sms, int* grid, int* nwarps, int* group, size_t* bytes) {
+  const long long n_tiles32 = (p.n_tiles16 + 1) >> 1;
+  const int gr = (int)(n_tiles32 < n_sms ? n_tiles32 : n_sms);
+  const long long tpc = (n_tiles32 + gr - 1) / gr;
+  const int c_up = (p.C + SPP_NCH - 1) / SPP_NCH * SPP_NCH;
+  int wmax = 0;
+  for (int w = (int)(tpc < SPP_MAX_WARPS ? tpc : SPP_MAX_WARPS); w >= 1; --w)
+    if (spred_bytes(p, pairs, SPP_NCH, w) <= BNN_MAX_DYN_SMEM) { wmax = w; break; }
+  if (!wmax) return false;
+  const long long rounds = (tpc + wmax - 1) / wmax;
+  const int w = (int)((tpc + rounds - 1) / rounds);
+  int gch = SPP_NCH;
+  while (gch + SPP_NCH <= c_up && spred_bytes(p, pairs, gch + SPP_NCH, w) <= BNN_MAX_DYN_SMEM) gch += SPP_NCH;
+  *grid = gr; *nwarps = w; *group = gch; *bytes = spred_bytes(p, pairs, gch, w);
+  return true;
+}
+
+bool bnn_sparse_predict_fits(const FwdParams& p) {
+  return p.g.O <= SP_MAX_O && spred_bytes(p, p.sp.pair_nc1 != 0, SPP_NCH, 1) <= BNN_MAX_DYN_SMEM;
+}
+
+template <int ACT, int NR1, int NR2, int NC1 = 0>
+static cudaError_t launch_pred(const FwdParams& p0, int n_sms, cudaStream_t st) {
+  if constexpr (NR1 > 0 && NC1 == 0)
+    if (p0.sp.pair_nc1 == 1) return launch_pred<ACT, NR1, NR2, 1>(p0, n_sms, st);
+  auto kern = k_pred_sparse<ACT, NR1, NR2, NC1>;
+  FwdParams p = p0;
+  int grid = 0, nwarps = 0, group = 0;
+  size_t bytes = 0;
+  if (!spred_plan(p, NR1 > 0, n_sms, &grid, &nwarps, &group, &bytes)) return cudaErrorInvalidConfiguration;
+  p.sp.group = group;
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
+  kern<<<grid, nwarps * 32, bytes, st>>>(p);
+  return cudaGetLastError();
+}
+
+template <int ACT>
+static cudaError_t launch_sparse_predict_t(const FwdParams& p, int n_sms, cudaStream_t st, const char** which) {
+  if (p.sp.pair_nc1) {
+    if (which) *which = "k_fwd_sparse<pairs,predict>";
+    cudaError_t e = cudaErrorInvalidConfiguration;
+    with_pair_shape(p.sp.pair_nr1, p.sp.pair_nr2, [&](auto s) {
+      e = launch_pred<ACT, decltype(s)::nr1, decltype(s)::nr2>(p, n_sms, st);
+    });
+    return e;
+  }
+  if (which) *which = "k_fwd_sparse<predict>";
+  return launch_pred<ACT, 0, 0>(p, n_sms, st);
+}
+
+cudaError_t bnn_launch_sparse_predict(const FwdParams& p, int n_sms, cudaStream_t st, const char** which) {
+  return bnn_with_act(p.g.act, [&](auto a) { return launch_sparse_predict_t<decltype(a)::value>(p, n_sms, st, which); });
+}
+
+// *flag = 1 if an entry the mask drops is nonzero in any of the n_sets canonical weight sets w [n_sets, P]
+__global__ void k_mask_violations(const double* __restrict__ w, long long n, int P, const double* __restrict__ mask,
+                                  int* flag) {
+  bool bad = false;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+    bad |= (__ldg(mask + i % P) == 0.0) && (__ldg(w + i) != 0.0);      // (NaN counts as nonzero)
+  if (__any_sync(FULL_MASK, bad) && (threadIdx.x & 31) == 0) *flag = 1;
+}
+
+cudaError_t bnn_launch_mask_violations(const double* w, int n_sets, int P, const double* mask, int* flag, int n_sms,
+                                       cudaStream_t st) {
+  if (cudaError_t e = cudaMemsetAsync(flag, 0, sizeof(int), st)) return e;
+  const long long n = (long long)n_sets * P;
+  const long long blocks = (n + 255) / 256;
+  k_mask_violations<<<(int)(blocks < 4LL * n_sms ? blocks : 4LL * n_sms), 256, 0, st>>>(w, n, P, mask, flag);
+  return cudaGetLastError();
+}

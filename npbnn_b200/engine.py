@@ -472,11 +472,23 @@ class Engine:
         torch.cuda.current_stream(self.device).synchronize()
 
     # ---------------------------------------------------------------- prediction
-    def predict(self, x, weight_sets, alphas=None, override=None, mean=True, votes=False, dense=False, device_out=False):
+    def _set_pattern(self, pattern):
+        """Zero pattern [n_params] (0/1) of the weight sets of this call (predshard.zero_pattern), or None: dense kernels.
+        Set on every call, so a cached engine never carries one network's pattern into the next network's call."""
+        pt = None
+        if pattern is not None:
+            pt = np.ascontiguousarray(pattern, dtype=np.float64)
+            assert pt.shape == (self.net.n_params,), pt.shape
+        L.check(self.lib.bnn_set_predict_mask(self._h, _np_ptr(pt)))
+
+    def predict(self, x, weight_sets, alphas=None, override=None, mean=True, votes=False, dense=False, device_out=False,
+                pattern=None):
         """Posterior prediction over rows of x for every weight set (reference BNN_lib.py:376-392).
-        override: (cols, vals) PDP column overwrite (BNN_pdp.py:65).  Returns dict of numpy arrays (device_out: of
-        tensors on this engine's device)."""
+        override: (cols, vals) PDP column overwrite (BNN_pdp.py:65).  pattern: zero pattern of the weight sets (a
+        block-masked network then runs the block-sparse kernels; None: dense kernels).  Returns dict of numpy arrays
+        (device_out: of tensors on this engine's device)."""
         w = self._as_sets(weight_sets)
+        self._set_pattern(pattern)
         with torch.cuda.device(self.device):
             xd = self._dev(x, torch.float64)
             wd = self._dev(w, torch.float64)
@@ -505,13 +517,14 @@ class Engine:
             return out if device_out else {k: v.cpu().numpy() for k, v in out.items()}
 
     def predict_sample(self, x, weight_sets, u=None, alphas=None, post_predictions=True, seed=None, row0=0, set0=0,
-                       device_out=False):
+                       device_out=False, pattern=None):
         """sample_from_categorical (BNN_lib.py:682-713) fused into the prediction pass.  u [n, S]: the reference's
         uniforms (np.random.random(S) per instance); u=None: uniforms generated in the kernel from `seed` (Philox,
         nothing of size n x S is stored), keyed on (row0 + row, set0 + set): rows row0... and sets set0... of a larger
         call draw that call's uniforms.  Returns dict(predictions [n,K], class_counts [S,K], post_predictions [n,S]
-        or None) of numpy arrays (device_out: of float64 tensors on this engine's device)."""
+        or None) of numpy arrays (device_out: of float64 tensors on this engine's device).  pattern: as in predict."""
         w = self._as_sets(weight_sets)
+        self._set_pattern(pattern)
         with torch.cuda.device(self.device):
             xd, wd, ad = self._dev(x, torch.float64), self._dev(w, torch.float64), self._dev(alphas, torch.float64)
             n, S = xd.shape[0], wd.shape[0]

@@ -87,6 +87,7 @@ def predict_sharded(engine, x_rows, weight_sets, n_rows_total: int, rank: int, w
     S = len(weight_sets)
     rows, sets, grid, rg, sg = partition(n_rows_total, S, world, rank, grid)
     w = engine._as_sets(weight_sets)[sets[0]:sets[1]]
+    engine._set_pattern(None)                 # the dense kernels, whatever pattern the engine's last call used
     n_loc = sets[1] - sets[0]
     with torch.cuda.device(engine.device):
         xd = engine._dev(x_rows, torch.float64)
@@ -137,6 +138,48 @@ def predict_sharded(engine, x_rows, weight_sets, n_rows_total: int, rank: int, w
         if votes:
             out["votes"] = combine(vsum, S, world, rank, grid)
     return out
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# zero pattern of the posterior samples (block-masked networks run the block-sparse prediction kernels)
+# ---------------------------------------------------------------------------------------------------------------------
+def zero_pattern(weight_sets, net) -> Optional[np.ndarray]:
+    """The union over the posterior samples of `w != 0`, as a canonical 0/1 vector [n_params] for
+    Engine.predict(pattern=...), or None when the prediction should stay on the dense kernels.  Entries that are zero in
+    every sample contribute nothing, so skipping them only changes the order of the sums.
+    weight_sets: a list of per-layer weight lists, or an array / tensor [S, n_params].  The block cover of the pattern
+    has at least as many multiply-adds as sample 0 has nonzero hidden-layer weights, and the program builder declines a
+    cover above a quarter of the dense work: when sample 0 alone is past that, this returns None after looking at that
+    one sample (dense networks pay O(n_params), not O(S n_params))."""
+    shapes, hb = net.shapes, net.has_bias()
+    if len(shapes) < 2 or len(weight_sets) == 0:
+        return None
+    dense = sum(r * (c - b) for (r, c), b in zip(shapes, hb))
+    last = shapes[-1][0] * (shapes[-1][1] - hb[-1])
+    flat = isinstance(weight_sets, (np.ndarray, torch.Tensor))
+    host = (lambda t: t.detach().cpu().numpy()) if isinstance(weight_sets, torch.Tensor) else np.asarray
+    if flat:
+        w0 = host(weight_sets[0])                    # (a tensor is copied to the host only past the shortcut)
+        offs = np.cumsum([0] + [r * c for r, c in shapes])
+        layers0 = [w0[offs[l]:offs[l + 1]].reshape(shapes[l]) for l in range(len(shapes))]
+    else:
+        layers0 = [np.asarray(w) for w in weight_sets[0]]
+    nnz = sum(int(np.count_nonzero(w[:, b:])) for w, b in zip(layers0[:-1], hb[:-1]))
+    if 4 * (nnz + last) > dense:
+        return None
+    if flat:
+        return np.any(host(weight_sets) != 0, axis=0).astype(np.float64)
+    pat = [w != 0 for w in layers0]
+    for s in weight_sets[1:]:
+        for l, w in enumerate(s):
+            pat[l] |= np.asarray(w) != 0
+    return np.concatenate([p.ravel() for p in pat]).astype(np.float64)
+
+
+def engine_pattern(engine, weight_sets) -> Optional[np.ndarray]:
+    """zero_pattern for `engine`'s network; None for an engine whose network declares no layer shapes (it scores
+    densely and is never handed a pattern)."""
+    return zero_pattern(weight_sets, engine.net) if hasattr(engine.net, "shapes") else None
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -204,7 +247,8 @@ _OUTPUTS = ("mean", "votes", "predictions", "class_counts", "post_predictions", 
 
 
 def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False, votes=False, dense=False,
-                  sample=None, post_predictions=False, shuffle=(), draw=None, grid: Optional[Tuple[int, int]] = None):
+                  sample=None, post_predictions=False, shuffle=(), draw=None, grid: Optional[Tuple[int, int]] = None,
+                  pattern="auto"):
     """Posterior prediction of all N rows of x over all S posterior samples, split over the ranks of the default process
     group.  Collective: every rank passes the same arguments (checked first, ValueError on every rank otherwise) and
     returns the same dict of host arrays as the engine calls over the whole problem:
@@ -215,7 +259,10 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
     (cols, vals) column overwrite.  sample: None, "host" (reference uniforms) or "philox" (in-kernel uniforms, keyed on
     the global (row, sample) so the split does not change them).  shuffle: feature selectors whose rows are permuted.
     draw(): run on rank 0 only, returns (permutations of range(N), one per shuffle entry; uniforms [N, S] or None; seed
-    or None) drawn from rank 0's numpy stream, which every rank then receives.
+    or None) drawn from rank 0's numpy stream, which every rank then receives.  The engine scores with the zero pattern
+    of all S samples: `pattern`, or zero_pattern(weight_sets) with pattern="auto" (callers that score the same samples
+    many times compute it once and pass it).  Every rank computes the same pattern from the same full sample list, so a
+    block-masked network runs the same block-sparse program on every rank.
 
     The rank scores rows x samples block `partition(N, S, world, rank, grid)`; a rank with an empty block makes no kernel
     call but joins every collective.  Combination (one all-gather of every rank's block): means are sums over each sample
@@ -257,13 +304,16 @@ def predict_ranks(engine, x, weight_sets, alphas=None, override=None, mean=False
         xb = permuted_rows(x, a, b, shuffle, perms) if shuffle else x[a:b]
         w = weight_sets[c:d]
         al = None if alphas is None else np.asarray(alphas)[c:d]
+        # (passed only when there is one)
+        pat = engine_pattern(engine, weight_sets) if isinstance(pattern, str) else pattern
+        kw = {} if pat is None else {"pattern": pat}
         if mean or votes or dense:
             out.update(engine.predict(xb, w, alphas=al, override=override, mean=mean, votes=votes, dense=dense,
-                                      device_out=world > 1))
+                                      device_out=world > 1, **kw))
         if sample:
             out.update(engine.predict_sample(xb, w, None if u is None else u[a:b, c:d], alphas=al,
                                              post_predictions=post_predictions, seed=seed, row0=a, set0=c,
-                                             device_out=world > 1))
+                                             device_out=world > 1, **kw))
     if world == 1:
         return out
 
