@@ -288,6 +288,12 @@ static int ensure_wp_scratch(bnn_ctx* c, const NetGeom& g, size_t n_sets, cudaSt
   return 0;
 }
 
+// Every network must run on k_fwd_generic, which stages a warp's hidden activations in shared memory: it fits when one
+// warp per CTA does in both modes -- a full pass of likelihood counters, and the prediction accumulators.
+static bool generic_fits(const NetGeom& g) {
+  return bnn_generic_warps(g, sets_per_pass(g), false) && bnn_generic_warps(g, 1, true);
+}
+
 extern "C" {
 
 const char* bnn_last_error(void) { return g_last_error.c_str(); }
@@ -398,6 +404,13 @@ int bnn_set_net(bnn_ctx* c, const bnn_net_spec* s) {
     g.K = g.O / 2;
   } else {
     g.K = g.O;
+  }
+  if (!generic_fits(g)) {
+    NetGeom h = g;
+    while (h.max_w > 8 && !generic_fits(h)) h.max_w -= 8;
+    return fail("bnn_set_net: a hidden layer of " + std::to_string(g.max_w) + " (padded) units is wider than the forward "
+                "kernel supports with this output layer: at most " + std::to_string(generic_fits(h) ? h.max_w : 0) +
+                " units per hidden layer");
   }
   c->g = g;
   c->g_base = g;

@@ -23,13 +23,33 @@
 // =============================================================================================
 // generic kernel
 // =============================================================================================
-constexpr int GEN_WARPS = 4;
+constexpr int GEN_WARPS = 4;      // warps per CTA where the staging fits (bnn_generic_warps); 2 or 1 for wider layers
 
+// Dynamic shared memory of a k_fwd_generic CTA of `warps` warps: exp table, per-warp staging (two hidden-layer buffers
+// of 16 rows x max_w, the output rows, prediction accumulators) and the ints (likelihood: the counters of C sets;
+// prediction: per-warp votes).
+size_t bnn_generic_smem_bytes(const NetGeom& g, int C, bool predict, int warps) {
+  const int ZS = g.l[g.L - 1].out_pad + 1;
+  const int PW = (g.lik == BNN_LIK_CATEGORICAL) ? g.K : g.O;
+  const size_t per_warp = 2 * 16 * (size_t)g.max_w + 16 * ZS + (predict ? 16 * PW : 0);
+  const size_t ints = predict ? (size_t)warps * 16 * PW : bnn_smem_counts(g, C);
+  return (GEN_TAB_SIZE + warps * per_warp) * sizeof(double) + ints * sizeof(int);
+}
+
+// Most warps per CTA (4, 2 or 1) whose staging fits; 0 when not even one warp's does.
+int bnn_generic_warps(const NetGeom& g, int C, bool predict) {
+  for (int w = GEN_WARPS; w >= 1; w >>= 1)
+    if (bnn_generic_smem_bytes(g, C, predict, w) <= BNN_MAX_DYN_SMEM) return w;
+  return 0;
+}
+
+// The warp count is blockDim.x / 32 (bnn_generic_warps): every (tile, set) is computed by one warp with the same
+// instruction sequence whatever the count, so results do not depend on it.
 template <int ACT, bool PREDICT>
 __global__ void __launch_bounds__(GEN_WARPS * 32) k_fwd_generic(const __grid_constant__ FwdParams p) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const NetGeom& g = p.g;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, n_warps = blockDim.x >> 5;
   const int gq = lane >> 2;
   const int ZS = g.l[g.L - 1].out_pad + 1;        // the last layer may be padded beyond round_up(O, 8) (k_fwd3 width families)
   const int PW = bnn_pred_width(g);
@@ -41,7 +61,7 @@ __global__ void __launch_bounds__(GEN_WARPS * 32) k_fwd_generic(const __grid_con
   double* h1 = h0 + 16 * g.max_w;
   double* zs = h1 + 16 * g.max_w;
   double* pacc = zs + 16 * ZS;
-  int* ibase = reinterpret_cast<int*>(hbase + GEN_WARPS * per_warp);
+  int* ibase = reinterpret_cast<int*>(hbase + n_warps * per_warp);
   int* pvote = ibase + warp * (PREDICT ? 16 * PW : 0);
   int* cnt = ibase;   // likelihood mode: [C][2+2K]
   const int n_cnt = PREDICT ? 0 : bnn_smem_counts(g, p.C);
@@ -54,8 +74,8 @@ __global__ void __launch_bounds__(GEN_WARPS * 32) k_fwd_generic(const __grid_con
   // gridDim.y as well (every (tile, set) still has exactly one owner); prediction accumulates over sets per tile
   const int c_beg = PREDICT ? 0 : (int)((long long)p.C * blockIdx.y / gridDim.y);
   const int c_end = PREDICT ? p.C : (int)((long long)p.C * (blockIdx.y + 1) / gridDim.y);
-  const long long total_warps = (long long)gridDim.x * GEN_WARPS;
-  for (long long wt = (long long)blockIdx.x * GEN_WARPS + warp; wt < p.n_tiles16; wt += total_warps) {
+  const long long total_warps = (long long)gridDim.x * n_warps;
+  for (long long wt = (long long)blockIdx.x * n_warps + warp; wt < p.n_tiles16; wt += total_warps) {
     if (PREDICT) {
       for (int i = lane; i < 16 * PW; i += 32) { pacc[i] = 0.0; pvote[i] = 0; }
       __syncwarp();
@@ -985,16 +1005,12 @@ int bnn_fwd3_family(const NetGeom& g) {
 template <int ACT, bool PREDICT>
 static cudaError_t launch_generic_t(const FwdParams& p, int n_sms, cudaStream_t st) {
   auto kern = k_fwd_generic<ACT, PREDICT>;
-  const int ZS = p.g.l[p.g.L - 1].out_pad + 1;
-  const int PW = (p.g.lik == BNN_LIK_CATEGORICAL) ? p.g.K : p.g.O;
-  size_t per_warp = 2 * 16 * (size_t)p.g.max_w + 16 * ZS + (PREDICT ? 16 * PW : 0);
-  size_t bytes = (GEN_TAB_SIZE + GEN_WARPS * per_warp) * sizeof(double);
-  size_t ints = PREDICT ? (size_t)GEN_WARPS * 16 * PW : bnn_smem_counts(p.g, p.C);
-  bytes += ints * sizeof(int);
-  if (bytes > BNN_MAX_DYN_SMEM) return cudaErrorInvalidConfiguration;
+  const int warps = bnn_generic_warps(p.g, p.C, PREDICT);
+  if (!warps) return cudaErrorInvalidConfiguration;       // (bnn_set_net refuses such networks)
+  const size_t bytes = bnn_generic_smem_bytes(p.g, p.C, PREDICT, warps);
   if (bytes > 48 * 1024)
     if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
-  long long ctas = (p.n_tiles16 + GEN_WARPS - 1) / GEN_WARPS;
+  long long ctas = (p.n_tiles16 + warps - 1) / warps;
   // resident CTAs per SM limited by shared memory; cap the grid at a few waves of resident CTAs
   long long max_grid = (long long)n_sms * 8;
   int grid = (int)(ctas < max_grid ? ctas : max_grid);
@@ -1003,7 +1019,7 @@ static cudaError_t launch_generic_t(const FwdParams& p, int n_sms, cudaStream_t 
     const int want = (n_sms * 4 + grid - 1) / grid;
     ny = want < p.C ? want : p.C;
   }
-  kern<<<dim3(grid, ny), GEN_WARPS * 32, bytes, st>>>(p);
+  kern<<<dim3(grid, ny), warps * 32, bytes, st>>>(p);
   return cudaGetLastError();
 }
 

@@ -96,6 +96,10 @@ cudaError_t bnn_launch_mask_violations(const double* w, int n_sets, int P, const
 // softmax, FP64 accumulation over the samples; summaries of the 64-64-32-16 categorical family only
 bool bnn_pred_tf32_fits(const FwdParams& p);
 cudaError_t bnn_launch_pred_tf32(const FwdParams& p, int n_sms, int passes, cudaStream_t st, const char** which);
+// Dynamic shared memory of a k_fwd_generic CTA of `warps` warps running C sets (likelihood) or posterior prediction, and
+// the most warps (4, 2, 1) whose CTA fits BNN_MAX_DYN_SMEM: 0 when none does (the network is too wide for the kernel)
+size_t bnn_generic_smem_bytes(const NetGeom& g, int C, bool predict, int warps);
+int bnn_generic_warps(const NetGeom& g, int C, bool predict);
 // k_fwd3 width family the padded geometry matches exactly: 1 = 64->64->32, 2 = 32->32->16, 0 = none (generic kernel)
 int bnn_fwd3_family(const NetGeom& g);
 cudaError_t bnn_launch_pack_x(const double* x, double* xs, long long n, long long n_pad, int F, int F_pad, int swz,

@@ -31,15 +31,19 @@ __global__ void k_pack_x(const double* __restrict__ x, double* __restrict__ xs, 
   xs[r * F_pad + (c ^ ((int)(r & 1) * swz))] = v;
 }
 
-// canonical weight sets [n_sets, P] -> packed [n_sets, PB] (padding entries are pre-zeroed, never written)
-__global__ void k_pack_w(const __grid_constant__ NetGeom g, const double* __restrict__ w, double* __restrict__ wp) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= g.P) return;
+// canonical weight sets [n_sets, P] -> packed [n_sets, PB] (padding entries are pre-zeroed, never written); one thread
+// per entry of all sets (a 1-D grid: a set count in gridDim.y would stop at 65,535)
+__global__ void k_pack_w(const __grid_constant__ NetGeom g, const double* __restrict__ w, double* __restrict__ wp,
+                         long long n_entries) {
+  const long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= n_entries) return;
+  const long long set = e / g.P;
+  const int i = (int)(e - set * g.P);
   int l = layer_of(g, i);
   const LayerGeom& lg = g.l[l];
   int cols = lg.in + lg.bias;
   int r = (i - lg.c_off) / cols, cc = (i - lg.c_off) % cols;
-  wp[(long long)blockIdx.y * g.PB + bnn_packed_index(lg, r, cc)] = w[(long long)blockIdx.y * g.P + i];
+  wp[set * g.PB + bnn_packed_index(lg, r, cc)] = w[e];
 }
 
 
@@ -130,8 +134,8 @@ cudaError_t bnn_launch_pack_x(const double* x, double* xs, long long n, long lon
   return cudaGetLastError();
 }
 cudaError_t bnn_launch_pack_w(const NetGeom& g, const double* w, double* wp, int n_sets, cudaStream_t st) {
-  dim3 grid((g.P + 255) / 256, n_sets);
-  k_pack_w<<<grid, 256, 0, st>>>(g, w, wp);
+  const long long n = (long long)n_sets * g.P;
+  k_pack_w<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(g, w, wp, n);
   return cudaGetLastError();
 }
 cudaError_t bnn_launch_finalize_lik(const NetGeom& g, const double* part, int NF, long long nt, long long n_train,

@@ -124,7 +124,7 @@ class Engine:
         spec = L.NetSpec()
         spec.n_layers, spec.n_features = net.n_layers, net.n_features
         hb = net.has_bias()
-        for i, (r, c) in enumerate(net.shapes):
+        for i, (r, c) in enumerate(net.shapes[:L.MAX_LAYERS]):      # (deeper networks: bnn_set_net refuses n_layers)
             spec.out_dim[i], spec.has_bias[i] = int(r), int(hb[i])
         spec.act, spec.lik = L.ACT[net.act], net.lik
         L.check(self.lib.bnn_set_net(h, C.byref(spec)))
