@@ -299,7 +299,8 @@ int bnn_predict(bnn_ctx* ctx, const double* x_dev, int64_t n, const double* w_de
  * asynchronous).  The program is built per pattern and padded layout and kept while the pattern does not change;
  * bnn_set_net clears the pattern.  When the pattern's block cover is not thin enough (or
  * the network has no hidden layer, more than 8 outputs, or a program too large for shared memory) the call succeeds and
- * prediction stays dense.  Option "predict_tf32" does not apply to the block-sparse kernels. */
+ * prediction stays dense.  Option "predict_tf32" does not apply to the block-sparse kernels: with a pattern in use,
+ * prediction runs them in FP64 whatever the option. */
 int bnn_set_predict_mask(bnn_ctx* ctx, const double* mask_host);
 
 /* Number of kernel launches issued by this context so far (bench.py's gpu_launches). */
@@ -369,10 +370,16 @@ int bnn_debug_read_part(bnn_ctx* ctx, double* out_host, int64_t n_doubles);
  * thread-block cluster per chain) where that beats one launch pair per iteration, 2 = wherever the problem fits, 0 = never
  * (results are bit-identical either way);
  * "chain_loop_cluster" = 1 | 2 | 4 | 8 | 16 caps the cluster size of that kernel (default 16);
- * "predict_tf32" = 1 (default 0) evaluates bnn_predict summaries (mean / votes) of the 64-64-32-16 categorical family on the
- * TF32 tensor cores in error-compensated 3xTF32 form with FP32 activations: class probabilities agree with the FP64 kernel
- * to ~1e-6 absolute (stated tolerance 5e-6); 2 = plain TF32 (one product, ~1e-4, stated 5e-3); bnn_mh_steps and the
- * likelihood calls never use reduced precision.  Any other name is refused. */
+ * "predict_tf32" = 1 (default 0) evaluates the prediction calls of every dense network -- bnn_predict summaries (mean /
+ * votes, every likelihood) and the resampling of bnn_predict_sample / bnn_predict_sample_philox(_at) -- on the TF32 tensor
+ * cores in error-compensated 3xTF32 form, with FP32 activations, softmax and softplus and FP64 sums over the sets in set
+ * order (bnn_last_kernel: "k_pred_tf32x3<act>" for the 64-64-32-16 categorical family, "k_pred_tf32x3_generic<act>" for
+ * every other network).  Stated tolerances against the FP64 kernels: class probabilities 5e-6 absolute; regression,
+ * sigma-head and count means 1e-5 * max(1, |y|); vote flips at most 1e-4 * n * n_sets; a drawn class differs from the FP64
+ * draw only where the FP64 running sum lies within 1e-5 of u at a class boundary.  2 = plain TF32 (one product,
+ * "k_pred_tf32x1...": 5e-3 in the same forms).  A call that asks for dense_dev, a call on the block-sparse kernels, and
+ * bnn_mh_steps and the likelihood calls always run in FP64; so do, under option 1 only, Gaussian and count outputs of
+ * networks padded to the 32-32-16 width family (measured slower in 3xTF32 than the FP64 kernel there).  Any other name is refused. */
 int bnn_set_option(bnn_ctx* ctx, const char* name, int value);
 
 #ifdef __cplusplus

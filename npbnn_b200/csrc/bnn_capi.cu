@@ -1351,9 +1351,10 @@ static int predict_impl(bnn_ctx* c, const double* x_dev, int64_t n, const double
     }
   }
   if (class_counts_dev) CUDA_TRY(cudaMemsetAsync(class_counts_dev, 0, sizeof(int32_t) * (size_t)n_sets * g.K, st));
-  if (c->opt_pred_tf32 && !c->force_generic && !p.sp.prog && bnn_pred_tf32_fits(p)) {
-    // opt-in reduced precision (stated tolerance: class probabilities to ~1e-6 absolute); summaries only
-    CUDA_TRY(bnn_launch_pred_tf32(p, c->n_sms, c->opt_pred_tf32 >= 2 ? 1 : 3, st, &c->last_kernel));
+  const int tf32_passes = c->opt_pred_tf32 >= 2 ? 1 : 3;
+  if (c->opt_pred_tf32 && !c->force_generic && bnn_pred_tf32_fits(p, tf32_passes)) {
+    // opt-in reduced precision (stated tolerances: include/npbnn_b200.h); summaries and resampling of dense networks
+    CUDA_TRY(bnn_launch_pred_tf32(p, c->n_sms, tf32_passes, st, &c->last_kernel));
     c->launches += 3;
     return 0;
   }

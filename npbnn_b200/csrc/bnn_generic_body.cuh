@@ -32,8 +32,9 @@ __device__ __forceinline__ double softplus_ref(double z) {
 }
 
 // Per-warp epilogue on the staged outputs of one (warp tile, weight set).
-// (Its prediction branch is restated per thread, on outputs held in registers, by sparse_pred_epilogue in bnn_sparse.cu:
-// a change of the prediction rules here -- argmax ties, the resampling draw, the transforms -- belongs there too.)
+// (Its prediction branch is restated per thread, on outputs held in registers, by sparse_pred_epilogue in bnn_sparse.cu,
+// and in FP32 by lpg_epilogue in bnn_pred_lp.cu: a change of the prediction rules here -- argmax ties, the resampling
+// draw, the transforms -- belongs in both of them too.)
 //   zs  : [16][ZS] pre-transform outputs of the last layer (row-major, per warp)
 //   lane r < 16 owns row r of the tile.
 // Likelihood mode (PREDICT=false): writes part[(c*NF+slot)*n_tiles16 + wt] and bumps the CTA counters.

@@ -92,9 +92,13 @@ bool bnn_sparse_predict_fits(const FwdParams& p);
 cudaError_t bnn_launch_sparse_predict(const FwdParams& p, int n_sms, cudaStream_t st, const char** which);
 cudaError_t bnn_launch_mask_violations(const double* w, int n_sets, int P, const double* mask, int* flag, int n_sms,
                                        cudaStream_t st);
-// opt-in reduced-precision posterior prediction (bnn_pred_lp.cu): 3xTF32 tensor-core contractions, FP32 activations /
-// softmax, FP64 accumulation over the samples; summaries of the 64-64-32-16 categorical family only
-bool bnn_pred_tf32_fits(const FwdParams& p);
+// opt-in reduced-precision posterior prediction (bnn_pred_lp.cu): 3xTF32 (passes = 3) or TF32 (passes = 1) tensor-core
+// contractions, FP32 activations / softmax / softplus, FP64 accumulation over the samples in set order.  Summaries
+// (mean / votes) and resampling of every dense network: k_pred_tf32x3 for the 64-64-32-16 categorical family,
+// k_pred_tf32_generic for the others.  bnn_pred_tf32_fits: the call is one of those (no dense tensor, no block-sparse
+// program) and not of the shape class measured slower than FP64 at that pass count.  The launcher converts the packed
+// weight sets in p.wp to (hi, lo) TF32 pairs in place.
+bool bnn_pred_tf32_fits(const FwdParams& p, int passes);
 cudaError_t bnn_launch_pred_tf32(const FwdParams& p, int n_sms, int passes, cudaStream_t st, const char** which);
 // Dynamic shared memory of a k_fwd_generic CTA of `warps` warps running C sets (likelihood) or posterior prediction, and
 // the most warps (4, 2, 1) whose CTA fits BNN_MAX_DYN_SMEM: 0 when none does (the network is too wide for the kernel)
