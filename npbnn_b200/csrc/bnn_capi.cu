@@ -67,6 +67,9 @@ struct bnn_ctx {
   NetGeom wp_geom{};                // layout the zero padding of wp_scratch was prepared for
   // staged data
   DevBuf xs, labels, targets, lgk1, inst_w, class_w;     // lgk1: lgamma(k + 1) of the targets (count likelihoods)
+  // 64 -> 64 -> 32 family: int8 digits of the rows (null: the data set runs the FP64 first layer, bnn_set_data), the
+  // per-feature power-of-two divisors the rows were staged with, and the digits of a pass's layer-1 weights
+  DevBuf x_i8, x_i8_scale, x_i8_wmul, w1_i8;
   bool has_iw = false, has_cw = false;
   long long n_train = 0, n_test = 0, n_total = 0, n_pad = 0, n_tiles16 = 0;
   // workspaces
@@ -214,6 +217,12 @@ static FwdParams base_params(const bnn_ctx* c) {
   p.lgk1 = c->lgk1.as<double>();
   p.inst_w = c->has_iw ? c->inst_w.as<double>() : nullptr;
   p.class_w = c->has_cw ? c->class_w.as<double>() : nullptr;
+  if (c->x_i8.p) {
+    p.x_i8 = c->x_i8.as<int8_t>();
+    p.x_i8_scale = c->x_i8_scale.as<double>();
+    p.x_i8_wmul = c->x_i8_wmul.as<double>();
+    p.w1_i8 = c->w1_i8.as<int8_t>();
+  }
   return p;
 }
 
@@ -452,6 +461,45 @@ int bnn_set_data(bnn_ctx* c, const double* x_dev, int64_t n_train, int64_t n_tes
   CUDA_TRY(c->xs.ensure(sizeof(double) * c->n_pad * g.F_pad, false, st));
   CUDA_TRY(bnn_launch_pack_x(x_dev, c->xs.as<double>(), c->n_total, c->n_pad, g.F, g.F_pad, g.x_swz, nullptr, nullptr, 0, st));
   c->launches++;
+  // 64 -> 64 -> 32 family: the likelihood kernel runs layer 1 on the int8 tensor cores (k_fwd3i, bnn_forward.cu) when
+  // every feature's largest magnitude is finite and in [2^-500, 2^500], and at least half of its nonzero entries are
+  // within 2^6 of it (or the feature is zero): then its error bound is small against the products; other data sets
+  // run the FP64 layer 1
+  bool i8 = false;
+  double wmul[64];
+  if (bnn_fwd3_family(g) == 1) {
+    CUDA_TRY(c->x_i8_wmul.ensure(3 * 64 * sizeof(double), false, st));
+    CUDA_TRY(bnn_launch_feature_stats(c->xs.as<double>(), c->n_total, g.x_swz, c->x_i8_wmul.as<double>(), st));
+    c->launches++;
+    double fs[192];
+    CUDA_TRY(cudaMemcpyAsync(fs, c->x_i8_wmul.p, sizeof(fs), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    i8 = true;
+    for (int k = 0; k < 64; ++k) {
+      const double m = fs[k];
+      if (m == 0.0) { wmul[k] = 1.0; continue; }
+      if (!(m >= 0x1p-500 && m <= 0x1p500 && 2.0 * fs[128 + k] >= fs[64 + k])) i8 = false;
+      int ex;
+      std::frexp(m, &ex);
+      wmul[k] = std::ldexp(1.0, ex);
+    }
+  }
+  if (i8) {
+    const size_t blocks = (size_t)bnn_i8_blocks(c->n_tiles16);
+    CUDA_TRY(cudaMemcpyAsync(c->x_i8_wmul.p, wmul, sizeof(wmul), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(c->x_i8.ensure(blocks * BNN_I8_XBLK_BYTES, false, st));
+    CUDA_TRY(c->x_i8_scale.ensure(blocks * 128 * sizeof(double), false, st));
+    CUDA_TRY(c->w1_i8.ensure((size_t)BNN_MAX_SETS_PER_PASS * BNN_I8_WSET_BYTES, false, st));
+    CUDA_TRY(bnn_launch_slice_x(c->xs.as<double>(), c->n_pad, g.x_swz, c->x_i8_wmul.as<double>(), c->x_i8.as<int8_t>(),
+                                c->x_i8_scale.as<double>(), st));
+    c->launches++;
+    CUDA_TRY(cudaStreamSynchronize(st));       // wmul lives on this stack frame
+  } else {
+    c->x_i8_wmul.release();
+    c->x_i8.release();
+    c->x_i8_scale.release();
+    c->w1_i8.release();
+  }
   if (g.lik == BNN_LIK_CATEGORICAL) {
     CUDA_TRY(c->labels.ensure(sizeof(int) * c->n_total, false, st));
     CUDA_TRY(cudaMemcpyAsync(c->labels.p, labels_dev, sizeof(int) * c->n_total, cudaMemcpyDeviceToDevice, st));
@@ -521,7 +569,7 @@ int bnn_forward_lik(bnn_ctx* c, const double* w_dev, int32_t n_sets, const doubl
     CUDA_TRY(timed_forward(c, p, false, st));
     CUDA_TRY(bnn_launch_finalize_lik(g, p.part, p.NF, c->n_tiles16, c->n_train, lik_temp, sigma_mode, sigma_dev,
                                      loglik_dev, sums_dev, s0, n, st));
-    c->launches += 2;
+    c->launches += 1 + bnn_forward_launches(p, false, c->force_generic);
   }
   return 0;
 }
@@ -662,7 +710,7 @@ static int chains_forward(bnn_ctx* c, cudaStream_t st) {
     p.part = c->part.as<double>() + (size_t)s0 * p.NF * c->n_tiles16;
     p.counts = c->counts_prop.as<int>() + (size_t)s0 * NC;
     CUDA_TRY(timed_forward(c, p, false, st));
-    c->launches++;
+    c->launches += bnn_forward_launches(p, false, c->force_generic);
   }
   if (const int ns = bnn_part_slices(c->n_tiles16)) {
     if (!c->rowshard) {              // (row-sharded chains fold the full partials in k_rowshard_local)

@@ -12,6 +12,8 @@
 //   k_fwd3        3-layer nets with compile-time padded widths: X warp tile in shared memory (bulk
 //                 async copy), weight sets streamed through a 2-deep shared-memory ring by bulk async
 //                 copies + mbarriers, hidden activations never leave registers.
+//   k_fwd3i       likelihood modes of the 64 -> 64 -> 32 family: layer 1 on the int8 tensor cores (tcgen05, exact
+//                 Ozaki split), layers 2 / 3 and the epilogues shared with k_fwd3.
 //   k_fwd_generic any depth/width: hidden activations staged in per-warp shared memory, weights read
 //                 through L1/L2.
 #include <mutex>
@@ -535,6 +537,97 @@ enum { FWD3_LIK = 0, FWD3_LIK_W = 1, FWD3_PRED = 2 };
 // 2 count likelihoods (likelihood modes only: their prediction is the Gaussian instantiation's identity output)
 enum { FWD3_CAT = 0, FWD3_GAUSS = 1, FWD3_COUNT = 2 };
 
+// Layers 2 and 3 of one (warp tile, weight set), from the first layer's pre-activations acc1 (m16n8 fragments) to the
+// last layer's accumulators acc3.  W23 indexes the packed weight set with Fwd3Geom's offsets (W2_OFF ... B3_OFF).
+// The activation of k-group kg+1 is independent of the MMAs of k-group kg, so its FP64 chains fill the issue slots
+// between the DMMAs instead of running as a separate latency-bound phase.  Two straight-line copies per layer: one
+// warp vote decides whether any pre-activation needs the guarded evaluation (frag_needs_care); the common copy carries
+// no clamp / NaN fix-up instructions.
+template <int ACT, int KP0, int N1, int N2, int N3>
+__device__ __forceinline__ void fwd3_layers23(double (&acc1)[N1 / 8][4], const double* W23, double a1, double a2,
+                                              const double* tab, int gq, int t, double (&acc3)[N3 / 8][4]) {
+  using G3 = Fwd3Geom<KP0, N1, N2, N3>;
+  // ---------------- layer 2: [16 x N1] x [N1 x N2]   (A operand = activated acc1, no data movement)
+  double acc2[N2 / 8][4];
+#pragma unroll
+  for (int j = 0; j < N2 / 8; ++j) {
+    const double2 bb = *reinterpret_cast<const double2*>(W23 + G3::B2_OFF + 8 * j + 2 * t);
+    acc2[j][0] = bb.x; acc2[j][1] = bb.y; acc2[j][2] = bb.x; acc2[j][3] = bb.y;
+  }
+  auto layer2 = [&](auto fast_tag) {
+    constexpr bool FAST = decltype(fast_tag)::value;
+    const double* wr = W23 + G3::W2_OFF + gq * N1;
+    const int sw = (gq & 1) * G3::SW1;
+    act_tile<ACT, FAST>(acc1[0], a1, tab);
+#pragma unroll
+    for (int kg = 0; kg < N1 / 8 - 2; ++kg) {
+      act_tile<ACT, FAST>(acc1[kg + 1], a1, tab);
+      const int col = (8 * kg + 2 * t) ^ sw;
+#pragma unroll
+      for (int j = 0; j < N2 / 8; ++j) {
+        const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + col);
+        dmma16x8x8(acc2[j], acc1[kg][0], acc1[kg][2], acc1[kg][1], acc1[kg][3], bb.x, bb.y);
+      }
+    }
+    {
+      constexpr int k0 = N1 / 8 - 2, k1 = N1 / 8 - 1;
+      act_tile<ACT, FAST>(acc1[k1], a1, tab);
+      const int c0 = (8 * k0 + 2 * t) ^ sw, c1 = (8 * k1 + 2 * t) ^ sw;
+#pragma unroll
+      for (int j = 0; j < N2 / 8; ++j) {
+        const double2 b0 = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + c0);
+        const double2 b1 = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + c1);
+        dmma16x8x8(acc2[j], acc1[k0][0], acc1[k0][2], acc1[k0][1], acc1[k0][3], b0.x, b0.y);
+        dmma16x8x8(acc2[j], acc1[k1][0], acc1[k1][2], acc1[k1][1], acc1[k1][3], b1.x, b1.y);
+      }
+    }
+  };
+  if (frag_needs_care<ACT, N1 / 8>(acc1)) layer2(std::false_type{});
+  else layer2(std::true_type{});
+  // ---------------- layer 3: [16 x N2] x [N2 x N3]
+#pragma unroll
+  for (int j = 0; j < N3 / 8; ++j) {
+    const double2 bb = *reinterpret_cast<const double2*>(W23 + G3::B3_OFF + 8 * j + 2 * t);
+    acc3[j][0] = bb.x; acc3[j][1] = bb.y; acc3[j][2] = bb.x; acc3[j][3] = bb.y;
+  }
+  auto layer3 = [&](auto fast_tag) {
+    constexpr bool FAST = decltype(fast_tag)::value;
+    const double* wr = W23 + G3::W3_OFF + gq * N2;
+    const int sw = (gq & 1) * G3::SW2;
+    act_tile<ACT, FAST>(acc2[0], a2, tab);
+#pragma unroll
+    for (int kg = 0; kg < N2 / 8; ++kg) {
+      if (kg + 1 < N2 / 8) act_tile<ACT, FAST>(acc2[kg + 1], a2, tab);
+      const int col = (8 * kg + 2 * t) ^ sw;
+#pragma unroll
+      for (int j = 0; j < N3 / 8; ++j) {
+        const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N2 + col);
+        dmma16x8x8(acc3[j], acc2[kg][0], acc2[kg][2], acc2[kg][1], acc2[kg][3], bb.x, bb.y);
+      }
+    }
+  };
+  if (frag_needs_care<ACT, N2 / 8>(acc2)) layer3(std::false_type{});
+  else layer3(std::true_type{});
+}
+
+// The epilogue of one (warp tile, weight set) that is not software-pipelined into the next set: prediction, and the
+// Gaussian / count likelihoods.  (The categorical likelihood runs quad_softmax_stats / quad_lik_finish / _commit.)
+template <int N3, int MODE, int LIKK>
+__device__ __forceinline__ void fwd3_set_epilogue(const FwdParams& p, int c, long long wt, int lane,
+                                                  const double (&acc3)[N3 / 8][4], const double* tab,
+                                                  double (&pacc)[2][N3 / 4], int (&pvote)[2][N3 / 4]) {
+  constexpr bool PREDICT = (MODE == FWD3_PRED);
+  if constexpr (LIKK == FWD3_CAT) {
+    if (PREDICT) quad_epilogue_pred<N3>(p, c, wt, lane, acc3, tab, pacc, pvote);
+  } else if constexpr (LIKK == FWD3_COUNT) {
+    static_assert(!PREDICT, "count prediction runs the FWD3_GAUSS instantiation");
+    quad_count_lik<N3>(p, c, wt, lane, acc3);
+  } else {
+    if (PREDICT) quad_gauss_pred<N3>(p, c, wt, lane, acc3, pacc, tab);
+    else quad_gauss_lik<N3>(p, c, wt, lane, acc3, tab);
+  }
+}
+
 template <int ACT, int KP0, int N1, int N2, int N3, int NWARPS, int MODE, int LIKK = FWD3_CAT>
 __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__ FwdParams p) {
   using G3 = Fwd3Geom<KP0, N1, N2, N3>;
@@ -807,71 +900,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
             x_prefetched = true;
           }
         }
-        // ---------------- layer 2: [16 x N1] x [N1 x N2]   (A operand = activated acc1, no data movement).
-        // The activation of k-group kg+1 is independent of the MMAs of k-group kg, so its FP64 chains fill
-        // the issue slots between the DMMAs instead of running as a separate latency-bound phase.
-        // Two straight-line copies per layer: one warp vote decides whether any pre-activation needs the guarded
-        // evaluation (frag_needs_care); the common copy carries no clamp / NaN fix-up instructions.
-        double acc2[N2 / 8][4];
-#pragma unroll
-        for (int j = 0; j < N2 / 8; ++j) {
-          const double2 bb = *reinterpret_cast<const double2*>(W23 + G3::B2_OFF + 8 * j + 2 * t);
-          acc2[j][0] = bb.x; acc2[j][1] = bb.y; acc2[j][2] = bb.x; acc2[j][3] = bb.y;
-        }
-        auto layer2 = [&](auto fast_tag) {
-          constexpr bool FAST = decltype(fast_tag)::value;
-          const double* wr = W23 + G3::W2_OFF + gq * N1;
-          const int sw = (gq & 1) * G3::SW1;
-          act_tile<ACT, FAST>(acc1[0], a1, tab);
-#pragma unroll
-          for (int kg = 0; kg < N1 / 8 - 2; ++kg) {
-            act_tile<ACT, FAST>(acc1[kg + 1], a1, tab);
-            const int col = (8 * kg + 2 * t) ^ sw;
-#pragma unroll
-            for (int j = 0; j < N2 / 8; ++j) {
-              const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + col);
-              dmma16x8x8(acc2[j], acc1[kg][0], acc1[kg][2], acc1[kg][1], acc1[kg][3], bb.x, bb.y);
-            }
-          }
-          {
-            constexpr int k0 = N1 / 8 - 2, k1 = N1 / 8 - 1;
-            act_tile<ACT, FAST>(acc1[k1], a1, tab);
-            const int c0 = (8 * k0 + 2 * t) ^ sw, c1 = (8 * k1 + 2 * t) ^ sw;
-#pragma unroll
-            for (int j = 0; j < N2 / 8; ++j) {
-              const double2 b0 = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + c0);
-              const double2 b1 = *reinterpret_cast<const double2*>(wr + j * 8 * N1 + c1);
-              dmma16x8x8(acc2[j], acc1[k0][0], acc1[k0][2], acc1[k0][1], acc1[k0][3], b0.x, b0.y);
-              dmma16x8x8(acc2[j], acc1[k1][0], acc1[k1][2], acc1[k1][1], acc1[k1][3], b1.x, b1.y);
-            }
-          }
-        };
-        if (frag_needs_care<ACT, N1 / 8>(acc1)) layer2(std::false_type{});
-        else layer2(std::true_type{});
-        // ---------------- layer 3: [16 x N2] x [N2 x N3]
-#pragma unroll
-        for (int j = 0; j < N3 / 8; ++j) {
-          const double2 bb = *reinterpret_cast<const double2*>(W23 + G3::B3_OFF + 8 * j + 2 * t);
-          acc3[j][0] = bb.x; acc3[j][1] = bb.y; acc3[j][2] = bb.x; acc3[j][3] = bb.y;
-        }
-        auto layer3 = [&](auto fast_tag) {
-          constexpr bool FAST = decltype(fast_tag)::value;
-          const double* wr = W23 + G3::W3_OFF + gq * N2;
-          const int sw = (gq & 1) * G3::SW2;
-          act_tile<ACT, FAST>(acc2[0], a2, tab);
-#pragma unroll
-          for (int kg = 0; kg < N2 / 8; ++kg) {
-            if (kg + 1 < N2 / 8) act_tile<ACT, FAST>(acc2[kg + 1], a2, tab);
-            const int col = (8 * kg + 2 * t) ^ sw;
-#pragma unroll
-            for (int j = 0; j < N3 / 8; ++j) {
-              const double2 bb = *reinterpret_cast<const double2*>(wr + j * 8 * N2 + col);
-              dmma16x8x8(acc3[j], acc2[kg][0], acc2[kg][2], acc2[kg][1], acc2[kg][3], bb.x, bb.y);
-            }
-          }
-        };
-        if (frag_needs_care<ACT, N2 / 8>(acc2)) layer3(std::false_type{});
-        else layer3(std::true_type{});
+        fwd3_layers23<ACT, KP0, N1, N2, N3>(acc1, W23, a1, a2, tab, gq, t, acc3);
         // weights of this use are no longer needed by this warp
         __syncwarp();
         release_part(1, q);
@@ -881,15 +910,7 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
           ep_y[0] = y[0]; ep_y[1] = y[1];
           if (MODE == FWD3_LIK_W) { ep_wgt[0] = wgt[0]; ep_wgt[1] = wgt[1]; }
         }
-        if constexpr (CAT) {
-          if (PREDICT) quad_epilogue_pred<N3>(p, c, wt, lane, acc3, tab, pacc, pvote);
-        } else if constexpr (LIKK == FWD3_COUNT) {
-          static_assert(!PREDICT, "count prediction runs the FWD3_GAUSS instantiation");
-          quad_count_lik<N3>(p, c, wt, lane, acc3);
-        } else {
-          if (PREDICT) quad_gauss_pred<N3>(p, c, wt, lane, acc3, pacc, tab);
-          else quad_gauss_lik<N3>(p, c, wt, lane, acc3, tab);
-        }
+        fwd3_set_epilogue<N3, MODE, LIKK>(p, c, wt, lane, acc3, tab, pacc, pvote);
       } else {
         // (a warp without a tile waits for both parts before releasing them, so that its releases cannot run ahead)
         mbar_wait(&full23[b], (uint32_t)((q >> 1) & 1));
@@ -928,6 +949,498 @@ __global__ void __launch_bounds__(NWARPS * 32, 1) k_fwd3(const __grid_constant__
     for (int i = threadIdx.x; i < n_cnt; i += blockDim.x)
       if (cnt[i]) atomicAdd(&p.counts[i], cnt[i]);
   }
+}
+
+// =============================================================================================
+// 64 -> 64 -> 32 family, likelihood modes: layer 1 on the int8 tensor cores (k_fwd3i)
+// =============================================================================================
+// Layer 1 (64 -> 64, 62 % of the family's DMMAs) is evaluated in integer arithmetic (Ozaki split).  bnn_set_data first
+// equalises the features: feature k is divided by 2^s_k, its largest magnitude over the rows rounded up to a power of
+// two, and W1's input column k is multiplied by 2^s_k (both exact, so X W1^T is unchanged).  Every row of the scaled X
+// and every unit's row of the scaled W1 is then scaled by a power of two 2^-e so that its largest magnitude lies in
+// [2^45, 2^46), rounded to an integer and cut into 6 balanced base-256 digits (each in [-128, 127], most significant
+// first).  The products of digit i of X and digit j of W1 with i + j = d <= 5 (21 of the 36 pairs) are summed by
+// tcgen05.mma.kind::i8 into one S32 accumulator per "diagonal" d, exactly (|sum| <= 6 * 64 * 2^14).  The compute warp
+// that owns the rows recombines v = sum_d acc_d * 256^(5 - d) exactly in 64-bit integers (|v| < 2^61; the sum of
+// products is 2^40 v) and forms z = fma(double(v) * sx_row, sw_unit, bias), with sx = 2^(e_x + 20), sw = 2^(e_w + 20).
+// Error of a pre-activation (rounding of both operands to 46 bits below their row's / unit's largest magnitude, and
+// the dropped diagonals): |z - z_exact| <= 2^-39 * max_k (c_k |w_k|), c_k = the largest |x| of feature k over the
+// rows, times the row's largest |x_k| / c_k.  That is small against the products themselves only when no feature has
+// rare values far above its typical ones, so bnn_set_data stages the digits (and this kernel runs) only when, for
+// every feature, at least half of its nonzero entries are within 2^6 of its largest magnitude (the median test) and
+// that magnitude lies in [2^-500, 2^500] (or the feature is zero): standardised features, counts, binary features,
+// timestamps.  Other data sets (rare outliers, heavy tails), and any with a non-finite entry, run k_fwd3.
+// A non-finite entry of W1 makes every pre-activation of its unit NaN.
+__device__ __forceinline__ int i8_scale_exp(double amax) {
+  if (!(amax > 0.0)) return 0;
+  int ex;
+  frexp(amax, &ex);                                 // amax in [2^(ex-1), 2^ex)
+  return max(ex - 46, -1042);                       // 2^(e + 20) stays a normal double (tiny W1 units)
+}
+// the 6 balanced base-256 digits of round(v * 2^-e), most significant first
+__device__ __forceinline__ void i8_digits(double v, int e, int (&dg)[BNN_I8_DIGITS]) {
+  long long iv = __double2ll_rn(ldexp(v, -e));
+#pragma unroll
+  for (int i = BNN_I8_DIGITS - 1; i >= 0; --i) {
+    const int d = (int)(signed char)(iv & 0xff);
+    dg[i] = d;
+    iv = (iv - d) >> 8;
+  }
+}
+// byte offset of (row r, input k) in a K-major tile of 64 inputs: 8-row groups 512 bytes apart, 16-byte core-matrix
+// columns 128 bytes apart (tcgen05 shared-memory descriptor, no swizzle: SBO = 512, LBO = 128)
+__host__ __device__ __forceinline__ int i8_kmajor(int r, int k) { return (r >> 3) * 512 + (k >> 4) * 128 + (r & 7) * 16 + (k & 15); }
+
+// Writes the digits of one row (or unit) of 64 values v(k) into the tile at `tile` (digit stride `dstride`).
+template <typename F>
+__device__ __forceinline__ double i8_split_row(F v, int r, int8_t* tile, int dstride) {
+  double amax = 0.0;
+  bool finite = true;
+  for (int k = 0; k < 64; ++k) {
+    const double a = fabs(v(k));
+    finite = finite && a <= 1.7976931348623157e308;
+    amax = fmax(amax, a);
+  }
+  const int e = finite ? i8_scale_exp(amax) : 0;
+  for (int kc = 0; kc < 4; ++kc) {
+    uint32_t w[BNN_I8_DIGITS][4] = {};
+    for (int k = 0; k < 16; ++k) {
+      int dg[BNN_I8_DIGITS];
+      i8_digits(finite ? v(16 * kc + k) : 0.0, e, dg);
+#pragma unroll
+      for (int i = 0; i < BNN_I8_DIGITS; ++i) w[i][k >> 2] |= (uint32_t)(dg[i] & 0xff) << (8 * (k & 3));
+    }
+#pragma unroll
+    for (int i = 0; i < BNN_I8_DIGITS; ++i)
+      *reinterpret_cast<uint4*>(tile + i * dstride + i8_kmajor(r, 16 * kc)) = make_uint4(w[i][0], w[i][1], w[i][2], w[i][3]);
+  }
+  return finite ? ldexp(1.0, e + 20) : __longlong_as_double(0x7ff8000000000000LL);
+}
+
+// staged rows (swizzled, n_pad16 of them, F_pad = 64) -> digits [n_blk][6][8 KB] + row scales; rows past n_pad16 are 0
+__global__ void k_slice_x(const double* __restrict__ xs, long long n_pad16, int swz, long long n_rows,
+                          const double* __restrict__ wmul, int8_t* x_i8, double* x_i8_scale) {
+  const long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n_rows) return;
+  const double* row = xs + r * 64;
+  const int sw = (int)(r & 1) * swz;
+  const bool live = r < n_pad16;
+  x_i8_scale[r] = i8_split_row([&](int k) { return live ? row[k ^ sw] / wmul[k] : 0.0; }, (int)(r & 127),
+                               x_i8 + (r >> 7) * BNN_I8_XBLK_BYTES, 128 * 64);
+}
+
+// Per feature of the staged rows (one CTA per feature, fixed reduction order): out[k] = largest magnitude over the n
+// rows (NaN if an entry is not finite), out[64 + k] = rows where it is nonzero, out[128 + k] = rows where it is at
+// least 2^-6 of that largest magnitude -- the statistics bnn_set_data decides the int8 first layer with.
+__global__ void __launch_bounds__(256) k_feature_stats(const double* __restrict__ xs, long long n, int swz, double* out) {
+  __shared__ double smax[256];
+  __shared__ long long snz[256], sbig[256];
+  const int k = blockIdx.x;
+  double m = 0.0;
+  bool finite = true;
+  for (long long r = threadIdx.x; r < n; r += blockDim.x) {
+    const double v = fabs(xs[r * 64 + (k ^ ((int)(r & 1) * swz))]);
+    finite = finite && v <= 1.7976931348623157e308;
+    m = fmax(m, v);
+  }
+  smax[threadIdx.x] = finite ? m : __longlong_as_double(0x7ff8000000000000LL);
+  __syncthreads();
+  for (int s = 128; s > 0; s >>= 1) {
+    if (threadIdx.x < s) {
+      const double a = smax[threadIdx.x], b = smax[threadIdx.x + s];
+      smax[threadIdx.x] = (a != a || b != b) ? a + b : fmax(a, b);
+    }
+    __syncthreads();
+  }
+  const double lim = smax[0] * 0x1p-6;
+  long long nz = 0, big = 0;
+  for (long long r = threadIdx.x; r < n; r += blockDim.x) {
+    const double v = fabs(xs[r * 64 + (k ^ ((int)(r & 1) * swz))]);
+    nz += v != 0.0;
+    big += v >= lim && v != 0.0;
+  }
+  __syncthreads();
+  snz[threadIdx.x] = nz;
+  sbig[threadIdx.x] = big;
+  __syncthreads();
+  for (int s = 128; s > 0; s >>= 1) {
+    if (threadIdx.x < s) { snz[threadIdx.x] += snz[threadIdx.x + s]; sbig[threadIdx.x] += sbig[threadIdx.x + s]; }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) { out[k] = smax[0]; out[64 + k] = (double)snz[0]; out[128 + k] = (double)sbig[0]; }
+}
+
+// packed weight sets [C, PB] -> per set the digits of W1, the unit scales and the layer-1 biases (BNN_I8_WSET_BYTES)
+__global__ void __launch_bounds__(64) k_slice_w1(const double* __restrict__ wp, int PB, const double* __restrict__ wmul,
+                                                  int8_t* w1_i8) {
+  using G3 = Fwd3Geom<64, 64, 32, 16>;            // (layer-1 offsets are the same for N3 = 8)
+  const int n = threadIdx.x, c = blockIdx.x;
+  const double* W = wp + (long long)c * PB;
+  const int sw = (n & 1) * G3::SW0;
+  int8_t* out = w1_i8 + (long long)c * BNN_I8_WSET_BYTES;
+  double* aux = reinterpret_cast<double*>(out + BNN_I8_DIGITS * BNN_I8_WDIG_BYTES);
+  aux[n] = i8_split_row([&](int k) { return W[G3::W1_OFF + n * 64 + (k ^ sw)] * wmul[k]; }, n, out, BNN_I8_WDIG_BYTES);
+  aux[64 + n] = W[G3::B1_OFF + n];
+}
+
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// shared-memory matrix descriptor: K-major, no swizzle, LBO = 128, SBO = 512, descriptor version 1 (sm_100)
+__device__ __forceinline__ uint64_t i8_desc(uint32_t saddr) {
+  return (uint64_t)((saddr >> 4) & 0x3fff) | ((uint64_t)(128 >> 4) << 16) | ((uint64_t)(512 >> 4) << 32) | ((uint64_t)1 << 46);
+}
+// instruction descriptor: S32 accumulator, signed A and B, K-major, M = 128, N = 64
+constexpr uint32_t I8_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((64u >> 3) << 17) | ((128u >> 4) << 24);
+__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t acc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}\n" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(I8_IDESC), "r"(acc)
+      : "memory");
+}
+__device__ __forceinline__ void umma_commit(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+// 16 TMEM lanes x 8 columns -> the m16n8 accumulator fragment (v0 = (g, 2t), v1 = (g, 2t+1), v2 = (g+8, 2t), v3 = (g+8, 2t+1))
+__device__ __forceinline__ void tmem_ld_frag(uint32_t addr, int (&v)[4]) {
+  asm volatile("tcgen05.ld.sync.aligned.16x256b.x1.b32 {%0,%1,%2,%3}, [%4];"
+               : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(addr));
+}
+
+constexpr int I8_WARPS = 8;     // compute warps; warp I8_WARPS issues the MMAs and the copies of the int8 operands
+
+// Per-phase clocks of k_fwd3i: empty here; tools/fwd3i_phases.py compiles this file with BNN_FWD3I_PHASES defined
+// (lane 0 of every warp adds the clock64 difference of each phase to a global counter) and reads the counters back.
+#ifdef BNN_FWD3I_PHASES
+__device__ unsigned long long g_fwd3i_phase[16];
+#define FWD3I_CLOCK(v) const long long v = clock64()
+#define FWD3I_PHASE(i, a, b) do { if (lane == 0) atomicAdd(&g_fwd3i_phase[i], (unsigned long long)((b) - (a))); } while (0)
+extern "C" int bnn_fwd3i_phase_clocks(unsigned long long* out, int reset) {
+  if (cudaMemcpyFromSymbol(out, g_fwd3i_phase, sizeof(g_fwd3i_phase)) != cudaSuccess) return 1;
+  static const unsigned long long zero[16] = {};
+  if (reset && cudaMemcpyToSymbol(g_fwd3i_phase, zero, sizeof(zero)) != cudaSuccess) return 1;
+  return 0;
+}
+#else
+#define FWD3I_CLOCK(v)
+#define FWD3I_PHASE(i, a, b)
+#endif
+
+template <int N3, int MODE>
+static constexpr size_t fwd3i_smem_bytes_fixed() {
+  using G3 = Fwd3Geom<64, 64, 32, N3>;
+  return 2 * (size_t)BNN_I8_XBLK_BYTES + 2 * (size_t)BNN_I8_WSET_BYTES + 2 * (size_t)(G3::PB - G3::W2_OFF) * 8 +
+         BNN_EXP_TAB_SIZE * 8 + 8 * sizeof(uint64_t) + 4 * sizeof(int);
+}
+
+// One CTA per SM, 8 compute warps + 1 MMA warp.  A CTA runs (128-row block, weight set) pairs with the decomposition of
+// k_fwd3 (16-row tile groups of 8 tiles = one block); compute warp w owns the 16-row tile 2 (w % 4) + w / 4 of the
+// block, i.e. TMEM lanes 32 (w % 4) + 16 (w / 4) ..., the lanes its warp may read.  Per pair the MMA warp issues the
+// 42 MMAs (21 digit pairs x 2 k-steps of 32) into 6 x 64 TMEM columns; every compute warp drains its 16 rows into the
+// m16n8 fragments of k_fwd3's acc1 and continues exactly as k_fwd3 (fwd3_layers23, the categorical epilogue
+// software-pipelined into the drain of the next pair, or fwd3_set_epilogue), while the MMAs of the next pair run.
+//
+// Buffers the tensor core reads asynchronously are released by the tcgen05.commit of the MMAs that read them, never
+// by their issue:
+//   * TMEM accumulators: the compute warps run tcgen05.wait::ld, tcgen05.fence::before_thread_sync, then arrive on
+//     `tempty`; the MMA thread waits on `tempty` and runs tcgen05.fence::after_thread_sync before it issues the MMAs
+//     that overwrite them.  The compute warps read them after waiting on `tfull` (the commit) and
+//     tcgen05.fence::after_thread_sync.
+//   * X digit tiles (2 blocks) and W1 digit slots (2 sets): refilled by the MMA thread only after `tempty` of the
+//     pair that last read them, which the compute warps arrive on after `tfull` of that pair, i.e. after its commit.
+//     The unit scales and biases in a W1 slot are read by the compute warps before their `tempty` arrival.
+//   * Layers 2/3 (generic loads only) go through k_fwd3's two-slot ring, refilled by the last warp that releases.
+template <int ACT, int MODE, int LIKK>
+__global__ void __launch_bounds__((I8_WARPS + 1) * 32, 1) k_fwd3i(const __grid_constant__ FwdParams p) {
+  constexpr int KP0 = 64, N1 = 64, N2 = 32, N3 = (LIKK == FWD3_CAT) ? 16 : 8, NW = I8_WARPS;
+  using G3 = Fwd3Geom<KP0, N1, N2, N3>;
+  static_assert(MODE != FWD3_PRED, "prediction runs k_fwd3");
+  constexpr bool DEFER = (LIKK == FWD3_CAT);
+  extern __shared__ __align__(128) unsigned char smem_raw[];
+  const NetGeom& g = p.g;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int gq = lane >> 2, t = lane & 3;
+
+  constexpr int W23_D = G3::PB - G3::W2_OFF;
+  int8_t* xbuf = reinterpret_cast<int8_t*>(smem_raw);                          // [2][BNN_I8_XBLK_BYTES]
+  int8_t* wbuf = xbuf + 2 * BNN_I8_XBLK_BYTES;                                 // [2][BNN_I8_WSET_BYTES]
+  double* w23buf = reinterpret_cast<double*>(wbuf + 2 * BNN_I8_WSET_BYTES);    // [2][W23_D]
+  double* tab = w23buf + 2 * W23_D;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(tab + BNN_EXP_TAB_SIZE);
+  uint64_t* xfull = bars;           // [2] X digit tiles
+  uint64_t* wfull = bars + 2;       // [2] W1 digit slots
+  uint64_t* full23 = bars + 4;      // [2] layers 2/3
+  uint64_t* tfull = bars + 6;       // accumulators written (tcgen05.commit)
+  uint64_t* tempty = bars + 7;      // accumulators drained (NW arrivals)
+  int* rel = reinterpret_cast<int*>(bars + 8);             // [2] release counters of the layers-2/3 ring
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(rel + 2);
+  int* cnt = rel + 4;
+  const int n_cnt = DEFER ? p.C * bnn_n_counts(g.K) : 0;
+
+  for (int i = threadIdx.x; i < BNN_EXP_TAB_SIZE; i += blockDim.x) tab[i] = p.exp_tab[i];
+  for (int i = threadIdx.x; i < n_cnt; i += blockDim.x) cnt[i] = 0;
+  if (threadIdx.x == 0) {
+    rel[0] = rel[1] = 0;
+    for (int i = 0; i < 7; ++i) mbar_init(&bars[i], 1);
+    mbar_init(tempty, NW);
+    mbar_fence_init();
+  }
+  if (warp == NW) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "r"(512u) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_slot;
+
+  // work decomposition of k_fwd3 with groups of NW tiles (one 128-row block)
+  const long long total_warps = (long long)gridDim.x * NW;
+  const long long n_full = p.n_tiles16 / total_warps;
+  const long long tail_base = n_full * total_warps;
+  const long long rem = p.n_tiles16 - tail_base;
+  int seg_tg[2] = {0, 0}, seg_lo[2] = {0, 0}, seg_hi[2] = {0, 0};
+  if (rem > 0) {
+    const long long groups = (rem + NW - 1) / NW;
+    const long long pairs = groups * p.C;
+    const long long per_cta = (pairs + gridDim.x - 1) / gridDim.x;
+    const long long s0 = (long long)blockIdx.x * per_cta;
+    const long long s1 = (s0 + per_cta < pairs) ? s0 + per_cta : pairs;
+    if (s0 < s1) {
+      seg_tg[0] = (int)(s0 / p.C);
+      seg_lo[0] = (int)(s0 % p.C);
+      const long long n0 = ((s1 - s0) < (long long)(p.C - seg_lo[0])) ? (s1 - s0) : (long long)(p.C - seg_lo[0]);
+      seg_hi[0] = seg_lo[0] + (int)n0;
+      if (s1 - s0 > n0) { seg_tg[1] = seg_tg[0] + 1; seg_hi[1] = (int)(s1 - s0 - n0); }
+    }
+  }
+  const long long q_seg0 = n_full * p.C;
+  const long long q_seg1 = q_seg0 + (seg_hi[0] - seg_lo[0]);
+  const long long total_q = q_seg1 + (seg_hi[1] - seg_lo[1]);
+  const long long n_iter = n_full + (seg_hi[0] > seg_lo[0] ? 1 : 0) + (seg_hi[1] > seg_lo[1] ? 1 : 0);
+  auto set_of = [&](long long qq) -> long long {
+    return qq < q_seg0 ? qq % p.C : (qq < q_seg1 ? seg_lo[0] + (qq - q_seg0) : seg_lo[1] + (qq - q_seg1));
+  };
+  auto block_of = [&](long long i) -> long long {            // 128-row block of iteration i
+    const int s2 = (int)(i - n_full);
+    return s2 < 0 ? i * gridDim.x + blockIdx.x : n_full * gridDim.x + (s2 == 0 ? seg_tg[0] : seg_tg[1]);
+  };
+  auto c_range = [&](long long i, int& lo, int& hi) {
+    const int s2 = (int)(i - n_full);
+    lo = s2 < 0 ? 0 : (s2 == 0 ? seg_lo[0] : seg_lo[1]);
+    hi = s2 < 0 ? p.C : (s2 == 0 ? seg_hi[0] : seg_hi[1]);
+  };
+  constexpr uint32_t W23_BYTES = W23_D * sizeof(double);
+  static_assert(W23_BYTES % 16 == 0, "bulk copies move multiples of 16 bytes");
+  auto load23 = [&](long long qq) {
+    const int b = (int)(qq & 1);
+    mbar_arrive_expect_tx(&full23[b], W23_BYTES);
+    bulk_g2s(w23buf + b * W23_D, p.wp + set_of(qq) * G3::PB + G3::W2_OFF, W23_BYTES, &full23[b]);
+  };
+
+  if (warp == NW) {
+    // ---------------- MMA warp: one thread issues the operand copies and the MMAs
+    if (lane == 0 && total_q > 0) {
+      auto load_x = [&](long long i) {
+        const int b = (int)(i & 1);
+        mbar_arrive_expect_tx(&xfull[b], BNN_I8_XBLK_BYTES);
+        bulk_g2s(xbuf + b * BNN_I8_XBLK_BYTES, p.x_i8 + block_of(i) * BNN_I8_XBLK_BYTES, BNN_I8_XBLK_BYTES, &xfull[b]);
+      };
+      auto load_w = [&](long long qq) {
+        const int b = (int)(qq & 1);
+        mbar_arrive_expect_tx(&wfull[b], BNN_I8_WSET_BYTES);
+        bulk_g2s(wbuf + b * BNN_I8_WSET_BYTES, p.w1_i8 + set_of(qq) * BNN_I8_WSET_BYTES, BNN_I8_WSET_BYTES, &wfull[b]);
+      };
+      load_x(0);
+      load_w(0);
+      if (total_q > 1) load_w(1);
+      long long q = 0;
+      for (long long it = 0; it < n_iter; ++it) {
+        int c_lo, c_hi;
+        c_range(it, c_lo, c_hi);
+        for (int c = c_lo; c < c_hi; ++c, ++q) {
+          FWD3I_CLOCK(m0);
+          if (q > 0) {
+            mbar_wait(tempty, (uint32_t)((q - 1) & 1));      // pair q-1 drained => its MMAs are complete
+            tc_fence_after();
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            if (q + 1 < total_q) load_w(q + 1);                // slot of pair q-1
+          }
+          if (c == c_lo) {
+            mbar_wait(&xfull[it & 1], (uint32_t)((it >> 1) & 1));
+            if (it + 1 < n_iter) load_x(it + 1);               // buffer of block it-1, last read by pair q-1
+          }
+          mbar_wait(&wfull[q & 1], (uint32_t)((q >> 1) & 1));
+          tc_fence_after();
+          FWD3I_CLOCK(m1);
+          const uint32_t xa = smem_u32(xbuf + (it & 1) * BNN_I8_XBLK_BYTES);
+          const uint32_t wa = smem_u32(wbuf + (q & 1) * BNN_I8_WSET_BYTES);
+#pragma unroll
+          for (int d = 0; d < BNN_I8_DIGITS; ++d)
+#pragma unroll
+            for (int i = 0; i <= d; ++i)
+#pragma unroll
+              for (int ks = 0; ks < 2; ++ks)
+                umma_i8(tmem + 64 * d, i8_desc(xa + i * 128 * 64 + ks * 256), i8_desc(wa + (d - i) * BNN_I8_WDIG_BYTES + ks * 256),
+                        (i | ks) ? 1u : 0u);
+          umma_commit(tfull);
+          FWD3I_CLOCK(m2);
+          FWD3I_PHASE(6, m0, m1);
+          FWD3I_PHASE(7, m1, m2);
+          FWD3I_PHASE(9, 0, 1);
+        }
+      }
+    }
+  } else {
+    // ---------------- compute warps
+    if (threadIdx.x == 0)
+      for (long long qq = 0; qq < 2 && qq < total_q; ++qq) load23(qq);
+    auto release23 = [&](long long qq) {
+      if (lane == 0) {
+        int* r = &rel[(int)(qq & 1)];
+        __threadfence_block();
+        const int old = atomicAdd(r, 1);
+        if (old == NW - 1) {
+          *r = 0;
+          if (qq + 2 < total_q) {
+            __threadfence_block();
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            load23(qq + 2);
+          }
+        }
+      }
+    };
+    const int tile_in_blk = 2 * (warp & 3) + (warp >> 2);
+    const uint32_t tm_rows = tmem + ((uint32_t)(32 * (warp & 3) + 16 * (warp >> 2)) << 16);
+    double acc3[N3 / 8][4];
+    bool prev_valid = false;
+    long long ep_wt = 0;
+    int ep_c = 0;
+    int ep_y[2] = {0, 0};
+    double ep_wgt[2] = {1.0, 1.0};
+#pragma unroll
+    for (int j = 0; j < N3 / 8; ++j) acc3[j][0] = acc3[j][1] = acc3[j][2] = acc3[j][3] = 0.0;
+    long long q = 0;
+    for (long long it = 0; it < n_iter; ++it) {
+      int c_lo, c_hi;
+      c_range(it, c_lo, c_hi);
+      const long long blk = block_of(it);
+      const long long wt = blk * NW + tile_in_blk;
+      const bool have_tile = wt < p.n_tiles16;
+      int y[2] = {0, 0};
+      double wgt[2] = {1.0, 1.0}, sx[2] = {0.0, 0.0};
+      if (have_tile) {
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const long long row = wt * 16 + gq + 8 * h;
+          sx[h] = p.x_i8_scale[row];
+          if (DEFER && row < p.n_total) {
+            y[h] = p.labels[row];
+            if (MODE == FWD3_LIK_W) {
+              if (p.class_w) wgt[h] *= p.class_w[y[h]];
+              if (p.inst_w && row < p.n_train) wgt[h] *= p.inst_w[row];
+            }
+          }
+        }
+      }
+      for (int c = c_lo; c < c_hi; ++c, ++q) {
+        const int b = (int)(q & 1);
+        FWD3I_CLOCK(t0);
+        __syncwarp();
+        mbar_wait(tfull, (uint32_t)(q & 1));
+        tc_fence_after();
+        mbar_wait(&wfull[b], (uint32_t)((q >> 1) & 1));
+        FWD3I_CLOCK(t1);
+        double acc1[N1 / 8][4];
+        if (have_tile) {
+          // ---------------- drain: 6 diagonals -> exact 64-bit sums -> FP64 pre-activations (+ pending epilogue)
+          const double* aux = reinterpret_cast<const double*>(wbuf + b * BNN_I8_WSET_BYTES + BNN_I8_DIGITS * BNN_I8_WDIG_BYTES);
+          RowStats<N3> rs;
+          LikRow lr;
+          const int K = g.K;
+#pragma unroll
+          for (int j = 0; j < N1 / 8; ++j) {
+            int v[BNN_I8_DIGITS][4];
+#pragma unroll
+            for (int d = 0; d < BNN_I8_DIGITS; ++d) tmem_ld_frag(tm_rows + 64 * d + 8 * j, v[d]);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            if (DEFER) {
+              if (j == 0) qs_max<N3>(acc3, K, t, rs);
+              else if (j == 2) qs_exp<N3, 0, true>(acc3, K, t, ep_y, tab, rs);
+              else if (j == 4) qs_exp<N3, 1, true>(acc3, K, t, ep_y, tab, rs);
+              else if (j == 6) {
+                qs_reduce<N3, true>(rs);
+                lr = quad_lik_finish<N3, MODE == FWD3_LIK_W>(p, ep_wt, lane, rs, ep_y, ep_wgt, prev_valid);
+              }
+            }
+            const int col = 8 * j + 2 * t;
+            const double2 sw = *reinterpret_cast<const double2*>(aux + col);
+            const double2 bb = *reinterpret_cast<const double2*>(aux + 64 + col);
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              long long s = v[0][e];
+#pragma unroll
+              for (int d = 1; d < BNN_I8_DIGITS; ++d) s = s * 256 + v[d][e];
+              acc1[j][e] = fma((double)s * sx[e >> 1], (e & 1) ? sw.y : sw.x, (e & 1) ? bb.y : bb.x);
+            }
+          }
+          if (DEFER) quad_lik_commit<N3>(p, ep_c, ep_wt, lane, cnt, lr, prev_valid);
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(tempty);
+        FWD3I_CLOCK(t2);
+        mbar_wait(&full23[b], (uint32_t)((q >> 1) & 1));
+        FWD3I_CLOCK(t3);
+        if (have_tile) {
+          const double* W23 = w23buf + b * W23_D - G3::W2_OFF;
+          const double a1 = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[c * 3 + 0] : 0.0;
+          const double a2 = (ACT == BNN_ACT_LEAKY && p.alpha) ? p.alpha[c * 3 + 1] : 0.0;
+          fwd3_layers23<ACT, KP0, N1, N2, N3>(acc1, W23, a1, a2, tab, gq, t, acc3);
+          FWD3I_CLOCK(t4);
+          FWD3I_PHASE(3, t3, t4);
+          __syncwarp();
+          release23(q);
+          if (DEFER) {
+            prev_valid = true;
+            ep_wt = wt; ep_c = c;
+            ep_y[0] = y[0]; ep_y[1] = y[1];
+            if (MODE == FWD3_LIK_W) { ep_wgt[0] = wgt[0]; ep_wgt[1] = wgt[1]; }
+          } else {
+            double pacc[2][N3 / 4];
+            int pvote[2][N3 / 4];
+            fwd3_set_epilogue<N3, MODE, LIKK>(p, c, wt, lane, acc3, tab, pacc, pvote);
+          }
+        } else {
+          release23(q);
+        }
+        FWD3I_CLOCK(t5);
+        FWD3I_PHASE(0, t0, t1);
+        FWD3I_PHASE(1, t1, t2);
+        FWD3I_PHASE(2, t2, t3);
+        FWD3I_PHASE(4, t0, t5);
+        FWD3I_PHASE(8, 0, 1);
+      }
+    }
+    if (DEFER && prev_valid) {
+      RowStats<N3> rs;
+      quad_softmax_stats<N3, true>(acc3, g.K, t, ep_y, tab, rs);
+      const LikRow lr = quad_lik_finish<N3, MODE == FWD3_LIK_W>(p, ep_wt, lane, rs, ep_y, ep_wgt, true);
+      quad_lik_commit<N3>(p, ep_c, ep_wt, lane, cnt, lr, true);
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == NW) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512u) : "memory");
+  }
+  if (n_cnt)
+    for (int i = threadIdx.x; i < n_cnt; i += blockDim.x)
+      if (cnt[i]) atomicAdd(&p.counts[i], cnt[i]);
 }
 
 // =============================================================================================
@@ -970,11 +1483,40 @@ static cudaError_t launch_fwd3(const FwdParams& p, int n_sms, cudaStream_t st) {
 }
 
 // k_fwd3 instantiations: two padded width families x four activations x {categorical (N3 = 16: likelihood, weighted
-// likelihood, prediction), Gaussian / sigma head (N3 = 8: likelihood, prediction), count (N3 = 8: likelihood)}
+// likelihood, prediction), Gaussian / sigma head (N3 = 8: likelihood, prediction), count (N3 = 8: likelihood)}; the
+// likelihood modes of family A run k_fwd3i instead
 //   family A   64 -> 64 -> 32 -> N3   12 warps per SM (BASELINE config 4 / 5 is its swish / categorical member)
 //   family B   32 -> 32 -> 16 -> N3   16 warps per SM
+static bool bnn_fwd3_uses_i8(const FwdParams& p, bool predict) {
+  return !predict && p.x_i8 && !(p.g.lik == BNN_LIK_CATEGORICAL && (p.class_w || p.inst_w));
+}
+
+template <int ACT, int MODE, int LIKK>
+static cudaError_t launch_fwd3i(const FwdParams& p, int n_sms, cudaStream_t st) {
+  auto kern = k_fwd3i<ACT, MODE, LIKK>;
+  constexpr int N3 = (LIKK == FWD3_CAT) ? 16 : 8;
+  const size_t smem = fwd3i_smem_bytes_fixed<N3, MODE>() + (LIKK == FWD3_CAT ? bnn_smem_counts(p.g, p.C) : 0) * sizeof(int);
+  if (smem > BNN_MAX_DYN_SMEM) return cudaErrorInvalidConfiguration;
+  if (p.C > BNN_MAX_SETS_PER_PASS) return cudaErrorInvalidValue;           // w1_i8 holds one pass
+  if (cudaError_t e = bnn_prepare_kernel((const void*)kern, BNN_MAX_DYN_SMEM)) return e;
+  k_slice_w1<<<p.C, 64, 0, st>>>(p.wp, p.g.PB, p.x_i8_wmul, p.w1_i8);
+  long long ctas = (p.n_tiles16 + I8_WARPS - 1) / I8_WARPS * p.C;
+  const int grid = (int)(ctas < n_sms ? ctas : n_sms);
+  kern<<<grid, (I8_WARPS + 1) * 32, smem, st>>>(p);
+  return cudaGetLastError();
+}
+
 template <int ACT, int KP0, int N1, int N2, int NWARPS>
 static cudaError_t launch_fwd3_family(const FwdParams& p, bool predict, int n_sms, cudaStream_t st) {
+  if constexpr (KP0 == 64) {
+    // 64 -> 64 -> 32: the unweighted likelihoods on data staged as int8 digits run k_fwd3i; the weighted likelihood
+    // stays on k_fwd3 (k_fwd3i measured 3-5 % slower there, profiles/r03_fwd3i_modes.json)
+    if (bnn_fwd3_uses_i8(p, predict)) {
+      if (p.g.lik == BNN_LIK_CATEGORICAL) return launch_fwd3i<ACT, FWD3_LIK, FWD3_CAT>(p, n_sms, st);
+      if (bnn_lik_is_count(p.g.lik)) return launch_fwd3i<ACT, FWD3_LIK, FWD3_COUNT>(p, n_sms, st);
+      return launch_fwd3i<ACT, FWD3_LIK, FWD3_GAUSS>(p, n_sms, st);
+    }
+  }
   if (p.g.lik == BNN_LIK_CATEGORICAL) {
     if (predict) return launch_fwd3<ACT, KP0, N1, N2, 16, NWARPS, FWD3_PRED, FWD3_CAT>(p, n_sms, st);
     if (p.class_w || p.inst_w) return launch_fwd3<ACT, KP0, N1, N2, 16, NWARPS, FWD3_LIK_W, FWD3_CAT>(p, n_sms, st);
@@ -990,6 +1532,18 @@ static cudaError_t launch_fwd3_act(const FwdParams& p, bool predict, int n_sms, 
   return bnn_with_act(p.g.act, [&](auto a) {
     return launch_fwd3_family<decltype(a)::value, KP0, N1, N2, NWARPS>(p, predict, n_sms, st);
   });
+}
+
+cudaError_t bnn_launch_feature_stats(const double* xs, long long n, int swz, double* out, cudaStream_t st) {
+  k_feature_stats<<<64, 256, 0, st>>>(xs, n, swz, out);
+  return cudaGetLastError();
+}
+cudaError_t bnn_launch_slice_x(const double* xs, long long n_pad16, int swz, const double* wmul, int8_t* x_i8,
+                               double* x_i8_scale, cudaStream_t st) {
+  const long long n_rows = bnn_i8_blocks(n_pad16 / 16) * 128;
+  if (n_rows == 0) return cudaSuccess;
+  k_slice_x<<<(unsigned)((n_rows + 127) / 128), 128, 0, st>>>(xs, n_pad16, swz, n_rows, wmul, x_i8, x_i8_scale);
+  return cudaGetLastError();
 }
 
 // which k_fwd3 family the padded geometry matches exactly: 1 = A, 2 = B, 0 = none
@@ -1028,6 +1582,10 @@ static cudaError_t launch_generic(const FwdParams& p, int n_sms, cudaStream_t st
   return bnn_with_act(p.g.act, [&](auto a) { return launch_generic_t<decltype(a)::value, PREDICT>(p, n_sms, st); });
 }
 
+int bnn_forward_launches(const FwdParams& p, bool predict, int force_generic) {
+  return (!force_generic && !p.samp_u && !p.sp.prog && bnn_fwd3_family(p.g) == 1 && bnn_fwd3_uses_i8(p, predict)) ? 2 : 1;
+}
+
 // Dispatch: specialised kernel when the padded shape is one of the compiled instantiations.
 // force_generic != 0 disables the specialised path (used by the tests to cross-check both kernels).
 cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int force_generic, cudaStream_t st,
@@ -1035,12 +1593,14 @@ cudaError_t bnn_launch_forward(const FwdParams& p, bool predict, int n_sms, int 
   const NetGeom& g = p.g;
   if (p.sp.prog) return predict ? bnn_launch_sparse_predict(p, n_sms, st, which) : bnn_launch_sparse(p, n_sms, st, which);
   if (!force_generic && !p.samp_u) {
-    static const char* const names[2][4] = {
+    static const char* const names[3][4] = {
         {"k_fwd3<relu,64,64,32>", "k_fwd3<leaky,64,64,32>", "k_fwd3<swish,64,64,32,16>", "k_fwd3<tanh,64,64,32>"},
-        {"k_fwd3<relu,32,32,16>", "k_fwd3<leaky,32,32,16>", "k_fwd3<swish,32,32,16>", "k_fwd3<tanh,32,32,16>"}};
+        {"k_fwd3<relu,32,32,16>", "k_fwd3<leaky,32,32,16>", "k_fwd3<swish,32,32,16>", "k_fwd3<tanh,32,32,16>"},
+        {"k_fwd3<relu,64,64,32,i8l1>", "k_fwd3<leaky,64,64,32,i8l1>", "k_fwd3<swish,64,64,32,16,i8l1>",
+         "k_fwd3<tanh,64,64,32,i8l1>"}};
     const int fam = bnn_fwd3_family(g);
     if (fam) {
-      if (which) *which = names[fam - 1][g.act];
+      if (which) *which = names[(fam == 1 && bnn_fwd3_uses_i8(p, predict)) ? 2 : fam - 1][g.act];
       return fam == 1 ? launch_fwd3_act<64, 64, 32, 12>(p, predict, n_sms, st)
                       : launch_fwd3_act<32, 32, 16, 16>(p, predict, n_sms, st);
     }

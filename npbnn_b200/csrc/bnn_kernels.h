@@ -106,6 +106,15 @@ size_t bnn_generic_smem_bytes(const NetGeom& g, int C, bool predict, int warps);
 int bnn_generic_warps(const NetGeom& g, int C, bool predict);
 // k_fwd3 width family the padded geometry matches exactly: 1 = 64->64->32, 2 = 32->32->16, 0 = none (generic kernel)
 int bnn_fwd3_family(const NetGeom& g);
+// kernels bnn_launch_forward enqueues for these parameters (the int8 first layer adds the slicing of W1)
+int bnn_forward_launches(const FwdParams& p, bool predict, int force_generic);
+// 64 -> 64 -> 32 family: out[k] = largest |x| of feature k over the n staged rows (NaN if one is not finite),
+// out[64 + k] = its nonzero entries, out[128 + k] = its nonzero entries of at least 2^-6 out[k]; then the rows divided by wmul [64] as the base-256 digits and row scales the
+// likelihood kernel k_fwd3i reads (FwdParams::x_i8 / x_i8_scale), sized for bnn_i8_blocks(n_tiles16) blocks of 128 rows
+inline long long bnn_i8_blocks(long long n_tiles16) { return (n_tiles16 + 7) / 8; }
+cudaError_t bnn_launch_feature_stats(const double* xs, long long n, int swz, double* out, cudaStream_t st);
+cudaError_t bnn_launch_slice_x(const double* xs, long long n_pad16, int swz, const double* wmul, int8_t* x_i8,
+                               double* x_i8_scale, cudaStream_t st);
 cudaError_t bnn_launch_pack_x(const double* x, double* xs, long long n, long long n_pad, int F, int F_pad, int swz,
                               const int* ov_cols, const double* ov_vals, int n_ov, cudaStream_t st);
 // *flag |= 1 if a training label is outside [0, K) or a test label is negative (the reference raises IndexError there)
